@@ -7,6 +7,7 @@
   python bench.py --scaling strong --gpus 8                           # the config's batch split across the ranks (shard_range)
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...   # the reference's CPU pipeline (real cv2 calls + cv2.dnn) on the host cores
+  python bench.py --dump-outputs DIR ... # also writes the results of the last timed step as DIR/<name>.npy
 
 Frames are independent, so the batch shards across ranks with no collective on the data path.  Default scaling is
 weak (the config's batch PER GPU); `--scaling strong` keeps the config's batch as the job total.
@@ -34,6 +35,7 @@ sys.path.insert(0, str(ROOT))
 
 METRIC = "images/sec BlazeFace detect (pre+infer+NMS)"
 PERIOD = 64            # unique synthetic frames; the batch tiles them
+DUMP_BYTES = 64 * 10**6 - 64 * 1024    # --dump-outputs budget, less room for the .npy headers
 
 CONFIGS = {
     # BASELINE.json configs[1]: the configuration the metric is quoted on
@@ -109,6 +111,34 @@ def peaks():
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
 
 
+def dump_outputs(out_dir: Path, counts: np.ndarray, faces: np.ndarray, mesh=None):
+    """Writes one step's results as .npy files: counts [B] and the valid slots of `faces` (fdt_face records, [B, max_faces])
+    and `mesh` ([B, max_faces, 468, 3] or None), in frame then slot order.  When the faces of every frame could exceed
+    DUMP_BYTES, only those of a seeded sample of frames are written; the sample depends on B and max_faces alone, so
+    two builds given the same arguments write the same frames."""
+    B, mf = faces.shape
+    per_face = 19 * 8 + (8 + mesh[0, 0].nbytes if mesh is not None else 0)
+    k = min(B, max(0, (DUMP_BYTES - 16 * B) // (mf * per_face)))
+    frames = np.arange(B) if k == B else np.sort(np.random.default_rng(0).choice(B, k, replace=False))
+    fi, slot = np.nonzero(np.arange(mf)[None, :] < counts[frames][:, None])
+    fb = frames[fi]
+    f = faces[fb, slot]
+    out = {"counts": counts.astype(np.float64),                        # faces per frame, every frame of the step
+           "sample_frames": frames.astype(np.float64),                 # the frames whose faces follow
+           "face_frame": fb.astype(np.float64),
+           "face_box": np.stack([f["xmin"], f["ymin"], f["xmax"], f["ymax"]], 1),
+           "face_score": f["score"],
+           "face_keypoints": f["keypoints"].reshape(-1, 6, 2),
+           "face_anchor_index": f["anchor_index"].astype(np.float64)}
+    if mesh is not None:
+        out["face_mesh_score"] = f["mesh_score"]
+        out["face_mesh"] = mesh[fb, slot]
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in out.items():
+        np.save(out_dir / (name + ".npy"), np.ascontiguousarray(a))
+    return sum(a.nbytes for a in out.values())
+
+
 def cpu_reference(cfg_name: str, steps: int, warmup: int, sample: int):
     """The reference's CPU path (oracle/cpu_bench.py: real cv2 resize / copyMakeBorder / warpAffine + cv2.dnn forward +
     vectorised candidate scan + restated decode / NMS) on all host cores."""
@@ -144,7 +174,13 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=0)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path, default=None,
+                    help="after the timed steps, write what the last one returned (rank 0's frames) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm returns face counts only)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     cfg = CONFIGS[args.config]
     W, H = cfg["w"], cfg["h"]
@@ -257,6 +293,18 @@ def main():
     else:
         check(lib.fdt_copy_to_host(h, host_counts.ctypes.data, pc.value, B * 4))
     faces_found = int(host_counts[:B].sum())
+    dumped = None
+    if args.dump_outputs is not None and rank == 0:
+        face_dtype = np.dtype(_ffi.FdtFace)
+        if standard:      # fdt_detect_batch filled the pinned host buffers of the last step
+            faces = np.ctypeslib.as_array(C.cast(out_faces, C.POINTER(C.c_uint8)), (B * mf * face_sz,)).view(face_dtype)
+            mesh = np.ctypeslib.as_array(mptr, (B * mf * _ffi.FDT_MESH_FLOATS,)).reshape(B, mf, -1, 3)
+        else:             # the device buffers fdt_detect_batch_device returned hold it until the next call
+            faces = np.empty(B * mf, face_dtype)
+            check(lib.fdt_copy_to_host(h, faces.ctypes.data, pf.value, B * mf * face_sz))
+            mesh = None
+        nbytes = dump_outputs(args.dump_outputs, host_counts[:B], faces.reshape(B, mf), mesh)
+        dumped = {"dir": str(args.dump_outputs), "bytes": nbytes}
 
     # ---- end to end: pinned host frames -> fdt_detect_batch -> host results ------------------------------
     e2e = None
@@ -291,7 +339,7 @@ def main():
         for _ in range(2):
             step_e2e()
         barrier()
-        e_steps = max(2, min(args.steps, 5))
+        e_steps = args.steps
         lib.fdt_timer_begin(h)
         t0 = time.perf_counter()
         for _ in range(e_steps):
@@ -444,6 +492,8 @@ def main():
                 "gpu_launches": launches_per_step * args.steps, "faces_per_step": faces_found,
                 "faces_per_s": faces_found * (world if args.scaling == "weak" else 1) * args.steps / (t_ms / 1e3) if standard else None,
                 "roofline": roofline, "cpu_baseline": cpu, "kernels": kernels}
+        if dumped:
+            line["outputs"] = dumped
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
