@@ -11,6 +11,8 @@ LIB_PATH = PKG / "libfdt_cuda.so"
 
 FDT_OK, FDT_ERR_NOT_READY, FDT_ERR_BAD_ARG, FDT_ERR_SIZE_MISMATCH, FDT_ERR_MODEL, FDT_ERR_CUDA, FDT_ERR_UNSUPPORTED, FDT_ERR_FORMAT = range(8)
 FDT_MAT_8UC1, FDT_MAT_8UC3, FDT_MAT_8UC4 = 0, 16, 24
+FDT_FMT_YUV_NV12, FDT_FMT_YUV_NV21, FDT_FMT_YUV_I420 = 0x1000, 0x1001, 0x1002   # YUV 4:2:0, height * rowStride * 3 / 2 bytes
+YUV_FORMATS = (FDT_FMT_YUV_NV12, FDT_FMT_YUV_NV21, FDT_FMT_YUV_I420)
 FDT_MEM_HOST, FDT_MEM_DEVICE = 0, 1
 FDT_MAX_FACES = 100
 FDT_MESH_FLOATS = 1404

@@ -91,6 +91,12 @@ struct LbTables {
   bool sparse = false;
   int r0 = 0, run = 0, period = 0, rows_c = 0;
   int *y0c = nullptr, *y1c = nullptr;
+  // YUV 4:2:0 frames (even sizes, resizing): chroma rows of y0 / y1 (y / 2), and the same sparse rule applied to the
+  // h / 2 rows of one chroma plane (c_rows_c: compacted rows per plane)
+  int *cy0 = nullptr, *cy1 = nullptr;
+  bool c_sparse = false;
+  int c_r0 = 0, c_run = 0, c_period = 0, c_rows_c = 0;
+  int *cy0c = nullptr, *cy1c = nullptr;
 };
 
 template <typename T> T* dev_upload(const std::vector<T>& v) {
@@ -187,6 +193,46 @@ int channels_of(int mat_type) {
   }
 }
 
+bool is_yuv(int mat_type) { return mat_type == FDT_FMT_YUV_NV12 || mat_type == FDT_FMT_YUV_NV21 || mat_type == FDT_FMT_YUV_I420; }
+
+// Where the bytes of one input frame are.  Packed formats: height rows of row_stride bytes.  YUV 4:2:0: the Y plane, then the
+// chroma area at c_off: c_rows rows of c_row_bytes (NV12 / NV21: h / 2 interleaved rows; I420: the h / 2 rows of U, then those
+// of V), the chroma of pixel (x, y) at row y / 2 (+ h / 2 for V of I420), byte (x / 2) * c_step + u_off / v_off.
+struct FrameLayout {
+  int channels = 0;          // packed formats; 0 for YUV
+  bool yuv = false;
+  long long frame_bytes = 0;
+  long long c_off = 0;
+  int c_row_bytes = 0, c_rows = 0, c_step = 0, u_off = 0, v_off = 0;
+  bool planar = false;       // I420: V is a plane of its own, h / 2 rows behind U
+};
+
+// Validates the frame arguments (w, hh > 0 checked by the caller); *msg names the failure.
+int frame_layout(int mat_type, int w, int hh, int row_stride, FrameLayout* L, const char** msg) {
+  *L = FrameLayout();
+  if (!is_yuv(mat_type)) {
+    L->channels = channels_of(mat_type);
+    if (L->channels == 0) { *msg = "bad frame arguments"; return FDT_ERR_BAD_ARG; }
+    if (row_stride < w * L->channels) { *msg = "row_stride smaller than width * channels"; return FDT_ERR_SIZE_MISMATCH; }
+    L->frame_bytes = (long long)hh * row_stride;
+    return FDT_OK;
+  }
+  if ((w & 1) || (hh & 1)) { *msg = "YUV 4:2:0 frames need an even width and height"; return FDT_ERR_BAD_ARG; }
+  if (row_stride < w) { *msg = "row_stride smaller than width"; return FDT_ERR_SIZE_MISMATCH; }
+  L->yuv = true;
+  L->frame_bytes = (long long)hh * row_stride * 3 / 2;
+  L->c_off = (long long)hh * row_stride;
+  if (mat_type == FDT_FMT_YUV_I420) {
+    if (row_stride & 1) { *msg = "I420 frames need an even row_stride"; return FDT_ERR_BAD_ARG; }
+    L->planar = true;
+    L->c_row_bytes = row_stride / 2; L->c_rows = hh; L->c_step = 1; L->u_off = 0; L->v_off = hh / 2 * L->c_row_bytes;
+  } else {
+    L->c_row_bytes = row_stride; L->c_rows = hh / 2; L->c_step = 2;
+    L->u_off = mat_type == FDT_FMT_YUV_NV12 ? 0 : 1; L->v_off = 1 - L->u_off;
+  }
+  return FDT_OK;
+}
+
 template <typename T> bool dalloc(fdt_handle* h, T** p, size_t n) {
   void* q = nullptr;
   if (cudaMalloc(&q, std::max<size_t>(n, 1) * sizeof(T)) != cudaSuccess) return false;
@@ -202,6 +248,27 @@ template <typename T> bool palloc(fdt_handle* h, T** p, size_t n) {
   return true;
 }
 
+// The rows `need` marks are `run` consecutive rows every `period` (rows first .. first + run - 1 of each period), all the way
+// down, with the plane height a multiple of the period and at most half of each period needed: worth a strided upload.
+bool periodic_rows(const std::vector<char>& need, int* first_out, int* run_out, int* period_out) {
+  const int hh = (int)need.size();
+  int first = 0;
+  while (first < hh && !need[first]) ++first;
+  int run = 0;
+  while (first + run < hh && need[first + run]) ++run;
+  int next = first + run;
+  while (next < hh && !need[next]) ++next;
+  int period = next < hh ? next - first : 0;
+  bool ok = period > run && hh % period == 0 && first + run <= period;
+  for (int r = 0; ok && r < hh; ++r) {
+    int ph = r % period;
+    ok = (need[r] != 0) == (ph >= first && ph < first + run);
+  }
+  if (!ok || run * 2 > period) return false;
+  *first_out = first; *run_out = run; *period_out = period;
+  return true;
+}
+
 const LbTables* get_tables(fdt_handle* h, int w, int hh) {
   for (const LbTables& t : h->tables)
     if (t.w == w && t.h == hh) return &t;
@@ -209,7 +276,7 @@ const LbTables* get_tables(fdt_handle* h, int w, int hh) {
   if (h->tables.size() >= 16) {
     LbTables& t = h->tables.front();
     for (int i = 0; i < kSlots; ++i) cudaStreamSynchronize(h->slots[i].stream);
-    void* tp[] = {t.x0, t.x1, t.y0, t.y1, t.ax0, t.ax1, t.by0, t.by1, t.y0c, t.y1c};
+    void* tp[] = {t.x0, t.x1, t.y0, t.y1, t.ax0, t.ax1, t.by0, t.by1, t.y0c, t.y1c, t.cy0, t.cy1, t.cy0c, t.cy1c};
     for (void* p : tp) if (p) cudaFree(p);
     h->tables.erase(h->tables.begin());
   }
@@ -227,24 +294,28 @@ const LbTables* get_tables(fdt_handle* h, int w, int hh) {
   if (!t.identity) {
     std::vector<char> need(hh, 0);
     for (int i = 0; i < t.lp.new_h; ++i) { need[y0[i]] = 1; need[y1[i]] = 1; }
-    int first = 0;
-    while (first < hh && !need[first]) ++first;
-    int run = 0;
-    while (first + run < hh && need[first + run]) ++run;
-    int next = first + run;
-    while (next < hh && !need[next]) ++next;
-    int period = next < hh ? next - first : 0;
-    bool ok = period > run && hh % period == 0 && first + run <= period;
-    for (int r = 0; ok && r < hh; ++r) {
-      int ph = r % period;
-      ok = (need[r] != 0) == (ph >= first && ph < first + run);
-    }
-    if (ok && run * 2 <= period) {
+    int first = 0, run = 0, period = 0;
+    if (periodic_rows(need, &first, &run, &period)) {
       std::vector<int> y0c(t.lp.new_h), y1c(t.lp.new_h);
       auto compact = [&](int r) { return (r / period) * run + (r % period - first); };
       for (int i = 0; i < t.lp.new_h; ++i) { y0c[i] = compact(y0[i]); y1c[i] = compact(y1[i]); }
       t.y0c = dev_upload(y0c); t.y1c = dev_upload(y1c);
       if (t.y0c && t.y1c) { t.sparse = true; t.r0 = first; t.run = run; t.period = period; t.rows_c = hh / period * run; }
+    }
+    if (hh % 2 == 0 && w % 2 == 0) {
+      // YUV 4:2:0 chroma rows: the rows of one chroma plane (h / 2 of them) the taps read, same sparse rule
+      const int ch = hh / 2;
+      std::vector<int> cy0(t.lp.new_h), cy1(t.lp.new_h);
+      std::vector<char> cneed(ch, 0);
+      for (int i = 0; i < t.lp.new_h; ++i) { cy0[i] = y0[i] >> 1; cy1[i] = y1[i] >> 1; cneed[cy0[i]] = 1; cneed[cy1[i]] = 1; }
+      t.cy0 = dev_upload(cy0); t.cy1 = dev_upload(cy1);
+      if (!t.cy0 || !t.cy1) return nullptr;
+      if (periodic_rows(cneed, &first, &run, &period)) {
+        auto compact = [&](int r) { return (r / period) * run + (r % period - first); };
+        for (int i = 0; i < t.lp.new_h; ++i) { cy0[i] = compact(cy0[i]); cy1[i] = compact(cy1[i]); }
+        t.cy0c = dev_upload(cy0); t.cy1c = dev_upload(cy1);
+        if (t.cy0c && t.cy1c) { t.c_sparse = true; t.c_r0 = first; t.c_run = run; t.c_period = period; t.c_rows_c = ch / period * run; }
+      }
     }
   }
   h->tables.push_back(t);
@@ -293,6 +364,43 @@ void fill_letterbox(LetterboxP& lb, const LbTables* tb, const uint8_t* d_fr, lon
   lb.identity = tb->identity ? 1 : 0;
 }
 
+// YUV frames: the Y planes at d_y (y_stride bytes apart, compacted when y_sparse), the chroma areas at d_c (c_stride apart,
+// compacted when c_sparse); for whole frames d_c = d_y + c_off and both strides are the frame size.
+void fill_letterbox_yuv(LetterboxYuvP& p, const LbTables* tb, const FrameLayout& L, const uint8_t* d_y, long long y_stride,
+                        bool y_sparse, const uint8_t* d_c, long long c_stride, bool c_sparse, int row_stride, int w, int hh,
+                        uint8_t* out, int S_w, int S_h) {
+  fill_letterbox(p.lb, tb, d_y, y_stride, row_stride, 0, w, hh, out, S_w, S_h, y_sparse);
+  p.chroma = d_c; p.c_frame_stride = c_stride;
+  p.c_row_stride = L.c_row_bytes; p.c_step = L.c_step; p.u_off = L.u_off;
+  // I420: V follows U, whose rows are compacted like V's
+  p.v_off = L.planar ? (c_sparse ? tb->c_rows_c : hh / 2) * L.c_row_bytes : L.v_off;
+  p.cy0 = c_sparse ? tb->cy0c : tb->cy0; p.cy1 = c_sparse ? tb->cy1c : tb->cy1;
+}
+
+void set_warp_layout(WarpP& wp, const FrameLayout& L) {
+  wp.yuv = L.yuv ? 1 : 0; wp.c_off = L.c_off; wp.c_row_stride = L.c_row_bytes; wp.c_step = L.c_step;
+  wp.u_off = L.u_off; wp.v_off = L.v_off;
+}
+
+// `run` rows of every `period` of one plane (row_bytes per row, `groups` periods) of each of n frames fb bytes apart, src =
+// the first needed row of frame 0, into dst as [n][groups * run][row_bytes].  One 3-D copy when the frame size is a whole number
+// of periods (the host side is then one pitched volume), else one 2-D copy per frame.
+void upload_rows(uint8_t* dst, const uint8_t* src, size_t row_bytes, int run, int period, int groups, size_t fb, int n, cudaStream_t s) {
+  const size_t pitch = (size_t)period * row_bytes, width = (size_t)run * row_bytes;
+  if (fb % pitch == 0) {
+    cudaMemcpy3DParms c = {};
+    c.srcPtr = make_cudaPitchedPtr(const_cast<uint8_t*>(src), pitch, width, fb / pitch);
+    c.dstPtr = make_cudaPitchedPtr(dst, width, width, (size_t)groups);
+    c.extent = make_cudaExtent(width, (size_t)groups, (size_t)n);
+    c.kind = cudaMemcpyHostToDevice;
+    cudaMemcpy3DAsync(&c, s);
+  } else {
+    for (int f = 0; f < n; ++f)
+      cudaMemcpy2DAsync(dst + (size_t)f * width * groups, width, src + (size_t)f * fb, pitch, width, (size_t)groups,
+                        cudaMemcpyHostToDevice, s);
+  }
+}
+
 void fill_decode(DecodeP& d, fdt_handle* h, const Slot& sl, const LbTables* tb, int w, int hh) {
   const Plan& dp = h->det.plan();
   const int S_w = h->det.in_w(), S_h = h->det.in_h();
@@ -311,6 +419,7 @@ void fill_decode(DecodeP& d, fdt_handle* h, const Slot& sl, const LbTables* tb, 
 
 struct CallArgs {
   const uint8_t* frames; int batch, w, hh, row_stride, channels, mode, mem_kind;
+  FrameLayout lay;
   fdt_face* out_faces; int32_t* out_counts; float* out_mesh; float* out_iris;
   bool keep_on_device;
   const LbTables* tb;
@@ -325,9 +434,14 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
   cudaStream_t s = sl.stream;
   const LbTables* tb = a.tb;
   const int S_w = h->det.in_w(), S_h = h->det.in_h();
-  const bool sparse = a.mem_kind == FDT_MEM_HOST && a.mode == FDT_MODE_FAST && tb->sparse;
+  const bool fast_host = a.mem_kind == FDT_MEM_HOST && a.mode == FDT_MODE_FAST;
+  const bool sparse = fast_host && !a.lay.yuv && tb->sparse;
+  // YUV frames: the Y plane and the chroma area go up independently, each compacted when its tap rows are periodic
+  const bool y_sparse = fast_host && a.lay.yuv && tb->sparse, c_sparse = fast_host && a.lay.yuv && tb->c_sparse;
   long long dev_frame_stride = a.frame_stride;
   const uint8_t* d_fr;
+  const uint8_t* d_c = nullptr;
+  long long y_stride = a.frame_stride, c_stride = a.frame_stride;
   if (a.mem_kind == FDT_MEM_HOST) {
     size_t need = (size_t)h->chunk * a.frame_stride;
     if (sl.d_frames_cap < need) {
@@ -338,7 +452,30 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
       sl.d_frames_cap = need;
     }
     const uint8_t* src = a.frames + (size_t)off * a.frame_stride;
-    if (sparse) {
+    if (y_sparse || c_sparse) {
+      const FrameLayout& L = a.lay;
+      const size_t fb = (size_t)a.frame_stride, y_bytes = (size_t)a.hh * a.row_stride, c_bytes = (size_t)L.c_rows * L.c_row_bytes;
+      uint8_t* d_y = sl.d_frames;
+      if (y_sparse) {
+        upload_rows(d_y, src + (size_t)tb->r0 * a.row_stride, a.row_stride, tb->run, tb->period, a.hh / tb->period, fb, n, s);
+        y_stride = (long long)tb->rows_c * a.row_stride;
+      } else {
+        cudaMemcpy2DAsync(d_y, y_bytes, src, fb, y_bytes, n, cudaMemcpyHostToDevice, s);
+        y_stride = (long long)y_bytes;
+      }
+      uint8_t* dc = d_y + (size_t)n * y_stride;
+      if (c_sparse) {
+        // I420: U and V stacked are one area of h rows with the same period (h / 2 is a multiple of it)
+        upload_rows(dc, src + L.c_off + (size_t)tb->c_r0 * L.c_row_bytes, L.c_row_bytes, tb->c_run, tb->c_period,
+                    L.c_rows / tb->c_period, fb, n, s);
+        c_stride = (long long)(L.c_rows / tb->c_period * tb->c_run) * L.c_row_bytes;
+      } else {
+        cudaMemcpy2DAsync(dc, c_bytes, src + L.c_off, fb, c_bytes, n, cudaMemcpyHostToDevice, s);
+        c_stride = (long long)c_bytes;
+      }
+      h->h2d_bytes += (long long)n * (y_stride + c_stride);
+      d_c = dc;
+    } else if (sparse) {
       // one strided DMA: `run` rows out of every `period`, for all n frames (frames are contiguous)
       size_t width_b = (size_t)tb->run * a.row_stride;
       cudaMemcpy2DAsync(sl.d_frames, width_b, src + (size_t)tb->r0 * a.row_stride, (size_t)tb->period * a.row_stride,
@@ -355,9 +492,16 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
   }
   {
     StageTimer t(h, 0, s);
-    LetterboxP lb;
-    fill_letterbox(lb, tb, d_fr, dev_frame_stride, a.row_stride, a.channels, a.w, a.hh, sl.d_lb, S_w, S_h, sparse);
-    launch_letterbox(lb, n, s);
+    if (a.lay.yuv) {
+      if (!d_c) d_c = d_fr + a.lay.c_off;     // whole frames
+      LetterboxYuvP lb;
+      fill_letterbox_yuv(lb, tb, a.lay, d_fr, y_stride, y_sparse, d_c, c_stride, c_sparse, a.row_stride, a.w, a.hh, sl.d_lb, S_w, S_h);
+      launch_letterbox_yuv(lb, n, s);
+    } else {
+      LetterboxP lb;
+      fill_letterbox(lb, tb, d_fr, dev_frame_stride, a.row_stride, a.channels, a.w, a.hh, sl.d_lb, S_w, S_h, sparse);
+      launch_letterbox(lb, n, s);
+    }
     t.launches = 1;
   }
   {
@@ -455,6 +599,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
       wp.frames = job.d_fr; wp.frame_stride = dev_frame_stride; wp.row_stride = a.row_stride; wp.channels = a.channels;
       wp.src_w = a.w; wp.src_h = a.hh; wp.crop_img = sl.d_crop_img; wp.affine = sl.d_affine; wp.ncrops = nf;
       wp.out_size = kMeshInput; wp.flip_odd = 0; wp.crops = sl.d_crops;
+      set_warp_layout(wp, a.lay);
       launch_warp_affine(wp, s);
       t.launches = 1;
     }
@@ -534,6 +679,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
           wp.frames = job.d_fr; wp.frame_stride = dev_frame_stride; wp.row_stride = a.row_stride; wp.channels = a.channels;
           wp.src_w = a.w; wp.src_h = a.hh; wp.crop_img = sl.d_eye_img; wp.affine = sl.d_eye_affine; wp.ncrops = ne;
           wp.out_size = kIrisInput; wp.flip_odd = 1; wp.crops = sl.d_eye_crops;
+          set_warp_layout(wp, a.lay);
           launch_warp_affine(wp, s);
           t.launches = 1;
         }
@@ -581,9 +727,10 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
 int detect_single(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh, int row_stride, int mat_type, int mode,
                   int mem_kind, fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris, bool keep_on_device) {
   if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
-  int channels = channels_of(mat_type);
-  if (!frames || batch < 0 || w <= 0 || hh <= 0 || channels == 0) return fail(h, FDT_ERR_BAD_ARG, "bad frame arguments");
-  if (row_stride < w * channels) return fail(h, FDT_ERR_SIZE_MISMATCH, "row_stride smaller than width * channels");
+  if (!frames || batch < 0 || w <= 0 || hh <= 0) return fail(h, FDT_ERR_BAD_ARG, "bad frame arguments");
+  FrameLayout lay;
+  const char* msg = nullptr;
+  if (int rc = frame_layout(mat_type, w, hh, row_stride, &lay, &msg)) return fail(h, rc, msg);
   if (mode != FDT_MODE_FAST && mode != FDT_MODE_STANDARD && mode != FDT_MODE_FULL) return fail(h, FDT_ERR_BAD_ARG, "unknown mode");
   if (mode != FDT_MODE_FAST && !h->has_mesh) return fail(h, FDT_ERR_NOT_READY, "standard / full mode needs the face_landmark model");
   if (mode == FDT_MODE_FULL && !h->has_iris) return fail(h, FDT_ERR_NOT_READY, "full mode needs the iris_landmark model");
@@ -596,12 +743,13 @@ int detect_single(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh
   if (batch == 0) return FDT_OK;
   if (!ensure_results(h, batch)) return FDT_ERR_CUDA;
   CallArgs a;
-  a.frames = frames; a.batch = batch; a.w = w; a.hh = hh; a.row_stride = row_stride; a.channels = channels; a.mode = mode;
+  a.frames = frames; a.batch = batch; a.w = w; a.hh = hh; a.row_stride = row_stride; a.channels = lay.channels; a.mode = mode;
+  a.lay = lay;
   a.mem_kind = mem_kind; a.out_faces = out_faces; a.out_counts = out_counts; a.out_mesh = out_mesh; a.out_iris = out_iris;
   a.keep_on_device = keep_on_device;
   a.tb = get_tables(h, w, hh);
   if (!a.tb) return fail(h, FDT_ERR_CUDA, "letterbox table upload failed");
-  a.frame_stride = (long long)hh * row_stride;
+  a.frame_stride = lay.frame_bytes;
   h->last_first_chunk = std::min(batch, h->chunk);
   h->last_mesh_faces = 0; h->last_iris_faces = 0;
 
@@ -642,7 +790,11 @@ int detect_multi(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh,
   if (batch <= 0 || !frames) return detect_single(h->shards[0], frames, batch, w, hh, row_stride, mat_type, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris, false);
   std::vector<int> rcs(g, FDT_OK);
   std::vector<std::thread> th;
-  const long long frame_stride = (long long)hh * row_stride;
+  FrameLayout lay;
+  const char* msg = nullptr;
+  if (w <= 0 || hh <= 0) return fail(h, FDT_ERR_BAD_ARG, "bad frame arguments");
+  if (int rc = frame_layout(mat_type, w, hh, row_stride, &lay, &msg)) return fail(h, rc, msg);
+  const long long frame_stride = lay.frame_bytes;
   for (int r = 0; r < g; ++r) {
     const int lo = (int)((long long)batch * r / g), hi = (int)((long long)batch * (r + 1) / g);   // sharding.shard_range
     if (hi <= lo) continue;
@@ -949,7 +1101,7 @@ int32_t fdt_destroy(fdt_handle* h) {
     void* dev[] = {h->d_faces, h->d_counts, h->d_anchors};
     for (void* p : dev) if (p) cudaFree(p);
     for (LbTables& t : h->tables) {
-      void* tp[] = {t.x0, t.x1, t.y0, t.y1, t.ax0, t.ax1, t.by0, t.by1, t.y0c, t.y1c};
+      void* tp[] = {t.x0, t.x1, t.y0, t.y1, t.ax0, t.ax1, t.by0, t.by1, t.y0c, t.y1c, t.cy0, t.cy1, t.cy0c, t.cy1c};
       for (void* p : tp) if (p) cudaFree(p);
     }
     if (h->ev[0]) cudaEventDestroy(h->ev[0]);
@@ -972,11 +1124,14 @@ int32_t fdt_detect_one(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int32
                        int32_t mode, fdt_face* out_faces, int32_t* out_count, float* out_mesh, float* out_iris) {
   if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
   std::lock_guard<std::mutex> g(h->mu);
-  int ch = channels_of(mat_type);
-  if (ch == 0 || width <= 0 || height <= 0) return fail(h, FDT_ERR_BAD_ARG, "bad frame arguments");
-  // matFromPackedBytes length check (lib/src/util/helpers.dart:440-447)
-  if (nbytes != (size_t)width * height * ch) return fail(h, FDT_ERR_SIZE_MISMATCH, "bytes length does not equal width * height * channels");
-  return detect_impl(h, bytes, 1, width, height, width * ch, mat_type, mode, FDT_MEM_HOST, out_faces, out_count, out_mesh, out_iris, false);
+  if (width <= 0 || height <= 0) return fail(h, FDT_ERR_BAD_ARG, "bad frame arguments");
+  const int row_stride = is_yuv(mat_type) ? width : width * channels_of(mat_type);
+  FrameLayout lay;
+  const char* msg = nullptr;
+  if (int rc = frame_layout(mat_type, width, height, row_stride, &lay, &msg)) return fail(h, rc, msg);
+  // matFromPackedBytes length check (lib/src/util/helpers.dart:440-447); YUV: width * height * 3 / 2
+  if (nbytes != (size_t)lay.frame_bytes) return fail(h, FDT_ERR_SIZE_MISMATCH, "bytes length does not equal the frame size (width * height * channels)");
+  return detect_impl(h, bytes, 1, width, height, row_stride, mat_type, mode, FDT_MEM_HOST, out_faces, out_count, out_mesh, out_iris, false);
 }
 
 int32_t fdt_detect_batch_device(fdt_handle* h, const uint8_t* d_frames, int32_t batch, int32_t width, int32_t height,
@@ -1469,10 +1624,12 @@ int32_t fdt_profile_chunk(fdt_handle* h, const uint8_t* d_frames, int32_t n, int
   if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
   h = primary(h);
   std::lock_guard<std::mutex> g(h->mu);
-  int channels = channels_of(mat_type);
   const int S = (int)h->det.plan().steps.size();
   if (out_launches) *out_launches = S + 2;
-  if (!d_frames || n <= 0 || n > h->chunk || channels == 0 || row_stride < width * channels || repeats <= 0)
+  FrameLayout lay;
+  const char* msg = nullptr;
+  if (!d_frames || n <= 0 || n > h->chunk || width <= 0 || height <= 0 || repeats <= 0 ||
+      frame_layout(mat_type, width, height, row_stride, &lay, &msg) != FDT_OK)
     return fail(h, FDT_ERR_BAD_ARG, "bad profile arguments");
   if (!out_ms || capacity < S + 2) return fail(h, FDT_ERR_SIZE_MISMATCH, "out_ms too small");
   cudaSetDevice(h->cfg.device);
@@ -1486,10 +1643,17 @@ int32_t fdt_profile_chunk(fdt_handle* h, const uint8_t* d_frames, int32_t n, int
   cudaStream_t s = sl.stream;
   const int S_w = h->det.in_w(), S_h = h->det.in_h();
   for (int r = 0; r < repeats; ++r) {
-    LetterboxP lb;
-    fill_letterbox(lb, tb, d_frames, (long long)height * row_stride, row_stride, channels, width, height, sl.d_lb, S_w, S_h, false);
     cudaEventRecord(ev[0], s);
-    launch_letterbox(lb, n, s);
+    if (lay.yuv) {
+      LetterboxYuvP lb;
+      fill_letterbox_yuv(lb, tb, lay, d_frames, lay.frame_bytes, false, d_frames + lay.c_off, lay.frame_bytes, false, row_stride,
+                         width, height, sl.d_lb, S_w, S_h);
+      launch_letterbox_yuv(lb, n, s);
+    } else {
+      LetterboxP lb;
+      fill_letterbox(lb, tb, d_frames, lay.frame_bytes, row_stride, lay.channels, width, height, sl.d_lb, S_w, S_h, false);
+      launch_letterbox(lb, n, s);
+    }
     h->det.run(sl.det_ctx, sl.d_lb, n, s, ev.data() + 1);
     DecodeP d;
     fill_decode(d, h, sl, tb, width, height);

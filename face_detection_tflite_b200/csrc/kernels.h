@@ -61,6 +61,17 @@ void launch_maxpool(const PoolP& p, int B, cudaStream_t s);
 void launch_resize_bilinear(const ResizeP& p, int B, cudaStream_t s);
 
 // ---- preprocessing ----
+#ifdef __CUDACC__
+// cv::cvtColor COLOR_YUV2BGR_NV12 / _NV21 / _I420 for one sample (BT.601 limited range, 20-bit fixed point, imgproc/color_yuv):
+// v[0..2] = B, G, R.
+__device__ __forceinline__ int sat_u8(int v) { return v < 0 ? 0 : (v > 255 ? 255 : v); }
+__device__ __forceinline__ void yuv_to_bgr(int Y, int U, int V, int* v) {
+  const int yy = max(Y - 16, 0) * 1220542 + (1 << 19), u = U - 128, w = V - 128;
+  v[0] = sat_u8((yy + 2116026 * u) >> 20);
+  v[1] = sat_u8((yy - 852492 * w - 409993 * u) >> 20);
+  v[2] = sat_u8((yy + 1673527 * w) >> 20);
+}
+#endif
 struct LetterboxP {
   const uint8_t* frames;   // [B][H][row_stride]
   long long frame_stride;  // bytes between frames
@@ -73,6 +84,19 @@ struct LetterboxP {
   int identity;            // 1: no resize (new == src)
 };
 void launch_letterbox(const LetterboxP& p, int B, cudaStream_t s);
+// YUV 4:2:0 frames (k_letterbox_yuv): lb.frames is the Y plane, lb.row_stride its row stride, lb.channels unused.  The chroma of
+// frame b starts at chroma + b * c_frame_stride; the chroma sample of pixel (x, y) sits in chroma row cy0 / cy1 (the rows of
+// lb.y0 / lb.y1, halved and, for a compacted upload, renumbered), byte (x >> 1) * c_step + u_off (U) / v_off (V):
+// NV12 c_step 2, u_off 0, v_off 1; NV21 2, 1, 0; I420 1, 0, offset of the V plane behind the U plane.
+// (A struct of its own: LetterboxP keeps its size, so k_letterbox keeps its parameter layout.)
+struct LetterboxYuvP {
+  LetterboxP lb;
+  const uint8_t* chroma;
+  long long c_frame_stride;
+  int c_row_stride, c_step, u_off, v_off;
+  const int* cy0; const int* cy1;
+};
+void launch_letterbox_yuv(const LetterboxYuvP& p, int B, cudaStream_t s);
 // u8 [B][S][S][4] BGRX -> f32 [B][S][S][3] RGB, v*(1/127.5)-1
 void launch_normalize(const uint8_t* in, TV out, int B, cudaStream_t s);
 
@@ -273,6 +297,10 @@ struct WarpP {
   int ncrops, out_size;
   int flip_odd;            // 1: odd crops are mirrored horizontally (cv.flip(rightEye, 1), face_detector_core.dart:567)
   uint8_t* crops;          // [ncrops][out][out][4] BGRX
+  // yuv = 1: YUV 4:2:0 frames (channels unused), `frames` dense: chroma at frame + c_off, addressed as in LetterboxP
+  int yuv = 0;
+  long long c_off = 0;
+  int c_row_stride = 0, c_step = 0, u_off = 0, v_off = 0;
 };
 void launch_warp_affine(const WarpP& p, cudaStream_t s);
 

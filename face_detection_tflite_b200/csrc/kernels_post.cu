@@ -2,7 +2,8 @@
 // operation by operation exactly like the reference's Dart doubles / OpenCV's C++:
 //   k_decode_nms       threshold -> ordered compaction -> decode -> sort -> weighted NMS ->
 //                      letterbox removal -> gates   (one block per image)
-//   k_warp_affine      cv::warpAffine(INTER_LINEAR, BORDER_CONSTANT 0) into square BGR crops (192 face / 64 eye)
+//   k_warp_affine      cv::warpAffine(INTER_LINEAR, BORDER_CONSTANT 0) into square BGR crops (192 face / 64 eye);
+//                      YUV 4:2:0 frames are converted tap by tap (in-frame taps only)
 //   k_mesh_post        _unpackLandmarks + transformMeshToAbsolute + face-flag sigmoid
 //   k_iris_post        _unpackLandmarks(clamp: false) + transformIrisNormToAbsolute + iris-centre eye keypoints
 #include "fdt_math.h"
@@ -238,7 +239,14 @@ __global__ void k_warp_affine(WarpP p) {
 #pragma unroll
     for (int t = 0; t < 4; ++t) {
       int yy = sy + (t >> 1), xx = sx + (t & 1);
-      if (yy < 0 || yy >= p.src_h || xx < 0 || xx >= p.src_w) continue;
+      if (yy < 0 || yy >= p.src_h || xx < 0 || xx >= p.src_w) continue;   // out-of-frame taps: BGR 0 (also for YUV frames)
+      if (p.yuv) {
+        const uint8_t* c = src + p.c_off + (size_t)(yy >> 1) * p.c_row_stride + (size_t)(xx >> 1) * p.c_step;
+        int v[3];
+        yuv_to_bgr(src[(size_t)yy * p.row_stride + xx], c[p.u_off], c[p.v_off], v);
+        acc[0] += v[0] * iw[t]; acc[1] += v[1] * iw[t]; acc[2] += v[2] * iw[t];
+        continue;
+      }
       const uint8_t* px = src + (size_t)yy * p.row_stride + (size_t)xx * p.channels;
       if (p.channels == 1) {
         acc[0] += px[0] * iw[t]; acc[1] += px[0] * iw[t]; acc[2] += px[0] * iw[t];

@@ -1,5 +1,5 @@
 // Preprocessing kernels: fused letterbox (cv::resize INTER_LINEAR 8U fixed point +
-// copyMakeBorder(0) + BGRA/GRAY->BGR) and the [-1,1] normalisation.
+// copyMakeBorder(0) + BGRA/GRAY->BGR, or cvtColor YUV2BGR for NV12 / NV21 / I420 frames) and the [-1,1] normalisation.
 // Reference: convertImageToTensor / bgrMatToSignedFloat32 (lib/src/util/helpers.dart:303-421).
 #include "kernels.h"
 
@@ -9,6 +9,15 @@ namespace {
 __device__ __forceinline__ void load_bgr(const uint8_t* px, int channels, int* v) {
   if (channels == 1) { v[0] = v[1] = v[2] = px[0]; }
   else { v[0] = px[0]; v[1] = px[1]; v[2] = px[2]; }
+}
+
+// HResizeLinear (11-bit) then VResizeLinear<uchar,int,short> fixed point (resize.cpp) of one channel of four taps
+__device__ __forceinline__ int resize_linear(int t00, int t01, int t10, int t11, int wa, int wb, int va, int vb) {
+  int h0 = t00 * wa + t01 * wb;
+  int h1 = t10 * wa + t11 * wb;
+  int v = ((va * (h0 >> 4)) >> 16) + ((vb * (h1 >> 4)) >> 16);
+  v = (v + 2) >> 2;
+  return v < 0 ? 0 : (v > 255 ? 255 : v);
 }
 
 // One thread per output pixel: four 3-byte taps (byte loads; neighbouring threads share the sectors through L1) and one uchar4
@@ -45,18 +54,56 @@ __global__ void __launch_bounds__(256) k_letterbox(LetterboxP p, int B) {
         load_bgr(r1 + (size_t)xb * p.channels, p.channels, t11);
         int res[3];
 #pragma unroll
-        for (int c = 0; c < 3; ++c) {
-          // HResizeLinear (11-bit) then VResizeLinear<uchar,int,short> fixed point (resize.cpp)
-          int h0 = t00[c] * wa + t01[c] * wb;
-          int h1 = t10[c] * wa + t11[c] * wb;
-          int v = ((va * (h0 >> 4)) >> 16) + ((vb * (h1 >> 4)) >> 16);
-          v = (v + 2) >> 2;
-          res[c] = v < 0 ? 0 : (v > 255 ? 255 : v);
-        }
+        for (int c = 0; c < 3; ++c) res[c] = resize_linear(t00[c], t01[c], t10[c], t11[c], wa, wb, va, vb);
         o = make_uchar3((unsigned char)res[0], (unsigned char)res[1], (unsigned char)res[2]);
       }
     }
     reinterpret_cast<uchar4*>(p.out)[((size_t)b * p.dst_h + y) * p.dst_w + x] = make_uchar4(o.x, o.y, o.z, 0);
+  }
+}
+
+// One YUV 4:2:0 tap: the Y byte and the chroma pair of its 2x2 block, converted to BGR (cvtColor first, then resize).
+__device__ __forceinline__ void load_yuv(const uint8_t* yrow, const uint8_t* crow, int x, const LetterboxYuvP& p, int* v) {
+  const uint8_t* c = crow + (size_t)(x >> 1) * p.c_step;
+  yuv_to_bgr(yrow[x], c[p.u_off], c[p.v_off], v);
+}
+
+// k_letterbox for NV12 / NV21 / I420 frames: same grid and fixed-point resize; every tap is converted before it is weighted
+// (the conversion is per pixel, so this equals resizing the converted frame).  Padding stays BGR 0.
+__global__ void __launch_bounds__(256) k_letterbox_yuv(LetterboxYuvP p, int B) {
+  const LetterboxP& q = p.lb;
+  const int x = blockIdx.x * 64 + (threadIdx.x & 63), y = blockIdx.y * 4 + (threadIdx.x >> 6);
+  if (x >= q.dst_w || y >= q.dst_h) return;
+  for (int b = blockIdx.z; b < B; b += gridDim.z) {
+    const int dy = y - q.pad_top, dx = x - q.pad_left;
+    uchar3 o = make_uchar3(0, 0, 0);
+    if (dy >= 0 && dy < q.new_h && dx >= 0 && dx < q.new_w) {
+      const uint8_t* ys = q.frames + (size_t)b * q.frame_stride;
+      const uint8_t* cs = p.chroma + (size_t)b * p.c_frame_stride;
+      if (q.identity) {
+        int v[3];
+        load_yuv(ys + (size_t)dy * q.row_stride, cs + (size_t)(dy >> 1) * p.c_row_stride, dx, p, v);
+        o = make_uchar3((unsigned char)v[0], (unsigned char)v[1], (unsigned char)v[2]);
+      } else {
+        const int xa = q.x0[dx], xb = q.x1[dx], wa = q.ax0[dx], wb = q.ax1[dx];
+        const int ya = q.y0[dy], yb = q.y1[dy], va = q.by0[dy], vb = q.by1[dy];
+        const int ca = p.cy0[dy], cb = p.cy1[dy];
+        int t00[3], t01[3], t10[3], t11[3];
+        const uint8_t* r0 = ys + (size_t)ya * q.row_stride;
+        const uint8_t* r1 = ys + (size_t)yb * q.row_stride;
+        const uint8_t* c0 = cs + (size_t)ca * p.c_row_stride;
+        const uint8_t* c1 = cs + (size_t)cb * p.c_row_stride;
+        load_yuv(r0, c0, xa, p, t00);
+        load_yuv(r0, c0, xb, p, t01);
+        load_yuv(r1, c1, xa, p, t10);
+        load_yuv(r1, c1, xb, p, t11);
+        int res[3];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) res[c] = resize_linear(t00[c], t01[c], t10[c], t11[c], wa, wb, va, vb);
+        o = make_uchar3((unsigned char)res[0], (unsigned char)res[1], (unsigned char)res[2]);
+      }
+    }
+    reinterpret_cast<uchar4*>(q.out)[((size_t)b * q.dst_h + y) * q.dst_w + x] = make_uchar4(o.x, o.y, o.z, 0);
   }
 }
 
@@ -80,6 +127,12 @@ void launch_letterbox(const LetterboxP& p, int B, cudaStream_t s) {
   if (B <= 0) return;
   dim3 grid((unsigned)((p.dst_w + 63) / 64), (unsigned)((p.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
   k_letterbox<<<grid, 256, 0, s>>>(p, B);
+}
+
+void launch_letterbox_yuv(const LetterboxYuvP& p, int B, cudaStream_t s) {
+  if (B <= 0) return;
+  dim3 grid((unsigned)((p.lb.dst_w + 63) / 64), (unsigned)((p.lb.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
+  k_letterbox_yuv<<<grid, 256, 0, s>>>(p, B);
 }
 
 void launch_normalize(const uint8_t* in, TV out, int B, cudaStream_t s) {

@@ -127,9 +127,12 @@ class FaceDetector:
     def detectFacesFromMatBytes(self, data, *, width: int, height: int, matType: int = 16,
                                 mode: FaceDetectionMode = FaceDetectionMode.full) -> List[Face]:
         """detectFacesFromMatBytes (face_detector.dart:588-609); the default mode is `full` like the reference's
-        (detector + mesh + iris; the blendshape classifier is outside this path)."""
+        (detector + mesh + iris; the blendshape classifier is outside this path).  matType may also be one of the YUV 4:2:0
+        formats FDT_FMT_YUV_NV12 / _NV21 / _I420: `data` is then width * height * 3 / 2 bytes (cv2's (3H/2) x W Mat)."""
         self._check()
         buf = np.ascontiguousarray(np.frombuffer(data, np.uint8) if not isinstance(data, np.ndarray) else data.reshape(-1))
+        if matType in _ffi.YUV_FORMATS and buf.size != width * height * 3 // 2:
+            raise ValueError("bytes length does not equal width * height * 3 / 2")        # helpers.dart:440-447
         faces = (_ffi.FdtFace * self._max_faces)()
         count = C.c_int32(0)
         mode = FaceDetectionMode(mode)
@@ -192,7 +195,8 @@ class FaceDetector:
 
     def detectFacesBatch(self, frames, *, count: int, width: int, height: int, matType: int = 16,
                          mode: FaceDetectionMode = FaceDetectionMode.fast) -> List[List[Face]]:
-        """New batched entry point: `frames` holds `count` packed frames (bytes / uint8 array)."""
+        """New batched entry point: `frames` holds `count` packed frames (bytes / uint8 array), or `count` YUV 4:2:0 frames of
+        width * height * 3 / 2 bytes with matType FDT_FMT_YUV_NV12 / _NV21 / _I420."""
         self._check()
         faces, counts, mesh, iris = self.detectBatchRaw(frames, count=count, width=width, height=height,
                                                         matType=matType, mode=mode, withIris=True)
@@ -208,16 +212,19 @@ class FaceDetector:
                        rowStride: Optional[int] = None, withIris: bool = False):
         """fdt_detect_batch with array outputs: (FdtFace array, counts int32[count], mesh f32 or None) and, with
         withIris=True, a fourth element iris f32 [count, max_faces, 152, 3] (None unless mode is full).
-        `frames` may be a numpy array / bytes (host) or an integer device pointer with memKind=FDT_MEM_DEVICE."""
+        `frames` may be a numpy array / bytes (host) or an integer device pointer with memKind=FDT_MEM_DEVICE.
+        YUV 4:2:0 formats: rowStride is the Y-plane stride (default: width) and a frame is height * rowStride * 3 / 2 bytes."""
         self._check()
-        ch = {_ffi.FDT_MAT_8UC1: 1, _ffi.FDT_MAT_8UC3: 3, _ffi.FDT_MAT_8UC4: 4}.get(matType, 0)
+        yuv = matType in _ffi.YUV_FORMATS
+        ch = 1 if yuv else {_ffi.FDT_MAT_8UC1: 1, _ffi.FDT_MAT_8UC3: 3, _ffi.FDT_MAT_8UC4: 4}.get(matType, 0)
         stride = rowStride if rowStride is not None else width * ch
+        frame_bytes = height * stride * 3 // 2 if yuv else height * stride
         if isinstance(frames, int):
             ptr = frames
         else:
             buf = np.ascontiguousarray(np.frombuffer(frames, np.uint8) if not isinstance(frames, np.ndarray) else frames.reshape(-1))
-            if buf.size != count * height * stride:
-                raise ValueError("frames length does not equal count * height * rowStride")   # helpers.dart:440-447
+            if buf.size != count * frame_bytes:
+                raise ValueError("frames length does not equal count * height * rowStride%s" % (" * 3 / 2" if yuv else ""))   # helpers.dart:440-447
             ptr = buf.ctypes.data
         faces = (_ffi.FdtFace * max(1, count * self._max_faces))()
         counts = np.zeros(max(1, count), np.int32)

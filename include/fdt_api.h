@@ -72,6 +72,18 @@ typedef enum fdt_mode {
  * colour conversion rule lib/src/util/helpers.dart:386-392). */
 enum { FDT_MAT_8UC1 = 0, FDT_MAT_8UC3 = 16, FDT_MAT_8UC4 = 24 };
 
+/* YUV 4:2:0 frames (camera frames, hardware video decoders), accepted wherever mat_type is, except by
+ * fdt_extract_aligned_squares.  The result equals cv::cvtColor(frame, COLOR_YUV2BGR_NV12 / _NV21 / _I420) followed
+ * by the BGR path; the conversion is fused into the letterbox and crop kernels (no host pass).
+ * width and height are the image size and must both be even (else FDT_ERR_BAD_ARG); row_stride is the Y-plane
+ * stride in bytes, >= width (else FDT_ERR_SIZE_MISMATCH).  One frame is height * row_stride * 3 / 2 bytes:
+ *   NV12 / NV21: Y plane, then the interleaved chroma plane (U,V / V,U) at height * row_stride, same row stride;
+ *   I420: Y plane, then the U plane at height * row_stride with row stride row_stride / 2 (row_stride must be even,
+ *         else FDT_ERR_BAD_ARG), then the V plane.
+ * With row_stride == width this is cv2's (3H/2) x W single-channel Mat.  The values cannot collide with a cv
+ * MatType (at most 4095). */
+enum { FDT_FMT_YUV_NV12 = 0x1000, FDT_FMT_YUV_NV21 = 0x1001, FDT_FMT_YUV_I420 = 0x1002 };
+
 enum { FDT_MEM_HOST = 0, FDT_MEM_DEVICE = 1 };
 
 enum { FDT_MAX_FACES = 100 };      /* weightedNms maxDet, lib/src/util/helpers.dart:187 */
@@ -130,7 +142,8 @@ FDT_EXPORT int32_t fdt_create_ex(const fdt_config* cfg, const uint8_t* det_tflit
 FDT_EXPORT int32_t fdt_destroy(fdt_handle* h);
 
 /* New batched entry point (Dart: detectFacesBatch).  `frames` is `batch` tightly laid out images
- * of height x row_stride bytes (row_stride >= width * channels(mat_type)), in host (pinned or
+ * of height x row_stride bytes (row_stride >= width * channels(mat_type); YUV formats: height * row_stride * 3 / 2
+ * bytes, see FDT_FMT_YUV_NV12), in host (pinned or
  * pageable) or device memory.  Replaces the per-frame sequence
  * _detectDetections -> applyDetectionGates -> computeFaceAlignment [-> extractAlignedSquare ->
  * FaceLandmark.callWithScore -> transformMeshToAbsolute]
@@ -147,7 +160,7 @@ FDT_EXPORT int32_t fdt_detect_batch(fdt_handle* h, const uint8_t* frames, int32_
 
 /* detectFacesFromMatBytes (lib/src/face_detector.dart:588-609): one packed frame of
  * `nbytes` bytes; FDT_ERR_SIZE_MISMATCH when nbytes != width*height*channels
- * (matFromPackedBytes, lib/src/util/helpers.dart:432-450). */
+ * (matFromPackedBytes, lib/src/util/helpers.dart:432-450), or != width*height*3/2 for the YUV formats. */
 FDT_EXPORT int32_t fdt_detect_one(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int32_t width,
                                   int32_t height, int32_t mat_type, int32_t mode, fdt_face* out_faces,
                                   int32_t* out_count, float* out_mesh, float* out_iris);
@@ -227,7 +240,8 @@ FDT_EXPORT int32_t fdt_debug_nms(fdt_handle* h, const double* dets17, int32_t n,
 FDT_EXPORT int64_t fdt_last_launch_count(fdt_handle* h);
 /* Bytes copied host->device by the last detect call.  In fast mode only the source rows the
  * INTER_LINEAR taps read are uploaded when they form a periodic pattern (e.g. 2 of every 10 rows
- * for 720 -> 72), so this can be far below batch * frame size. */
+ * for 720 -> 72), so this can be far below batch * frame size.  YUV frames: the same rule applies to the Y plane
+ * and to the chroma plane(s) independently (720 -> 72: Y rows 10k+4, 10k+5 and chroma rows 5k+2). */
 FDT_EXPORT int64_t fdt_last_h2d_bytes(fdt_handle* h);
 /* Device time in ms of the named stage summed over the last call when stage timing was enabled
  * with fdt_set_stage_timing(h,1) (adds cudaEvent records; off by default).

@@ -175,7 +175,8 @@ class FdtFaceDetector {
     }
   }
 
-  /// New batched entry point: [frames] holds [count] packed frames (count * height * width * channels bytes).
+  /// New batched entry point: [frames] holds [count] packed frames (count * height * width * channels bytes), or [count]
+  /// YUV 4:2:0 frames of width * height * 3 / 2 bytes with matType kFdtFmtYuvNv12 / kFdtFmtYuvNv21 / kFdtFmtYuvI420.
   /// One `fdt_detect_batch` call; results come back in frame order.  For sustained throughput keep the frames in a
   /// buffer from `fdt_alloc_pinned` (see [FdtPinnedFrames]) so the upload runs at PCIe speed.
   Future<List<List<Face>>> detectFacesBatch(
@@ -187,17 +188,16 @@ class FdtFaceDetector {
     FaceDetectionMode mode = FaceDetectionMode.fast,
   }) async {
     _check();
-    final int channels = matType == 0 ? 1 : (matType == 24 ? 4 : 3);
-    final int frameBytes = width * height * channels;
+    final int frameBytes = fdtFrameBytes(matType, width, height);
     if (frames.length != count * frameBytes) {
-      throw ArgumentError('frames length ${frames.length} does not equal count * width * height * channels');
+      throw ArgumentError('frames length ${frames.length} does not equal count * frame size ($frameBytes bytes)');
     }
     if (count == 0) return <List<Face>>[];
     final arena = Arena();
     try {
       final Pointer<Uint8> src = arena<Uint8>(frames.length);
       src.asTypedList(frames.length).setAll(0, frames);
-      return _detectBatchPtr(arena, src, count, width, height, width * channels, matType, mode);
+      return _detectBatchPtr(arena, src, count, width, height, fdtRowStride(matType, width), matType, mode);
     } finally {
       arena.releaseAll();
     }
@@ -213,13 +213,12 @@ class FdtFaceDetector {
     FaceDetectionMode mode = FaceDetectionMode.fast,
   }) async {
     _check();
-    final int channels = matType == 0 ? 1 : (matType == 24 ? 4 : 3);
-    if (count * width * height * channels > frames.lengthInBytes) {
-      throw ArgumentError('pinned buffer smaller than count * width * height * channels');
+    if (count * fdtFrameBytes(matType, width, height) > frames.lengthInBytes) {
+      throw ArgumentError('pinned buffer smaller than count * frame size');
     }
     final arena = Arena();
     try {
-      return _detectBatchPtr(arena, frames.pointer, count, width, height, width * channels, matType, mode);
+      return _detectBatchPtr(arena, frames.pointer, count, width, height, fdtRowStride(matType, width), matType, mode);
     } finally {
       arena.releaseAll();
     }

@@ -29,6 +29,19 @@ const int kFdtMeshFloats = 1404;
 const int kFdtIrisFloats = 456;
 const int kFdtMemHost = 0;
 const int kFdtMemDevice = 1;
+/// YUV 4:2:0 frame formats (fdt_api.h FDT_FMT_YUV_*), accepted wherever a matType is, except by extractAlignedSquares.
+/// A frame is height * rowStride * 3 / 2 bytes: the Y plane, then NV12 / NV21 interleaved chroma (same row stride) or the
+/// I420 U and V planes (rowStride / 2 per row).  width and height must be even.
+const int kFdtFmtYuvNv12 = 0x1000;
+const int kFdtFmtYuvNv21 = 0x1001;
+const int kFdtFmtYuvI420 = 0x1002;
+
+bool fdtIsYuv(int matType) => matType == kFdtFmtYuvNv12 || matType == kFdtFmtYuvNv21 || matType == kFdtFmtYuvI420;
+
+/// Row stride (Y-plane stride for the YUV formats) and size in bytes of one tightly packed frame of [matType].
+int fdtRowStride(int matType, int width) => fdtIsYuv(matType) ? width : width * (matType == 0 ? 1 : (matType == 24 ? 4 : 3));
+int fdtFrameBytes(int matType, int width, int height) =>
+    fdtIsYuv(matType) ? height * width * 3 ~/ 2 : height * fdtRowStride(matType, width);
 
 /// fdt_config: the named arguments of FaceDetector.create that touch the path (48 bytes).
 final class FdtConfig extends Struct {
