@@ -155,6 +155,7 @@ struct fdt_handle {
   long long h2d_bytes = 0;
   long long jpeg_launches = 0;
   int last_first_chunk = 0;                  // images of the last call's first chunk (debug taps)
+  bool slot0_first_chunk = true;             // slot 0 still holds that chunk: false once a third chunk reused the slot
   int last_mesh_faces = 0, last_mesh_slot = 0, last_iris_faces = 0, last_iris_slot = 0;
   bool stage_timing = false;
   float stage_ms[kNumStages] = {};
@@ -751,6 +752,7 @@ int detect_single(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh
   if (!a.tb) return fail(h, FDT_ERR_CUDA, "letterbox table upload failed");
   a.frame_stride = lay.frame_bytes;
   h->last_first_chunk = std::min(batch, h->chunk);
+  h->slot0_first_chunk = batch <= kSlots * h->chunk;     // chunk c runs on slot c % kSlots
   h->last_mesh_faces = 0; h->last_iris_faces = 0;
 
   ChunkJob jobs[kSlots];
@@ -1298,11 +1300,21 @@ static void unpack_bgrx(const std::vector<uint8_t>& tmp, size_t px, uint8_t* out
   for (size_t i = 0; i < px; ++i) { out[3 * i] = tmp[4 * i]; out[3 * i + 1] = tmp[4 * i + 1]; out[3 * i + 2] = tmp[4 * i + 2]; }
 }
 
+// The letterbox, input-tensor, raw-head and detector-tensor taps read slot 0's buffers.  A call of three or more chunks
+// ran its third chunk there, so those buffers no longer describe its first chunk (the candidate tap has buffers of its own).
+static int32_t check_first_chunk_tap(fdt_handle* h, int32_t n) {
+  if (!h->slot0_first_chunk)
+    return fail(h, FDT_ERR_BAD_ARG, "the last call ran more than two chunks, so a later chunk overwrote its first chunk's buffers");
+  if (n < 0 || n > h->last_first_chunk) return fail(h, FDT_ERR_BAD_ARG, "n exceeds the last call's first chunk");
+  return FDT_OK;
+}
+
 int32_t fdt_debug_get_letterboxed(fdt_handle* h, int32_t n, uint8_t* out) {
   if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
   h = primary(h);
   std::lock_guard<std::mutex> g(h->mu);
-  if (n < 0 || n > h->last_first_chunk || !out) return fail(h, FDT_ERR_BAD_ARG, "n exceeds the last call's first chunk");
+  if (!out) return fail(h, FDT_ERR_BAD_ARG, "null output buffer");
+  if (int32_t rc = check_first_chunk_tap(h, n)) return rc;
   cudaSetDevice(h->cfg.device);
   size_t px = (size_t)n * h->det.in_h() * h->det.in_w();
   std::vector<uint8_t> tmp(px * 4);
@@ -1315,7 +1327,8 @@ int32_t fdt_debug_get_input_tensor(fdt_handle* h, int32_t n, float* out) {
   if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
   h = primary(h);
   std::lock_guard<std::mutex> g(h->mu);
-  if (n < 0 || n > h->last_first_chunk || !out) return fail(h, FDT_ERR_BAD_ARG, "n exceeds the last call's first chunk");
+  if (!out) return fail(h, FDT_ERR_BAD_ARG, "null output buffer");
+  if (int32_t rc = check_first_chunk_tap(h, n)) return rc;
   cudaSetDevice(h->cfg.device);
   float* tmp = nullptr;
   size_t elems = (size_t)n * h->det.in_h() * h->det.in_w() * 3;
@@ -1333,7 +1346,7 @@ int32_t fdt_debug_get_raw_heads(fdt_handle* h, int32_t n, float* out_boxes, floa
   if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
   h = primary(h);
   std::lock_guard<std::mutex> g(h->mu);
-  if (n < 0 || n > h->last_first_chunk) return fail(h, FDT_ERR_BAD_ARG, "n exceeds the last call's first chunk");
+  if (int32_t rc = check_first_chunk_tap(h, n)) return rc;
   cudaSetDevice(h->cfg.device);
   const Plan& dp = h->det.plan();
   const EngineCtx& ctx = h->slots[0].det_ctx;
@@ -1373,8 +1386,12 @@ int32_t fdt_debug_get_tensor(fdt_handle* h, int32_t which, int32_t tflite_tensor
   auto it = p.tf2pt.find(tflite_tensor);
   if (it == p.tf2pt.end() || !p.tensors[it->second].materialized) return fail(h, FDT_ERR_BAD_ARG, "tensor is not materialised in this plan");
   if (p.fuse_level == 1 && p.tensors[it->second].root < 0) return fail(h, FDT_ERR_UNSUPPORTED, "activation buffers are reused at fuse_level 1; use 0 or 2");
-  int cap = which == 0 ? h->last_first_chunk : (which == 1 ? h->last_mesh_faces : 2 * h->last_iris_faces);
-  if (n < 0 || n > cap) return fail(h, FDT_ERR_BAD_ARG, "n exceeds the images of the last call");
+  if (which == 0) {
+    if (int32_t rc = check_first_chunk_tap(h, n)) return rc;
+  } else {
+    const int cap = which == 1 ? h->last_mesh_faces : 2 * h->last_iris_faces;
+    if (n < 0 || n > cap) return fail(h, FDT_ERR_BAD_ARG, "n exceeds the crops of the last call's last pass");
+  }
   cudaSetDevice(h->cfg.device);
   TV v = e.view(ctx, it->second);
   if (out_dims4) { out_dims4[0] = n; out_dims4[1] = v.H; out_dims4[2] = v.W; out_dims4[3] = v.C; }

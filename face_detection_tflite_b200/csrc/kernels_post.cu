@@ -185,6 +185,8 @@ __global__ void __launch_bounds__(kDecodeThreads) k_decode_nms(DecodeP p) {
     fc.mesh_score = nan("");
     fc.has_mesh = 0;
     fc.anchor_index = i;
+    fc.has_iris = 0;            // every byte of the record is defined: callers read has_iris, tests compare records bitwise
+    fc.reserved = 0;
     bool pass = true;
     if (p.min_score > 0.0 || p.min_face_size > 0.0) {
       pass = fc.score >= p.min_score &&

@@ -282,6 +282,10 @@ class FaceDetector:
         return crops[0]
 
     # -- parity taps (tests only) -----------------------------------------------------------------
+    # The detector taps describe the first n frames of the last call's first chunk (min(count, maxBatch) frames).  After a
+    # call of more than two chunks (count > 2 * maxBatch) a later chunk has overwritten that chunk's buffers, and
+    # debugLetterboxed, debugInputTensor, debugRawHeads and debugTensor(0, ...) raise ValueError; debugCandidates
+    # keeps the first chunk's index sets for any count.
     def debugLetterboxed(self, n: int) -> np.ndarray:
         out = np.empty((n, self.inputHeight, self.inputWidth, 3), np.uint8)
         self._rc(self._lib.fdt_debug_get_letterboxed(self._h, n, out.ctypes.data))
@@ -305,6 +309,8 @@ class FaceDetector:
         return idx[:n.value].copy()
 
     def debugTensor(self, which: int, tensor: int, n: int) -> np.ndarray:
+        """A materialised activation of the detector (which=0, first chunk), mesh (1) or iris (2) graph, dense NHWC f32.
+        The mesh and iris tensors hold the last call's last mesh / iris pass."""
         dims = (C.c_int32 * 4)()
         self._rc(self._lib.fdt_debug_get_tensor(self._h, which, tensor, n, None, 0, dims))
         out = np.empty(tuple(dims), np.float32)
@@ -312,6 +318,9 @@ class FaceDetector:
         return out
 
     def debugMeshStage(self, n: int):
+        """The first min(n, m) faces of the last call's LAST mesh pass, m being that pass's size (a pass holds up to
+        2 * maxBatch faces of one chunk, in frame then detection order): (crops u8 [., 192, 192, 3], raw mesh outputs
+        f32 [., 1404], face-flag logits f32 [.])."""
         crops = np.empty((n, 192, 192, 3), np.uint8)
         raw = np.empty((n, 1404), np.float32)
         flag = np.empty((n,), np.float32)
@@ -321,7 +330,9 @@ class FaceDetector:
         return crops[:m], raw[:m], flag[:m]
 
     def debugIrisStage(self, n: int):
-        """(eye crops u8 [2m,64,64,3], rois f64 [2m,4] = cx,cy,size,theta, contours f32 [2m,213], iris f32 [2m,15])."""
+        """The first m = min(n, faces) faces of the last call's LAST iris pass (the faces of the last mesh pass that passed
+        the presence gate and have two valid eye ROIs): (eye crops u8 [2m,64,64,3], rois f64 [2m,4] = cx,cy,size,theta,
+        contours f32 [2m,213], iris f32 [2m,15])."""
         crops = np.empty((2 * n, 64, 64, 3), np.uint8)
         rois = np.empty((2 * n, 4), np.float64)
         cont = np.empty((2 * n, 213), np.float32)

@@ -195,6 +195,10 @@ FDT_EXPORT int32_t fdt_copy_to_device(fdt_handle* h, void* dst, const void* src,
 FDT_EXPORT int32_t fdt_copy_to_host(fdt_handle* h, void* dst, const void* src, size_t nbytes);
 
 /* ---- parity taps (test / debug only; valid for the frames of the LAST detect call, first chunk) ----
+ * n (or image) may not exceed the first chunk's frames (min(batch, max_batch)).  Chunks alternate over two
+ * pipeline slots, so a call of more than two chunks (batch > 2 * max_batch) overwrites the first chunk's
+ * buffers: after such a call the letterbox, input-tensor, raw-head and detector-tensor (which=0) taps
+ * return FDT_ERR_BAD_ARG.  The candidate tap keeps the first chunk's index sets for any batch.
  * fdt_debug_get_letterboxed : u8 [n, S, S, 3] BGR after resize + copyMakeBorder
  *                             (convertImageToTensor u8 stage, lib/src/util/helpers.dart:303-347)
  * fdt_debug_get_input_tensor: f32 [n, S, S, 3] RGB in [-1,1] (bgrMatToSignedFloat32, :377-421)
@@ -202,8 +206,9 @@ FDT_EXPORT int32_t fdt_copy_to_host(fdt_handle* h, void* dst, const void* src, s
  *                             lib/src/models/face_detection_model.dart:19)
  * fdt_debug_get_candidates  : ascending anchor indices with raw score >= logit(minScore)
  *                             (_collectCandidateScores, face_detection_model.dart:477-492)
- * fdt_debug_get_tensor      : any materialised activation of the detector (which=0) or mesh (which=1)
- *                             graph by TFLite tensor index, as dense NHWC f32.                    */
+ * fdt_debug_get_tensor      : any materialised activation of the detector (which=0), mesh (which=1)
+ *                             or iris (which=2) graph by TFLite tensor index, as dense NHWC f32.
+ *                             The mesh and iris tensors hold the last call's last mesh / iris pass. */
 FDT_EXPORT int32_t fdt_debug_get_letterboxed(fdt_handle* h, int32_t n, uint8_t* out);
 FDT_EXPORT int32_t fdt_debug_get_input_tensor(fdt_handle* h, int32_t n, float* out);
 FDT_EXPORT int32_t fdt_debug_get_raw_heads(fdt_handle* h, int32_t n, float* out_boxes, float* out_scores);
@@ -212,10 +217,13 @@ FDT_EXPORT int32_t fdt_debug_get_candidates(fdt_handle* h, int32_t image, int32_
 FDT_EXPORT int32_t fdt_debug_get_tensor(fdt_handle* h, int32_t which, int32_t tflite_tensor, int32_t n,
                                         float* out, size_t out_capacity_floats, int32_t* out_dims4);
 /* Mesh stage taps: u8 [n,192,192,3] BGR crops (extractAlignedSquare, helpers.dart:583-625), raw
- * mesh outputs f32 [n,1404] + face-flag logits [n], for the first n faces of the last call. */
+ * mesh outputs f32 [n,1404] + face-flag logits [n], for the first n faces of the LAST mesh pass of the
+ * last call (a pass holds up to 2 * max_batch faces of one chunk, in frame then detection order).
+ * out_n receives the size of that pass. */
 FDT_EXPORT int32_t fdt_debug_get_mesh_stage(fdt_handle* h, int32_t n, uint8_t* out_crops,
                                             float* out_raw1404, float* out_flag, int32_t* out_n);
-/* Iris stage taps for the first n faces that reached it in the last call (last pass of the last chunk):
+/* Iris stage taps for the first n faces of the LAST iris pass of the last call (the faces of the last mesh
+ * pass that passed the presence gate and have two valid eye ROIs); out_n receives the faces of that pass:
  * u8 [2n,64,64,3] BGR eye crops (left, right-mirrored), the eye ROIs [2n,4] = cx, cy, size, theta
  * (eyeRoisFromMesh, face_geometry.dart:155-168), raw outputs f32 [2n,213] contours + [2n,15] iris. */
 FDT_EXPORT int32_t fdt_debug_get_iris_stage(fdt_handle* h, int32_t n, uint8_t* out_crops, double* out_rois,
