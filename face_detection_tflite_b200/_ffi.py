@@ -31,6 +31,12 @@ class FdtFace(C.Structure):
                 ("has_mesh", C.c_int32), ("anchor_index", C.c_int32), ("has_iris", C.c_int32), ("reserved", C.c_int32)]
 
 
+class FdtFrame(C.Structure):
+    """fdt_frame: one frame of a mixed batch (fdt_detect_frames)."""
+    _fields_ = [("data", C.c_void_p), ("width", C.c_int32), ("height", C.c_int32), ("row_stride", C.c_int32),
+                ("mat_type", C.c_int32)]
+
+
 # every symbol include/fdt_api.h declares: name -> (restype, argtypes)
 P = C.c_void_p
 u8p = C.POINTER(C.c_uint8)
@@ -45,6 +51,9 @@ SIGNATURES = {
     "fdt_destroy": (C.c_int32, [P]),
     "fdt_detect_batch": (C.c_int32, [P, P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                      C.POINTER(FdtFace), i32p, f32p, f32p]),
+    "fdt_detect_frames": (C.c_int32, [P, C.POINTER(FdtFrame), C.c_int32, C.c_int32, C.c_int32, C.POINTER(FdtFace), i32p, f32p, f32p]),
+    "fdt_detect_jpeg_batch": (C.c_int32, [P, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_int32, C.c_int32, C.POINTER(FdtFace),
+                                          i32p, f32p, f32p, i32p, i32p]),
     "fdt_detect_one": (C.c_int32, [P, P, C.c_size_t, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(FdtFace), i32p, f32p, f32p]),
     "fdt_detect_batch_device": (C.c_int32, [P, P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                             C.POINTER(P), C.POINTER(P)]),

@@ -13,6 +13,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -29,6 +30,7 @@ using namespace fdt;
 
 static_assert(sizeof(fdt_face) == 160, "fdt_face wire layout (bindings rely on it)");
 static_assert(sizeof(fdt_config) == 48, "fdt_config layout");
+static_assert(sizeof(fdt_frame) == 24, "fdt_frame layout (bindings rely on it)");
 
 namespace {
 
@@ -39,6 +41,10 @@ constexpr double kMinScore = 0.5;         // lib/src/shared/face_model_config.da
 constexpr double kMinSuppression = 0.3;   // lib/src/shared/face_model_config.dart:77
 constexpr int kNumStages = 9;
 constexpr int kEagerSlots = 4;            // result slots per frame copied to the host with the chunk (more on demand)
+// Mixed batches: a chunk of host frames (fdt_detect_frames) or of decoded JPEGs stages at most max_batch * this many bytes,
+// e.g. 256 frames of 1920x1080 BGRA; a larger frame runs as a chunk of its own.
+constexpr long long kStageBytesPerFrame = 8ll << 20;
+constexpr size_t kStageAlign = 256;       // staged frames start at multiples of this
 
 std::string g_create_error;
 std::mutex g_create_mu;
@@ -127,6 +133,11 @@ struct Slot {
   uint8_t* d_eye_crops = nullptr;
   float *d_iris_out = nullptr, *h_iris_out = nullptr;
   double *d_eye_kp = nullptr, *h_eye_kp = nullptr;
+  // mixed batches: per chunk one pinned blob (frame descriptors, tap tables, decode geometry) goes up in one copy;
+  // ev_blob follows that copy, and the next chunk on this slot waits on it before rewriting h_blob
+  uint8_t *h_blob = nullptr, *d_blob = nullptr; size_t blob_cap = 0;
+  cudaEvent_t ev_blob = nullptr;
+  double *h_eye_wh = nullptr, *d_eye_wh = nullptr;    // frame size per iris face [F][2]
 };
 
 }  // namespace
@@ -168,6 +179,7 @@ struct fdt_handle {
   uint8_t* d_jframe = nullptr; size_t jframe_cap = 0;
   uint16_t* d_jq = nullptr;
   int jw = 0, jh = 0;                        // size of the frame in d_jframe
+  uint8_t* d_jarena = nullptr; size_t jarena_cap = 0;   // fdt_detect_jpeg_batch: one chunk's decoded frames
   bool ready = false;
 };
 
@@ -231,6 +243,14 @@ int frame_layout(int mat_type, int w, int hh, int row_stride, FrameLayout* L, co
     L->c_row_bytes = row_stride; L->c_rows = hh / 2; L->c_step = 2;
     L->u_off = mat_type == FDT_FMT_YUV_NV12 ? 0 : 1; L->v_off = 1 - L->u_off;
   }
+  return FDT_OK;
+}
+
+// The mode and model-availability checks of every detect entry point.
+int check_mode(fdt_handle* h, int mode) {
+  if (mode != FDT_MODE_FAST && mode != FDT_MODE_STANDARD && mode != FDT_MODE_FULL) return fail(h, FDT_ERR_BAD_ARG, "unknown mode");
+  if (mode != FDT_MODE_FAST && !h->has_mesh) return fail(h, FDT_ERR_NOT_READY, "standard / full mode needs the face_landmark model");
+  if (mode == FDT_MODE_FULL && !h->has_iris) return fail(h, FDT_ERR_NOT_READY, "full mode needs the iris_landmark model");
   return FDT_OK;
 }
 
@@ -410,13 +430,49 @@ void fill_decode(DecodeP& d, fdt_handle* h, const Slot& sl, const LbTables* tb, 
   d.anchors = h->d_anchors; d.N = h->num_anchors; d.input_h = S_h;
   d.raw_thresh = std::log(kMinScore / (1.0 - kMinScore));
   d.score_thresh = kMinScore; d.iou_thresh = kMinSuppression;
-  d.pad_t = (double)tb->lp.pad_top / S_h; d.pad_b = (double)tb->lp.pad_bottom / S_h;
-  d.pad_l = (double)tb->lp.pad_left / S_w; d.pad_r = (double)tb->lp.pad_right / S_w;
+  d.pad_t = d.pad_b = d.pad_l = d.pad_r = 0.0;    // no tables: mixed chunks pass per-image geometry (DecodeP::geom)
+  if (tb) {
+    d.pad_t = (double)tb->lp.pad_top / S_h; d.pad_b = (double)tb->lp.pad_bottom / S_h;
+    d.pad_l = (double)tb->lp.pad_left / S_w; d.pad_r = (double)tb->lp.pad_right / S_w;
+  }
   d.min_score = h->cfg.min_score; d.min_face_size = h->cfg.min_face_size;
   d.img_w = w; d.img_h = hh; d.max_faces = h->max_faces;
   d.cand_idx = nullptr; d.cand_cap = 0; d.cand_n = nullptr;
   d.pre = nullptr; d.dbg_dec = nullptr; d.skip_roi = 0;
 }
+
+// Letterbox geometry and INTER_LINEAR taps of one frame size, as k_letterbox_multi reads them: x0, x1, ax0, ax1 (new_w each),
+// then y0, y1, by0, by1, cy0, cy1 (new_h each).  Built on the host with resize_linear_taps, like LbTables.
+struct SizeTaps {
+  LetterboxParams lp;
+  bool identity = false;
+  std::vector<int> t;
+};
+
+SizeTaps make_taps(int w, int hh, int S_w, int S_h) {
+  SizeTaps st;
+  st.lp = letterbox_params(w, hh, S_w, S_h);
+  st.identity = st.lp.new_w == w && st.lp.new_h == hh;
+  const int nw = st.lp.new_w, nh = st.lp.new_h;
+  st.t.resize((size_t)4 * nw + 6 * nh);
+  int* x = st.t.data();
+  int* y = x + 4 * nw;
+  std::vector<short> a0(std::max(nw, nh)), a1(std::max(nw, nh));
+  resize_linear_taps(w, nw, true, x, x + nw, a0.data(), a1.data());
+  for (int i = 0; i < nw; ++i) { x[2 * nw + i] = a0[i]; x[3 * nw + i] = a1[i]; }
+  resize_linear_taps(hh, nh, false, y, y + nh, a0.data(), a1.data());
+  for (int i = 0; i < nh; ++i) { y[2 * nh + i] = a0[i]; y[3 * nh + i] = a1[i]; y[4 * nh + i] = y[i] >> 1; y[5 * nh + i] = y[nh + i] >> 1; }
+  return st;
+}
+
+// One mixed call (fdt_detect_frames): the frames, their layouts and the taps of each distinct size.  The taps are computed once
+// per size within the call instead of going through the handle's table cache: a stream of distinct sizes would evict that
+// cache on every frame, and each eviction synchronises both slots.
+struct Ragged {
+  const fdt_frame* frames = nullptr;
+  std::vector<FrameLayout> lay;
+  std::map<std::pair<int, int>, SizeTaps> taps;
+};
 
 struct CallArgs {
   const uint8_t* frames; int batch, w, hh, row_stride, channels, mode, mem_kind;
@@ -425,13 +481,111 @@ struct CallArgs {
   bool keep_on_device;
   const LbTables* tb;
   long long frame_stride;
+  Ragged* rg = nullptr;                   // mixed call: per-frame sizes and layouts (the uniform fields above are unused)
 };
 
-struct ChunkJob { int off = 0, n = 0; const uint8_t* d_fr = nullptr; bool active = false; };
+// Size of frame i of the call: the mesh and iris stages map their points into it.
+void frame_size(const CallArgs& a, int i, double* w, double* hh) {
+  if (a.rg) { *w = a.rg->frames[i].width; *hh = a.rg->frames[i].height; }
+  else { *w = a.w; *hh = a.hh; }
+}
+
+// d_desc: a mixed chunk's frame descriptors on the device (the crop warps read the frames through them)
+struct ChunkJob { int off = 0, n = 0; const uint8_t* d_fr = nullptr; const FrameD* d_desc = nullptr; bool active = false; };
+
+size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// A mixed chunk on its slot's stream: host frames go up whole, one copy each at kStageAlign-aligned offsets; then the chunk's
+// blob (frame descriptors, concatenated tap tables, decode geometry) in one copy; then k_letterbox_multi.
+int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, const FrameD** d_desc, const double** d_geom) {
+  cudaStream_t s = sl.stream;
+  Ragged& rg = *a.rg;
+  const fdt_frame* fr = rg.frames + off;
+  const int S_w = h->det.in_w(), S_h = h->det.in_h();
+  std::vector<const uint8_t*> base(n);
+  if (a.mem_kind == FDT_MEM_HOST) {
+    std::vector<size_t> at(n);
+    size_t need = 0;
+    for (int i = 0; i < n; ++i) { at[i] = need; need += align_up((size_t)rg.lay[off + i].frame_bytes, kStageAlign); }
+    if (sl.d_frames_cap < need) {
+      cudaStreamSynchronize(s);
+      if (sl.d_frames) cudaFree(sl.d_frames);
+      sl.d_frames = nullptr; sl.d_frames_cap = 0;
+      if (!cuda_ok(h, cudaMalloc(&sl.d_frames, need), "cudaMalloc(frame staging)")) return FDT_ERR_CUDA;
+      sl.d_frames_cap = need;
+    }
+    for (int i = 0; i < n; ++i) {
+      const size_t fb = (size_t)rg.lay[off + i].frame_bytes;
+      cudaMemcpyAsync(sl.d_frames + at[i], fr[i].data, fb, cudaMemcpyHostToDevice, s);
+      h->h2d_bytes += (long long)fb;
+      base[i] = sl.d_frames + at[i];
+    }
+  } else {
+    for (int i = 0; i < n; ++i) base[i] = fr[i].data;
+  }
+  // the chunk's distinct sizes, each with its taps at an offset of the concatenated table
+  std::map<std::pair<int, int>, int> tap_at;
+  std::vector<const SizeTaps*> st(n);
+  size_t ntaps = 0;
+  for (int i = 0; i < n; ++i) {
+    const std::pair<int, int> key(fr[i].width, fr[i].height);
+    auto it = rg.taps.find(key);
+    if (it == rg.taps.end()) it = rg.taps.emplace(key, make_taps(key.first, key.second, S_w, S_h)).first;
+    st[i] = &it->second;
+    if (tap_at.emplace(key, (int)ntaps).second) ntaps += it->second.t.size();
+  }
+  const size_t taps_at = align_up((size_t)n * sizeof(FrameD), 16), geom_at = align_up(taps_at + ntaps * sizeof(int), 16);
+  const size_t bytes = geom_at + (size_t)n * 6 * sizeof(double);
+  if (sl.blob_cap < bytes) {
+    cudaStreamSynchronize(s);
+    if (sl.h_blob) cudaFreeHost(sl.h_blob);
+    if (sl.d_blob) cudaFree(sl.d_blob);
+    sl.h_blob = nullptr; sl.d_blob = nullptr; sl.blob_cap = 0;
+    const size_t cap = bytes + bytes / 4;
+    if (!cuda_ok(h, cudaMallocHost(&sl.h_blob, cap), "cudaMallocHost(chunk blob)") ||
+        !cuda_ok(h, cudaMalloc(&sl.d_blob, cap), "cudaMalloc(chunk blob)")) return FDT_ERR_CUDA;
+    sl.blob_cap = cap;
+  } else if (!cuda_ok(h, cudaEventSynchronize(sl.ev_blob), "chunk blob")) {
+    return FDT_ERR_CUDA;       // the blob of two chunks back may still be on its way up
+  }
+  FrameD* desc = reinterpret_cast<FrameD*>(sl.h_blob);
+  int* taps = reinterpret_cast<int*>(sl.h_blob + taps_at);
+  double* geom = reinterpret_cast<double*>(sl.h_blob + geom_at);
+  for (const auto& kv : tap_at) {
+    const std::vector<int>& t = rg.taps.at(kv.first).t;
+    std::memcpy(taps + kv.second, t.data(), t.size() * sizeof(int));
+  }
+  for (int i = 0; i < n; ++i) {
+    const FrameLayout& L = rg.lay[off + i];
+    const LetterboxParams& lp = st[i]->lp;
+    FrameD& d = desc[i];
+    d.y = base[i]; d.c = L.yuv ? base[i] + L.c_off : nullptr;
+    d.w = fr[i].width; d.h = fr[i].height; d.row_stride = fr[i].row_stride; d.channels = L.channels;
+    d.c_row_stride = L.c_row_bytes; d.c_step = L.c_step; d.u_off = L.u_off; d.v_off = L.v_off;
+    d.new_w = lp.new_w; d.new_h = lp.new_h; d.pad_top = lp.pad_top; d.pad_left = lp.pad_left; d.identity = st[i]->identity ? 1 : 0;
+    d.tx = tap_at[std::make_pair(d.w, d.h)]; d.ty = d.tx + 4 * lp.new_w;
+    // the values fill_decode derives from LbTables, computed the same way
+    double* g = geom + 6 * (size_t)i;
+    g[0] = (double)lp.pad_top / S_h; g[1] = (double)lp.pad_bottom / S_h;
+    g[2] = (double)lp.pad_left / S_w; g[3] = (double)lp.pad_right / S_w;
+    g[4] = d.w; g[5] = d.h;
+  }
+  cudaMemcpyAsync(sl.d_blob, sl.h_blob, bytes, cudaMemcpyHostToDevice, s);
+  cudaEventRecord(sl.ev_blob, s);
+  *d_desc = reinterpret_cast<const FrameD*>(sl.d_blob);
+  *d_geom = reinterpret_cast<const double*>(sl.d_blob + geom_at);
+  StageTimer t(h, 0, s);
+  LetterboxMultiP lb;
+  lb.fr = *d_desc; lb.taps = reinterpret_cast<const int*>(sl.d_blob + taps_at); lb.out = sl.d_lb; lb.dst_w = S_w; lb.dst_h = S_h;
+  launch_letterbox_multi(lb, n, s);
+  t.launches = 1;
+  return FDT_OK;
+}
 
 // Stage 1 of a chunk on its slot's stream: [H2D] -> letterbox -> detector -> decode + NMS -> [D2H of counts and the
 // first kEagerSlots result slots per frame].
-int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, bool first_chunk, ChunkJob* job) {
+// Uniform chunk: [H2D] -> k_letterbox / k_letterbox_yuv; *d_fr = the frames on the device.
+int stage_uniform(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, const uint8_t** d_fr_out) {
   cudaStream_t s = sl.stream;
   const LbTables* tb = a.tb;
   const int S_w = h->det.in_w(), S_h = h->det.in_h();
@@ -505,6 +659,17 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
     }
     t.launches = 1;
   }
+  *d_fr_out = d_fr;
+  return FDT_OK;
+}
+
+int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, bool first_chunk, ChunkJob* job) {
+  cudaStream_t s = sl.stream;
+  const uint8_t* d_fr = nullptr;
+  const FrameD* d_desc = nullptr;
+  const double* d_geom = nullptr;
+  const int rc = a.rg ? stage_ragged(h, sl, a, off, n, &d_desc, &d_geom) : stage_uniform(h, sl, a, off, n, &d_fr);
+  if (rc != FDT_OK) return rc;
   {
     StageTimer t(h, 1, s);
     t.launches = h->det.run(sl.det_ctx, sl.d_lb, n, s);
@@ -512,7 +677,8 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
   {
     StageTimer t(h, 2, s);
     DecodeP d;
-    fill_decode(d, h, sl, tb, a.w, a.hh);
+    fill_decode(d, h, sl, a.tb, a.w, a.hh);
+    d.geom = d_geom;
     d.faces = h->d_faces + (size_t)off * h->max_faces; d.counts = h->d_counts + off;
     if (first_chunk) { d.cand_idx = sl.d_cand_idx; d.cand_cap = h->cand_cap; d.cand_n = sl.d_cand_n; }
     launch_decode_nms(d, n, s);
@@ -531,7 +697,7 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
     cudaMemcpy2DAsync(a.out_faces + (size_t)off * h->max_faces, pitch, h->d_faces + (size_t)off * h->max_faces, pitch, eager, n,
                       cudaMemcpyDeviceToHost, s);
   }
-  job->off = off; job->n = n; job->d_fr = d_fr; job->active = true;
+  job->off = off; job->n = n; job->d_fr = d_fr; job->d_desc = d_desc; job->active = true;
   return FDT_OK;
 }
 
@@ -574,7 +740,6 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
   const long long total = (long long)list.size();
   const bool full = a.mode == FDT_MODE_FULL;
   const double gate = h->cfg.min_face_presence;
-  const int frame_stride_is_dev = 1; (void)frame_stride_is_dev;
   // the warp reads whole frames: host frames were uploaded unsparsified in these modes
   const long long dev_frame_stride = a.frame_stride;
   for (long long skip = 0; skip < total; skip += h->mesh_cap) {
@@ -583,8 +748,9 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
     for (int f = 0; f < nf; ++f) {
       const Ref r = list[(size_t)(skip + f)];
       const fdt_face& fc = sl.h_faces[(size_t)r.b * h->max_faces + r.j];
-      double theta, cx, cy, size;
-      face_alignment(fc.keypoints, (double)a.w, (double)a.hh, &theta, &cx, &cy, &size);
+      double theta, cx, cy, size, fw, fh;
+      frame_size(a, off + r.b, &fw, &fh);
+      face_alignment(fc.keypoints, fw, fh, &theta, &cx, &cy, &size);
       double* roi = sl.h_roi + 6 * f;
       roi[0] = theta; roi[1] = cx; roi[2] = cy; roi[3] = size; roi[4] = std::cos(theta); roi[5] = std::sin(theta);
       sl.h_crop_img[f] = r.b;
@@ -601,6 +767,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
       wp.src_w = a.w; wp.src_h = a.hh; wp.crop_img = sl.d_crop_img; wp.affine = sl.d_affine; wp.ncrops = nf;
       wp.out_size = kMeshInput; wp.flip_odd = 0; wp.crops = sl.d_crops;
       set_warp_layout(wp, a.lay);
+      wp.fr = job.d_desc;
       launch_warp_affine(wp, s);
       t.launches = 1;
     }
@@ -667,6 +834,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
           sl.h_eye_img[ne + e] = list[(size_t)(skip + f)].b;
         }
         ne += 2;
+        if (a.rg) frame_size(a, off + list[(size_t)(skip + f)].b, sl.h_eye_wh + 2 * run.size(), sl.h_eye_wh + 2 * run.size() + 1);
         run.push_back(f);
       }
       const int nfi = (int)run.size();
@@ -674,6 +842,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
         cudaMemcpyAsync(sl.d_eye_img, sl.h_eye_img, (size_t)ne * sizeof(int), cudaMemcpyHostToDevice, s);
         cudaMemcpyAsync(sl.d_eye_affine, sl.h_eye_affine, (size_t)ne * 6 * sizeof(double), cudaMemcpyHostToDevice, s);
         cudaMemcpyAsync(sl.d_eye_roi, sl.h_eye_roi, (size_t)ne * 6 * sizeof(double), cudaMemcpyHostToDevice, s);
+        if (a.rg) cudaMemcpyAsync(sl.d_eye_wh, sl.h_eye_wh, (size_t)nfi * 2 * sizeof(double), cudaMemcpyHostToDevice, s);
         {
           StageTimer t(h, 6, s);
           WarpP wp;
@@ -681,6 +850,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
           wp.src_w = a.w; wp.src_h = a.hh; wp.crop_img = sl.d_eye_img; wp.affine = sl.d_eye_affine; wp.ncrops = ne;
           wp.out_size = kIrisInput; wp.flip_odd = 1; wp.crops = sl.d_eye_crops;
           set_warp_layout(wp, a.lay);
+          wp.fr = job.d_desc;
           launch_warp_affine(wp, s);
           t.launches = 1;
         }
@@ -700,6 +870,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
           pp.contours = sl.iris_ctx.outputs[ci]; pp.contours_istride = ip.out_elems[ci];
           pp.iris = sl.iris_ctx.outputs[ii]; pp.iris_istride = ip.out_elems[ii];
           pp.roi = sl.d_eye_roi; pp.nfaces = nfi; pp.in_size = kIrisInput; pp.img_w = a.w; pp.img_h = a.hh;
+          if (a.rg) pp.img_wh = sl.d_eye_wh;
           pp.iris_out = sl.d_iris_out; pp.eye_kp = sl.d_eye_kp;
           launch_iris_post(pp, s);
           t.launches = 1;
@@ -725,6 +896,41 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
   return FDT_OK;
 }
 
+// The chunks of one call (chunk c = frames bounds[c] .. bounds[c + 1] - 1) through the two-slot software pipeline.
+int run_chunks(fdt_handle* h, const CallArgs& a, const std::vector<int>& bounds) {
+  const int nchunks = (int)bounds.size() - 1, mode = a.mode;
+  h->last_first_chunk = bounds[1] - bounds[0];
+  h->slot0_first_chunk = nchunks <= kSlots;             // chunk c runs on slot c % kSlots
+  h->last_mesh_faces = 0; h->last_iris_faces = 0;
+
+  ChunkJob jobs[kSlots];
+  int rc = FDT_OK;
+  for (int c = 0; c < nchunks && rc == FDT_OK; ++c) {
+    const int off = bounds[c], n = bounds[c + 1] - off;
+    Slot& sl = h->slots[c % kSlots];
+    // software pipeline: chunk c is queued on its slot, then the host turns to chunk c - 1 on the other slot
+    rc = enqueue_detect(h, sl, a, off, n, c == 0, &jobs[c % kSlots]);
+    if (rc == FDT_OK && mode != FDT_MODE_FAST && c > 0) {
+      ChunkJob& prev = jobs[(c - 1) % kSlots];
+      rc = finish_mesh(h, h->slots[(c - 1) % kSlots], a, prev);
+      prev.active = false;
+    }
+  }
+  if (rc == FDT_OK && mode != FDT_MODE_FAST) {
+    for (int i = 0; i < kSlots && rc == FDT_OK; ++i)
+      if (jobs[i].active) { rc = finish_mesh(h, h->slots[i], a, jobs[i]); jobs[i].active = false; }
+  }
+  if (rc != FDT_OK) { for (int i = 0; i < kSlots; ++i) cudaStreamSynchronize(h->slots[i].stream); return rc; }
+  if (!a.keep_on_device) {
+    for (int i = 0; i < kSlots; ++i)
+      if (!cuda_ok(h, cudaStreamSynchronize(h->slots[i].stream), "pipeline")) return FDT_ERR_CUDA;
+    if (mode == FDT_MODE_FAST && fetch_overflow_faces(h, a.out_counts, a.out_faces, 0, a.batch) != FDT_OK) return FDT_ERR_CUDA;
+  }
+  if (!cuda_ok(h, cudaGetLastError(), "kernel launch")) return FDT_ERR_CUDA;
+  if (h->det.failed() || h->mesh.failed() || h->iris.failed()) { h->err = "a kernel of the plan could not be launched (tensor map encoding / unsupported shape)"; return FDT_ERR_CUDA; }
+  return FDT_OK;
+}
+
 int detect_single(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh, int row_stride, int mat_type, int mode,
                   int mem_kind, fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris, bool keep_on_device) {
   if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
@@ -732,9 +938,7 @@ int detect_single(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh
   FrameLayout lay;
   const char* msg = nullptr;
   if (int rc = frame_layout(mat_type, w, hh, row_stride, &lay, &msg)) return fail(h, rc, msg);
-  if (mode != FDT_MODE_FAST && mode != FDT_MODE_STANDARD && mode != FDT_MODE_FULL) return fail(h, FDT_ERR_BAD_ARG, "unknown mode");
-  if (mode != FDT_MODE_FAST && !h->has_mesh) return fail(h, FDT_ERR_NOT_READY, "standard / full mode needs the face_landmark model");
-  if (mode == FDT_MODE_FULL && !h->has_iris) return fail(h, FDT_ERR_NOT_READY, "full mode needs the iris_landmark model");
+  if (int rc = check_mode(h, mode)) return rc;
   if (mode != FDT_MODE_FAST && keep_on_device) return fail(h, FDT_ERR_UNSUPPORTED, "device-resident results are fast-mode only");
   if (!keep_on_device && (!out_faces || !out_counts)) return fail(h, FDT_ERR_BAD_ARG, "null output buffers");
   cudaSetDevice(h->cfg.device);
@@ -751,36 +955,101 @@ int detect_single(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh
   a.tb = get_tables(h, w, hh);
   if (!a.tb) return fail(h, FDT_ERR_CUDA, "letterbox table upload failed");
   a.frame_stride = lay.frame_bytes;
-  h->last_first_chunk = std::min(batch, h->chunk);
-  h->slot0_first_chunk = batch <= kSlots * h->chunk;     // chunk c runs on slot c % kSlots
-  h->last_mesh_faces = 0; h->last_iris_faces = 0;
+  std::vector<int> bounds;
+  for (int off = 0; off < batch; off += h->chunk) bounds.push_back(off);
+  bounds.push_back(batch);
+  return run_chunks(h, a, bounds);
+}
 
-  ChunkJob jobs[kSlots];
-  int rc = FDT_OK;
-  for (int off = 0, c = 0; off < batch && rc == FDT_OK; off += h->chunk, ++c) {
-    const int n = std::min(h->chunk, batch - off);
-    Slot& sl = h->slots[c % kSlots];
-    // software pipeline: chunk c is queued on its slot, then the host turns to chunk c - 1 on the other slot
-    rc = enqueue_detect(h, sl, a, off, n, c == 0, &jobs[c % kSlots]);
-    if (rc == FDT_OK && mode != FDT_MODE_FAST && c > 0) {
-      ChunkJob& prev = jobs[(c - 1) % kSlots];
-      rc = finish_mesh(h, h->slots[(c - 1) % kSlots], a, prev);
-      prev.active = false;
-    }
+// fdt_detect_frames' argument checks, every frame before any work; *lay receives the frames' layouts.
+int check_frames(fdt_handle* h, const fdt_frame* frames, int n, int mode, int mem_kind, const fdt_face* out_faces,
+                 const int32_t* out_counts, std::vector<FrameLayout>* lay) {
+  if (n < 0 || (n > 0 && !frames)) return fail(h, FDT_ERR_BAD_ARG, "bad frame list");
+  if (mem_kind != FDT_MEM_HOST && mem_kind != FDT_MEM_DEVICE) return fail(h, FDT_ERR_BAD_ARG, "unknown mem_kind");
+  if (int rc = check_mode(h, mode)) return rc;
+  if (n > 0 && (!out_faces || !out_counts)) return fail(h, FDT_ERR_BAD_ARG, "null output buffers");
+  lay->assign(n, FrameLayout());
+  for (int i = 0; i < n; ++i) {
+    const fdt_frame& f = frames[i];
+    const char* msg = "bad frame arguments";
+    int rc = (!f.data || f.width <= 0 || f.height <= 0) ? FDT_ERR_BAD_ARG : frame_layout(f.mat_type, f.width, f.height, f.row_stride, &(*lay)[i], &msg);
+    if (rc != FDT_OK) return fail(h, rc, "frame " + std::to_string(i) + ": " + msg);
   }
-  if (rc == FDT_OK && mode != FDT_MODE_FAST) {
-    for (int i = 0; i < kSlots && rc == FDT_OK; ++i)
-      if (jobs[i].active) { rc = finish_mesh(h, h->slots[i], a, jobs[i]); jobs[i].active = false; }
-  }
-  if (rc != FDT_OK) { for (int i = 0; i < kSlots; ++i) cudaStreamSynchronize(h->slots[i].stream); return rc; }
-  if (!keep_on_device) {
-    for (int i = 0; i < kSlots; ++i)
-      if (!cuda_ok(h, cudaStreamSynchronize(h->slots[i].stream), "pipeline")) return FDT_ERR_CUDA;
-    if (mode == FDT_MODE_FAST && fetch_overflow_faces(h, out_counts, out_faces, 0, batch) != FDT_OK) return FDT_ERR_CUDA;
-  }
-  if (!cuda_ok(h, cudaGetLastError(), "kernel launch")) return FDT_ERR_CUDA;
-  if (h->det.failed() || h->mesh.failed() || h->iris.failed()) { h->err = "a kernel of the plan could not be launched (tensor map encoding / unsupported shape)"; return FDT_ERR_CUDA; }
   return FDT_OK;
+}
+
+int detect_frames_single(fdt_handle* h, const fdt_frame* frames, int n, int mode, int mem_kind, fdt_face* out_faces,
+                         int32_t* out_counts, float* out_mesh, float* out_iris) {
+  if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
+  Ragged rg;
+  if (int rc = check_frames(h, frames, n, mode, mem_kind, out_faces, out_counts, &rg.lay)) return rc;
+  cudaSetDevice(h->cfg.device);
+  if (mem_kind == FDT_MEM_DEVICE)
+    for (int i = 0; i < n; ++i) {
+      cudaPointerAttributes pa;
+      const bool ok = cudaPointerGetAttributes(&pa, frames[i].data) == cudaSuccess &&
+                      (pa.type == cudaMemoryTypeDevice || pa.type == cudaMemoryTypeManaged) && pa.device == h->cfg.device;
+      cudaGetLastError();
+      if (!ok) return fail(h, FDT_ERR_BAD_ARG, "frame " + std::to_string(i) + ": FDT_MEM_DEVICE frames must be in the handle's device memory");
+    }
+  h->launches = 0;
+  h->h2d_bytes = 0;
+  for (int i = 0; i < kNumStages; ++i) { h->stage_ms[i] = 0; h->stage_launches[i] = 0; }
+  if (n == 0) return FDT_OK;
+  if (!ensure_results(h, n)) return FDT_ERR_CUDA;
+  rg.frames = frames;
+  CallArgs a;
+  a.frames = nullptr; a.batch = n; a.w = 0; a.hh = 0; a.row_stride = 0; a.channels = 0; a.mode = mode; a.mem_kind = mem_kind;
+  a.out_faces = out_faces; a.out_counts = out_counts; a.out_mesh = out_mesh; a.out_iris = out_iris;
+  a.keep_on_device = false; a.tb = nullptr; a.frame_stride = 0; a.rg = &rg;
+  // a chunk closes at max_batch frames, or (host frames) before its staged bytes would pass the budget
+  const long long budget = (long long)h->chunk * kStageBytesPerFrame;
+  std::vector<int> bounds(1, 0);
+  long long staged = 0;
+  for (int i = 0; i < n; ++i) {
+    const long long fb = mem_kind == FDT_MEM_HOST ? (long long)align_up((size_t)rg.lay[i].frame_bytes, kStageAlign) : 0;
+    if (i - bounds.back() == h->chunk || (i > bounds.back() && staged + fb > budget)) { bounds.push_back(i); staged = 0; }
+    staged += fb;
+  }
+  bounds.push_back(n);
+  return run_chunks(h, a, bounds);
+}
+
+// Multi-device handle: items 0 .. n - 1 split contiguously (sharding.shard_range), one host thread per replica running
+// fn(replica, lo, hi) under the replica's lock; launches and h2d bytes are summed, the first failing replica's error reported.
+template <typename F> int on_shards(fdt_handle* h, int n, F fn) {
+  const int g = (int)h->shards.size();
+  std::vector<int> rcs(g, FDT_OK);
+  std::vector<std::thread> th;
+  for (int r = 0; r < g; ++r) {
+    const int lo = (int)((long long)n * r / g), hi = (int)((long long)n * (r + 1) / g);
+    if (hi <= lo) continue;
+    th.emplace_back([=, &rcs, &fn] {
+      fdt_handle* sh = h->shards[r];
+      std::lock_guard<std::mutex> gl(sh->mu);
+      rcs[r] = fn(sh, lo, hi);
+    });
+  }
+  for (auto& t : th) t.join();
+  h->launches = 0; h->h2d_bytes = 0;
+  for (int r = 0; r < g; ++r) {
+    h->launches += h->shards[r]->launches; h->h2d_bytes += h->shards[r]->h2d_bytes;
+    if (rcs[r] != FDT_OK) { h->err = "device " + std::to_string(h->shards[r]->cfg.device) + ": " + h->shards[r]->err; return rcs[r]; }
+  }
+  return FDT_OK;
+}
+
+int detect_frames_multi(fdt_handle* h, const fdt_frame* frames, int n, int mode, int mem_kind, fdt_face* out_faces,
+                        int32_t* out_counts, float* out_mesh, float* out_iris) {
+  std::vector<FrameLayout> lay;
+  if (int rc = check_frames(h, frames, n, mode, mem_kind, out_faces, out_counts, &lay)) return rc;
+  if (mem_kind != FDT_MEM_HOST) return fail(h, FDT_ERR_UNSUPPORTED, "a multi-device handle takes host frames (device memory belongs to one device)");
+  return on_shards(h, n, [=](fdt_handle* sh, int lo, int hi) {
+    const size_t mf = (size_t)sh->max_faces;
+    return detect_frames_single(sh, frames + lo, hi - lo, mode, mem_kind, out_faces + lo * mf, out_counts + lo,
+                                out_mesh ? out_mesh + lo * mf * FDT_MESH_FLOATS : nullptr,
+                                out_iris ? out_iris + lo * mf * FDT_IRIS_FLOATS : nullptr);
+  });
 }
 
 // Multi-device handle: contiguous split of the batch, one host thread per replica, results land in frame order.
@@ -848,34 +1117,32 @@ template <typename T> bool grow(fdt_handle* h, T** p, size_t* cap, size_t need) 
   return true;
 }
 
-// decodes into h->d_jframe (packed BGR, EXIF orientation applied); *w / *hh = the oriented size
-int jpeg_to_device(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int* w, int* hh) {
-  if (!bytes || nbytes == 0) return fail(h, FDT_ERR_FORMAT, "empty image buffer");
-  JpegImage img;
-  std::string e;
-  const JpegStatus st = jpeg_decode_coefficients(bytes, nbytes, &img, &e);
-  if (st == kJpegBad) return fail(h, FDT_ERR_FORMAT, e);
-  if (st == kJpegUnsupported) return fail(h, FDT_ERR_UNSUPPORTED, e);
-  cudaSetDevice(h->cfg.device);
-  cudaStream_t s = h->slots[0].stream;
+// size of the decoded frame: EXIF orientations 5-8 swap width and height
+void jpeg_oriented_size(const JpegImage& img, int* w, int* hh) {
+  const bool swap = img.orientation >= 5;
+  *w = swap ? img.height : img.width; *hh = swap ? img.width : img.height;
+}
+
+// Device half of one decode, queued on s: coefficients up, IDCT per component, colour conversion + orientation into `out`
+// (packed BGR).  Returns the kernel launches, or -1 (h->err set).
+int jpeg_decode_device(fdt_handle* h, const JpegImage& img, uint8_t* out, cudaStream_t s) {
   size_t ncoef = 0, nplane = 0, coff[3] = {0, 0, 0}, poff[3] = {0, 0, 0};
   for (int c = 0; c < img.ncomp; ++c) {
     coff[c] = ncoef; poff[c] = nplane;
     ncoef += img.comp[c].coef.size();
     nplane += (size_t)img.comp[c].bw * 8 * img.comp[c].bh * 8;
   }
-  const bool swap = img.orientation >= 5;
-  const int ow = swap ? img.height : img.width, oh = swap ? img.width : img.height;
-  if (!grow(h, &h->d_jcoef, &h->jcoef_cap, ncoef) || !grow(h, &h->d_jplanes, &h->jplanes_cap, nplane) ||
-      !grow(h, &h->d_jframe, &h->jframe_cap, (size_t)ow * oh * 3)) return FDT_ERR_CUDA;
-  if (!h->d_jq && !cuda_ok(h, cudaMalloc(reinterpret_cast<void**>(&h->d_jq), 3 * 64 * sizeof(uint16_t)), "cudaMalloc(jpeg q)")) return FDT_ERR_CUDA;
+  int ow = 0, oh = 0;
+  jpeg_oriented_size(img, &ow, &oh);
+  if (!grow(h, &h->d_jcoef, &h->jcoef_cap, ncoef) || !grow(h, &h->d_jplanes, &h->jplanes_cap, nplane)) return -1;
+  if (!h->d_jq && !cuda_ok(h, cudaMalloc(reinterpret_cast<void**>(&h->d_jq), 3 * 64 * sizeof(uint16_t)), "cudaMalloc(jpeg q)")) return -1;
   uint16_t q[3 * 64];
   for (int c = 0; c < img.ncomp; ++c) std::memcpy(q + 64 * c, img.qt[img.comp[c].tq], 64 * sizeof(uint16_t));
   // pageable sources: the copies are staged by the driver before the call returns, so the local buffers may go out of scope
-  if (!cuda_ok(h, cudaMemcpyAsync(h->d_jq, q, (size_t)img.ncomp * 64 * sizeof(uint16_t), cudaMemcpyHostToDevice, s), "jpeg q upload")) return FDT_ERR_CUDA;
+  if (!cuda_ok(h, cudaMemcpyAsync(h->d_jq, q, (size_t)img.ncomp * 64 * sizeof(uint16_t), cudaMemcpyHostToDevice, s), "jpeg q upload")) return -1;
   for (int c = 0; c < img.ncomp; ++c)
     if (!cuda_ok(h, cudaMemcpyAsync(h->d_jcoef + coff[c], img.comp[c].coef.data(), img.comp[c].coef.size() * sizeof(int16_t), cudaMemcpyHostToDevice, s), "jpeg coefficient upload"))
-      return FDT_ERR_CUDA;
+      return -1;
   h->h2d_bytes += (long long)(ncoef * sizeof(int16_t));
   for (int c = 0; c < img.ncomp; ++c) {
     JpegIdctP p;
@@ -891,13 +1158,130 @@ int jpeg_to_device(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int* w, i
     cp.cdw = img.comp[1].dw; cp.cdh = img.comp[1].dh; cp.hs = img.hmax / img.comp[1].h; cp.vs = img.vmax / img.comp[1].v;
   }
   cp.W = img.width; cp.H = img.height; cp.ncomp = img.ncomp; cp.orientation = img.orientation;
-  cp.out = h->d_jframe; cp.out_w = ow;
+  cp.out = out; cp.out_w = ow;
   launch_jpeg_color(cp, s);
-  h->jpeg_launches = img.ncomp + 1;
+  return img.ncomp + 1;
+}
+
+// decodes into h->d_jframe (packed BGR, EXIF orientation applied); *w / *hh = the oriented size
+int jpeg_to_device(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int* w, int* hh) {
+  if (!bytes || nbytes == 0) return fail(h, FDT_ERR_FORMAT, "empty image buffer");
+  JpegImage img;
+  std::string e;
+  const JpegStatus st = jpeg_decode_coefficients(bytes, nbytes, &img, &e);
+  if (st == kJpegBad) return fail(h, FDT_ERR_FORMAT, e);
+  if (st == kJpegUnsupported) return fail(h, FDT_ERR_UNSUPPORTED, e);
+  cudaSetDevice(h->cfg.device);
+  cudaStream_t s = h->slots[0].stream;
+  int ow = 0, oh = 0;
+  jpeg_oriented_size(img, &ow, &oh);
+  if (!grow(h, &h->d_jframe, &h->jframe_cap, (size_t)ow * oh * 3)) return FDT_ERR_CUDA;
+  const int launches = jpeg_decode_device(h, img, h->d_jframe, s);
+  if (launches < 0) return FDT_ERR_CUDA;
+  h->jpeg_launches = launches;
   if (!cuda_ok(h, cudaStreamSynchronize(s), "jpeg decode")) return FDT_ERR_CUDA;   // the coefficient vectors die with this frame
   *w = ow; *hh = oh;
   h->jw = ow; h->jh = oh;
   return FDT_OK;
+}
+
+// fdt_detect_jpeg_batch on one replica.  The host parses and Huffman-decodes the images in waves of one image per thread;
+// the device decodes each into h->d_jarena (packed BGR at kStageAlign-aligned offsets); a chunk of arena frames (max_batch
+// images, max_batch * kStageBytesPerFrame bytes) then runs through detect_frames_single as device frames.  The host decode of
+// the next chunk does not overlap the device work of this one.
+int jpeg_batch_single(fdt_handle* h, const uint8_t* const* images, const size_t* sizes, int n, int mode, fdt_face* out_faces,
+                      int32_t* out_counts, float* out_mesh, float* out_iris, int32_t* out_wh, int32_t* out_status) {
+  cudaSetDevice(h->cfg.device);
+  cudaStream_t s = h->slots[0].stream;
+  const size_t mf = (size_t)h->max_faces, budget = (size_t)h->chunk * kStageBytesPerFrame;
+  long long launches = 0, h2d = 0;
+  std::vector<int> idx;                       // the images in the arena, in list order
+  std::vector<fdt_frame> fr;                  // their frames (data = arena offset until the chunk runs)
+  size_t used = 0;
+  std::vector<fdt_face> tf;                   // a chunk with failed images between its own runs into these, then scatters
+  std::vector<int32_t> tc;
+  std::vector<float> tm, ti;
+  auto run_chunk = [&]() -> int {
+    const int k = (int)idx.size();
+    if (k == 0) return FDT_OK;
+    if (!cuda_ok(h, cudaStreamSynchronize(s), "jpeg decode")) return FDT_ERR_CUDA;     // detection reads the arena on both slots
+    for (fdt_frame& f : fr) f.data = h->d_jarena + reinterpret_cast<size_t>(f.data);
+    const size_t i0 = (size_t)idx[0];
+    int rc;
+    if (idx.back() - idx[0] + 1 == k) {
+      rc = detect_frames_single(h, fr.data(), k, mode, FDT_MEM_DEVICE, out_faces + i0 * mf, out_counts + i0,
+                                out_mesh ? out_mesh + i0 * mf * FDT_MESH_FLOATS : nullptr, out_iris ? out_iris + i0 * mf * FDT_IRIS_FLOATS : nullptr);
+    } else {
+      tf.resize(k * mf); tc.resize(k);
+      if (out_mesh) tm.resize(k * mf * FDT_MESH_FLOATS);
+      if (out_iris) ti.resize(k * mf * FDT_IRIS_FLOATS);
+      rc = detect_frames_single(h, fr.data(), k, mode, FDT_MEM_DEVICE, tf.data(), tc.data(), out_mesh ? tm.data() : nullptr,
+                                out_iris ? ti.data() : nullptr);
+      for (int j = 0; j < k && rc == FDT_OK; ++j) {
+        const size_t i = (size_t)idx[j], c = (size_t)tc[j];
+        out_counts[i] = tc[j];
+        std::memcpy(out_faces + i * mf, tf.data() + j * mf, c * sizeof(fdt_face));
+        if (out_mesh) std::memcpy(out_mesh + i * mf * FDT_MESH_FLOATS, tm.data() + j * mf * FDT_MESH_FLOATS, c * FDT_MESH_FLOATS * sizeof(float));
+        if (out_iris) std::memcpy(out_iris + i * mf * FDT_IRIS_FLOATS, ti.data() + j * mf * FDT_IRIS_FLOATS, c * FDT_IRIS_FLOATS * sizeof(float));
+      }
+    }
+    launches += h->launches; h2d += h->h2d_bytes;
+    idx.clear(); fr.clear(); used = 0;
+    return rc;
+  };
+  const int nth = std::max(1, std::min(n, (int)std::thread::hardware_concurrency()));
+  std::vector<JpegImage> imgs(nth);
+  std::vector<JpegStatus> st(nth);
+  for (int w0 = 0; w0 < n; w0 += nth) {
+    const int m = std::min(nth, n - w0);
+    {
+      // jpeg_decode_coefficients keeps no state between calls: one image per thread
+      std::vector<std::thread> pool;
+      for (int t = 0; t < m; ++t)
+        pool.emplace_back([&, t] {
+          const int i = w0 + t;
+          std::string e;
+          imgs[t] = JpegImage();
+          st[t] = (!images[i] || sizes[i] == 0) ? kJpegBad : jpeg_decode_coefficients(images[i], sizes[i], &imgs[t], &e);
+        });
+      for (auto& t : pool) t.join();
+    }
+    for (int t = 0; t < m; ++t) {
+      const int i = w0 + t;
+      out_counts[i] = 0;
+      if (out_wh) { out_wh[2 * i] = 0; out_wh[2 * i + 1] = 0; }
+      if (st[t] != kJpegOk) { out_status[i] = st[t] == kJpegBad ? FDT_ERR_FORMAT : FDT_ERR_UNSUPPORTED; continue; }
+      int ow = 0, oh = 0;
+      jpeg_oriented_size(imgs[t], &ow, &oh);
+      const size_t fb = (size_t)ow * oh * 3;
+      if (!idx.empty() && ((int)idx.size() == h->chunk || align_up(used, kStageAlign) + fb > budget))
+        if (int rc = run_chunk()) return rc;
+      const size_t pos = align_up(used, kStageAlign);
+      if (pos + fb > h->jarena_cap) {
+        // grow, keeping the frames already decoded into the arena
+        const size_t want = std::max(pos + fb, std::min(budget, 2 * h->jarena_cap));
+        uint8_t* p = nullptr;
+        if (!cuda_ok(h, cudaMalloc(&p, want), "cudaMalloc(jpeg arena)")) return FDT_ERR_CUDA;
+        if (used) cudaMemcpyAsync(p, h->d_jarena, used, cudaMemcpyDeviceToDevice, s);
+        if (!cuda_ok(h, cudaStreamSynchronize(s), "jpeg arena")) { cudaFree(p); return FDT_ERR_CUDA; }
+        if (h->d_jarena) cudaFree(h->d_jarena);
+        h->d_jarena = p; h->jarena_cap = want;
+      }
+      h->h2d_bytes = 0;
+      const int l = jpeg_decode_device(h, imgs[t], h->d_jarena + pos, s);
+      if (l < 0) return FDT_ERR_CUDA;
+      launches += l; h2d += h->h2d_bytes;
+      fdt_frame f;
+      f.data = reinterpret_cast<const uint8_t*>(pos); f.width = ow; f.height = oh; f.row_stride = ow * 3; f.mat_type = FDT_MAT_8UC3;
+      idx.push_back(i); fr.push_back(f);
+      used = pos + fb;
+      out_status[i] = FDT_OK;
+      if (out_wh) { out_wh[2 * i] = ow; out_wh[2 * i + 1] = oh; }
+    }
+  }
+  const int rc = run_chunk();
+  h->launches = launches; h->h2d_bytes = h2d;
+  return rc;
 }
 }  // namespace
 
@@ -1032,7 +1416,8 @@ int create_single(const fdt_config& cfg, const uint8_t* det_tflite, size_t det_l
   for (int i = 0; i < kSlots; ++i) {
     Slot& sl = h->slots[i];
     if (cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking) != cudaSuccess) return bail(FDT_ERR_CUDA, "stream creation failed");
-    if (cudaEventCreateWithFlags(&sl.ev_det, cudaEventDisableTiming) != cudaSuccess) return bail(FDT_ERR_CUDA, "event creation failed");
+    if (cudaEventCreateWithFlags(&sl.ev_det, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&sl.ev_blob, cudaEventDisableTiming) != cudaSuccess) return bail(FDT_ERR_CUDA, "event creation failed");
     if (!h->det.make_ctx(h->chunk, &sl.det_ctx, &err)) return bail(FDT_ERR_CUDA, err);
     bool ok = dalloc(h, &sl.d_lb, (size_t)h->chunk * h->det.in_h() * h->det.in_w() * 4) &&     // BGRX
               dalloc(h, &sl.d_cand_idx, (size_t)h->chunk * h->cand_cap) && dalloc(h, &sl.d_cand_n, (size_t)h->chunk) &&
@@ -1055,7 +1440,8 @@ int create_single(const fdt_config& cfg, const uint8_t* det_tflite, size_t det_l
       ok = dalloc(h, &sl.d_eye_img, ec) && palloc(h, &sl.h_eye_img, ec) && dalloc(h, &sl.d_eye_affine, ec * 6) && palloc(h, &sl.h_eye_affine, ec * 6) &&
            dalloc(h, &sl.d_eye_roi, ec * 6) && palloc(h, &sl.h_eye_roi, ec * 6) && dalloc(h, &sl.d_eye_crops, ec * kIrisInput * kIrisInput * 4) &&
            dalloc(h, &sl.d_iris_out, (ec / 2) * FDT_IRIS_FLOATS) && palloc(h, &sl.h_iris_out, (ec / 2) * FDT_IRIS_FLOATS) &&
-           dalloc(h, &sl.d_eye_kp, (ec / 2) * 4) && palloc(h, &sl.h_eye_kp, (ec / 2) * 4);
+           dalloc(h, &sl.d_eye_kp, (ec / 2) * 4) && palloc(h, &sl.h_eye_kp, (ec / 2) * 4) &&
+           dalloc(h, &sl.d_eye_wh, ec) && palloc(h, &sl.h_eye_wh, ec);
       if (!ok) return bail(FDT_ERR_CUDA, "iris stage allocation failed");
     }
   }
@@ -1093,12 +1479,16 @@ int32_t fdt_destroy(fdt_handle* h) {
       if (sl.d_frames) cudaFree(sl.d_frames);
       if (sl.stream) cudaStreamDestroy(sl.stream);
       if (sl.ev_det) cudaEventDestroy(sl.ev_det);
+      if (sl.ev_blob) cudaEventDestroy(sl.ev_blob);
+      if (sl.h_blob) cudaFreeHost(sl.h_blob);
+      if (sl.d_blob) cudaFree(sl.d_blob);
     }
     for (void* p : h->dev_allocs) cudaFree(p);
     if (h->d_jcoef) cudaFree(h->d_jcoef);
     if (h->d_jplanes) cudaFree(h->d_jplanes);
     if (h->d_jframe) cudaFree(h->d_jframe);
     if (h->d_jq) cudaFree(h->d_jq);
+    if (h->d_jarena) cudaFree(h->d_jarena);
     for (void* p : h->pin_allocs) cudaFreeHost(p);
     void* dev[] = {h->d_faces, h->d_counts, h->d_anchors};
     for (void* p : dev) if (p) cudaFree(p);
@@ -1192,6 +1582,33 @@ int32_t fdt_detect_jpeg(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int3
   }
   if (p != h) { h->err = p->err; h->launches = p->launches; h->h2d_bytes = p->h2d_bytes; }
   return rc;
+}
+
+int32_t fdt_detect_frames(fdt_handle* h, const fdt_frame* frames, int32_t n, int32_t mode, int32_t mem_kind, fdt_face* out_faces,
+                          int32_t* out_counts, float* out_mesh, float* out_iris) {
+  if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
+  std::lock_guard<std::mutex> g(h->mu);
+  if (!h->shards.empty()) return detect_frames_multi(h, frames, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
+  return detect_frames_single(h, frames, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
+}
+
+int32_t fdt_detect_jpeg_batch(fdt_handle* h, const uint8_t* const* images, const size_t* sizes, int32_t n, int32_t mode,
+                              fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris, int32_t* out_wh,
+                              int32_t* out_status) {
+  if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
+  std::lock_guard<std::mutex> g(h->mu);
+  if (!h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
+  if (n < 0 || (n > 0 && (!images || !sizes || !out_faces || !out_counts || !out_status))) return fail(h, FDT_ERR_BAD_ARG, "bad image list");
+  if (int rc = check_mode(h, mode)) return rc;
+  h->launches = 0; h->h2d_bytes = 0;
+  if (n == 0) return FDT_OK;
+  if (h->shards.empty()) return jpeg_batch_single(h, images, sizes, n, mode, out_faces, out_counts, out_mesh, out_iris, out_wh, out_status);
+  return on_shards(h, n, [=](fdt_handle* sh, int lo, int hi) {
+    const size_t mf = (size_t)sh->max_faces;
+    return jpeg_batch_single(sh, images + lo, sizes + lo, hi - lo, mode, out_faces + lo * mf, out_counts + lo,
+                             out_mesh ? out_mesh + lo * mf * FDT_MESH_FLOATS : nullptr,
+                             out_iris ? out_iris + lo * mf * FDT_IRIS_FLOATS : nullptr, out_wh ? out_wh + 2 * lo : nullptr, out_status + lo);
+  });
 }
 
 int32_t fdt_host_jpeg_info(const uint8_t* bytes, size_t nbytes, int32_t* info8) {

@@ -97,6 +97,26 @@ struct LetterboxYuvP {
   const int* cy0; const int* cy1;
 };
 void launch_letterbox_yuv(const LetterboxYuvP& p, int B, cudaStream_t s);
+// Ragged batches (fdt_detect_frames): one descriptor per frame of a chunk.  It says where the frame's bytes are and how the
+// letterbox maps it; the crop warps read the same table, indexed by WarpP::crop_img.
+struct FrameD {
+  const uint8_t* y;        // the packed frame, or the Y plane
+  const uint8_t* c;        // YUV 4:2:0: the chroma area, addressed as in LetterboxYuvP (v_off relative to it)
+  int w, h, row_stride;
+  int channels;            // 1 / 3 / 4; 0: YUV 4:2:0
+  int c_row_stride, c_step, u_off, v_off;
+  int new_w, new_h, pad_top, pad_left, identity;
+  int tx, ty;              // offsets (ints) of the frame's x taps [4][new_w] and y taps [6][new_h] in the chunk's tap table
+};
+// k_letterbox_multi: k_letterbox / k_letterbox_yuv per frame.  taps (host-built, resize_linear_taps): per distinct size
+// x0, x1, ax0, ax1 (new_w each), then y0, y1, by0, by1, cy0, cy1 (new_h each; cy = y / 2, read for YUV frames only).
+struct LetterboxMultiP {
+  const FrameD* fr;        // [B]
+  const int* taps;
+  uint8_t* out;            // [B][S_h][S_w][4] BGRX
+  int dst_w, dst_h;
+};
+void launch_letterbox_multi(const LetterboxMultiP& p, int B, cudaStream_t s);
 // u8 [B][S][S][4] BGRX -> f32 [B][S][S][3] RGB, v*(1/127.5)-1
 void launch_normalize(const uint8_t* in, TV out, int B, cudaStream_t s);
 
@@ -283,6 +303,8 @@ struct DecodeP {
   const double* pre;                              // [B][N][17] already decoded detections (box4, score, kp12): skips threshold + decode
   double* dbg_dec;                                // [B][N][18] decoded candidates in anchor order: box4, score, kp12, kept flag
   int skip_roi;                                   // 1: keep faces whose alignment ROI is degenerate (round(size) <= 0)
+  // ragged batches: [B][6] = pad_t, pad_b, pad_l, pad_r, img_w, img_h per image; null: the scalars above
+  const double* geom = nullptr;
 };
 size_t decode_smem_bytes(int N);
 void launch_decode_nms(const DecodeP& p, int B, cudaStream_t s);
@@ -301,6 +323,8 @@ struct WarpP {
   int yuv = 0;
   long long c_off = 0;
   int c_row_stride = 0, c_step = 0, u_off = 0, v_off = 0;
+  // ragged batches: the frame of crop f is fr[crop_img[f]] (its layout and size replace the fields above); null: uniform
+  const FrameD* fr = nullptr;
 };
 void launch_warp_affine(const WarpP& p, cudaStream_t s);
 
@@ -322,7 +346,8 @@ struct IrisPostP {
   const double* roi;                                   // [2F][6] theta, cx, cy, size, cos, sin per eye (even = left, odd = right/flipped)
   int nfaces, in_size;
   double img_w, img_h;
-  float* iris_out;                                     // [F][456] 76 points of the left eye then 76 of the right, absolute pixels
+  const double* img_wh = nullptr;                      // ragged batches: [F][2] frame size per face; null: img_w, img_h
+  float* iris_out;                                    // [F][456] 76 points of the left eye then 76 of the right, absolute pixels
   double* eye_kp;                                      // [F][4] iris-refined leftEye / rightEye keypoints, normalised
 };
 void launch_iris_post(const IrisPostP& p, cudaStream_t s);

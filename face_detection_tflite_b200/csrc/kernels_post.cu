@@ -165,7 +165,10 @@ __global__ void __launch_bounds__(kDecodeThreads) k_decode_nms(DecodeP p) {
 
   // 5. letterbox removal (helpers.dart:101-136), gates (face_gates.dart:130-146), ROI check
   //    (face_detector_core.dart:255-265 / helpers.dart:591-592)
-  const double sx = 1.0 - (p.pad_l + p.pad_r), sy = 1.0 - (p.pad_t + p.pad_b);
+  const double* g = p.geom ? p.geom + 6 * (size_t)b : nullptr;
+  const double pad_t = g ? g[0] : p.pad_t, pad_b = g ? g[1] : p.pad_b, pad_l = g ? g[2] : p.pad_l, pad_r = g ? g[3] : p.pad_r;
+  const double img_w = g ? g[4] : p.img_w, img_h = g ? g[5] : p.img_h;
+  const double sx = 1.0 - (pad_l + pad_r), sy = 1.0 - (pad_t + pad_b);
   for (int f = tid; f < nout; f += kDecodeThreads) {
     const NmsOut& o = s_out[f];
     int i = s_idx[o.cand];
@@ -173,14 +176,14 @@ __global__ void __launch_bounds__(kDecodeThreads) k_decode_nms(DecodeP p) {
     if (pre) { for (int k = 0; k < 12; ++k) kp[k] = pre[(size_t)i * 17 + 5 + k]; }
     else decode_box(boxes + (size_t)i * 16, p.anchors[2 * i], p.anchors[2 * i + 1], (double)p.input_h, box, kp);
     fdt_face fc;
-    fc.xmin = (o.box[0] - p.pad_l) / sx;
-    fc.ymin = (o.box[1] - p.pad_t) / sy;
-    fc.xmax = (o.box[2] - p.pad_l) / sx;
-    fc.ymax = (o.box[3] - p.pad_t) / sy;
+    fc.xmin = (o.box[0] - pad_l) / sx;
+    fc.ymin = (o.box[1] - pad_t) / sy;
+    fc.xmax = (o.box[2] - pad_l) / sx;
+    fc.ymax = (o.box[3] - pad_t) / sy;
     fc.score = o.score;
     for (int k = 0; k < 12; k += 2) {
-      fc.keypoints[k] = (kp[k] - p.pad_l) / sx;
-      fc.keypoints[k + 1] = (kp[k + 1] - p.pad_t) / sy;
+      fc.keypoints[k] = (kp[k] - pad_l) / sx;
+      fc.keypoints[k + 1] = (kp[k + 1] - pad_t) / sy;
     }
     fc.mesh_score = nan("");
     fc.has_mesh = 0;
@@ -190,10 +193,10 @@ __global__ void __launch_bounds__(kDecodeThreads) k_decode_nms(DecodeP p) {
     bool pass = true;
     if (p.min_score > 0.0 || p.min_face_size > 0.0) {
       pass = fc.score >= p.min_score &&
-             (p.min_face_size <= 0.0 || visible_width_fraction(fc.xmin, fc.xmax, p.img_w) >= p.min_face_size);
+             (p.min_face_size <= 0.0 || visible_width_fraction(fc.xmin, fc.xmax, img_w) >= p.min_face_size);
     }
     double theta, cx, cy, size;
-    face_alignment(fc.keypoints, p.img_w, p.img_h, &theta, &cx, &cy, &size);
+    face_alignment(fc.keypoints, img_w, img_h, &theta, &cx, &cy, &size);
     if (!p.skip_roi && !(dart_round(size) > 0)) pass = false;
     s_face[f] = fc;
     s_pass[f] = pass ? 1 : 0;
@@ -217,12 +220,16 @@ __device__ __forceinline__ long long sat_round_ll(double v) { return (long long)
 
 // One thread per output pixel; blockIdx.y = crop.  The per-row / per-column fixed-point terms of
 // imgproc/imgwarp.cpp WarpAffineInvoker (AB_BITS = 10, INTER_BITS = 5) are evaluated per pixel: two f64 rint each.
+// kRagged: the crop's frame, its layout and size come from the descriptor table p.fr (chunks of frames of different sizes).
+template <bool kRagged>
 __global__ void k_warp_affine(WarpP p) {
   const int f = blockIdx.y;
   if (f >= p.ncrops) return;
   const int S = p.out_size;
   const double* A = p.affine + 6 * f;
-  const uint8_t* src = p.frames + (size_t)p.crop_img[f] * p.frame_stride;
+  // every per-frame value is written as (kRagged ? descriptor : parameter), so the uniform instantiation is the plain kernel
+  const FrameD* d = kRagged ? p.fr + p.crop_img[f] : nullptr;
+  const uint8_t* src = kRagged ? d->y : p.frames + (size_t)p.crop_img[f] * p.frame_stride;
   const bool flip = p.flip_odd && (f & 1);
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < S * S; i += gridDim.x * blockDim.x) {
     int y = i / S, x = i - y * S;
@@ -241,16 +248,19 @@ __global__ void k_warp_affine(WarpP p) {
 #pragma unroll
     for (int t = 0; t < 4; ++t) {
       int yy = sy + (t >> 1), xx = sx + (t & 1);
-      if (yy < 0 || yy >= p.src_h || xx < 0 || xx >= p.src_w) continue;   // out-of-frame taps: BGR 0 (also for YUV frames)
-      if (p.yuv) {
-        const uint8_t* c = src + p.c_off + (size_t)(yy >> 1) * p.c_row_stride + (size_t)(xx >> 1) * p.c_step;
+      if (yy < 0 || yy >= (kRagged ? d->h : p.src_h) || xx < 0 || xx >= (kRagged ? d->w : p.src_w)) continue;   // out-of-frame taps: BGR 0 (also for YUV frames)
+      const int row_stride = kRagged ? d->row_stride : p.row_stride;
+      if (kRagged ? d->channels == 0 : p.yuv) {
+        const uint8_t* c = (kRagged ? d->c : src + p.c_off) + (size_t)(yy >> 1) * (kRagged ? d->c_row_stride : p.c_row_stride) +
+                           (size_t)(xx >> 1) * (kRagged ? d->c_step : p.c_step);
         int v[3];
-        yuv_to_bgr(src[(size_t)yy * p.row_stride + xx], c[p.u_off], c[p.v_off], v);
+        yuv_to_bgr(src[(size_t)yy * row_stride + xx], c[kRagged ? d->u_off : p.u_off], c[kRagged ? d->v_off : p.v_off], v);
         acc[0] += v[0] * iw[t]; acc[1] += v[1] * iw[t]; acc[2] += v[2] * iw[t];
         continue;
       }
-      const uint8_t* px = src + (size_t)yy * p.row_stride + (size_t)xx * p.channels;
-      if (p.channels == 1) {
+      const int channels = kRagged ? d->channels : p.channels;
+      const uint8_t* px = src + (size_t)yy * row_stride + (size_t)xx * channels;
+      if (channels == 1) {
         acc[0] += px[0] * iw[t]; acc[1] += px[0] * iw[t]; acc[2] += px[0] * iw[t];
       } else {
         acc[0] += px[0] * iw[t]; acc[1] += px[1] * iw[t]; acc[2] += px[2] * iw[t];
@@ -340,8 +350,9 @@ __global__ void k_iris_post(IrisPostP p) {
       const double dx = s_xy[t][k][0] - mx, dy = s_xy[t][k][1] - my, d = dx * dx + dy * dy;
       if (d < bd) { bd = d; best = k; }
     }
-    p.eye_kp[4 * f + 2 * t] = s_xy[t][best][0] / p.img_w;
-    p.eye_kp[4 * f + 2 * t + 1] = s_xy[t][best][1] / p.img_h;
+    const double iw = p.img_wh ? p.img_wh[2 * f] : p.img_w, ih = p.img_wh ? p.img_wh[2 * f + 1] : p.img_h;
+    p.eye_kp[4 * f + 2 * t] = s_xy[t][best][0] / iw;
+    p.eye_kp[4 * f + 2 * t + 1] = s_xy[t][best][1] / ih;
   }
 }
 
@@ -360,7 +371,8 @@ void launch_decode_nms(const DecodeP& p, int B, cudaStream_t s) {
 void launch_warp_affine(const WarpP& p, cudaStream_t s) {
   if (p.ncrops <= 0) return;
   dim3 grid((p.out_size * p.out_size + 255) / 256, p.ncrops);
-  k_warp_affine<<<grid, 256, 0, s>>>(p);
+  if (p.fr) k_warp_affine<true><<<grid, 256, 0, s>>>(p);
+  else k_warp_affine<false><<<grid, 256, 0, s>>>(p);
 }
 
 void launch_mesh_post(const MeshPostP& p, cudaStream_t s) {

@@ -1,5 +1,6 @@
 // Preprocessing kernels: fused letterbox (cv::resize INTER_LINEAR 8U fixed point +
-// copyMakeBorder(0) + BGRA/GRAY->BGR, or cvtColor YUV2BGR for NV12 / NV21 / I420 frames) and the [-1,1] normalisation.
+// copyMakeBorder(0) + BGRA/GRAY->BGR, or cvtColor YUV2BGR for NV12 / NV21 / I420 frames; k_letterbox_multi for chunks of
+// frames of different sizes and formats) and the [-1,1] normalisation.
 // Reference: convertImageToTensor / bgrMatToSignedFloat32 (lib/src/util/helpers.dart:303-421).
 #include "kernels.h"
 
@@ -67,6 +68,11 @@ __device__ __forceinline__ void load_yuv(const uint8_t* yrow, const uint8_t* cro
   const uint8_t* c = crow + (size_t)(x >> 1) * p.c_step;
   yuv_to_bgr(yrow[x], c[p.u_off], c[p.v_off], v);
 }
+// the same for a frame of a ragged chunk
+__device__ __forceinline__ void load_yuv(const uint8_t* yrow, const uint8_t* crow, int x, const FrameD& f, int* v) {
+  const uint8_t* c = crow + (size_t)(x >> 1) * f.c_step;
+  yuv_to_bgr(yrow[x], c[f.u_off], c[f.v_off], v);
+}
 
 // k_letterbox for NV12 / NV21 / I420 frames: same grid and fixed-point resize; every tap is converted before it is weighted
 // (the conversion is per pixel, so this equals resizing the converted frame).  Padding stays BGR 0.
@@ -107,6 +113,51 @@ __global__ void __launch_bounds__(256) k_letterbox_yuv(LetterboxYuvP p, int B) {
   }
 }
 
+// Ragged batches: the grid of k_letterbox, one frame per blockIdx.z step, its geometry and layout from a descriptor table.  The
+// format is the same for every thread of a block, so the packed / YUV branch does not diverge; the arithmetic is that of
+// k_letterbox / k_letterbox_yuv, so a frame letterboxes to the same bytes in a ragged chunk as in a uniform one.
+__global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int B) {
+  const int x = blockIdx.x * 64 + (threadIdx.x & 63), y = blockIdx.y * 4 + (threadIdx.x >> 6);
+  if (x >= p.dst_w || y >= p.dst_h) return;
+  for (int b = blockIdx.z; b < B; b += gridDim.z) {
+    const FrameD f = p.fr[b];
+    const int dy = y - f.pad_top, dx = x - f.pad_left;
+    uchar3 o = make_uchar3(0, 0, 0);
+    if (dy >= 0 && dy < f.new_h && dx >= 0 && dx < f.new_w) {
+      int res[3];
+      if (f.identity) {
+        if (f.channels) load_bgr(f.y + (size_t)dy * f.row_stride + (size_t)dx * f.channels, f.channels, res);
+        else load_yuv(f.y + (size_t)dy * f.row_stride, f.c + (size_t)(dy >> 1) * f.c_row_stride, dx, f, res);
+      } else {
+        const int* tx = p.taps + f.tx;
+        const int* ty = p.taps + f.ty;
+        const int xa = tx[dx], xb = tx[f.new_w + dx], wa = tx[2 * f.new_w + dx], wb = tx[3 * f.new_w + dx];
+        const int ya = ty[dy], yb = ty[f.new_h + dy], va = ty[2 * f.new_h + dy], vb = ty[3 * f.new_h + dy];
+        int t00[3], t01[3], t10[3], t11[3];
+        const uint8_t* r0 = f.y + (size_t)ya * f.row_stride;
+        const uint8_t* r1 = f.y + (size_t)yb * f.row_stride;
+        if (f.channels) {
+          load_bgr(r0 + (size_t)xa * f.channels, f.channels, t00);
+          load_bgr(r0 + (size_t)xb * f.channels, f.channels, t01);
+          load_bgr(r1 + (size_t)xa * f.channels, f.channels, t10);
+          load_bgr(r1 + (size_t)xb * f.channels, f.channels, t11);
+        } else {
+          const uint8_t* c0 = f.c + (size_t)ty[4 * f.new_h + dy] * f.c_row_stride;
+          const uint8_t* c1 = f.c + (size_t)ty[5 * f.new_h + dy] * f.c_row_stride;
+          load_yuv(r0, c0, xa, f, t00);
+          load_yuv(r0, c0, xb, f, t01);
+          load_yuv(r1, c1, xa, f, t10);
+          load_yuv(r1, c1, xb, f, t11);
+        }
+#pragma unroll
+        for (int c = 0; c < 3; ++c) res[c] = resize_linear(t00[c], t01[c], t10[c], t11[c], wa, wb, va, vb);
+      }
+      o = make_uchar3((unsigned char)res[0], (unsigned char)res[1], (unsigned char)res[2]);
+    }
+    reinterpret_cast<uchar4*>(p.out)[((size_t)b * p.dst_h + y) * p.dst_w + x] = make_uchar4(o.x, o.y, o.z, 0);
+  }
+}
+
 __global__ void k_normalize(const uint8_t* in, TV out, long long total) {
   for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total;
        idx += (long long)gridDim.x * blockDim.x) {
@@ -133,6 +184,12 @@ void launch_letterbox_yuv(const LetterboxYuvP& p, int B, cudaStream_t s) {
   if (B <= 0) return;
   dim3 grid((unsigned)((p.lb.dst_w + 63) / 64), (unsigned)((p.lb.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
   k_letterbox_yuv<<<grid, 256, 0, s>>>(p, B);
+}
+
+void launch_letterbox_multi(const LetterboxMultiP& p, int B, cudaStream_t s) {
+  if (B <= 0) return;
+  dim3 grid((unsigned)((p.dst_w + 63) / 64), (unsigned)((p.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
+  k_letterbox_multi<<<grid, 256, 0, s>>>(p, B);
 }
 
 void launch_normalize(const uint8_t* in, TV out, int B, cudaStream_t s) {

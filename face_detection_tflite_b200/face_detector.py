@@ -41,6 +41,44 @@ def _raise(lib, handle, code: int):
     raise RuntimeError(msg)
 
 
+_PACKED = {_ffi.FDT_MAT_8UC1: 1, _ffi.FDT_MAT_8UC3: 3, _ffi.FDT_MAT_8UC4: 4}
+
+
+def _mat_type(m, i: int) -> int:
+    if not isinstance(m, np.ndarray) or m.dtype != np.uint8 or m.ndim not in (2, 3) or m.shape[0] <= 0 or m.shape[1] <= 0:
+        raise ValueError("mat %d: expected an HxW, HxWx3 or HxWx4 uint8 array" % i)
+    mt = {1: _ffi.FDT_MAT_8UC1, 3: _ffi.FDT_MAT_8UC3, 4: _ffi.FDT_MAT_8UC4}.get(1 if m.ndim == 2 else m.shape[2])
+    if mt is None:
+        raise ValueError("mat %d: unsupported Mat type" % i)
+    return mt
+
+
+def _rows_in_buffer(m: np.ndarray) -> bool:
+    """True when height * strides[0] bytes from the view's start stay inside the memory it views (the library reads a frame
+    as height whole rows of the row stride)."""
+    root = m
+    while isinstance(root.base, np.ndarray):
+        root = root.base
+    byte_bounds = getattr(np, "byte_bounds", None) or np.lib.array_utils.byte_bounds
+    return m.ctypes.data + m.shape[0] * m.strides[0] <= byte_bounds(root)[1]
+
+
+def _frame_geometry(i: int, w, h, mt, stride):
+    """(row stride, frame bytes) of one fdt_frame; ValueError for arguments the library cannot take."""
+    if not all(isinstance(v, (int, np.integer)) for v in (w, h, mt)) or w <= 0 or h <= 0:
+        raise ValueError("frame %d: width, height and matType must be positive integers" % i)
+    yuv = mt in _ffi.YUV_FORMATS
+    ch = 1 if yuv else _PACKED.get(mt)
+    if ch is None:
+        raise ValueError("frame %d: unknown matType %r" % (i, mt))
+    stride = w * ch if stride is None else stride
+    if not isinstance(stride, (int, np.integer)) or stride < w * ch:
+        raise ValueError("frame %d: rowStride smaller than width * channels" % i)
+    if yuv and (w % 2 or h % 2):
+        raise ValueError("frame %d: YUV 4:2:0 frames need an even width and height" % i)
+    return int(stride), (h * stride * 3 // 2 if yuv else h * stride)
+
+
 class FaceDetector:
     modelVersion = "1.1.1"   # lib/src/face_detector.dart:54-64
 
@@ -240,6 +278,107 @@ class FaceDetector:
         if rc != _ffi.FDT_OK:
             _raise(self._lib, self._h, rc)
         return (faces, counts[:count], mesh, iris) if withIris else (faces, counts[:count], mesh)
+
+    # -- mixed batches: frames of different sizes and formats, and encoded images, in one call ----------------------------
+    def detectFacesFromMats(self, mats, *, mode: FaceDetectionMode = FaceDetectionMode.full) -> List[List[Face]]:
+        """detectFacesFromMat over a list of HxW / HxWx3 / HxWx4 uint8 arrays of any sizes, in one batched call
+        (fdt_detect_frames).  A row-padded view (e.g. a crop of a larger array) goes in uncopied with strides[0] as its row
+        stride.  Returns one list of faces per mat, each normalised to its own mat."""
+        frames, keep = [], []
+        for i, m in enumerate(mats):
+            mt = _mat_type(m, i)
+            if m.strides[-1] != 1 or (m.ndim == 3 and m.strides[1] != m.shape[2]) or m.strides[0] < m.shape[1] * m.strides[1] \
+                    or not _rows_in_buffer(m):
+                m = np.ascontiguousarray(m)
+            keep.append(m)
+            frames.append((m.ctypes.data, m.shape[1], m.shape[0], m.strides[0], mt))
+        self._check()
+        faces, counts, mesh, iris = self._detect_frames(frames, mode, _ffi.FDT_MEM_HOST)
+        return self._faces_per_frame(faces, counts, mesh, iris, [(f[1], f[2]) for f in frames])
+
+    def detectFramesRaw(self, frames, *, mode: FaceDetectionMode = FaceDetectionMode.fast, memKind: int = _ffi.FDT_MEM_HOST):
+        """fdt_detect_frames with array outputs.  `frames` is a list of (data, width, height, matType[, rowStride]) tuples: data
+        is a numpy array / bytes of exactly height * rowStride bytes (YUV 4:2:0: height * rowStride * 3 / 2), or an integer
+        device pointer with memKind=FDT_MEM_DEVICE.  rowStride defaults to width * channels (YUV: width).  Returns
+        (FdtFace array [n * max_faces], counts int32 [n], mesh f32 [n, max_faces, 468, 3] or None,
+        iris f32 [n, max_faces, 152, 3] or None)."""
+        if memKind not in (_ffi.FDT_MEM_HOST, _ffi.FDT_MEM_DEVICE):
+            raise ValueError("memKind must be FDT_MEM_HOST or FDT_MEM_DEVICE")
+        descs, keep = [], []
+        for i, fr in enumerate(frames):
+            if not isinstance(fr, (tuple, list)) or len(fr) not in (4, 5):
+                raise ValueError("frame %d: expected (data, width, height, matType[, rowStride])" % i)
+            data, w, h, mt = fr[:4]
+            stride, nbytes = _frame_geometry(i, w, h, mt, fr[4] if len(fr) == 5 else None)
+            if memKind == _ffi.FDT_MEM_DEVICE:
+                if not isinstance(data, int):
+                    raise ValueError("frame %d: FDT_MEM_DEVICE frames are integer device pointers" % i)
+                ptr = data
+            else:
+                if isinstance(data, int):
+                    raise ValueError("frame %d: host frames are numpy arrays or bytes" % i)
+                buf = np.ascontiguousarray(np.frombuffer(data, np.uint8) if not isinstance(data, np.ndarray) else data.reshape(-1))
+                if buf.dtype != np.uint8 or buf.size != nbytes:
+                    raise ValueError("frame %d: data length does not equal height * rowStride%s" % (i, " * 3 / 2" if mt in _ffi.YUV_FORMATS else ""))
+                keep.append(buf)
+                ptr = buf.ctypes.data
+            descs.append((ptr, w, h, stride, mt))
+        self._check()
+        return self._detect_frames(descs, mode, memKind)
+
+    def detectFacesFromBytesBatch(self, images, *, mode: FaceDetectionMode = FaceDetectionMode.full) -> List[Optional[List[Face]]]:
+        """detectFacesFromBytes over a list of encoded images (JPEG) in one call (fdt_detect_jpeg_batch).  An image that
+        cannot be decoded gives None in its place instead of raising, so one bad photo does not discard the batch."""
+        faces, counts, mesh, iris, wh, status = self.detectBytesBatchRaw(images, mode=mode)
+        out = self._faces_per_frame(faces, counts, mesh, iris, [tuple(x) for x in wh])
+        return [f if status[i] == _ffi.FDT_OK else None for i, f in enumerate(out)]
+
+    def detectBytesBatchRaw(self, images, *, mode: FaceDetectionMode = FaceDetectionMode.full):
+        """fdt_detect_jpeg_batch with array outputs: (FdtFace array, counts, mesh or None, iris or None, wh int32 [n, 2],
+        status int32 [n]); status is FDT_OK, FDT_ERR_FORMAT or FDT_ERR_UNSUPPORTED per image."""
+        bufs = []
+        for i, im in enumerate(images):
+            if not isinstance(im, (bytes, bytearray, memoryview, np.ndarray)):
+                raise ValueError("image %d: expected encoded bytes" % i)
+            bufs.append(np.frombuffer(bytes(im), np.uint8) if not isinstance(im, np.ndarray) else np.ascontiguousarray(im, np.uint8).reshape(-1))
+        self._check()
+        n = len(bufs)
+        ptrs = (C.c_void_p * max(1, n))(*[b.ctypes.data if b.size else None for b in bufs])
+        sizes = (C.c_size_t * max(1, n))(*[b.size for b in bufs])
+        faces, counts, mesh, iris = self._outputs(n, mode)
+        wh = np.zeros((max(1, n), 2), np.int32)
+        status = np.zeros(max(1, n), np.int32)
+        rc = self._lib.fdt_detect_jpeg_batch(self._h, ptrs, sizes, n, int(mode), faces, counts.ctypes.data_as(_ffi.i32p),
+                                             mesh.ctypes.data_as(_ffi.f32p) if mesh is not None else None,
+                                             iris.ctypes.data_as(_ffi.f32p) if iris is not None else None,
+                                             wh.ctypes.data_as(_ffi.i32p), status.ctypes.data_as(_ffi.i32p))
+        if rc != _ffi.FDT_OK:
+            _raise(self._lib, self._h, rc)
+        return faces, counts[:n], mesh, iris, wh[:n], status[:n]
+
+    def _outputs(self, n: int, mode):
+        mode = FaceDetectionMode(mode)
+        faces = (_ffi.FdtFace * max(1, n * self._max_faces))()
+        counts = np.zeros(max(1, n), np.int32)
+        mesh = np.zeros((n, self._max_faces, 468, 3), np.float32) if mode != FaceDetectionMode.fast else None
+        iris = np.zeros((n, self._max_faces, 152, 3), np.float32) if mode == FaceDetectionMode.full else None
+        return faces, counts, mesh, iris
+
+    def _detect_frames(self, descs, mode, memKind):
+        n = len(descs)
+        arr = (_ffi.FdtFrame * max(1, n))(*[_ffi.FdtFrame(*d) for d in descs])   # (data, width, height, row_stride, mat_type)
+        faces, counts, mesh, iris = self._outputs(n, mode)
+        rc = self._lib.fdt_detect_frames(self._h, arr, n, int(FaceDetectionMode(mode)), memKind, faces, counts.ctypes.data_as(_ffi.i32p),
+                                         mesh.ctypes.data_as(_ffi.f32p) if mesh is not None else None,
+                                         iris.ctypes.data_as(_ffi.f32p) if iris is not None else None)
+        if rc != _ffi.FDT_OK:
+            _raise(self._lib, self._h, rc)
+        return faces, counts[:n], mesh, iris
+
+    def _faces_per_frame(self, faces, counts, mesh, iris, sizes):
+        mf = self._max_faces
+        return [[self._to_face(faces[b * mf + j], mesh[b, j] if mesh is not None else None, w, h, iris[b, j] if iris is not None else None)
+                 for j in range(int(counts[b]))] for b, (w, h) in enumerate(sizes)]
 
     @staticmethod
     def _to_face(f, mesh, width, height, iris=None) -> Face:

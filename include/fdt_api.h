@@ -158,6 +158,37 @@ FDT_EXPORT int32_t fdt_detect_batch(fdt_handle* h, const uint8_t* frames, int32_
                                     int32_t mem_kind, fdt_face* out_faces, int32_t* out_counts,
                                     float* out_mesh, float* out_iris);
 
+/* One frame of a mixed batch (fdt_detect_frames): its own size and format. */
+typedef struct fdt_frame {
+  const uint8_t* data;       /* host or device memory, per the call's mem_kind                                   */
+  int32_t width, height;     /* image size                                                                        */
+  int32_t row_stride;        /* as fdt_detect_batch: >= width * channels; YUV: the Y-plane stride                 */
+  int32_t mat_type;          /* FDT_MAT_8UC1 / _8UC3 / _8UC4 or FDT_FMT_YUV_NV12 / _NV21 / _I420                 */
+} fdt_frame;                 /* 24 bytes */
+
+/* detectFacesFromMat over a list of frames of different sizes and formats (photos, mixed camera feeds), batched like
+ * fdt_detect_batch: the frames run in chunks of up to max_batch through the same kernels, launches and two-slot pipeline.
+ * Host frames also close a chunk when its staged bytes would pass max_batch * 8 MiB (a larger frame is a chunk of its own);
+ * they go up whole (no sparse row upload), so fdt_last_h2d_bytes is the sum of the frames' sizes.  Device frames must be in
+ * the handle's device memory; a multi-device handle takes host frames only and splits the list contiguously.
+ * Outputs as fdt_detect_batch: faces [n][max_faces], counts [n], mesh [n][max_faces][1404], iris [n][max_faces][456]; each
+ * frame's faces are normalised to its own size, mesh and iris points are in its own pixels.  Results are bitwise those of
+ * fdt_detect_batch on each frame alone.  Every descriptor is checked before any work: the first bad one returns the code
+ * fdt_detect_batch would return for it, and fdt_last_error names its index.  n == 0 returns FDT_OK. */
+FDT_EXPORT int32_t fdt_detect_frames(fdt_handle* h, const fdt_frame* frames, int32_t n, int32_t mode, int32_t mem_kind,
+                                     fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris);
+
+/* fdt_detect_jpeg over n encoded images in one call.  The host parses and Huffman-decodes them on a pool of
+ * min(n, hardware threads) threads; the device decodes them into a handle-owned frame arena and detects them as one mixed
+ * batch (chunks of up to max_batch images and max_batch * 8 MiB of decoded BGR).  out_status[i] is FDT_OK, FDT_ERR_FORMAT
+ * (not a decodable JPEG; also NULL or empty buffers) or FDT_ERR_UNSUPPORTED; a failed image gets count 0 and out_wh 0, 0
+ * and does not stop the others.  The call returns FDT_OK unless an argument or CUDA error stops the whole batch.
+ * out_wh: [n][2] decoded width, height, or NULL.  Outputs otherwise as fdt_detect_frames; a multi-device handle splits the
+ * list contiguously over its replicas. */
+FDT_EXPORT int32_t fdt_detect_jpeg_batch(fdt_handle* h, const uint8_t* const* images, const size_t* sizes, int32_t n,
+                                         int32_t mode, fdt_face* out_faces, int32_t* out_counts, float* out_mesh,
+                                         float* out_iris, int32_t* out_wh, int32_t* out_status);
+
 /* detectFacesFromMatBytes (lib/src/face_detector.dart:588-609): one packed frame of
  * `nbytes` bytes; FDT_ERR_SIZE_MISMATCH when nbytes != width*height*channels
  * (matFromPackedBytes, lib/src/util/helpers.dart:432-450), or != width*height*3/2 for the YUV formats. */

@@ -247,6 +247,100 @@ class FdtFaceDetector {
     return out;
   }
 
+  /// detectFacesFromMat over a list of frames of any sizes and formats (photos, mixed camera feeds) in one batched
+  /// `fdt_detect_frames` call.  Each mat is packed bytes of its own width, height and matType (kFdtFmtYuv* included);
+  /// each result list is normalised to its own mat.
+  Future<List<List<Face>>> detectFacesFromMats(
+    List<({Uint8List bytes, int width, int height, int matType})> mats, {
+    FaceDetectionMode mode = FaceDetectionMode.full,
+  }) async {
+    _check();
+    for (int i = 0; i < mats.length; i++) {
+      final m = mats[i];
+      if (m.bytes.length != fdtFrameBytes(m.matType, m.width, m.height)) {
+        throw ArgumentError('mat $i: bytes length does not equal its frame size');
+      }
+    }
+    final int n = mats.length;
+    if (n == 0) return <List<Face>>[];
+    final arena = Arena();
+    try {
+      final Pointer<FdtFrame> frames = arena<FdtFrame>(n);
+      for (int i = 0; i < n; i++) {
+        final m = mats[i];
+        final Pointer<Uint8> src = arena<Uint8>(m.bytes.length);
+        src.asTypedList(m.bytes.length).setAll(0, m.bytes);
+        frames[i].data = src;
+        frames[i].width = m.width;
+        frames[i].height = m.height;
+        frames[i].rowStride = fdtRowStride(m.matType, m.width);
+        frames[i].matType = m.matType;
+      }
+      final out = _outputs(arena, n, mode);
+      final int rc = _lib.detectFrames(_h, frames, n, mode.index, kFdtMemHost, out.faces, out.counts, out.mesh, out.iris);
+      if (rc != FdtStatus.ok) {
+        _lib.throwFor(rc, _h); // ArgumentError naming the first bad mat
+      }
+      return <List<Face>>[for (int b = 0; b < n; b++) _facesOf(out, b, mats[b].width, mats[b].height)];
+    } finally {
+      arena.releaseAll();
+    }
+  }
+
+  /// detectFacesFromBytes over a list of encoded images (JPEG) in one `fdt_detect_jpeg_batch` call.  An image that cannot
+  /// be decoded gives `null` in its place instead of throwing, so one bad photo does not discard the batch.
+  Future<List<List<Face>?>> detectFacesFromBytesBatch(
+    List<Uint8List> images, {
+    FaceDetectionMode mode = FaceDetectionMode.full,
+  }) async {
+    _check();
+    final int n = images.length;
+    if (n == 0) return <List<Face>?>[];
+    final arena = Arena();
+    try {
+      final Pointer<Pointer<Uint8>> ptrs = arena<Pointer<Uint8>>(n);
+      final Pointer<Size> sizes = arena<Size>(n);
+      for (int i = 0; i < n; i++) {
+        final Pointer<Uint8> src = arena<Uint8>(images[i].length + 1);
+        src.asTypedList(images[i].length).setAll(0, images[i]);
+        ptrs[i] = src;
+        sizes[i] = images[i].length;
+      }
+      final Pointer<Int32> wh = arena<Int32>(2 * n);
+      final Pointer<Int32> status = arena<Int32>(n);
+      final out = _outputs(arena, n, mode);
+      final int rc = _lib.detectJpegBatch(_h, ptrs, sizes, n, mode.index, out.faces, out.counts, out.mesh, out.iris, wh, status);
+      if (rc != FdtStatus.ok) {
+        _lib.throwFor(rc, _h);
+      }
+      return <List<Face>?>[
+        for (int b = 0; b < n; b++) status[b] == FdtStatus.ok ? _facesOf(out, b, wh[2 * b], wh[2 * b + 1]) : null,
+      ];
+    } finally {
+      arena.releaseAll();
+    }
+  }
+
+  ({Pointer<FdtFace> faces, Pointer<Int32> counts, Pointer<Float> mesh, Pointer<Float> iris}) _outputs(
+      Arena arena, int n, FaceDetectionMode mode) {
+    final bool wantMesh = mode != FaceDetectionMode.fast;
+    final bool wantIris = mode == FaceDetectionMode.full;
+    return (
+      faces: arena<FdtFace>(n * _maxFaces),
+      counts: arena<Int32>(n),
+      mesh: wantMesh ? arena<Float>(n * _maxFaces * kFdtMeshFloats) : nullptr,
+      iris: wantIris ? arena<Float>(n * _maxFaces * kFdtIrisFloats) : nullptr,
+    );
+  }
+
+  List<Face> _facesOf(({Pointer<FdtFace> faces, Pointer<Int32> counts, Pointer<Float> mesh, Pointer<Float> iris}) out, int b,
+      int width, int height) {
+    return <Face>[
+      for (int j = 0; j < out.counts[b]; j++)
+        _toFace(out.faces[b * _maxFaces + j], out.mesh, out.iris, b * _maxFaces + j, width, height),
+    ];
+  }
+
   /// The aligned crop getFaceEmbeddingFromEyesDirect feeds the embedding model (face_detector_core.dart:419-452):
   /// computeEmbeddingAlignment on the (iris-refined) eye landmarks, then extractAlignedSquare(..., -theta, outSize).
   /// Returns `outSize * outSize * 3` BGR bytes.

@@ -91,6 +91,19 @@ final class FdtFace extends Struct {
   external int reserved;
 }
 
+/// fdt_frame: one frame of a mixed batch (fdt_detect_frames); 24 bytes.
+final class FdtFrame extends Struct {
+  external Pointer<Uint8> data;
+  @Int32()
+  external int width;
+  @Int32()
+  external int height;
+  @Int32()
+  external int rowStride;
+  @Int32()
+  external int matType;
+}
+
 typedef _DefaultConfigC = Void Function(Pointer<FdtConfig>);
 typedef _DefaultConfigD = void Function(Pointer<FdtConfig>);
 typedef _CreateExC = Int32 Function(Pointer<FdtConfig>, Pointer<Uint8>, Size, Pointer<Uint8>, Size, Pointer<Uint8>, Size,
@@ -124,6 +137,14 @@ typedef _DetectJpegC = Int32 Function(Pointer<Void>, Pointer<Uint8>, Size, Int32
     Pointer<Float>, Pointer<Float>, Pointer<Int32>);
 typedef _DetectJpegD = int Function(Pointer<Void>, Pointer<Uint8>, int, int, Pointer<FdtFace>, Pointer<Int32>,
     Pointer<Float>, Pointer<Float>, Pointer<Int32>);
+typedef _DetectFramesC = Int32 Function(Pointer<Void>, Pointer<FdtFrame>, Int32, Int32, Int32, Pointer<FdtFace>, Pointer<Int32>,
+    Pointer<Float>, Pointer<Float>);
+typedef _DetectFramesD = int Function(Pointer<Void>, Pointer<FdtFrame>, int, int, int, Pointer<FdtFace>, Pointer<Int32>,
+    Pointer<Float>, Pointer<Float>);
+typedef _DetectJpegBatchC = Int32 Function(Pointer<Void>, Pointer<Pointer<Uint8>>, Pointer<Size>, Int32, Int32, Pointer<FdtFace>,
+    Pointer<Int32>, Pointer<Float>, Pointer<Float>, Pointer<Int32>, Pointer<Int32>);
+typedef _DetectJpegBatchD = int Function(Pointer<Void>, Pointer<Pointer<Uint8>>, Pointer<Size>, int, int, Pointer<FdtFace>,
+    Pointer<Int32>, Pointer<Float>, Pointer<Float>, Pointer<Int32>, Pointer<Int32>);
 typedef _NumDevicesC = Int32 Function(Pointer<Void>);
 typedef _NumDevicesD = int Function(Pointer<Void>);
 
@@ -142,6 +163,8 @@ class FdtLibrary {
         extractAlignedSquares = _lib.lookupFunction<_ExtractSquaresC, _ExtractSquaresD>('fdt_extract_aligned_squares'),
         hostEmbeddingRoi = _lib.lookupFunction<_EmbeddingRoiC, _EmbeddingRoiD>('fdt_host_embedding_roi'),
         detectJpeg = _lib.lookupFunction<_DetectJpegC, _DetectJpegD>('fdt_detect_jpeg'),
+        detectFrames = _lib.lookupFunction<_DetectFramesC, _DetectFramesD>('fdt_detect_frames'),
+        detectJpegBatch = _lib.lookupFunction<_DetectJpegBatchC, _DetectJpegBatchD>('fdt_detect_jpeg_batch'),
         numDevices = _lib.lookupFunction<_NumDevicesC, _NumDevicesD>('fdt_num_devices');
 
   final DynamicLibrary _lib;
@@ -157,6 +180,8 @@ class FdtLibrary {
   final _ExtractSquaresD extractAlignedSquares;
   final _EmbeddingRoiD hostEmbeddingRoi;
   final _DetectJpegD detectJpeg;
+  final _DetectFramesD detectFrames;
+  final _DetectJpegBatchD detectJpegBatch;
   final _NumDevicesD numDevices;
 
   static FdtLibrary? _instance;
