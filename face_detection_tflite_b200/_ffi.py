@@ -14,6 +14,10 @@ FDT_MAT_8UC1, FDT_MAT_8UC3, FDT_MAT_8UC4 = 0, 16, 24
 FDT_FMT_YUV_NV12, FDT_FMT_YUV_NV21, FDT_FMT_YUV_I420 = 0x1000, 0x1001, 0x1002   # YUV 4:2:0, height * rowStride * 3 / 2 bytes
 YUV_FORMATS = (FDT_FMT_YUV_NV12, FDT_FMT_YUV_NV21, FDT_FMT_YUV_I420)
 FDT_MEM_HOST, FDT_MEM_DEVICE = 0, 1
+# EXIF orientation of a stored frame (fdt_detect_batch_oriented / fdt_detect_frames_oriented): the upright image is
+# oracle.jpeg_ops.exif_transform(stored, orientation)
+(FDT_ORIENT_UPRIGHT, FDT_ORIENT_MIRROR_H, FDT_ORIENT_ROT180, FDT_ORIENT_MIRROR_V, FDT_ORIENT_TRANSPOSE, FDT_ORIENT_ROT90_CW,
+ FDT_ORIENT_TRANSVERSE, FDT_ORIENT_ROT90_CCW) = range(1, 9)
 FDT_MAX_FACES = 100
 FDT_MESH_FLOATS = 1404
 FDT_IRIS_FLOATS = 456
@@ -52,6 +56,10 @@ SIGNATURES = {
     "fdt_detect_batch": (C.c_int32, [P, P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                      C.POINTER(FdtFace), i32p, f32p, f32p]),
     "fdt_detect_frames": (C.c_int32, [P, C.POINTER(FdtFrame), C.c_int32, C.c_int32, C.c_int32, C.POINTER(FdtFace), i32p, f32p, f32p]),
+    "fdt_detect_batch_oriented": (C.c_int32, [P, P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                              C.c_int32, C.POINTER(FdtFace), i32p, f32p, f32p]),
+    "fdt_detect_frames_oriented": (C.c_int32, [P, C.POINTER(FdtFrame), i32p, C.c_int32, C.c_int32, C.c_int32, C.POINTER(FdtFace),
+                                               i32p, f32p, f32p]),
     "fdt_detect_jpeg_batch": (C.c_int32, [P, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_int32, C.c_int32, C.POINTER(FdtFace),
                                           i32p, f32p, f32p, i32p, i32p]),
     "fdt_detect_one": (C.c_int32, [P, P, C.c_size_t, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(FdtFace), i32p, f32p, f32p]),

@@ -14,6 +14,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <tuple>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -86,19 +87,20 @@ std::vector<double> generate_anchors(const SsdOptions& o) {
 }
 
 struct LbTables {
-  int w = 0, h = 0;
+  int w = 0, h = 0, o = 1;   // stored size, EXIF orientation; lp and the taps are those of the upright image (fdt_detect_batch_oriented)
+  bool transposed = false;   // orientations 5-8: the x taps name stored rows, the y taps stored columns (k_letterbox_tr)
   LetterboxParams lp;
   int *x0 = nullptr, *x1 = nullptr, *y0 = nullptr, *y1 = nullptr;
   short *ax0 = nullptr, *ax1 = nullptr, *by0 = nullptr, *by1 = nullptr;
   bool identity = false;
-  // Sparse upload (host frames, fast mode): INTER_LINEAR only reads the rows y0/y1 name.  When those
+  // Sparse upload (host frames, fast mode): INTER_LINEAR only reads the rows y0/y1 name (x0/x1 when transposed).  When those
   // rows form a periodic pattern (`run` consecutive rows every `period`, e.g. rows 10y+4,10y+5 for
-  // 720 -> 72) a single strided DMA copies just them; y0c/y1c index the compacted frame.
+  // 720 -> 72) a single strided DMA copies just them; y0c/y1c are those row taps renumbered into the compacted frame.
   bool sparse = false;
   int r0 = 0, run = 0, period = 0, rows_c = 0;
   int *y0c = nullptr, *y1c = nullptr;
-  // YUV 4:2:0 frames (even sizes, resizing): chroma rows of y0 / y1 (y / 2), and the same sparse rule applied to the
-  // h / 2 rows of one chroma plane (c_rows_c: compacted rows per plane)
+  // YUV 4:2:0 frames (even sizes, resizing): chroma rows of the row taps (y0 / y1, or x0 / x1 when transposed, halved), and
+  // the same sparse rule applied to the h / 2 rows of one chroma plane (c_rows_c: compacted rows per plane)
   int *cy0 = nullptr, *cy1 = nullptr;
   bool c_sparse = false;
   int c_r0 = 0, c_run = 0, c_period = 0, c_rows_c = 0;
@@ -290,9 +292,23 @@ bool periodic_rows(const std::vector<char>& need, int* first_out, int* run_out, 
   return true;
 }
 
-const LbTables* get_tables(fdt_handle* h, int w, int hh) {
+// EXIF orientation (fdt_detect_batch_oriented): the upright image U = exif_transform(stored, o) is the stored frame transposed
+// for 5-8, then read backwards along U's x axis for 2, 3, 6, 7 and along U's y axis for 3, 4, 7, 8.
+bool orient_transposed(int o) { return o >= 5; }
+bool orient_flips_x(int o) { return o == 2 || o == 3 || o == 6 || o == 7; }
+bool orient_flips_y(int o) { return o == 3 || o == 4 || o == 7 || o == 8; }
+void upright_size(int w, int hh, int o, int* uw, int* uh) {
+  *uw = orient_transposed(o) ? hh : w;
+  *uh = orient_transposed(o) ? w : hh;
+}
+// Folds a flip into one axis' taps: tap i of an axis of n source pixels reads pixel n - 1 - i instead, weights unchanged.
+void fold_flip(int* i0, int* i1, int taps, int n) {
+  for (int i = 0; i < taps; ++i) { i0[i] = n - 1 - i0[i]; i1[i] = n - 1 - i1[i]; }
+}
+
+const LbTables* get_tables(fdt_handle* h, int w, int hh, int o) {
   for (const LbTables& t : h->tables)
-    if (t.w == w && t.h == hh) return &t;
+    if (t.w == w && t.h == hh && t.o == o) return &t;
   // the cache is bounded: a stream of distinct resolutions recycles the oldest entry
   if (h->tables.size() >= 16) {
     LbTables& t = h->tables.front();
@@ -302,38 +318,48 @@ const LbTables* get_tables(fdt_handle* h, int w, int hh) {
     h->tables.erase(h->tables.begin());
   }
   LbTables t;
-  t.w = w; t.h = hh;
-  t.lp = letterbox_params(w, hh, h->det.in_w(), h->det.in_h());
-  t.identity = t.lp.new_w == w && t.lp.new_h == hh;
+  t.w = w; t.h = hh; t.o = o; t.transposed = orient_transposed(o);
+  // U's letterbox and U's taps: the x axis rule for U's x taps even when they address stored rows (the axes clamp differently
+  // at the borders).  Rotated / mirrored frames always take the tap path; at equal sizes it returns the pixels exactly.
+  int uw = 0, uh = 0;
+  upright_size(w, hh, o, &uw, &uh);
+  t.lp = letterbox_params(uw, uh, h->det.in_w(), h->det.in_h());
+  t.identity = o == 1 && t.lp.new_w == w && t.lp.new_h == hh;
   std::vector<int> x0(t.lp.new_w), x1(t.lp.new_w), y0(t.lp.new_h), y1(t.lp.new_h);
   std::vector<short> ax0(t.lp.new_w), ax1(t.lp.new_w), by0(t.lp.new_h), by1(t.lp.new_h);
-  resize_linear_taps(w, t.lp.new_w, true, x0.data(), x1.data(), ax0.data(), ax1.data());
-  resize_linear_taps(hh, t.lp.new_h, false, y0.data(), y1.data(), by0.data(), by1.data());
+  resize_linear_taps(uw, t.lp.new_w, true, x0.data(), x1.data(), ax0.data(), ax1.data());
+  resize_linear_taps(uh, t.lp.new_h, false, y0.data(), y1.data(), by0.data(), by1.data());
+  if (orient_flips_x(o)) fold_flip(x0.data(), x1.data(), t.lp.new_w, uw);
+  if (orient_flips_y(o)) fold_flip(y0.data(), y1.data(), t.lp.new_h, uh);
   t.x0 = dev_upload(x0); t.x1 = dev_upload(x1); t.ax0 = dev_upload(ax0); t.ax1 = dev_upload(ax1);
   t.y0 = dev_upload(y0); t.y1 = dev_upload(y1); t.by0 = dev_upload(by0); t.by1 = dev_upload(by1);
   if (!t.x0 || !t.x1 || !t.ax0 || !t.ax1 || !t.y0 || !t.y1 || !t.by0 || !t.by1) return nullptr;
   if (!t.identity) {
+    // the stored rows the taps read: named by the y taps, or by the x taps of a transposed frame
+    const std::vector<int>& r0v = t.transposed ? x0 : y0;
+    const std::vector<int>& r1v = t.transposed ? x1 : y1;
+    const int nr = (int)r0v.size();
     std::vector<char> need(hh, 0);
-    for (int i = 0; i < t.lp.new_h; ++i) { need[y0[i]] = 1; need[y1[i]] = 1; }
+    for (int i = 0; i < nr; ++i) { need[r0v[i]] = 1; need[r1v[i]] = 1; }
     int first = 0, run = 0, period = 0;
     if (periodic_rows(need, &first, &run, &period)) {
-      std::vector<int> y0c(t.lp.new_h), y1c(t.lp.new_h);
+      std::vector<int> y0c(nr), y1c(nr);
       auto compact = [&](int r) { return (r / period) * run + (r % period - first); };
-      for (int i = 0; i < t.lp.new_h; ++i) { y0c[i] = compact(y0[i]); y1c[i] = compact(y1[i]); }
+      for (int i = 0; i < nr; ++i) { y0c[i] = compact(r0v[i]); y1c[i] = compact(r1v[i]); }
       t.y0c = dev_upload(y0c); t.y1c = dev_upload(y1c);
       if (t.y0c && t.y1c) { t.sparse = true; t.r0 = first; t.run = run; t.period = period; t.rows_c = hh / period * run; }
     }
     if (hh % 2 == 0 && w % 2 == 0) {
       // YUV 4:2:0 chroma rows: the rows of one chroma plane (h / 2 of them) the taps read, same sparse rule
       const int ch = hh / 2;
-      std::vector<int> cy0(t.lp.new_h), cy1(t.lp.new_h);
+      std::vector<int> cy0(nr), cy1(nr);
       std::vector<char> cneed(ch, 0);
-      for (int i = 0; i < t.lp.new_h; ++i) { cy0[i] = y0[i] >> 1; cy1[i] = y1[i] >> 1; cneed[cy0[i]] = 1; cneed[cy1[i]] = 1; }
+      for (int i = 0; i < nr; ++i) { cy0[i] = r0v[i] >> 1; cy1[i] = r1v[i] >> 1; cneed[cy0[i]] = 1; cneed[cy1[i]] = 1; }
       t.cy0 = dev_upload(cy0); t.cy1 = dev_upload(cy1);
       if (!t.cy0 || !t.cy1) return nullptr;
       if (periodic_rows(cneed, &first, &run, &period)) {
         auto compact = [&](int r) { return (r / period) * run + (r % period - first); };
-        for (int i = 0; i < t.lp.new_h; ++i) { cy0[i] = compact(cy0[i]); cy1[i] = compact(cy1[i]); }
+        for (int i = 0; i < nr; ++i) { cy0[i] = compact(cy0[i]); cy1[i] = compact(cy1[i]); }
         t.cy0c = dev_upload(cy0); t.cy1c = dev_upload(cy1);
         if (t.cy0c && t.cy1c) { t.c_sparse = true; t.c_r0 = first; t.c_run = run; t.c_period = period; t.c_rows_c = ch / period * run; }
       }
@@ -380,8 +406,10 @@ void fill_letterbox(LetterboxP& lb, const LbTables* tb, const uint8_t* d_fr, lon
   lb.frames = d_fr; lb.frame_stride = frame_stride; lb.row_stride = row_stride; lb.channels = channels;
   lb.src_w = w; lb.src_h = hh; lb.out = out; lb.dst_w = S_w; lb.dst_h = S_h;
   lb.new_w = tb->lp.new_w; lb.new_h = tb->lp.new_h; lb.pad_top = tb->lp.pad_top; lb.pad_left = tb->lp.pad_left;
-  lb.x0 = tb->x0; lb.x1 = tb->x1; lb.ax0 = tb->ax0; lb.ax1 = tb->ax1;
-  lb.y0 = sparse ? tb->y0c : tb->y0; lb.y1 = sparse ? tb->y1c : tb->y1; lb.by0 = tb->by0; lb.by1 = tb->by1;
+  // a compacted upload renumbers the taps that address rows: the y taps, or the x taps of a transposed frame
+  const bool xs = sparse && tb->transposed, ys = sparse && !tb->transposed;
+  lb.x0 = xs ? tb->y0c : tb->x0; lb.x1 = xs ? tb->y1c : tb->x1; lb.ax0 = tb->ax0; lb.ax1 = tb->ax1;
+  lb.y0 = ys ? tb->y0c : tb->y0; lb.y1 = ys ? tb->y1c : tb->y1; lb.by0 = tb->by0; lb.by1 = tb->by1;
   lb.identity = tb->identity ? 1 : 0;
 }
 
@@ -441,18 +469,21 @@ void fill_decode(DecodeP& d, fdt_handle* h, const Slot& sl, const LbTables* tb, 
   d.pre = nullptr; d.dbg_dec = nullptr; d.skip_roi = 0;
 }
 
-// Letterbox geometry and INTER_LINEAR taps of one frame size, as k_letterbox_multi reads them: x0, x1, ax0, ax1 (new_w each),
-// then y0, y1, by0, by1, cy0, cy1 (new_h each).  Built on the host with resize_linear_taps, like LbTables.
+// Letterbox geometry and INTER_LINEAR taps of one frame size and orientation, as k_letterbox_multi reads them: x0, x1, ax0, ax1
+// (new_w each), then y0, y1, by0, by1, cy0, cy1 (new_h each).  Built on the host with resize_linear_taps for the upright size,
+// flips folded in, like LbTables.
 struct SizeTaps {
   LetterboxParams lp;
   bool identity = false;
   std::vector<int> t;
 };
 
-SizeTaps make_taps(int w, int hh, int S_w, int S_h) {
+SizeTaps make_taps(int sw, int sh, int o, int S_w, int S_h) {
   SizeTaps st;
+  int w = 0, hh = 0;
+  upright_size(sw, sh, o, &w, &hh);
   st.lp = letterbox_params(w, hh, S_w, S_h);
-  st.identity = st.lp.new_w == w && st.lp.new_h == hh;
+  st.identity = o == 1 && st.lp.new_w == w && st.lp.new_h == hh;
   const int nw = st.lp.new_w, nh = st.lp.new_h;
   st.t.resize((size_t)4 * nw + 6 * nh);
   int* x = st.t.data();
@@ -460,7 +491,9 @@ SizeTaps make_taps(int w, int hh, int S_w, int S_h) {
   std::vector<short> a0(std::max(nw, nh)), a1(std::max(nw, nh));
   resize_linear_taps(w, nw, true, x, x + nw, a0.data(), a1.data());
   for (int i = 0; i < nw; ++i) { x[2 * nw + i] = a0[i]; x[3 * nw + i] = a1[i]; }
+  if (orient_flips_x(o)) fold_flip(x, x + nw, nw, w);
   resize_linear_taps(hh, nh, false, y, y + nh, a0.data(), a1.data());
+  if (orient_flips_y(o)) fold_flip(y, y + nh, nh, hh);
   for (int i = 0; i < nh; ++i) { y[2 * nh + i] = a0[i]; y[3 * nh + i] = a1[i]; y[4 * nh + i] = y[i] >> 1; y[5 * nh + i] = y[nh + i] >> 1; }
   return st;
 }
@@ -470,8 +503,10 @@ SizeTaps make_taps(int w, int hh, int S_w, int S_h) {
 // cache on every frame, and each eviction synchronises both slots.
 struct Ragged {
   const fdt_frame* frames = nullptr;
+  const int32_t* orientations = nullptr;   // [n] EXIF 1..8, or null: all upright
   std::vector<FrameLayout> lay;
-  std::map<std::pair<int, int>, SizeTaps> taps;
+  std::map<std::tuple<int, int, int>, SizeTaps> taps;   // (stored width, height, orientation)
+  int orientation(int i) const { return orientations ? orientations[i] : 1; }
 };
 
 struct CallArgs {
@@ -482,22 +517,33 @@ struct CallArgs {
   const LbTables* tb;
   long long frame_stride;
   Ragged* rg = nullptr;                   // mixed call: per-frame sizes and layouts (the uniform fields above are unused)
+  int orientation = 1;                    // EXIF orientation of every frame; w, hh are the stored size, uw, uh the upright one
+  int uw = 0, uh = 0;
 };
 
-// Size of frame i of the call: the mesh and iris stages map their points into it.
+// Upright size of frame i of the call: faces are normalised to it, the mesh and iris stages map their points into it.
 void frame_size(const CallArgs& a, int i, double* w, double* hh) {
-  if (a.rg) { *w = a.rg->frames[i].width; *hh = a.rg->frames[i].height; }
-  else { *w = a.w; *hh = a.hh; }
+  if (a.rg) {
+    int uw = 0, uh = 0;
+    upright_size(a.rg->frames[i].width, a.rg->frames[i].height, a.rg->orientation(i), &uw, &uh);
+    *w = uw; *hh = uh;
+  } else {
+    *w = a.uw; *hh = a.uh;
+  }
 }
 
-// d_desc: a mixed chunk's frame descriptors on the device (the crop warps read the frames through them)
-struct ChunkJob { int off = 0, n = 0; const uint8_t* d_fr = nullptr; const FrameD* d_desc = nullptr; bool active = false; };
+// d_desc: a mixed chunk's frame descriptors on the device (the crop warps read the frames through them); orientation: as
+// WarpP::orientation
+struct ChunkJob {
+  int off = 0, n = 0; const uint8_t* d_fr = nullptr; const FrameD* d_desc = nullptr; bool active = false; int orientation = 1;
+};
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 // A mixed chunk on its slot's stream: host frames go up whole, one copy each at kStageAlign-aligned offsets; then the chunk's
 // blob (frame descriptors, concatenated tap tables, decode geometry) in one copy; then k_letterbox_multi.
-int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, const FrameD** d_desc, const double** d_geom) {
+int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, const FrameD** d_desc, const double** d_geom,
+                 int* orientation) {
   cudaStream_t s = sl.stream;
   Ragged& rg = *a.rg;
   const fdt_frame* fr = rg.frames + off;
@@ -523,17 +569,22 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
   } else {
     for (int i = 0; i < n; ++i) base[i] = fr[i].data;
   }
-  // the chunk's distinct sizes, each with its taps at an offset of the concatenated table
-  std::map<std::pair<int, int>, int> tap_at;
+  // the chunk's distinct sizes and orientations, each with its taps at an offset of the concatenated table
+  std::map<std::tuple<int, int, int>, int> tap_at;
   std::vector<const SizeTaps*> st(n);
   size_t ntaps = 0;
+  bool upright = true, transposed = false;
   for (int i = 0; i < n; ++i) {
-    const std::pair<int, int> key(fr[i].width, fr[i].height);
+    const int o = rg.orientation(off + i);
+    upright = upright && o == 1;
+    transposed = transposed || orient_transposed(o);
+    const std::tuple<int, int, int> key(fr[i].width, fr[i].height, o);
     auto it = rg.taps.find(key);
-    if (it == rg.taps.end()) it = rg.taps.emplace(key, make_taps(key.first, key.second, S_w, S_h)).first;
+    if (it == rg.taps.end()) it = rg.taps.emplace(key, make_taps(fr[i].width, fr[i].height, o, S_w, S_h)).first;
     st[i] = &it->second;
     if (tap_at.emplace(key, (int)ntaps).second) ntaps += it->second.t.size();
   }
+  *orientation = upright ? 1 : 0;
   const size_t taps_at = align_up((size_t)n * sizeof(FrameD), 16), geom_at = align_up(taps_at + ntaps * sizeof(int), 16);
   const size_t bytes = geom_at + (size_t)n * 6 * sizeof(double);
   if (sl.blob_cap < bytes) {
@@ -563,12 +614,15 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
     d.w = fr[i].width; d.h = fr[i].height; d.row_stride = fr[i].row_stride; d.channels = L.channels;
     d.c_row_stride = L.c_row_bytes; d.c_step = L.c_step; d.u_off = L.u_off; d.v_off = L.v_off;
     d.new_w = lp.new_w; d.new_h = lp.new_h; d.pad_top = lp.pad_top; d.pad_left = lp.pad_left; d.identity = st[i]->identity ? 1 : 0;
-    d.tx = tap_at[std::make_pair(d.w, d.h)]; d.ty = d.tx + 4 * lp.new_w;
+    d.orientation = rg.orientation(off + i);
+    d.tx = tap_at[std::make_tuple(d.w, d.h, d.orientation)]; d.ty = d.tx + 4 * lp.new_w;
     // the values fill_decode derives from LbTables, computed the same way
     double* g = geom + 6 * (size_t)i;
     g[0] = (double)lp.pad_top / S_h; g[1] = (double)lp.pad_bottom / S_h;
     g[2] = (double)lp.pad_left / S_w; g[3] = (double)lp.pad_right / S_w;
-    g[4] = d.w; g[5] = d.h;
+    int uw = 0, uh = 0;
+    upright_size(d.w, d.h, d.orientation, &uw, &uh);
+    g[4] = uw; g[5] = uh;
   }
   cudaMemcpyAsync(sl.d_blob, sl.h_blob, bytes, cudaMemcpyHostToDevice, s);
   cudaEventRecord(sl.ev_blob, s);
@@ -577,7 +631,7 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
   StageTimer t(h, 0, s);
   LetterboxMultiP lb;
   lb.fr = *d_desc; lb.taps = reinterpret_cast<const int*>(sl.d_blob + taps_at); lb.out = sl.d_lb; lb.dst_w = S_w; lb.dst_h = S_h;
-  launch_letterbox_multi(lb, n, s);
+  launch_letterbox_multi(lb, n, transposed, s);
   t.launches = 1;
   return FDT_OK;
 }
@@ -647,7 +701,18 @@ int stage_uniform(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, co
   }
   {
     StageTimer t(h, 0, s);
-    if (a.lay.yuv) {
+    if (tb->transposed) {
+      LetterboxTrP lb;
+      lb.yuv = a.lay.yuv ? 1 : 0;
+      if (a.lay.yuv) {
+        if (!d_c) d_c = d_fr + a.lay.c_off;
+        fill_letterbox_yuv(lb.yp, tb, a.lay, d_fr, y_stride, y_sparse, d_c, c_stride, c_sparse, a.row_stride, a.w, a.hh, sl.d_lb, S_w, S_h);
+      } else {
+        lb.yp = LetterboxYuvP();
+        fill_letterbox(lb.yp.lb, tb, d_fr, dev_frame_stride, a.row_stride, a.channels, a.w, a.hh, sl.d_lb, S_w, S_h, sparse);
+      }
+      launch_letterbox_tr(lb, n, s);
+    } else if (a.lay.yuv) {
       if (!d_c) d_c = d_fr + a.lay.c_off;     // whole frames
       LetterboxYuvP lb;
       fill_letterbox_yuv(lb, tb, a.lay, d_fr, y_stride, y_sparse, d_c, c_stride, c_sparse, a.row_stride, a.w, a.hh, sl.d_lb, S_w, S_h);
@@ -668,7 +733,8 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
   const uint8_t* d_fr = nullptr;
   const FrameD* d_desc = nullptr;
   const double* d_geom = nullptr;
-  const int rc = a.rg ? stage_ragged(h, sl, a, off, n, &d_desc, &d_geom) : stage_uniform(h, sl, a, off, n, &d_fr);
+  int orientation = a.orientation;
+  const int rc = a.rg ? stage_ragged(h, sl, a, off, n, &d_desc, &d_geom, &orientation) : stage_uniform(h, sl, a, off, n, &d_fr);
   if (rc != FDT_OK) return rc;
   {
     StageTimer t(h, 1, s);
@@ -677,7 +743,7 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
   {
     StageTimer t(h, 2, s);
     DecodeP d;
-    fill_decode(d, h, sl, a.tb, a.w, a.hh);
+    fill_decode(d, h, sl, a.tb, a.uw, a.uh);
     d.geom = d_geom;
     d.faces = h->d_faces + (size_t)off * h->max_faces; d.counts = h->d_counts + off;
     if (first_chunk) { d.cand_idx = sl.d_cand_idx; d.cand_cap = h->cand_cap; d.cand_n = sl.d_cand_n; }
@@ -697,7 +763,7 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
     cudaMemcpy2DAsync(a.out_faces + (size_t)off * h->max_faces, pitch, h->d_faces + (size_t)off * h->max_faces, pitch, eager, n,
                       cudaMemcpyDeviceToHost, s);
   }
-  job->off = off; job->n = n; job->d_fr = d_fr; job->d_desc = d_desc; job->active = true;
+  job->off = off; job->n = n; job->d_fr = d_fr; job->d_desc = d_desc; job->active = true; job->orientation = orientation;
   return FDT_OK;
 }
 
@@ -764,10 +830,10 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
       StageTimer t(h, 3, s);
       WarpP wp;
       wp.frames = job.d_fr; wp.frame_stride = dev_frame_stride; wp.row_stride = a.row_stride; wp.channels = a.channels;
-      wp.src_w = a.w; wp.src_h = a.hh; wp.crop_img = sl.d_crop_img; wp.affine = sl.d_affine; wp.ncrops = nf;
+      wp.src_w = a.uw; wp.src_h = a.uh; wp.crop_img = sl.d_crop_img; wp.affine = sl.d_affine; wp.ncrops = nf;
       wp.out_size = kMeshInput; wp.flip_odd = 0; wp.crops = sl.d_crops;
       set_warp_layout(wp, a.lay);
-      wp.fr = job.d_desc;
+      wp.fr = job.d_desc; wp.orientation = job.orientation;
       launch_warp_affine(wp, s);
       t.launches = 1;
     }
@@ -847,10 +913,10 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
           StageTimer t(h, 6, s);
           WarpP wp;
           wp.frames = job.d_fr; wp.frame_stride = dev_frame_stride; wp.row_stride = a.row_stride; wp.channels = a.channels;
-          wp.src_w = a.w; wp.src_h = a.hh; wp.crop_img = sl.d_eye_img; wp.affine = sl.d_eye_affine; wp.ncrops = ne;
+          wp.src_w = a.uw; wp.src_h = a.uh; wp.crop_img = sl.d_eye_img; wp.affine = sl.d_eye_affine; wp.ncrops = ne;
           wp.out_size = kIrisInput; wp.flip_odd = 1; wp.crops = sl.d_eye_crops;
           set_warp_layout(wp, a.lay);
-          wp.fr = job.d_desc;
+          wp.fr = job.d_desc; wp.orientation = job.orientation;
           launch_warp_affine(wp, s);
           t.launches = 1;
         }
@@ -869,7 +935,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
           IrisPostP pp;
           pp.contours = sl.iris_ctx.outputs[ci]; pp.contours_istride = ip.out_elems[ci];
           pp.iris = sl.iris_ctx.outputs[ii]; pp.iris_istride = ip.out_elems[ii];
-          pp.roi = sl.d_eye_roi; pp.nfaces = nfi; pp.in_size = kIrisInput; pp.img_w = a.w; pp.img_h = a.hh;
+          pp.roi = sl.d_eye_roi; pp.nfaces = nfi; pp.in_size = kIrisInput; pp.img_w = a.uw; pp.img_h = a.uh;
           if (a.rg) pp.img_wh = sl.d_eye_wh;
           pp.iris_out = sl.d_iris_out; pp.eye_kp = sl.d_eye_kp;
           launch_iris_post(pp, s);
@@ -931,8 +997,9 @@ int run_chunks(fdt_handle* h, const CallArgs& a, const std::vector<int>& bounds)
   return FDT_OK;
 }
 
-int detect_single(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh, int row_stride, int mat_type, int mode,
-                  int mem_kind, fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris, bool keep_on_device) {
+int detect_single(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh, int row_stride, int mat_type, int orientation,
+                  int mode, int mem_kind, fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris,
+                  bool keep_on_device) {
   if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
   if (!frames || batch < 0 || w <= 0 || hh <= 0) return fail(h, FDT_ERR_BAD_ARG, "bad frame arguments");
   FrameLayout lay;
@@ -952,7 +1019,9 @@ int detect_single(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh
   a.lay = lay;
   a.mem_kind = mem_kind; a.out_faces = out_faces; a.out_counts = out_counts; a.out_mesh = out_mesh; a.out_iris = out_iris;
   a.keep_on_device = keep_on_device;
-  a.tb = get_tables(h, w, hh);
+  a.orientation = orientation;
+  upright_size(w, hh, orientation, &a.uw, &a.uh);
+  a.tb = get_tables(h, w, hh, orientation);
   if (!a.tb) return fail(h, FDT_ERR_CUDA, "letterbox table upload failed");
   a.frame_stride = lay.frame_bytes;
   std::vector<int> bounds;
@@ -962,8 +1031,8 @@ int detect_single(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh
 }
 
 // fdt_detect_frames' argument checks, every frame before any work; *lay receives the frames' layouts.
-int check_frames(fdt_handle* h, const fdt_frame* frames, int n, int mode, int mem_kind, const fdt_face* out_faces,
-                 const int32_t* out_counts, std::vector<FrameLayout>* lay) {
+int check_frames(fdt_handle* h, const fdt_frame* frames, const int32_t* orientations, int n, int mode, int mem_kind,
+                 const fdt_face* out_faces, const int32_t* out_counts, std::vector<FrameLayout>* lay) {
   if (n < 0 || (n > 0 && !frames)) return fail(h, FDT_ERR_BAD_ARG, "bad frame list");
   if (mem_kind != FDT_MEM_HOST && mem_kind != FDT_MEM_DEVICE) return fail(h, FDT_ERR_BAD_ARG, "unknown mem_kind");
   if (int rc = check_mode(h, mode)) return rc;
@@ -973,16 +1042,20 @@ int check_frames(fdt_handle* h, const fdt_frame* frames, int n, int mode, int me
     const fdt_frame& f = frames[i];
     const char* msg = "bad frame arguments";
     int rc = (!f.data || f.width <= 0 || f.height <= 0) ? FDT_ERR_BAD_ARG : frame_layout(f.mat_type, f.width, f.height, f.row_stride, &(*lay)[i], &msg);
+    if (rc == FDT_OK && orientations && (orientations[i] < 1 || orientations[i] > 8)) {
+      rc = FDT_ERR_BAD_ARG;
+      msg = "orientation must be an EXIF value 1..8";
+    }
     if (rc != FDT_OK) return fail(h, rc, "frame " + std::to_string(i) + ": " + msg);
   }
   return FDT_OK;
 }
 
-int detect_frames_single(fdt_handle* h, const fdt_frame* frames, int n, int mode, int mem_kind, fdt_face* out_faces,
-                         int32_t* out_counts, float* out_mesh, float* out_iris) {
+int detect_frames_single(fdt_handle* h, const fdt_frame* frames, const int32_t* orientations, int n, int mode, int mem_kind,
+                         fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris) {
   if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
   Ragged rg;
-  if (int rc = check_frames(h, frames, n, mode, mem_kind, out_faces, out_counts, &rg.lay)) return rc;
+  if (int rc = check_frames(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, &rg.lay)) return rc;
   cudaSetDevice(h->cfg.device);
   if (mem_kind == FDT_MEM_DEVICE)
     for (int i = 0; i < n; ++i) {
@@ -998,6 +1071,7 @@ int detect_frames_single(fdt_handle* h, const fdt_frame* frames, int n, int mode
   if (n == 0) return FDT_OK;
   if (!ensure_results(h, n)) return FDT_ERR_CUDA;
   rg.frames = frames;
+  rg.orientations = orientations;
   CallArgs a;
   a.frames = nullptr; a.batch = n; a.w = 0; a.hh = 0; a.row_stride = 0; a.channels = 0; a.mode = mode; a.mem_kind = mem_kind;
   a.out_faces = out_faces; a.out_counts = out_counts; a.out_mesh = out_mesh; a.out_iris = out_iris;
@@ -1039,26 +1113,27 @@ template <typename F> int on_shards(fdt_handle* h, int n, F fn) {
   return FDT_OK;
 }
 
-int detect_frames_multi(fdt_handle* h, const fdt_frame* frames, int n, int mode, int mem_kind, fdt_face* out_faces,
-                        int32_t* out_counts, float* out_mesh, float* out_iris) {
+int detect_frames_multi(fdt_handle* h, const fdt_frame* frames, const int32_t* orientations, int n, int mode, int mem_kind,
+                        fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris) {
   std::vector<FrameLayout> lay;
-  if (int rc = check_frames(h, frames, n, mode, mem_kind, out_faces, out_counts, &lay)) return rc;
+  if (int rc = check_frames(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, &lay)) return rc;
   if (mem_kind != FDT_MEM_HOST) return fail(h, FDT_ERR_UNSUPPORTED, "a multi-device handle takes host frames (device memory belongs to one device)");
   return on_shards(h, n, [=](fdt_handle* sh, int lo, int hi) {
     const size_t mf = (size_t)sh->max_faces;
-    return detect_frames_single(sh, frames + lo, hi - lo, mode, mem_kind, out_faces + lo * mf, out_counts + lo,
+    return detect_frames_single(sh, frames + lo, orientations ? orientations + lo : nullptr, hi - lo, mode, mem_kind,
+                                out_faces + lo * mf, out_counts + lo,
                                 out_mesh ? out_mesh + lo * mf * FDT_MESH_FLOATS : nullptr,
                                 out_iris ? out_iris + lo * mf * FDT_IRIS_FLOATS : nullptr);
   });
 }
 
 // Multi-device handle: contiguous split of the batch, one host thread per replica, results land in frame order.
-int detect_multi(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh, int row_stride, int mat_type, int mode,
-                 int mem_kind, fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris) {
+int detect_multi(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh, int row_stride, int mat_type, int orientation,
+                 int mode, int mem_kind, fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris) {
   if (mem_kind != FDT_MEM_HOST) return fail(h, FDT_ERR_UNSUPPORTED, "a multi-device handle takes host frames (device memory belongs to one device)");
   if (!out_faces || !out_counts) return fail(h, FDT_ERR_BAD_ARG, "null output buffers");
   const int g = (int)h->shards.size();
-  if (batch <= 0 || !frames) return detect_single(h->shards[0], frames, batch, w, hh, row_stride, mat_type, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris, false);
+  if (batch <= 0 || !frames) return detect_single(h->shards[0], frames, batch, w, hh, row_stride, mat_type, orientation, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris, false);
   std::vector<int> rcs(g, FDT_OK);
   std::vector<std::thread> th;
   FrameLayout lay;
@@ -1073,7 +1148,7 @@ int detect_multi(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh,
       fdt_handle* sh = h->shards[r];
       std::lock_guard<std::mutex> gl(sh->mu);
       const int mf = sh->max_faces;
-      rcs[r] = detect_single(sh, frames + (size_t)lo * frame_stride, hi - lo, w, hh, row_stride, mat_type, mode, mem_kind,
+      rcs[r] = detect_single(sh, frames + (size_t)lo * frame_stride, hi - lo, w, hh, row_stride, mat_type, orientation, mode, mem_kind,
                              out_faces + (size_t)lo * mf, out_counts + lo, out_mesh ? out_mesh + (size_t)lo * mf * FDT_MESH_FLOATS : nullptr,
                              out_iris ? out_iris + (size_t)lo * mf * FDT_IRIS_FLOATS : nullptr, false);
     });
@@ -1088,12 +1163,13 @@ int detect_multi(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh,
 }
 
 int detect_impl(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh, int row_stride, int mat_type, int mode,
-                int mem_kind, fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris, bool keep_on_device) {
+                int mem_kind, fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris, bool keep_on_device,
+                int orientation = 1) {
   if (h && !h->shards.empty()) {
     if (keep_on_device) return fail(h, FDT_ERR_UNSUPPORTED, "device-resident results need a single-device handle");
-    return detect_multi(h, frames, batch, w, hh, row_stride, mat_type, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
+    return detect_multi(h, frames, batch, w, hh, row_stride, mat_type, orientation, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
   }
-  return detect_single(h, frames, batch, w, hh, row_stride, mat_type, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris, keep_on_device);
+  return detect_single(h, frames, batch, w, hh, row_stride, mat_type, orientation, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris, keep_on_device);
 }
 
 // the replica debug taps and profiling entries address (replica 0 of a multi-device handle)
@@ -1209,13 +1285,13 @@ int jpeg_batch_single(fdt_handle* h, const uint8_t* const* images, const size_t*
     const size_t i0 = (size_t)idx[0];
     int rc;
     if (idx.back() - idx[0] + 1 == k) {
-      rc = detect_frames_single(h, fr.data(), k, mode, FDT_MEM_DEVICE, out_faces + i0 * mf, out_counts + i0,
+      rc = detect_frames_single(h, fr.data(), nullptr, k, mode, FDT_MEM_DEVICE, out_faces + i0 * mf, out_counts + i0,
                                 out_mesh ? out_mesh + i0 * mf * FDT_MESH_FLOATS : nullptr, out_iris ? out_iris + i0 * mf * FDT_IRIS_FLOATS : nullptr);
     } else {
       tf.resize(k * mf); tc.resize(k);
       if (out_mesh) tm.resize(k * mf * FDT_MESH_FLOATS);
       if (out_iris) ti.resize(k * mf * FDT_IRIS_FLOATS);
-      rc = detect_frames_single(h, fr.data(), k, mode, FDT_MEM_DEVICE, tf.data(), tc.data(), out_mesh ? tm.data() : nullptr,
+      rc = detect_frames_single(h, fr.data(), nullptr, k, mode, FDT_MEM_DEVICE, tf.data(), tc.data(), out_mesh ? tm.data() : nullptr,
                                 out_iris ? ti.data() : nullptr);
       for (int j = 0; j < k && rc == FDT_OK; ++j) {
         const size_t i = (size_t)idx[j], c = (size_t)tc[j];
@@ -1507,9 +1583,18 @@ int32_t fdt_destroy(fdt_handle* h) {
 int32_t fdt_detect_batch(fdt_handle* h, const uint8_t* frames, int32_t batch, int32_t width, int32_t height,
                          int32_t row_stride, int32_t mat_type, int32_t mode, int32_t mem_kind, fdt_face* out_faces,
                          int32_t* out_counts, float* out_mesh, float* out_iris) {
+  return fdt_detect_batch_oriented(h, frames, batch, width, height, row_stride, mat_type, FDT_ORIENT_UPRIGHT, mode, mem_kind,
+                                   out_faces, out_counts, out_mesh, out_iris);
+}
+
+int32_t fdt_detect_batch_oriented(fdt_handle* h, const uint8_t* frames, int32_t batch, int32_t width, int32_t height,
+                                  int32_t row_stride, int32_t mat_type, int32_t orientation, int32_t mode, int32_t mem_kind,
+                                  fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris) {
   if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
   std::lock_guard<std::mutex> g(h->mu);
-  return detect_impl(h, frames, batch, width, height, row_stride, mat_type, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris, false);
+  if (orientation < 1 || orientation > 8) return fail(h, FDT_ERR_BAD_ARG, "orientation must be an EXIF value 1..8");
+  return detect_impl(h, frames, batch, width, height, row_stride, mat_type, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris,
+                     false, orientation);
 }
 
 int32_t fdt_detect_one(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int32_t width, int32_t height, int32_t mat_type,
@@ -1577,7 +1662,7 @@ int32_t fdt_detect_jpeg(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int3
   if (rc == FDT_OK) {
     if (out_wh) { out_wh[0] = w; out_wh[1] = hh; }
     const long long jl = p->jpeg_launches;
-    rc = detect_single(p, p->d_jframe, 1, w, hh, w * 3, FDT_MAT_8UC3, mode, FDT_MEM_DEVICE, out_faces, out_count, out_mesh, out_iris, false);
+    rc = detect_single(p, p->d_jframe, 1, w, hh, w * 3, FDT_MAT_8UC3, 1, mode, FDT_MEM_DEVICE, out_faces, out_count, out_mesh, out_iris, false);
     p->launches += jl;
   }
   if (p != h) { h->err = p->err; h->launches = p->launches; h->h2d_bytes = p->h2d_bytes; }
@@ -1586,10 +1671,15 @@ int32_t fdt_detect_jpeg(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int3
 
 int32_t fdt_detect_frames(fdt_handle* h, const fdt_frame* frames, int32_t n, int32_t mode, int32_t mem_kind, fdt_face* out_faces,
                           int32_t* out_counts, float* out_mesh, float* out_iris) {
+  return fdt_detect_frames_oriented(h, frames, nullptr, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
+}
+
+int32_t fdt_detect_frames_oriented(fdt_handle* h, const fdt_frame* frames, const int32_t* orientations, int32_t n, int32_t mode,
+                                   int32_t mem_kind, fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris) {
   if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
   std::lock_guard<std::mutex> g(h->mu);
-  if (!h->shards.empty()) return detect_frames_multi(h, frames, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
-  return detect_frames_single(h, frames, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
+  if (!h->shards.empty()) return detect_frames_multi(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
+  return detect_frames_single(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
 }
 
 int32_t fdt_detect_jpeg_batch(fdt_handle* h, const uint8_t* const* images, const size_t* sizes, int32_t n, int32_t mode,
@@ -2068,7 +2158,7 @@ int32_t fdt_profile_chunk(fdt_handle* h, const uint8_t* d_frames, int32_t n, int
   if (!out_ms || capacity < S + 2) return fail(h, FDT_ERR_SIZE_MISMATCH, "out_ms too small");
   cudaSetDevice(h->cfg.device);
   if (!ensure_results(h, n)) return FDT_ERR_CUDA;
-  const LbTables* tb = get_tables(h, width, height);
+  const LbTables* tb = get_tables(h, width, height, 1);
   if (!tb) return fail(h, FDT_ERR_CUDA, "letterbox table upload failed");
   std::vector<cudaEvent_t> ev(S + 3);
   for (auto& e : ev) cudaEventCreate(&e);

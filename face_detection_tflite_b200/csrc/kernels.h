@@ -97,6 +97,16 @@ struct LetterboxYuvP {
   const int* cy0; const int* cy1;
 };
 void launch_letterbox_yuv(const LetterboxYuvP& p, int B, cudaStream_t s);
+// Frames stored transposed (EXIF orientations 5-8, see fdt_detect_batch_oriented), k_letterbox_tr: the letterbox of the upright
+// image U.  The tables are U's (x taps from U's width, y taps from U's height, flips folded in on the host), but the x taps,
+// indexed by the output column, name stored ROWS and the y taps, indexed by the output row, stored COLUMNS.  YUV frames (yuv = 1):
+// yp.cy0 / yp.cy1 are the chroma rows of lb.x0 / lb.x1 (indexed by the output column); a chroma byte sits at
+// (column >> 1) * c_step.  (A struct of its own: LetterboxP and LetterboxYuvP keep their layouts.)
+struct LetterboxTrP {
+  LetterboxYuvP yp;
+  int yuv;
+};
+void launch_letterbox_tr(const LetterboxTrP& p, int B, cudaStream_t s);
 // Ragged batches (fdt_detect_frames): one descriptor per frame of a chunk.  It says where the frame's bytes are and how the
 // letterbox maps it; the crop warps read the same table, indexed by WarpP::crop_img.
 struct FrameD {
@@ -107,16 +117,19 @@ struct FrameD {
   int c_row_stride, c_step, u_off, v_off;
   int new_w, new_h, pad_top, pad_left, identity;
   int tx, ty;              // offsets (ints) of the frame's x taps [4][new_w] and y taps [6][new_h] in the chunk's tap table
+  int orientation;         // EXIF 1..8: the upright image is exif_transform(stored frame, orientation); w, h are the stored size
 };
-// k_letterbox_multi: k_letterbox / k_letterbox_yuv per frame.  taps (host-built, resize_linear_taps): per distinct size
-// x0, x1, ax0, ax1 (new_w each), then y0, y1, by0, by1, cy0, cy1 (new_h each; cy = y / 2, read for YUV frames only).
+// k_letterbox_multi: k_letterbox / k_letterbox_yuv per frame.  taps (host-built, resize_linear_taps): per distinct size and
+// orientation x0, x1, ax0, ax1 (new_w each), then y0, y1, by0, by1, cy0, cy1 (new_h each; cy = y / 2, read for YUV frames only),
+// all of the upright image with the flips folded in.  transposed = true launches the variant that also takes frames of
+// orientations 5-8 (their x taps name stored rows, as in k_letterbox_tr); a chunk without such frames runs the plain one.
 struct LetterboxMultiP {
   const FrameD* fr;        // [B]
   const int* taps;
   uint8_t* out;            // [B][S_h][S_w][4] BGRX
   int dst_w, dst_h;
 };
-void launch_letterbox_multi(const LetterboxMultiP& p, int B, cudaStream_t s);
+void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s);
 // u8 [B][S][S][4] BGRX -> f32 [B][S][S][3] RGB, v*(1/127.5)-1
 void launch_normalize(const uint8_t* in, TV out, int B, cudaStream_t s);
 
@@ -325,6 +338,10 @@ struct WarpP {
   int c_row_stride = 0, c_step = 0, u_off = 0, v_off = 0;
   // ragged batches: the frame of crop f is fr[crop_img[f]] (its layout and size replace the fields above); null: uniform
   const FrameD* fr = nullptr;
+  // EXIF orientation of the frames (fdt_detect_batch_oriented): src_w / src_h are then the upright size, and each in-frame tap
+  // of the upright image is mapped to its stored pixel right before the load.  Ragged: 1 when every frame of the chunk is
+  // upright, else 0 (each frame's own FrameD::orientation applies).  Anything but 1 launches the oriented instantiation.
+  int orientation = 1;
 };
 void launch_warp_affine(const WarpP& p, cudaStream_t s);
 

@@ -221,7 +221,10 @@ __device__ __forceinline__ long long sat_round_ll(double v) { return (long long)
 // One thread per output pixel; blockIdx.y = crop.  The per-row / per-column fixed-point terms of
 // imgproc/imgwarp.cpp WarpAffineInvoker (AB_BITS = 10, INTER_BITS = 5) are evaluated per pixel: two f64 rint each.
 // kRagged: the crop's frame, its layout and size come from the descriptor table p.fr (chunks of frames of different sizes).
-template <bool kRagged>
+// kOriented: the frame is stored rotated / mirrored (EXIF orientation, p.orientation or the descriptor's).  Coordinates, weights
+// and bounds are those of the upright image U; only each in-frame tap's address is mapped to the stored pixel (and chroma
+// sample) it is.  Folding the orientation into the affine map instead would change the rint rounding above.
+template <bool kRagged, bool kOriented>
 __global__ void k_warp_affine(WarpP p) {
   const int f = blockIdx.y;
   if (f >= p.ncrops) return;
@@ -231,6 +234,8 @@ __global__ void k_warp_affine(WarpP p) {
   const FrameD* d = kRagged ? p.fr + p.crop_img[f] : nullptr;
   const uint8_t* src = kRagged ? d->y : p.frames + (size_t)p.crop_img[f] * p.frame_stride;
   const bool flip = p.flip_odd && (f & 1);
+  const int orient = kOriented ? (kRagged ? d->orientation : p.orientation) : 1;
+  const bool tr = orient >= 5;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < S * S; i += gridDim.x * blockDim.x) {
     int y = i / S, x = i - y * S;
     long long adelta = sat_round_ll(A[0] * x * 1024.0);
@@ -248,7 +253,16 @@ __global__ void k_warp_affine(WarpP p) {
 #pragma unroll
     for (int t = 0; t < 4; ++t) {
       int yy = sy + (t >> 1), xx = sx + (t & 1);
-      if (yy < 0 || yy >= (kRagged ? d->h : p.src_h) || xx < 0 || xx >= (kRagged ? d->w : p.src_w)) continue;   // out-of-frame taps: BGR 0 (also for YUV frames)
+      // bounds of U: the uniform src_w / src_h already are U's size; a descriptor holds the stored size
+      if (yy < 0 || yy >= (kRagged ? (tr ? d->w : d->h) : p.src_h) || xx < 0 || xx >= (kRagged ? (tr ? d->h : d->w) : p.src_w)) continue;   // out-of-frame taps: BGR 0 (also for YUV frames)
+      if (kOriented) {
+        // U(xx, yy) = stored(column, row): flips first (2, 3, 6, 7 run U's x backwards, 3, 4, 7, 8 its y), then the transpose
+        const int uw = kRagged ? (tr ? d->h : d->w) : p.src_w, uh = kRagged ? (tr ? d->w : d->h) : p.src_h;
+        const int fx = (orient == 2 || orient == 3 || orient == 6 || orient == 7) ? uw - 1 - xx : xx;
+        const int fy = (orient == 3 || orient == 4 || orient == 7 || orient == 8) ? uh - 1 - yy : yy;
+        xx = tr ? fy : fx;
+        yy = tr ? fx : fy;
+      }
       const int row_stride = kRagged ? d->row_stride : p.row_stride;
       if (kRagged ? d->channels == 0 : p.yuv) {
         const uint8_t* c = (kRagged ? d->c : src + p.c_off) + (size_t)(yy >> 1) * (kRagged ? d->c_row_stride : p.c_row_stride) +
@@ -371,8 +385,13 @@ void launch_decode_nms(const DecodeP& p, int B, cudaStream_t s) {
 void launch_warp_affine(const WarpP& p, cudaStream_t s) {
   if (p.ncrops <= 0) return;
   dim3 grid((p.out_size * p.out_size + 255) / 256, p.ncrops);
-  if (p.fr) k_warp_affine<true><<<grid, 256, 0, s>>>(p);
-  else k_warp_affine<false><<<grid, 256, 0, s>>>(p);
+  if (p.orientation != 1) {
+    if (p.fr) k_warp_affine<true, true><<<grid, 256, 0, s>>>(p);
+    else k_warp_affine<false, true><<<grid, 256, 0, s>>>(p);
+  } else {
+    if (p.fr) k_warp_affine<true, false><<<grid, 256, 0, s>>>(p);
+    else k_warp_affine<false, false><<<grid, 256, 0, s>>>(p);
+  }
 }
 
 void launch_mesh_post(const MeshPostP& p, cudaStream_t s) {

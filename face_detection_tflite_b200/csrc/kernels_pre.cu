@@ -1,6 +1,6 @@
 // Preprocessing kernels: fused letterbox (cv::resize INTER_LINEAR 8U fixed point +
 // copyMakeBorder(0) + BGRA/GRAY->BGR, or cvtColor YUV2BGR for NV12 / NV21 / I420 frames; k_letterbox_multi for chunks of
-// frames of different sizes and formats) and the [-1,1] normalisation.
+// frames of different sizes and formats; k_letterbox_tr for frames stored transposed) and the [-1,1] normalisation.
 // Reference: convertImageToTensor / bgrMatToSignedFloat32 (lib/src/util/helpers.dart:303-421).
 #include "kernels.h"
 
@@ -113,9 +113,56 @@ __global__ void __launch_bounds__(256) k_letterbox_yuv(LetterboxYuvP p, int B) {
   }
 }
 
+// Frames stored transposed (orientations 5-8): the grid and fixed-point resize of k_letterbox over the upright image U, whose
+// pixel (x, y) is the stored pixel (row x', column y') - x' from the x taps, y' from the y taps, flips already folded into both.
+// So U's four taps t00 = U(xa, ya), t01 = U(xb, ya), t10 = U(xa, yb), t11 = U(xb, yb) are read from stored rows xa / xb and stored
+// columns ya / yb, and resize_linear weights them exactly as it weights an upright frame's taps: the output bytes are those of
+// letterboxing U itself.  No identity branch: at equal sizes the taps are (i, weight 2048 / 0), which resize_linear returns exactly.
+template <bool kYuv>
+__global__ void __launch_bounds__(256) k_letterbox_tr(LetterboxTrP p, int B) {
+  const LetterboxP& q = p.yp.lb;
+  const int x = blockIdx.x * 64 + (threadIdx.x & 63), y = blockIdx.y * 4 + (threadIdx.x >> 6);
+  if (x >= q.dst_w || y >= q.dst_h) return;
+  for (int b = blockIdx.z; b < B; b += gridDim.z) {
+    const int dy = y - q.pad_top, dx = x - q.pad_left;
+    uchar3 o = make_uchar3(0, 0, 0);
+    if (dy >= 0 && dy < q.new_h && dx >= 0 && dx < q.new_w) {
+      const uint8_t* src = q.frames + (size_t)b * q.frame_stride;
+      const int ra = q.x0[dx], rb = q.x1[dx], wa = q.ax0[dx], wb = q.ax1[dx];   // stored rows, U's x weights
+      const int ca = q.y0[dy], cb = q.y1[dy], va = q.by0[dy], vb = q.by1[dy];   // stored columns, U's y weights
+      int t00[3], t01[3], t10[3], t11[3];
+      const uint8_t* r0 = src + (size_t)ra * q.row_stride;
+      const uint8_t* r1 = src + (size_t)rb * q.row_stride;
+      if (kYuv) {
+        const uint8_t* cs = p.yp.chroma + (size_t)b * p.yp.c_frame_stride;
+        const uint8_t* c0 = cs + (size_t)p.yp.cy0[dx] * p.yp.c_row_stride;
+        const uint8_t* c1 = cs + (size_t)p.yp.cy1[dx] * p.yp.c_row_stride;
+        load_yuv(r0, c0, ca, p.yp, t00);
+        load_yuv(r1, c1, ca, p.yp, t01);
+        load_yuv(r0, c0, cb, p.yp, t10);
+        load_yuv(r1, c1, cb, p.yp, t11);
+      } else {
+        load_bgr(r0 + (size_t)ca * q.channels, q.channels, t00);
+        load_bgr(r1 + (size_t)ca * q.channels, q.channels, t01);
+        load_bgr(r0 + (size_t)cb * q.channels, q.channels, t10);
+        load_bgr(r1 + (size_t)cb * q.channels, q.channels, t11);
+      }
+      int res[3];
+#pragma unroll
+      for (int c = 0; c < 3; ++c) res[c] = resize_linear(t00[c], t01[c], t10[c], t11[c], wa, wb, va, vb);
+      o = make_uchar3((unsigned char)res[0], (unsigned char)res[1], (unsigned char)res[2]);
+    }
+    reinterpret_cast<uchar4*>(q.out)[((size_t)b * q.dst_h + y) * q.dst_w + x] = make_uchar4(o.x, o.y, o.z, 0);
+  }
+}
+
 // Ragged batches: the grid of k_letterbox, one frame per blockIdx.z step, its geometry and layout from a descriptor table.  The
 // format is the same for every thread of a block, so the packed / YUV branch does not diverge; the arithmetic is that of
 // k_letterbox / k_letterbox_yuv, so a frame letterboxes to the same bytes in a ragged chunk as in a uniform one.
+// kTransposed: the chunk also holds frames of orientations 5-8, gathered as in k_letterbox_tr (block-uniform branch; their
+// chroma rows are the stored rows halved, mixed calls upload whole frames).  Orientations 2-4 need nothing here: their flips are
+// folded into the taps.
+template <bool kTransposed>
 __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int B) {
   const int x = blockIdx.x * 64 + (threadIdx.x & 63), y = blockIdx.y * 4 + (threadIdx.x >> 6);
   if (x >= p.dst_w || y >= p.dst_h) return;
@@ -125,7 +172,30 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
     uchar3 o = make_uchar3(0, 0, 0);
     if (dy >= 0 && dy < f.new_h && dx >= 0 && dx < f.new_w) {
       int res[3];
-      if (f.identity) {
+      if (kTransposed && f.orientation >= 5) {
+        const int* tx = p.taps + f.tx;
+        const int* ty = p.taps + f.ty;
+        const int ra = tx[dx], rb = tx[f.new_w + dx], wa = tx[2 * f.new_w + dx], wb = tx[3 * f.new_w + dx];
+        const int ca = ty[dy], cb = ty[f.new_h + dy], va = ty[2 * f.new_h + dy], vb = ty[3 * f.new_h + dy];
+        int t00[3], t01[3], t10[3], t11[3];
+        const uint8_t* r0 = f.y + (size_t)ra * f.row_stride;
+        const uint8_t* r1 = f.y + (size_t)rb * f.row_stride;
+        if (f.channels) {
+          load_bgr(r0 + (size_t)ca * f.channels, f.channels, t00);
+          load_bgr(r1 + (size_t)ca * f.channels, f.channels, t01);
+          load_bgr(r0 + (size_t)cb * f.channels, f.channels, t10);
+          load_bgr(r1 + (size_t)cb * f.channels, f.channels, t11);
+        } else {
+          const uint8_t* c0 = f.c + (size_t)(ra >> 1) * f.c_row_stride;
+          const uint8_t* c1 = f.c + (size_t)(rb >> 1) * f.c_row_stride;
+          load_yuv(r0, c0, ca, f, t00);
+          load_yuv(r1, c1, ca, f, t01);
+          load_yuv(r0, c0, cb, f, t10);
+          load_yuv(r1, c1, cb, f, t11);
+        }
+#pragma unroll
+        for (int c = 0; c < 3; ++c) res[c] = resize_linear(t00[c], t01[c], t10[c], t11[c], wa, wb, va, vb);
+      } else if (f.identity) {
         if (f.channels) load_bgr(f.y + (size_t)dy * f.row_stride + (size_t)dx * f.channels, f.channels, res);
         else load_yuv(f.y + (size_t)dy * f.row_stride, f.c + (size_t)(dy >> 1) * f.c_row_stride, dx, f, res);
       } else {
@@ -186,10 +256,18 @@ void launch_letterbox_yuv(const LetterboxYuvP& p, int B, cudaStream_t s) {
   k_letterbox_yuv<<<grid, 256, 0, s>>>(p, B);
 }
 
-void launch_letterbox_multi(const LetterboxMultiP& p, int B, cudaStream_t s) {
+void launch_letterbox_tr(const LetterboxTrP& p, int B, cudaStream_t s) {
+  if (B <= 0) return;
+  dim3 grid((unsigned)((p.yp.lb.dst_w + 63) / 64), (unsigned)((p.yp.lb.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
+  if (p.yuv) k_letterbox_tr<true><<<grid, 256, 0, s>>>(p, B);
+  else k_letterbox_tr<false><<<grid, 256, 0, s>>>(p, B);
+}
+
+void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s) {
   if (B <= 0) return;
   dim3 grid((unsigned)((p.dst_w + 63) / 64), (unsigned)((p.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
-  k_letterbox_multi<<<grid, 256, 0, s>>>(p, B);
+  if (transposed) k_letterbox_multi<true><<<grid, 256, 0, s>>>(p, B);
+  else k_letterbox_multi<false><<<grid, 256, 0, s>>>(p, B);
 }
 
 void launch_normalize(const uint8_t* in, TV out, int B, cudaStream_t s) {

@@ -79,6 +79,27 @@ def _frame_geometry(i: int, w, h, mt, stride):
     return int(stride), (h * stride * 3 // 2 if yuv else h * stride)
 
 
+def _orientation(o, what: str = "orientation") -> int:
+    """An EXIF orientation 1..8 as an int; ValueError otherwise."""
+    if isinstance(o, bool) or not isinstance(o, (int, np.integer)) or not 1 <= o <= 8:
+        raise ValueError("%s must be an EXIF orientation 1..8, got %r" % (what, o))
+    return int(o)
+
+
+def _orientations(orientations, n: int):
+    """A per-frame orientation list as int32 [n] (None: all upright, passed on as None); ValueError otherwise."""
+    if orientations is None:
+        return None
+    if isinstance(orientations, (str, bytes)) or not hasattr(orientations, "__len__") or len(orientations) != n:
+        raise ValueError("orientations must be a list of one EXIF orientation per frame (%d)" % n)
+    return np.array([_orientation(o, "orientations[%d]" % i) for i, o in enumerate(orientations)], np.int32)
+
+
+def _upright(w, h, orientation) -> tuple:
+    """Size of the upright image of a w x h frame stored in `orientation`: 5-8 swap the axes."""
+    return (h, w) if orientation >= 5 else (w, h)
+
+
 class FaceDetector:
     modelVersion = "1.1.1"   # lib/src/face_detector.dart:54-64
 
@@ -163,10 +184,16 @@ class FaceDetector:
 
     # -- detection ------------------------------------------------------------------------------
     def detectFacesFromMatBytes(self, data, *, width: int, height: int, matType: int = 16,
-                                mode: FaceDetectionMode = FaceDetectionMode.full) -> List[Face]:
+                                mode: FaceDetectionMode = FaceDetectionMode.full, orientation: int = 1) -> List[Face]:
         """detectFacesFromMatBytes (face_detector.dart:588-609); the default mode is `full` like the reference's
         (detector + mesh + iris; the blendshape classifier is outside this path).  matType may also be one of the YUV 4:2:0
-        formats FDT_FMT_YUV_NV12 / _NV21 / _I420: `data` is then width * height * 3 / 2 bytes (cv2's (3H/2) x W Mat)."""
+        formats FDT_FMT_YUV_NV12 / _NV21 / _I420: `data` is then width * height * 3 / 2 bytes (cv2's (3H/2) x W Mat).
+        orientation (EXIF 1..8, FDT_ORIENT_*): the frame is stored rotated / mirrored; width and height are the stored size,
+        the faces are those of the upright image exif_transform(frame, orientation), normalised to its size."""
+        if _orientation(orientation) != 1:
+            self._check()
+            return self.detectFacesBatch(data, count=1, width=width, height=height, matType=matType, mode=mode,
+                                         orientation=orientation)[0]
         self._check()
         buf = np.ascontiguousarray(np.frombuffer(data, np.uint8) if not isinstance(data, np.ndarray) else data.reshape(-1))
         if matType in _ffi.YUV_FORMATS and buf.size != width * height * 3 // 2:
@@ -222,36 +249,44 @@ class FaceDetector:
             _raise(self._lib, self._h, rc)
         return out
 
-    def detectFacesFromMat(self, mat: np.ndarray, *, mode: FaceDetectionMode = FaceDetectionMode.full) -> List[Face]:
-        """detectFacesFromMat (face_detector.dart:559-572): `mat` is an HxW[xC] uint8 array (cv.Mat)."""
+    def detectFacesFromMat(self, mat: np.ndarray, *, mode: FaceDetectionMode = FaceDetectionMode.full,
+                           orientation: int = 1) -> List[Face]:
+        """detectFacesFromMat (face_detector.dart:559-572): `mat` is an HxW[xC] uint8 array (cv.Mat), stored in EXIF
+        `orientation` (see detectFacesFromMatBytes)."""
         ch = 1 if mat.ndim == 2 else mat.shape[2]
         mt = {1: _ffi.FDT_MAT_8UC1, 3: _ffi.FDT_MAT_8UC3, 4: _ffi.FDT_MAT_8UC4}.get(ch)
         if mt is None or mat.dtype != np.uint8:
             raise ValueError("unsupported Mat type")
         return self.detectFacesFromMatBytes(np.ascontiguousarray(mat), width=mat.shape[1], height=mat.shape[0],
-                                            matType=mt, mode=mode)
+                                            matType=mt, mode=mode, orientation=orientation)
 
     def detectFacesBatch(self, frames, *, count: int, width: int, height: int, matType: int = 16,
-                         mode: FaceDetectionMode = FaceDetectionMode.fast) -> List[List[Face]]:
+                         mode: FaceDetectionMode = FaceDetectionMode.fast, orientation: int = 1) -> List[List[Face]]:
         """New batched entry point: `frames` holds `count` packed frames (bytes / uint8 array), or `count` YUV 4:2:0 frames of
-        width * height * 3 / 2 bytes with matType FDT_FMT_YUV_NV12 / _NV21 / _I420."""
+        width * height * 3 / 2 bytes with matType FDT_FMT_YUV_NV12 / _NV21 / _I420.  orientation: EXIF 1..8 of every frame
+        (see detectBatchRaw); the faces refer to the upright image."""
+        uw, uh = _upright(width, height, _orientation(orientation))
         self._check()
         faces, counts, mesh, iris = self.detectBatchRaw(frames, count=count, width=width, height=height,
-                                                        matType=matType, mode=mode, withIris=True)
+                                                        matType=matType, mode=mode, withIris=True, orientation=orientation)
         out = []
         for b in range(count):
-            out.append([self._to_face(faces[b * self._max_faces + j], mesh[b, j] if mesh is not None else None, width, height,
+            out.append([self._to_face(faces[b * self._max_faces + j], mesh[b, j] if mesh is not None else None, uw, uh,
                                       iris[b, j] if iris is not None else None)
                         for j in range(int(counts[b]))])
         return out
 
     def detectBatchRaw(self, frames, *, count: int, width: int, height: int, matType: int = 16,
                        mode: FaceDetectionMode = FaceDetectionMode.fast, memKind: int = _ffi.FDT_MEM_HOST,
-                       rowStride: Optional[int] = None, withIris: bool = False):
+                       rowStride: Optional[int] = None, withIris: bool = False, orientation: int = 1):
         """fdt_detect_batch with array outputs: (FdtFace array, counts int32[count], mesh f32 or None) and, with
         withIris=True, a fourth element iris f32 [count, max_faces, 152, 3] (None unless mode is full).
         `frames` may be a numpy array / bytes (host) or an integer device pointer with memKind=FDT_MEM_DEVICE.
-        YUV 4:2:0 formats: rowStride is the Y-plane stride (default: width) and a frame is height * rowStride * 3 / 2 bytes."""
+        YUV 4:2:0 formats: rowStride is the Y-plane stride (default: width) and a frame is height * rowStride * 3 / 2 bytes.
+        orientation (EXIF 1..8, FDT_ORIENT_*; fdt_detect_batch_oriented): every frame is stored rotated / mirrored.  width,
+        height and rowStride describe the stored frames; faces are normalised to the upright image exif_transform(frame,
+        orientation) and mesh / iris points are in its pixels."""
+        orientation = _orientation(orientation)
         self._check()
         yuv = matType in _ffi.YUV_FORMATS
         ch = 1 if yuv else {_ffi.FDT_MAT_8UC1: 1, _ffi.FDT_MAT_8UC3: 3, _ffi.FDT_MAT_8UC4: 4}.get(matType, 0)
@@ -271,19 +306,26 @@ class FaceDetector:
         want_iris = mode == FaceDetectionMode.full
         mesh = np.zeros((count, self._max_faces, 468, 3), np.float32) if want_mesh else None
         iris = np.zeros((count, self._max_faces, 152, 3), np.float32) if want_iris else None
-        rc = self._lib.fdt_detect_batch(self._h, ptr, count, width, height, stride, matType, int(mode), memKind, faces,
-                                        counts.ctypes.data_as(_ffi.i32p),
-                                        mesh.ctypes.data_as(_ffi.f32p) if want_mesh else None,
-                                        iris.ctypes.data_as(_ffi.f32p) if want_iris else None)
+        outs = (faces, counts.ctypes.data_as(_ffi.i32p), mesh.ctypes.data_as(_ffi.f32p) if want_mesh else None,
+                iris.ctypes.data_as(_ffi.f32p) if want_iris else None)
+        if orientation == 1:
+            rc = self._lib.fdt_detect_batch(self._h, ptr, count, width, height, stride, matType, int(mode), memKind, *outs)
+        else:
+            rc = self._lib.fdt_detect_batch_oriented(self._h, ptr, count, width, height, stride, matType, orientation, int(mode),
+                                                     memKind, *outs)
         if rc != _ffi.FDT_OK:
             _raise(self._lib, self._h, rc)
         return (faces, counts[:count], mesh, iris) if withIris else (faces, counts[:count], mesh)
 
     # -- mixed batches: frames of different sizes and formats, and encoded images, in one call ----------------------------
-    def detectFacesFromMats(self, mats, *, mode: FaceDetectionMode = FaceDetectionMode.full) -> List[List[Face]]:
+    def detectFacesFromMats(self, mats, *, mode: FaceDetectionMode = FaceDetectionMode.full,
+                            orientations=None) -> List[List[Face]]:
         """detectFacesFromMat over a list of HxW / HxWx3 / HxWx4 uint8 arrays of any sizes, in one batched call
         (fdt_detect_frames).  A row-padded view (e.g. a crop of a larger array) goes in uncopied with strides[0] as its row
-        stride.  Returns one list of faces per mat, each normalised to its own mat."""
+        stride.  Returns one list of faces per mat, each normalised to its own mat.  orientations: one EXIF orientation 1..8
+        per mat (fdt_detect_frames_oriented), or None for all upright; faces then refer to each mat's upright image."""
+        mats = list(mats)
+        orients = _orientations(orientations, len(mats))
         frames, keep = [], []
         for i, m in enumerate(mats):
             mt = _mat_type(m, i)
@@ -293,17 +335,22 @@ class FaceDetector:
             keep.append(m)
             frames.append((m.ctypes.data, m.shape[1], m.shape[0], m.strides[0], mt))
         self._check()
-        faces, counts, mesh, iris = self._detect_frames(frames, mode, _ffi.FDT_MEM_HOST)
-        return self._faces_per_frame(faces, counts, mesh, iris, [(f[1], f[2]) for f in frames])
+        faces, counts, mesh, iris = self._detect_frames(frames, mode, _ffi.FDT_MEM_HOST, orients)
+        sizes = [_upright(f[1], f[2], 1 if orients is None else orients[i]) for i, f in enumerate(frames)]
+        return self._faces_per_frame(faces, counts, mesh, iris, sizes)
 
-    def detectFramesRaw(self, frames, *, mode: FaceDetectionMode = FaceDetectionMode.fast, memKind: int = _ffi.FDT_MEM_HOST):
+    def detectFramesRaw(self, frames, *, mode: FaceDetectionMode = FaceDetectionMode.fast, memKind: int = _ffi.FDT_MEM_HOST,
+                        orientations=None):
         """fdt_detect_frames with array outputs.  `frames` is a list of (data, width, height, matType[, rowStride]) tuples: data
         is a numpy array / bytes of exactly height * rowStride bytes (YUV 4:2:0: height * rowStride * 3 / 2), or an integer
         device pointer with memKind=FDT_MEM_DEVICE.  rowStride defaults to width * channels (YUV: width).  Returns
         (FdtFace array [n * max_faces], counts int32 [n], mesh f32 [n, max_faces, 468, 3] or None,
-        iris f32 [n, max_faces, 152, 3] or None)."""
+        iris f32 [n, max_faces, 152, 3] or None).  orientations: one EXIF orientation 1..8 per frame
+        (fdt_detect_frames_oriented; results refer to each frame's upright image), or None for all upright."""
         if memKind not in (_ffi.FDT_MEM_HOST, _ffi.FDT_MEM_DEVICE):
             raise ValueError("memKind must be FDT_MEM_HOST or FDT_MEM_DEVICE")
+        frames = list(frames)
+        orients = _orientations(orientations, len(frames))
         descs, keep = [], []
         for i, fr in enumerate(frames):
             if not isinstance(fr, (tuple, list)) or len(fr) not in (4, 5):
@@ -324,7 +371,7 @@ class FaceDetector:
                 ptr = buf.ctypes.data
             descs.append((ptr, w, h, stride, mt))
         self._check()
-        return self._detect_frames(descs, mode, memKind)
+        return self._detect_frames(descs, mode, memKind, orients)
 
     def detectFacesFromBytesBatch(self, images, *, mode: FaceDetectionMode = FaceDetectionMode.full) -> List[Optional[List[Face]]]:
         """detectFacesFromBytes over a list of encoded images (JPEG) in one call (fdt_detect_jpeg_batch).  An image that
@@ -364,13 +411,17 @@ class FaceDetector:
         iris = np.zeros((n, self._max_faces, 152, 3), np.float32) if mode == FaceDetectionMode.full else None
         return faces, counts, mesh, iris
 
-    def _detect_frames(self, descs, mode, memKind):
+    def _detect_frames(self, descs, mode, memKind, orients=None):
         n = len(descs)
         arr = (_ffi.FdtFrame * max(1, n))(*[_ffi.FdtFrame(*d) for d in descs])   # (data, width, height, row_stride, mat_type)
         faces, counts, mesh, iris = self._outputs(n, mode)
-        rc = self._lib.fdt_detect_frames(self._h, arr, n, int(FaceDetectionMode(mode)), memKind, faces, counts.ctypes.data_as(_ffi.i32p),
-                                         mesh.ctypes.data_as(_ffi.f32p) if mesh is not None else None,
-                                         iris.ctypes.data_as(_ffi.f32p) if iris is not None else None)
+        outs = (faces, counts.ctypes.data_as(_ffi.i32p), mesh.ctypes.data_as(_ffi.f32p) if mesh is not None else None,
+                iris.ctypes.data_as(_ffi.f32p) if iris is not None else None)
+        if orients is None:
+            rc = self._lib.fdt_detect_frames(self._h, arr, n, int(FaceDetectionMode(mode)), memKind, *outs)
+        else:
+            rc = self._lib.fdt_detect_frames_oriented(self._h, arr, orients.ctypes.data_as(_ffi.i32p), n,
+                                                      int(FaceDetectionMode(mode)), memKind, *outs)
         if rc != _ffi.FDT_OK:
             _raise(self._lib, self._h, rc)
         return faces, counts[:n], mesh, iris

@@ -86,6 +86,20 @@ enum { FDT_FMT_YUV_NV12 = 0x1000, FDT_FMT_YUV_NV21 = 0x1001, FDT_FMT_YUV_I420 = 
 
 enum { FDT_MEM_HOST = 0, FDT_MEM_DEVICE = 1 };
 
+/* Frame orientation (fdt_detect_batch_oriented, fdt_detect_frames_oriented): the EXIF Orientation value of the STORED frame,
+ * meaning what OpenCV's ExifTransform and fdt_detect_jpeg apply.  The upright image U is the stored frame transformed:
+ *   1 as stored              2 mirrored left-right      3 rotated 180 degrees              4 mirrored top-bottom
+ *   5 transposed (U[r][c] = stored[c][r])              6 rotated 90 degrees clockwise
+ *   7 transverse (U[r][c] = stored[H-1-c][W-1-r])      8 rotated 90 degrees counter-clockwise
+ * For orientations 5-8 U's width is the stored height.
+ * Camera callers: a frame that must be rotated R degrees clockwise to display upright (Android's rotationDegrees, a video
+ * stream's display rotation) has orientation 1, 6, 3, 8 for R = 0, 90, 180, 270.  A frame that must be rotated R degrees
+ * clockwise and THEN mirrored left-right (a front camera preview) has 2, 5, 4, 7 for R = 0, 90, 180, 270. */
+enum {
+  FDT_ORIENT_UPRIGHT = 1, FDT_ORIENT_MIRROR_H = 2, FDT_ORIENT_ROT180 = 3, FDT_ORIENT_MIRROR_V = 4,
+  FDT_ORIENT_TRANSPOSE = 5, FDT_ORIENT_ROT90_CW = 6, FDT_ORIENT_TRANSVERSE = 7, FDT_ORIENT_ROT90_CCW = 8
+};
+
 enum { FDT_MAX_FACES = 100 };      /* weightedNms maxDet, lib/src/util/helpers.dart:187 */
 enum { FDT_MESH_POINTS = 468, FDT_MESH_FLOATS = 1404 };
 enum { FDT_IRIS_POINTS = 152, FDT_IRIS_FLOATS = 456 }; /* 76 per eye: 71 contour + 5 iris (face_detector.dart:1888-1893) */
@@ -177,6 +191,24 @@ typedef struct fdt_frame {
  * fdt_detect_batch would return for it, and fdt_last_error names its index.  n == 0 returns FDT_OK. */
 FDT_EXPORT int32_t fdt_detect_frames(fdt_handle* h, const fdt_frame* frames, int32_t n, int32_t mode, int32_t mem_kind,
                                      fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris);
+
+/* Rotated and mirrored frames (video coded sideways, sensor-orientation camera frames, decoded photos with an EXIF tag) without a
+ * rotation pass: fdt_detect_batch / fdt_detect_frames on frames stored in one of the eight FDT_ORIENT_* orientations.  width,
+ * height, row_stride and mat_type (and every fdt_frame field) describe the STORED frame and are checked as before; YUV frames need
+ * an even stored size.  Every result refers to the upright image U: faces are normalised to U's width and height, mesh and iris
+ * points are in U's pixels, and the letterbox tap shows U letterboxed.  Results are bitwise those of the same call on U itself.
+ * The letterbox and crop kernels read each stored pixel where U's tap falls; no rotated copy is made, and the kernel launch count
+ * is that of orientation 1.  An orientation outside 1..8 returns FDT_ERR_BAD_ARG before any work (fdt_detect_frames_oriented:
+ * fdt_last_error names the first bad index).  orientations: int32 [n], or NULL for all FDT_ORIENT_UPRIGHT.  fdt_detect_batch
+ * is fdt_detect_batch_oriented with FDT_ORIENT_UPRIGHT, fdt_detect_frames is fdt_detect_frames_oriented with NULL.
+ * Multi-device handles split the frames (and the orientations with them) contiguously, as the plain calls do. */
+FDT_EXPORT int32_t fdt_detect_batch_oriented(fdt_handle* h, const uint8_t* frames, int32_t batch, int32_t width,
+                                             int32_t height, int32_t row_stride, int32_t mat_type, int32_t orientation,
+                                             int32_t mode, int32_t mem_kind, fdt_face* out_faces, int32_t* out_counts,
+                                             float* out_mesh, float* out_iris);
+FDT_EXPORT int32_t fdt_detect_frames_oriented(fdt_handle* h, const fdt_frame* frames, const int32_t* orientations, int32_t n,
+                                              int32_t mode, int32_t mem_kind, fdt_face* out_faces, int32_t* out_counts,
+                                              float* out_mesh, float* out_iris);
 
 /* fdt_detect_jpeg over n encoded images in one call.  The host parses and Huffman-decodes them on a pool of
  * min(n, hardware threads) threads; the device decodes them into a handle-owned frame arena and detects them as one mixed
@@ -280,7 +312,11 @@ FDT_EXPORT int64_t fdt_last_launch_count(fdt_handle* h);
 /* Bytes copied host->device by the last detect call.  In fast mode only the source rows the
  * INTER_LINEAR taps read are uploaded when they form a periodic pattern (e.g. 2 of every 10 rows
  * for 720 -> 72), so this can be far below batch * frame size.  YUV frames: the same rule applies to the Y plane
- * and to the chroma plane(s) independently (720 -> 72: Y rows 10k+4, 10k+5 and chroma rows 5k+2). */
+ * and to the chroma plane(s) independently (720 -> 72: Y rows 10k+4, 10k+5 and chroma rows 5k+2).
+ * Oriented frames (fdt_detect_batch_oriented): the rule is "the stored rows the upright image's taps read" - U's y taps for
+ * orientations 1-4, U's x taps for 5-8 (a 1280x720 frame stored sideways still uploads 2 rows in 10), after the flips.  The two
+ * axes clamp differently at the borders, so at some sizes that set differs from orientation 1's.  Mixed calls upload whole
+ * frames. */
 FDT_EXPORT int64_t fdt_last_h2d_bytes(fdt_handle* h);
 /* Device time in ms of the named stage summed over the last call when stage timing was enabled
  * with fdt_set_stage_timing(h,1) (adds cudaEvent records; off by default).

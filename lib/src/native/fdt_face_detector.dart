@@ -110,6 +110,13 @@ class FdtFaceDetector {
     }
   }
 
+  /// An EXIF orientation (kFdtOrient*) must be 1..8; checked before any library call.
+  static void _checkOrientation(int orientation) {
+    if (orientation < 1 || orientation > 8) {
+      throw ArgumentError.value(orientation, 'orientation', 'must be an EXIF orientation 1..8');
+    }
+  }
+
   void _check() {
     if (_h == nullptr) {
       throw StateError('FaceDetector not initialized. Call initialize() first.'); // :1083-1089
@@ -123,7 +130,14 @@ class FdtFaceDetector {
     required int height,
     int matType = 16,
     FaceDetectionMode mode = FaceDetectionMode.full,
+    int orientation = kFdtOrientUpright,
   }) async {
+    _checkOrientation(orientation);
+    if (orientation != kFdtOrientUpright) {
+      // a stored-rotated frame: fdt_detect_batch_oriented with one frame; faces refer to the upright image
+      return (await detectFacesBatch(bytes, count: 1, width: width, height: height, matType: matType, mode: mode,
+          orientation: orientation))[0];
+    }
     _check();
     final arena = Arena();
     try {
@@ -177,7 +191,8 @@ class FdtFaceDetector {
 
   /// New batched entry point: [frames] holds [count] packed frames (count * height * width * channels bytes), or [count]
   /// YUV 4:2:0 frames of width * height * 3 / 2 bytes with matType kFdtFmtYuvNv12 / kFdtFmtYuvNv21 / kFdtFmtYuvI420.
-  /// One `fdt_detect_batch` call; results come back in frame order.  For sustained throughput keep the frames in a
+  /// One `fdt_detect_batch` call; results come back in frame order.  [orientation]: the EXIF orientation (kFdtOrient*) every
+  /// frame is stored in (`fdt_detect_batch_oriented`); width / height are the stored size, faces refer to the upright image.  For sustained throughput keep the frames in a
   /// buffer from `fdt_alloc_pinned` (see [FdtPinnedFrames]) so the upload runs at PCIe speed.
   Future<List<List<Face>>> detectFacesBatch(
     Uint8List frames, {
@@ -186,7 +201,9 @@ class FdtFaceDetector {
     required int height,
     int matType = 16,
     FaceDetectionMode mode = FaceDetectionMode.fast,
+    int orientation = kFdtOrientUpright,
   }) async {
+    _checkOrientation(orientation);
     _check();
     final int frameBytes = fdtFrameBytes(matType, width, height);
     if (frames.length != count * frameBytes) {
@@ -197,7 +214,7 @@ class FdtFaceDetector {
     try {
       final Pointer<Uint8> src = arena<Uint8>(frames.length);
       src.asTypedList(frames.length).setAll(0, frames);
-      return _detectBatchPtr(arena, src, count, width, height, fdtRowStride(matType, width), matType, mode);
+      return _detectBatchPtr(arena, src, count, width, height, fdtRowStride(matType, width), matType, mode, orientation);
     } finally {
       arena.releaseAll();
     }
@@ -211,37 +228,44 @@ class FdtFaceDetector {
     required int height,
     int matType = 16,
     FaceDetectionMode mode = FaceDetectionMode.fast,
+    int orientation = kFdtOrientUpright,
   }) async {
+    _checkOrientation(orientation);
     _check();
     if (count * fdtFrameBytes(matType, width, height) > frames.lengthInBytes) {
       throw ArgumentError('pinned buffer smaller than count * frame size');
     }
     final arena = Arena();
     try {
-      return _detectBatchPtr(arena, frames.pointer, count, width, height, fdtRowStride(matType, width), matType, mode);
+      return _detectBatchPtr(
+          arena, frames.pointer, count, width, height, fdtRowStride(matType, width), matType, mode, orientation);
     } finally {
       arena.releaseAll();
     }
   }
 
   List<List<Face>> _detectBatchPtr(Arena arena, Pointer<Uint8> src, int count, int width, int height, int rowStride,
-      int matType, FaceDetectionMode mode) {
+      int matType, FaceDetectionMode mode, int orientation) {
     final Pointer<FdtFace> faces = arena<FdtFace>(count * _maxFaces);
     final Pointer<Int32> counts = arena<Int32>(count);
     final bool wantMesh = mode != FaceDetectionMode.fast;
     final bool wantIris = mode == FaceDetectionMode.full;
     final Pointer<Float> mesh = wantMesh ? arena<Float>(count * _maxFaces * kFdtMeshFloats) : nullptr;
     final Pointer<Float> iris = wantIris ? arena<Float>(count * _maxFaces * kFdtIrisFloats) : nullptr;
-    final int rc = _lib.detectBatch(
-        _h, src, count, width, height, rowStride, matType, mode.index, kFdtMemHost, faces, counts, mesh, iris);
+    final int rc = orientation == kFdtOrientUpright
+        ? _lib.detectBatch(_h, src, count, width, height, rowStride, matType, mode.index, kFdtMemHost, faces, counts, mesh, iris)
+        : _lib.detectBatchOriented(
+            _h, src, count, width, height, rowStride, matType, orientation, mode.index, kFdtMemHost, faces, counts, mesh, iris);
     if (rc != FdtStatus.ok) {
       _lib.throwFor(rc, _h);
     }
+    // faces are normalised to the upright image: orientations 5-8 swap its axes
+    final int uw = orientation >= 5 ? height : width, uh = orientation >= 5 ? width : height;
     final List<List<Face>> out = <List<Face>>[];
     for (int b = 0; b < count; b++) {
       final int n = counts[b];
       out.add(<Face>[
-        for (int j = 0; j < n; j++) _toFace(faces[b * _maxFaces + j], mesh, iris, b * _maxFaces + j, width, height),
+        for (int j = 0; j < n; j++) _toFace(faces[b * _maxFaces + j], mesh, iris, b * _maxFaces + j, uw, uh),
       ]);
     }
     return out;
@@ -249,11 +273,19 @@ class FdtFaceDetector {
 
   /// detectFacesFromMat over a list of frames of any sizes and formats (photos, mixed camera feeds) in one batched
   /// `fdt_detect_frames` call.  Each mat is packed bytes of its own width, height and matType (kFdtFmtYuv* included);
-  /// each result list is normalised to its own mat.
+  /// each result list is normalised to its own mat.  [orientations]: one EXIF orientation (kFdtOrient*) per mat, or null
+  /// for all upright (`fdt_detect_frames_oriented`); each result list then refers to its mat's upright image.
   Future<List<List<Face>>> detectFacesFromMats(
     List<({Uint8List bytes, int width, int height, int matType})> mats, {
     FaceDetectionMode mode = FaceDetectionMode.full,
+    List<int>? orientations,
   }) async {
+    if (orientations != null) {
+      if (orientations.length != mats.length) {
+        throw ArgumentError('orientations: one EXIF orientation per mat (${mats.length})');
+      }
+      orientations.forEach(_checkOrientation);
+    }
     _check();
     for (int i = 0; i < mats.length; i++) {
       final m = mats[i];
@@ -277,11 +309,23 @@ class FdtFaceDetector {
         frames[i].matType = m.matType;
       }
       final out = _outputs(arena, n, mode);
-      final int rc = _lib.detectFrames(_h, frames, n, mode.index, kFdtMemHost, out.faces, out.counts, out.mesh, out.iris);
+      final int rc;
+      if (orientations == null) {
+        rc = _lib.detectFrames(_h, frames, n, mode.index, kFdtMemHost, out.faces, out.counts, out.mesh, out.iris);
+      } else {
+        final Pointer<Int32> ors = arena<Int32>(n);
+        ors.asTypedList(n).setAll(0, orientations);
+        rc = _lib.detectFramesOriented(_h, frames, ors, n, mode.index, kFdtMemHost, out.faces, out.counts, out.mesh, out.iris);
+      }
       if (rc != FdtStatus.ok) {
         _lib.throwFor(rc, _h); // ArgumentError naming the first bad mat
       }
-      return <List<Face>>[for (int b = 0; b < n; b++) _facesOf(out, b, mats[b].width, mats[b].height)];
+      return <List<Face>>[
+        for (int b = 0; b < n; b++)
+          (orientations != null && orientations[b] >= 5)
+              ? _facesOf(out, b, mats[b].height, mats[b].width)
+              : _facesOf(out, b, mats[b].width, mats[b].height),
+      ];
     } finally {
       arena.releaseAll();
     }

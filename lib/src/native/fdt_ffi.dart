@@ -36,6 +36,19 @@ const int kFdtFmtYuvNv12 = 0x1000;
 const int kFdtFmtYuvNv21 = 0x1001;
 const int kFdtFmtYuvI420 = 0x1002;
 
+/// Frame orientations (fdt_api.h FDT_ORIENT_*): the EXIF Orientation value of a stored frame, as OpenCV's ExifTransform
+/// applies it.  Results of the oriented calls refer to the upright image; for 5-8 its width is the stored height.  Camera
+/// frames that must be rotated R degrees clockwise to display: 1, 6, 3, 8 for R = 0, 90, 180, 270; rotated R degrees clockwise
+/// and then mirrored left-right: 2, 5, 4, 7.
+const int kFdtOrientUpright = 1;
+const int kFdtOrientMirrorH = 2;
+const int kFdtOrientRot180 = 3;
+const int kFdtOrientMirrorV = 4;
+const int kFdtOrientTranspose = 5;
+const int kFdtOrientRot90Cw = 6;
+const int kFdtOrientTransverse = 7;
+const int kFdtOrientRot90Ccw = 8;
+
 bool fdtIsYuv(int matType) => matType == kFdtFmtYuvNv12 || matType == kFdtFmtYuvNv21 || matType == kFdtFmtYuvI420;
 
 /// Row stride (Y-plane stride for the YUV formats) and size in bytes of one tightly packed frame of [matType].
@@ -141,6 +154,14 @@ typedef _DetectFramesC = Int32 Function(Pointer<Void>, Pointer<FdtFrame>, Int32,
     Pointer<Float>, Pointer<Float>);
 typedef _DetectFramesD = int Function(Pointer<Void>, Pointer<FdtFrame>, int, int, int, Pointer<FdtFace>, Pointer<Int32>,
     Pointer<Float>, Pointer<Float>);
+typedef _DetectBatchOrientedC = Int32 Function(Pointer<Void>, Pointer<Uint8>, Int32, Int32, Int32, Int32, Int32, Int32, Int32,
+    Int32, Pointer<FdtFace>, Pointer<Int32>, Pointer<Float>, Pointer<Float>);
+typedef _DetectBatchOrientedD = int Function(Pointer<Void>, Pointer<Uint8>, int, int, int, int, int, int, int, int,
+    Pointer<FdtFace>, Pointer<Int32>, Pointer<Float>, Pointer<Float>);
+typedef _DetectFramesOrientedC = Int32 Function(Pointer<Void>, Pointer<FdtFrame>, Pointer<Int32>, Int32, Int32, Int32,
+    Pointer<FdtFace>, Pointer<Int32>, Pointer<Float>, Pointer<Float>);
+typedef _DetectFramesOrientedD = int Function(Pointer<Void>, Pointer<FdtFrame>, Pointer<Int32>, int, int, int, Pointer<FdtFace>,
+    Pointer<Int32>, Pointer<Float>, Pointer<Float>);
 typedef _DetectJpegBatchC = Int32 Function(Pointer<Void>, Pointer<Pointer<Uint8>>, Pointer<Size>, Int32, Int32, Pointer<FdtFace>,
     Pointer<Int32>, Pointer<Float>, Pointer<Float>, Pointer<Int32>, Pointer<Int32>);
 typedef _DetectJpegBatchD = int Function(Pointer<Void>, Pointer<Pointer<Uint8>>, Pointer<Size>, int, int, Pointer<FdtFace>,
@@ -164,6 +185,8 @@ class FdtLibrary {
         hostEmbeddingRoi = _lib.lookupFunction<_EmbeddingRoiC, _EmbeddingRoiD>('fdt_host_embedding_roi'),
         detectJpeg = _lib.lookupFunction<_DetectJpegC, _DetectJpegD>('fdt_detect_jpeg'),
         detectFrames = _lib.lookupFunction<_DetectFramesC, _DetectFramesD>('fdt_detect_frames'),
+        detectBatchOriented = _lib.lookupFunction<_DetectBatchOrientedC, _DetectBatchOrientedD>('fdt_detect_batch_oriented'),
+        detectFramesOriented = _lib.lookupFunction<_DetectFramesOrientedC, _DetectFramesOrientedD>('fdt_detect_frames_oriented'),
         detectJpegBatch = _lib.lookupFunction<_DetectJpegBatchC, _DetectJpegBatchD>('fdt_detect_jpeg_batch'),
         numDevices = _lib.lookupFunction<_NumDevicesC, _NumDevicesD>('fdt_num_devices');
 
@@ -181,6 +204,8 @@ class FdtLibrary {
   final _EmbeddingRoiD hostEmbeddingRoi;
   final _DetectJpegD detectJpeg;
   final _DetectFramesD detectFrames;
+  final _DetectBatchOrientedD detectBatchOriented;
+  final _DetectFramesOrientedD detectFramesOriented;
   final _DetectJpegBatchD detectJpegBatch;
   final _NumDevicesD numDevices;
 
