@@ -13,6 +13,10 @@ FDT_OK, FDT_ERR_NOT_READY, FDT_ERR_BAD_ARG, FDT_ERR_SIZE_MISMATCH, FDT_ERR_MODEL
 FDT_MAT_8UC1, FDT_MAT_8UC3, FDT_MAT_8UC4 = 0, 16, 24
 FDT_FMT_YUV_NV12, FDT_FMT_YUV_NV21, FDT_FMT_YUV_I420 = 0x1000, 0x1001, 0x1002   # YUV 4:2:0, height * rowStride * 3 / 2 bytes
 YUV_FORMATS = (FDT_FMT_YUV_NV12, FDT_FMT_YUV_NV21, FDT_FMT_YUV_I420)
+# RGB-ordered frames: packed RGB / RGBA (height * rowStride bytes) and planar RGB, an R, a G and a B plane of height rows of
+# rowStride bytes each, back to back (3 * height * rowStride bytes; a contiguous [3, H, W] tensor has rowStride = W)
+FDT_FMT_RGB, FDT_FMT_RGBA, FDT_FMT_RGB_PLANAR = 0x1010, 0x1011, 0x1012
+RGB_FORMATS = (FDT_FMT_RGB, FDT_FMT_RGBA, FDT_FMT_RGB_PLANAR)
 FDT_MEM_HOST, FDT_MEM_DEVICE = 0, 1
 # EXIF orientation of a stored frame (fdt_detect_batch_oriented / fdt_detect_frames_oriented): the upright image is
 # oracle.jpeg_ops.exif_transform(stored, orientation)

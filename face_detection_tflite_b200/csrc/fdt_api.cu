@@ -140,6 +140,7 @@ struct Slot {
   uint8_t *h_blob = nullptr, *d_blob = nullptr; size_t blob_cap = 0;
   cudaEvent_t ev_blob = nullptr;
   double *h_eye_wh = nullptr, *d_eye_wh = nullptr;    // frame size per iris face [F][2]
+  PixFmt *h_pf = nullptr, *d_pf = nullptr;             // uniform RGB-family calls: the frames' pixel rule for the crop warps
 };
 
 }  // namespace
@@ -209,27 +210,55 @@ int channels_of(int mat_type) {
 }
 
 bool is_yuv(int mat_type) { return mat_type == FDT_FMT_YUV_NV12 || mat_type == FDT_FMT_YUV_NV21 || mat_type == FDT_FMT_YUV_I420; }
+bool is_rgb(int mat_type) { return mat_type == FDT_FMT_RGB || mat_type == FDT_FMT_RGBA || mat_type == FDT_FMT_RGB_PLANAR; }
+
+// Bytes of one pixel within a row: the packed formats' channels, 1 for planar RGB and YUV (a row is one plane's); 0: unknown.
+int row_step(int mat_type) {
+  if (is_yuv(mat_type) || mat_type == FDT_FMT_RGB_PLANAR) return 1;
+  if (mat_type == FDT_FMT_RGB) return 3;
+  if (mat_type == FDT_FMT_RGBA) return 4;
+  return channels_of(mat_type);
+}
 
 // Where the bytes of one input frame are.  Packed formats: height rows of row_stride bytes.  YUV 4:2:0: the Y plane, then the
 // chroma area at c_off: c_rows rows of c_row_bytes (NV12 / NV21: h / 2 interleaved rows; I420: the h / 2 rows of U, then those
 // of V), the chroma of pixel (x, y) at row y / 2 (+ h / 2 for V of I420), byte (x / 2) * c_step + u_off / v_off.
 struct FrameLayout {
-  int channels = 0;          // packed formats; 0 for YUV
+  int channels = 0;          // packed formats (RGB family: the pixel step); 0 for YUV
   bool yuv = false;
+  bool rgb = false;          // FDT_FMT_RGB / _RGBA / _RGB_PLANAR: read through px by k_letterbox_rgb and the format-aware warps
+  int planes = 1;            // planar RGB: 3 planes of height rows of row_stride, back to back
+  PixFmt px;                 // every non-YUV format: pixel step and B, G, R offsets, P = one plane of the whole frame
   long long frame_bytes = 0;
   long long c_off = 0;
   int c_row_bytes = 0, c_rows = 0, c_step = 0, u_off = 0, v_off = 0;
   bool planar = false;       // I420: V is a plane of its own, h / 2 rows behind U
 };
 
+// The pixel rule of a non-YUV format (kernels.h, PixFmt); plane = bytes of one plane where the frame lies.
+PixFmt pix_fmt(int mat_type, long long plane) {
+  PixFmt f;
+  f.step = row_step(mat_type);
+  if (mat_type == FDT_FMT_RGB_PLANAR) { f.b = 2 * plane; f.g = plane; f.r = 0; }
+  else if (mat_type == FDT_FMT_RGB || mat_type == FDT_FMT_RGBA) { f.b = 2; f.g = 1; f.r = 0; }
+  else if (f.step > 1) { f.b = 0; f.g = 1; f.r = 2; }
+  return f;
+}
+
 // Validates the frame arguments (w, hh > 0 checked by the caller); *msg names the failure.
 int frame_layout(int mat_type, int w, int hh, int row_stride, FrameLayout* L, const char** msg) {
   *L = FrameLayout();
   if (!is_yuv(mat_type)) {
-    L->channels = channels_of(mat_type);
+    L->channels = row_step(mat_type);
     if (L->channels == 0) { *msg = "bad frame arguments"; return FDT_ERR_BAD_ARG; }
-    if (row_stride < w * L->channels) { *msg = "row_stride smaller than width * channels"; return FDT_ERR_SIZE_MISMATCH; }
-    L->frame_bytes = (long long)hh * row_stride;
+    if (row_stride < w * L->channels) {
+      *msg = L->channels == 1 && is_rgb(mat_type) ? "row_stride smaller than width" : "row_stride smaller than width * channels";
+      return FDT_ERR_SIZE_MISMATCH;
+    }
+    L->rgb = is_rgb(mat_type);
+    L->planes = mat_type == FDT_FMT_RGB_PLANAR ? 3 : 1;
+    L->frame_bytes = (long long)L->planes * hh * row_stride;
+    L->px = pix_fmt(mat_type, (long long)hh * row_stride);
     return FDT_OK;
   }
   if ((w & 1) || (hh & 1)) { *msg = "YUV 4:2:0 frames need an even width and height"; return FDT_ERR_BAD_ARG; }
@@ -533,17 +562,19 @@ void frame_size(const CallArgs& a, int i, double* w, double* hh) {
 }
 
 // d_desc: a mixed chunk's frame descriptors on the device (the crop warps read the frames through them); orientation: as
-// WarpP::orientation
+// WarpP::orientation; d_pf: a mixed chunk's PixFmt table when it holds an RGB-family frame, else null
 struct ChunkJob {
   int off = 0, n = 0; const uint8_t* d_fr = nullptr; const FrameD* d_desc = nullptr; bool active = false; int orientation = 1;
+  const PixFmt* d_pf = nullptr;
 };
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 // A mixed chunk on its slot's stream: host frames go up whole, one copy each at kStageAlign-aligned offsets; then the chunk's
-// blob (frame descriptors, concatenated tap tables, decode geometry) in one copy; then k_letterbox_multi.
+// blob (frame descriptors, concatenated tap tables, decode geometry and, for a chunk with an RGB-family frame, every frame's
+// PixFmt) in one copy; then k_letterbox_multi.
 int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, const FrameD** d_desc, const double** d_geom,
-                 int* orientation) {
+                 int* orientation, const PixFmt** d_pf) {
   cudaStream_t s = sl.stream;
   Ragged& rg = *a.rg;
   const fdt_frame* fr = rg.frames + off;
@@ -573,8 +604,9 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
   std::map<std::tuple<int, int, int>, int> tap_at;
   std::vector<const SizeTaps*> st(n);
   size_t ntaps = 0;
-  bool upright = true, transposed = false;
+  bool upright = true, transposed = false, rgb = false;
   for (int i = 0; i < n; ++i) {
+    rgb = rgb || rg.lay[off + i].rgb;
     const int o = rg.orientation(off + i);
     upright = upright && o == 1;
     transposed = transposed || orient_transposed(o);
@@ -586,7 +618,9 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
   }
   *orientation = upright ? 1 : 0;
   const size_t taps_at = align_up((size_t)n * sizeof(FrameD), 16), geom_at = align_up(taps_at + ntaps * sizeof(int), 16);
-  const size_t bytes = geom_at + (size_t)n * 6 * sizeof(double);
+  // a chunk with an RGB-family frame also carries every frame's PixFmt (k_letterbox_multi<true, true>, k_warp_affine<., ., true>)
+  const size_t pf_at = align_up(geom_at + (size_t)n * 6 * sizeof(double), 16);
+  const size_t bytes = rgb ? pf_at + (size_t)n * sizeof(PixFmt) : geom_at + (size_t)n * 6 * sizeof(double);
   if (sl.blob_cap < bytes) {
     cudaStreamSynchronize(s);
     if (sl.h_blob) cudaFreeHost(sl.h_blob);
@@ -623,22 +657,24 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
     int uw = 0, uh = 0;
     upright_size(d.w, d.h, d.orientation, &uw, &uh);
     g[4] = uw; g[5] = uh;
+    if (rgb) reinterpret_cast<PixFmt*>(sl.h_blob + pf_at)[i] = L.px;
   }
   cudaMemcpyAsync(sl.d_blob, sl.h_blob, bytes, cudaMemcpyHostToDevice, s);
   cudaEventRecord(sl.ev_blob, s);
   *d_desc = reinterpret_cast<const FrameD*>(sl.d_blob);
   *d_geom = reinterpret_cast<const double*>(sl.d_blob + geom_at);
+  *d_pf = rgb ? reinterpret_cast<const PixFmt*>(sl.d_blob + pf_at) : nullptr;
   StageTimer t(h, 0, s);
   LetterboxMultiP lb;
   lb.fr = *d_desc; lb.taps = reinterpret_cast<const int*>(sl.d_blob + taps_at); lb.out = sl.d_lb; lb.dst_w = S_w; lb.dst_h = S_h;
-  launch_letterbox_multi(lb, n, transposed, s);
+  launch_letterbox_multi(lb, n, transposed, s, *d_pf);
   t.launches = 1;
   return FDT_OK;
 }
 
 // Stage 1 of a chunk on its slot's stream: [H2D] -> letterbox -> detector -> decode + NMS -> [D2H of counts and the
 // first kEagerSlots result slots per frame].
-// Uniform chunk: [H2D] -> k_letterbox / k_letterbox_yuv; *d_fr = the frames on the device.
+// Uniform chunk: [H2D] -> k_letterbox / k_letterbox_yuv / k_letterbox_tr / k_letterbox_rgb; *d_fr = the frames on the device.
 int stage_uniform(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, const uint8_t** d_fr_out) {
   cudaStream_t s = sl.stream;
   const LbTables* tb = a.tb;
@@ -685,12 +721,14 @@ int stage_uniform(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, co
       h->h2d_bytes += (long long)n * (y_stride + c_stride);
       d_c = dc;
     } else if (sparse) {
-      // one strided DMA: `run` rows out of every `period`, for all n frames (frames are contiguous)
+      // one strided DMA: `run` rows out of every `period`, for all n frames (frames are contiguous).  Planar RGB: the planes are
+      // 3 * hh stacked rows, and hh is a multiple of the period, so the pattern runs on through the G and B planes.
+      const int planes = a.lay.planes;
       size_t width_b = (size_t)tb->run * a.row_stride;
       cudaMemcpy2DAsync(sl.d_frames, width_b, src + (size_t)tb->r0 * a.row_stride, (size_t)tb->period * a.row_stride,
-                        width_b, (size_t)n * (a.hh / tb->period), cudaMemcpyHostToDevice, s);
-      dev_frame_stride = (long long)tb->rows_c * a.row_stride;
-      h->h2d_bytes += (long long)width_b * n * (a.hh / tb->period);
+                        width_b, (size_t)n * planes * (a.hh / tb->period), cudaMemcpyHostToDevice, s);
+      dev_frame_stride = (long long)planes * tb->rows_c * a.row_stride;
+      h->h2d_bytes += (long long)width_b * n * planes * (a.hh / tb->period);
     } else {
       cudaMemcpyAsync(sl.d_frames, src, (size_t)n * a.frame_stride, cudaMemcpyHostToDevice, s);
       h->h2d_bytes += (long long)n * a.frame_stride;
@@ -701,7 +739,13 @@ int stage_uniform(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, co
   }
   {
     StageTimer t(h, 0, s);
-    if (tb->transposed) {
+    if (a.lay.rgb) {
+      LetterboxRgbP lb;
+      fill_letterbox(lb.lb, tb, d_fr, dev_frame_stride, a.row_stride, a.channels, a.w, a.hh, sl.d_lb, S_w, S_h, sparse);
+      lb.pf = a.lay.px;
+      if (a.lay.planes > 1) lb.pf = pix_fmt(FDT_FMT_RGB_PLANAR, dev_frame_stride / a.lay.planes);   // the plane as uploaded
+      launch_letterbox_rgb(lb, n, tb->transposed, s);
+    } else if (tb->transposed) {
       LetterboxTrP lb;
       lb.yuv = a.lay.yuv ? 1 : 0;
       if (a.lay.yuv) {
@@ -734,7 +778,8 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
   const FrameD* d_desc = nullptr;
   const double* d_geom = nullptr;
   int orientation = a.orientation;
-  const int rc = a.rg ? stage_ragged(h, sl, a, off, n, &d_desc, &d_geom, &orientation) : stage_uniform(h, sl, a, off, n, &d_fr);
+  const PixFmt* d_pf = nullptr;
+  const int rc = a.rg ? stage_ragged(h, sl, a, off, n, &d_desc, &d_geom, &orientation, &d_pf) : stage_uniform(h, sl, a, off, n, &d_fr);
   if (rc != FDT_OK) return rc;
   {
     StageTimer t(h, 1, s);
@@ -764,6 +809,7 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
                       cudaMemcpyDeviceToHost, s);
   }
   job->off = off; job->n = n; job->d_fr = d_fr; job->d_desc = d_desc; job->active = true; job->orientation = orientation;
+  job->d_pf = d_pf;
   return FDT_OK;
 }
 
@@ -808,6 +854,13 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
   const double gate = h->cfg.min_face_presence;
   // the warp reads whole frames: host frames were uploaded unsparsified in these modes
   const long long dev_frame_stride = a.frame_stride;
+  // the crop warps' PixFmt: a mixed chunk's table, or for a uniform RGB-family call the frames' own (whole frames)
+  const PixFmt* d_pf = job.d_pf;
+  if (a.lay.rgb) {
+    *sl.h_pf = a.lay.px;
+    cudaMemcpyAsync(sl.d_pf, sl.h_pf, sizeof(PixFmt), cudaMemcpyHostToDevice, s);
+    d_pf = sl.d_pf;
+  }
   for (long long skip = 0; skip < total; skip += h->mesh_cap) {
     const int nf = (int)std::min<long long>(h->mesh_cap, total - skip);
     // ---- face ROIs on the host: computeFaceAlignment + extractAlignedSquare's matrix (face_detector_core.dart:478-507)
@@ -833,7 +886,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
       wp.src_w = a.uw; wp.src_h = a.uh; wp.crop_img = sl.d_crop_img; wp.affine = sl.d_affine; wp.ncrops = nf;
       wp.out_size = kMeshInput; wp.flip_odd = 0; wp.crops = sl.d_crops;
       set_warp_layout(wp, a.lay);
-      wp.fr = job.d_desc; wp.orientation = job.orientation;
+      wp.fr = job.d_desc; wp.orientation = job.orientation; wp.pf = d_pf;
       launch_warp_affine(wp, s);
       t.launches = 1;
     }
@@ -916,7 +969,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
           wp.src_w = a.uw; wp.src_h = a.uh; wp.crop_img = sl.d_eye_img; wp.affine = sl.d_eye_affine; wp.ncrops = ne;
           wp.out_size = kIrisInput; wp.flip_odd = 1; wp.crops = sl.d_eye_crops;
           set_warp_layout(wp, a.lay);
-          wp.fr = job.d_desc; wp.orientation = job.orientation;
+          wp.fr = job.d_desc; wp.orientation = job.orientation; wp.pf = d_pf;
           launch_warp_affine(wp, s);
           t.launches = 1;
         }
@@ -1507,7 +1560,7 @@ int create_single(const fdt_config& cfg, const uint8_t* det_tflite, size_t det_l
            dalloc(h, &sl.d_roi, mc * 6) && palloc(h, &sl.h_roi, mc * 6) && dalloc(h, &sl.d_crops, mc * kMeshInput * kMeshInput * 4) &&
            dalloc(h, &sl.d_mesh_out, mc * FDT_MESH_FLOATS) && palloc(h, &sl.h_mesh_out, mc * FDT_MESH_FLOATS) &&
            dalloc(h, &sl.d_mesh_score, mc) && palloc(h, &sl.h_mesh_score, mc) && dalloc(h, &sl.d_eye_corners, mc * 8) &&
-           palloc(h, &sl.h_eye_corners, mc * 8);
+           palloc(h, &sl.h_eye_corners, mc * 8) && dalloc(h, &sl.d_pf, 1) && palloc(h, &sl.h_pf, 1);
       if (!ok) return bail(FDT_ERR_CUDA, "mesh stage allocation failed");
     }
     if (with_iris) {
@@ -1602,11 +1655,11 @@ int32_t fdt_detect_one(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int32
   if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
   std::lock_guard<std::mutex> g(h->mu);
   if (width <= 0 || height <= 0) return fail(h, FDT_ERR_BAD_ARG, "bad frame arguments");
-  const int row_stride = is_yuv(mat_type) ? width : width * channels_of(mat_type);
+  const int row_stride = width * row_step(mat_type);
   FrameLayout lay;
   const char* msg = nullptr;
   if (int rc = frame_layout(mat_type, width, height, row_stride, &lay, &msg)) return fail(h, rc, msg);
-  // matFromPackedBytes length check (lib/src/util/helpers.dart:440-447); YUV: width * height * 3 / 2
+  // matFromPackedBytes length check (lib/src/util/helpers.dart:440-447); YUV: width * height * 3 / 2; planar RGB: 3 * width * height
   if (nbytes != (size_t)lay.frame_bytes) return fail(h, FDT_ERR_SIZE_MISMATCH, "bytes length does not equal the frame size (width * height * channels)");
   return detect_impl(h, bytes, 1, width, height, row_stride, mat_type, mode, FDT_MEM_HOST, out_faces, out_count, out_mesh, out_iris, false);
 }
@@ -2168,7 +2221,12 @@ int32_t fdt_profile_chunk(fdt_handle* h, const uint8_t* d_frames, int32_t n, int
   const int S_w = h->det.in_w(), S_h = h->det.in_h();
   for (int r = 0; r < repeats; ++r) {
     cudaEventRecord(ev[0], s);
-    if (lay.yuv) {
+    if (lay.rgb) {
+      LetterboxRgbP lb;
+      fill_letterbox(lb.lb, tb, d_frames, lay.frame_bytes, row_stride, lay.channels, width, height, sl.d_lb, S_w, S_h, false);
+      lb.pf = lay.px;
+      launch_letterbox_rgb(lb, n, false, s);
+    } else if (lay.yuv) {
       LetterboxYuvP lb;
       fill_letterbox_yuv(lb, tb, lay, d_frames, lay.frame_bytes, false, d_frames + lay.c_off, lay.frame_bytes, false, row_stride,
                          width, height, sl.d_lb, S_w, S_h);

@@ -107,13 +107,24 @@ struct LetterboxTrP {
   int yuv;
 };
 void launch_letterbox_tr(const LetterboxTrP& p, int B, cudaStream_t s);
+// RGB, RGBA and planar RGB frames (FDT_FMT_RGB / _RGBA / _RGB_PLANAR): every non-YUV format is a pixel step and the byte offsets
+// of its B, G and R samples from the pixel's first byte (row + x * step):
+//   BGR 3: 0, 1, 2   RGB 3: 2, 1, 0   BGRA 4: 0, 1, 2   RGBA 4: 2, 1, 0   GRAY 1: 0, 0, 0   planar RGB 1: 2P, P, 0
+// with P the bytes of one plane as it lies on the device (after a compacted upload, the compacted plane).
+struct PixFmt {
+  long long b = 0, g = 0, r = 0;
+  int step = 0;            // 0: no PixFmt (the existing formats' own kernels)
+};
+#ifdef __CUDACC__
+__device__ __forceinline__ void load_pix(const uint8_t* px, const PixFmt& f, int* v) { v[0] = px[f.b]; v[1] = px[f.g]; v[2] = px[f.r]; }
+#endif
 // Ragged batches (fdt_detect_frames): one descriptor per frame of a chunk.  It says where the frame's bytes are and how the
 // letterbox maps it; the crop warps read the same table, indexed by WarpP::crop_img.
 struct FrameD {
   const uint8_t* y;        // the packed frame, or the Y plane
   const uint8_t* c;        // YUV 4:2:0: the chroma area, addressed as in LetterboxYuvP (v_off relative to it)
   int w, h, row_stride;
-  int channels;            // 1 / 3 / 4; 0: YUV 4:2:0
+  int channels;            // 1 / 3 / 4 (RGB-family frames: their pixel step); 0: YUV 4:2:0
   int c_row_stride, c_step, u_off, v_off;
   int new_w, new_h, pad_top, pad_left, identity;
   int tx, ty;              // offsets (ints) of the frame's x taps [4][new_w] and y taps [6][new_h] in the chunk's tap table
@@ -129,7 +140,18 @@ struct LetterboxMultiP {
   uint8_t* out;            // [B][S_h][S_w][4] BGRX
   int dst_w, dst_h;
 };
-void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s);
+// pf (device, [B]): the chunk holds an RGB / RGBA / planar RGB frame, and pf[b] is frame b's PixFmt (offsets from FrameD::y, whole
+// frames; unused for YUV frames), FrameD::channels its pixel step.  Non-null launches the variant that reads every packed or planar
+// frame through pf, whatever its orientation.  (A kernel argument of its own, behind B: FrameD and LetterboxMultiP keep their
+// sizes, which the existing variants' code depends on.)
+void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s, const PixFmt* pf = nullptr);
+// k_letterbox_rgb: k_letterbox (transposed = 0) or k_letterbox_tr (transposed = 1, orientations 5-8) with every tap read through
+// pf; lb.channels unused.  (A struct of its own: the existing parameter blocks keep their layouts.)
+struct LetterboxRgbP {
+  LetterboxP lb;
+  PixFmt pf;
+};
+void launch_letterbox_rgb(const LetterboxRgbP& p, int B, bool transposed, cudaStream_t s);
 // u8 [B][S][S][4] BGRX -> f32 [B][S][S][3] RGB, v*(1/127.5)-1
 void launch_normalize(const uint8_t* in, TV out, int B, cudaStream_t s);
 
@@ -342,6 +364,11 @@ struct WarpP {
   // of the upright image is mapped to its stored pixel right before the load.  Ragged: 1 when every frame of the chunk is
   // upright, else 0 (each frame's own FrameD::orientation applies).  Anything but 1 launches the oriented instantiation.
   int orientation = 1;
+  // RGB / RGBA / planar RGB frames (device memory): uniform, pf[0] is the frames' PixFmt (whole frames); ragged, pf is the chunk's
+  // table (k_letterbox_multi's), indexed like fr.  Non-null launches the format-aware instantiation, which reads every packed or
+  // planar frame's taps through it; out-of-frame taps stay BGR 0.  (One pointer: a larger WarpP changes the code the compiler
+  // makes for the existing instantiations.)
+  const PixFmt* pf = nullptr;
 };
 void launch_warp_affine(const WarpP& p, cudaStream_t s);
 

@@ -3,7 +3,8 @@
 //   k_decode_nms       threshold -> ordered compaction -> decode -> sort -> weighted NMS ->
 //                      letterbox removal -> gates   (one block per image)
 //   k_warp_affine      cv::warpAffine(INTER_LINEAR, BORDER_CONSTANT 0) into square BGR crops (192 face / 64 eye);
-//                      YUV 4:2:0 frames are converted tap by tap (in-frame taps only)
+//                      YUV 4:2:0 frames are converted tap by tap (in-frame taps only); RGB, RGBA and planar RGB frames
+//                      are read through their PixFmt
 //   k_mesh_post        _unpackLandmarks + transformMeshToAbsolute + face-flag sigmoid
 //   k_iris_post        _unpackLandmarks(clamp: false) + transformIrisNormToAbsolute + iris-centre eye keypoints
 #include "fdt_math.h"
@@ -224,7 +225,9 @@ __device__ __forceinline__ long long sat_round_ll(double v) { return (long long)
 // kOriented: the frame is stored rotated / mirrored (EXIF orientation, p.orientation or the descriptor's).  Coordinates, weights
 // and bounds are those of the upright image U; only each in-frame tap's address is mapped to the stored pixel (and chroma
 // sample) it is.  Folding the orientation into the affine map instead would change the rint rounding above.
-template <bool kRagged, bool kOriented>
+// kFmt: the frame (uniform) or some frame of the chunk (ragged) is RGB / RGBA / planar RGB; every packed or planar frame's taps
+// are read through its PixFmt (p.pf[0], or p.pf[frame]), so a crop equals the crop of the BGR image.
+template <bool kRagged, bool kOriented, bool kFmt>
 __global__ void k_warp_affine(WarpP p) {
   const int f = blockIdx.y;
   if (f >= p.ncrops) return;
@@ -236,6 +239,8 @@ __global__ void k_warp_affine(WarpP p) {
   const bool flip = p.flip_odd && (f & 1);
   const int orient = kOriented ? (kRagged ? d->orientation : p.orientation) : 1;
   const bool tr = orient >= 5;
+  PixFmt pf;
+  if (kFmt) pf = p.pf[kRagged ? p.crop_img[f] : 0];
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < S * S; i += gridDim.x * blockDim.x) {
     int y = i / S, x = i - y * S;
     long long adelta = sat_round_ll(A[0] * x * 1024.0);
@@ -274,7 +279,11 @@ __global__ void k_warp_affine(WarpP p) {
       }
       const int channels = kRagged ? d->channels : p.channels;
       const uint8_t* px = src + (size_t)yy * row_stride + (size_t)xx * channels;
-      if (channels == 1) {
+      if (kFmt) {
+        int v[3];
+        load_pix(px, pf, v);
+        acc[0] += v[0] * iw[t]; acc[1] += v[1] * iw[t]; acc[2] += v[2] * iw[t];
+      } else if (channels == 1) {
         acc[0] += px[0] * iw[t]; acc[1] += px[0] * iw[t]; acc[2] += px[0] * iw[t];
       } else {
         acc[0] += px[0] * iw[t]; acc[1] += px[1] * iw[t]; acc[2] += px[2] * iw[t];
@@ -382,16 +391,21 @@ void launch_decode_nms(const DecodeP& p, int B, cudaStream_t s) {
   k_decode_nms<<<B, kDecodeThreads, smem, s>>>(p);
 }
 
+template <bool kFmt> void launch_warp(const WarpP& p, dim3 grid, cudaStream_t s) {
+  if (p.orientation != 1) {
+    if (p.fr) k_warp_affine<true, true, kFmt><<<grid, 256, 0, s>>>(p);
+    else k_warp_affine<false, true, kFmt><<<grid, 256, 0, s>>>(p);
+  } else {
+    if (p.fr) k_warp_affine<true, false, kFmt><<<grid, 256, 0, s>>>(p);
+    else k_warp_affine<false, false, kFmt><<<grid, 256, 0, s>>>(p);
+  }
+}
+
 void launch_warp_affine(const WarpP& p, cudaStream_t s) {
   if (p.ncrops <= 0) return;
   dim3 grid((p.out_size * p.out_size + 255) / 256, p.ncrops);
-  if (p.orientation != 1) {
-    if (p.fr) k_warp_affine<true, true><<<grid, 256, 0, s>>>(p);
-    else k_warp_affine<false, true><<<grid, 256, 0, s>>>(p);
-  } else {
-    if (p.fr) k_warp_affine<true, false><<<grid, 256, 0, s>>>(p);
-    else k_warp_affine<false, false><<<grid, 256, 0, s>>>(p);
-  }
+  if (p.pf) launch_warp<true>(p, grid, s);
+  else launch_warp<false>(p, grid, s);
 }
 
 void launch_mesh_post(const MeshPostP& p, cudaStream_t s) {

@@ -1,6 +1,7 @@
 // Preprocessing kernels: fused letterbox (cv::resize INTER_LINEAR 8U fixed point +
 // copyMakeBorder(0) + BGRA/GRAY->BGR, or cvtColor YUV2BGR for NV12 / NV21 / I420 frames; k_letterbox_multi for chunks of
-// frames of different sizes and formats; k_letterbox_tr for frames stored transposed) and the [-1,1] normalisation.
+// frames of different sizes and formats; k_letterbox_tr for frames stored transposed; k_letterbox_rgb for RGB, RGBA and planar
+// RGB frames, read through their PixFmt) and the [-1,1] normalisation.
 // Reference: convertImageToTensor / bgrMatToSignedFloat32 (lib/src/util/helpers.dart:303-421).
 #include "kernels.h"
 
@@ -162,12 +163,22 @@ __global__ void __launch_bounds__(256) k_letterbox_tr(LetterboxTrP p, int B) {
 // kTransposed: the chunk also holds frames of orientations 5-8, gathered as in k_letterbox_tr (block-uniform branch; their
 // chroma rows are the stored rows halved, mixed calls upload whole frames).  Orientations 2-4 need nothing here: their flips are
 // folded into the taps.
-template <bool kTransposed>
-__global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int B) {
+// kFmt: the chunk also holds RGB / RGBA / planar RGB frames; every packed or planar frame is read through its PixFmt pfs[b]
+// (launched with kTransposed = true, for a chunk of any orientations).
+template <bool kFmt>
+__device__ __forceinline__ void load_packed(const uint8_t* px, int channels, const PixFmt& pf, int* v) {
+  if (kFmt) load_pix(px, pf, v);
+  else load_bgr(px, channels, v);
+}
+
+template <bool kTransposed, bool kFmt>
+__global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int B, const PixFmt* pfs) {
   const int x = blockIdx.x * 64 + (threadIdx.x & 63), y = blockIdx.y * 4 + (threadIdx.x >> 6);
   if (x >= p.dst_w || y >= p.dst_h) return;
   for (int b = blockIdx.z; b < B; b += gridDim.z) {
     const FrameD f = p.fr[b];
+    PixFmt pf;
+    if (kFmt) pf = pfs[b];
     const int dy = y - f.pad_top, dx = x - f.pad_left;
     uchar3 o = make_uchar3(0, 0, 0);
     if (dy >= 0 && dy < f.new_h && dx >= 0 && dx < f.new_w) {
@@ -181,10 +192,10 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
         const uint8_t* r0 = f.y + (size_t)ra * f.row_stride;
         const uint8_t* r1 = f.y + (size_t)rb * f.row_stride;
         if (f.channels) {
-          load_bgr(r0 + (size_t)ca * f.channels, f.channels, t00);
-          load_bgr(r1 + (size_t)ca * f.channels, f.channels, t01);
-          load_bgr(r0 + (size_t)cb * f.channels, f.channels, t10);
-          load_bgr(r1 + (size_t)cb * f.channels, f.channels, t11);
+          load_packed<kFmt>(r0 + (size_t)ca * f.channels, f.channels, pf, t00);
+          load_packed<kFmt>(r1 + (size_t)ca * f.channels, f.channels, pf, t01);
+          load_packed<kFmt>(r0 + (size_t)cb * f.channels, f.channels, pf, t10);
+          load_packed<kFmt>(r1 + (size_t)cb * f.channels, f.channels, pf, t11);
         } else {
           const uint8_t* c0 = f.c + (size_t)(ra >> 1) * f.c_row_stride;
           const uint8_t* c1 = f.c + (size_t)(rb >> 1) * f.c_row_stride;
@@ -196,7 +207,7 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
 #pragma unroll
         for (int c = 0; c < 3; ++c) res[c] = resize_linear(t00[c], t01[c], t10[c], t11[c], wa, wb, va, vb);
       } else if (f.identity) {
-        if (f.channels) load_bgr(f.y + (size_t)dy * f.row_stride + (size_t)dx * f.channels, f.channels, res);
+        if (f.channels) load_packed<kFmt>(f.y + (size_t)dy * f.row_stride + (size_t)dx * f.channels, f.channels, pf, res);
         else load_yuv(f.y + (size_t)dy * f.row_stride, f.c + (size_t)(dy >> 1) * f.c_row_stride, dx, f, res);
       } else {
         const int* tx = p.taps + f.tx;
@@ -207,10 +218,10 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
         const uint8_t* r0 = f.y + (size_t)ya * f.row_stride;
         const uint8_t* r1 = f.y + (size_t)yb * f.row_stride;
         if (f.channels) {
-          load_bgr(r0 + (size_t)xa * f.channels, f.channels, t00);
-          load_bgr(r0 + (size_t)xb * f.channels, f.channels, t01);
-          load_bgr(r1 + (size_t)xa * f.channels, f.channels, t10);
-          load_bgr(r1 + (size_t)xb * f.channels, f.channels, t11);
+          load_packed<kFmt>(r0 + (size_t)xa * f.channels, f.channels, pf, t00);
+          load_packed<kFmt>(r0 + (size_t)xb * f.channels, f.channels, pf, t01);
+          load_packed<kFmt>(r1 + (size_t)xa * f.channels, f.channels, pf, t10);
+          load_packed<kFmt>(r1 + (size_t)xb * f.channels, f.channels, pf, t11);
         } else {
           const uint8_t* c0 = f.c + (size_t)ty[4 * f.new_h + dy] * f.c_row_stride;
           const uint8_t* c1 = f.c + (size_t)ty[5 * f.new_h + dy] * f.c_row_stride;
@@ -225,6 +236,52 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
       o = make_uchar3((unsigned char)res[0], (unsigned char)res[1], (unsigned char)res[2]);
     }
     reinterpret_cast<uchar4*>(p.out)[((size_t)b * p.dst_h + y) * p.dst_w + x] = make_uchar4(o.x, o.y, o.z, 0);
+  }
+}
+
+// RGB, RGBA and planar RGB frames (uniform chunks): the grid, taps and fixed-point resize of k_letterbox (kTransposed = false,
+// identity branch included) or of k_letterbox_tr (true, orientations 5-8: x taps name stored rows, y taps stored columns), with
+// every tap's B, G, R read through p.pf.  Swapping channels or reading three planes only changes which bytes a tap loads, so the
+// output equals letterboxing the BGR image.
+template <bool kTransposed>
+__global__ void __launch_bounds__(256) k_letterbox_rgb(LetterboxRgbP p, int B) {
+  const LetterboxP& q = p.lb;
+  const int x = blockIdx.x * 64 + (threadIdx.x & 63), y = blockIdx.y * 4 + (threadIdx.x >> 6);
+  if (x >= q.dst_w || y >= q.dst_h) return;
+  const int step = p.pf.step;
+  for (int b = blockIdx.z; b < B; b += gridDim.z) {
+    const int dy = y - q.pad_top, dx = x - q.pad_left;
+    uchar3 o = make_uchar3(0, 0, 0);
+    if (dy >= 0 && dy < q.new_h && dx >= 0 && dx < q.new_w) {
+      const uint8_t* src = q.frames + (size_t)b * q.frame_stride;
+      int res[3];
+      if (!kTransposed && q.identity) {
+        load_pix(src + (size_t)dy * q.row_stride + (size_t)dx * step, p.pf, res);
+      } else {
+        const int xa = q.x0[dx], xb = q.x1[dx], wa = q.ax0[dx], wb = q.ax1[dx];
+        const int ya = q.y0[dy], yb = q.y1[dy], va = q.by0[dy], vb = q.by1[dy];
+        int t00[3], t01[3], t10[3], t11[3];
+        if (kTransposed) {
+          const uint8_t* r0 = src + (size_t)xa * q.row_stride;
+          const uint8_t* r1 = src + (size_t)xb * q.row_stride;
+          load_pix(r0 + (size_t)ya * step, p.pf, t00);
+          load_pix(r1 + (size_t)ya * step, p.pf, t01);
+          load_pix(r0 + (size_t)yb * step, p.pf, t10);
+          load_pix(r1 + (size_t)yb * step, p.pf, t11);
+        } else {
+          const uint8_t* r0 = src + (size_t)ya * q.row_stride;
+          const uint8_t* r1 = src + (size_t)yb * q.row_stride;
+          load_pix(r0 + (size_t)xa * step, p.pf, t00);
+          load_pix(r0 + (size_t)xb * step, p.pf, t01);
+          load_pix(r1 + (size_t)xa * step, p.pf, t10);
+          load_pix(r1 + (size_t)xb * step, p.pf, t11);
+        }
+#pragma unroll
+        for (int c = 0; c < 3; ++c) res[c] = resize_linear(t00[c], t01[c], t10[c], t11[c], wa, wb, va, vb);
+      }
+      o = make_uchar3((unsigned char)res[0], (unsigned char)res[1], (unsigned char)res[2]);
+    }
+    reinterpret_cast<uchar4*>(q.out)[((size_t)b * q.dst_h + y) * q.dst_w + x] = make_uchar4(o.x, o.y, o.z, 0);
   }
 }
 
@@ -263,11 +320,19 @@ void launch_letterbox_tr(const LetterboxTrP& p, int B, cudaStream_t s) {
   else k_letterbox_tr<false><<<grid, 256, 0, s>>>(p, B);
 }
 
-void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s) {
+void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s, const PixFmt* pf) {
   if (B <= 0) return;
   dim3 grid((unsigned)((p.dst_w + 63) / 64), (unsigned)((p.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
-  if (transposed) k_letterbox_multi<true><<<grid, 256, 0, s>>>(p, B);
-  else k_letterbox_multi<false><<<grid, 256, 0, s>>>(p, B);
+  if (pf) k_letterbox_multi<true, true><<<grid, 256, 0, s>>>(p, B, pf);
+  else if (transposed) k_letterbox_multi<true, false><<<grid, 256, 0, s>>>(p, B, pf);
+  else k_letterbox_multi<false, false><<<grid, 256, 0, s>>>(p, B, pf);
+}
+
+void launch_letterbox_rgb(const LetterboxRgbP& p, int B, bool transposed, cudaStream_t s) {
+  if (B <= 0) return;
+  dim3 grid((unsigned)((p.lb.dst_w + 63) / 64), (unsigned)((p.lb.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
+  if (transposed) k_letterbox_rgb<true><<<grid, 256, 0, s>>>(p, B);
+  else k_letterbox_rgb<false><<<grid, 256, 0, s>>>(p, B);
 }
 
 void launch_normalize(const uint8_t* in, TV out, int B, cudaStream_t s) {

@@ -41,15 +41,42 @@ def _raise(lib, handle, code: int):
     raise RuntimeError(msg)
 
 
-_PACKED = {_ffi.FDT_MAT_8UC1: 1, _ffi.FDT_MAT_8UC3: 3, _ffi.FDT_MAT_8UC4: 4}
+_PACKED = {_ffi.FDT_MAT_8UC1: 1, _ffi.FDT_MAT_8UC3: 3, _ffi.FDT_MAT_8UC4: 4, _ffi.FDT_FMT_RGB: 3, _ffi.FDT_FMT_RGBA: 4}
+LAYOUTS = ("bgr", "rgb", "rgb_planar")
 
 
-def _mat_type(m, i: int) -> int:
+def _row_step(mt) -> int:
+    """Bytes of one pixel within a row: the packed formats' channels, 1 for YUV and planar RGB (a row is one plane's); 0 when
+    matType is unknown."""
+    return 1 if mt in _ffi.YUV_FORMATS or mt == _ffi.FDT_FMT_RGB_PLANAR else _PACKED.get(mt, 0)
+
+
+def _frame_bytes(mt, h, stride) -> int:
+    if mt in _ffi.YUV_FORMATS:
+        return h * stride * 3 // 2
+    return 3 * h * stride if mt == _ffi.FDT_FMT_RGB_PLANAR else h * stride
+
+
+def _layout(layout) -> str:
+    if not isinstance(layout, str) or layout not in LAYOUTS:
+        raise ValueError("layout must be one of %s, got %r" % (", ".join(LAYOUTS), layout))
+    return layout
+
+
+def _mat_type(m, i: int, layout: str = "bgr") -> int:
+    """The matType of a mat in `layout`: "bgr" (cv.Mat: HxW gray, HxWx3 BGR, HxWx4 BGRA), "rgb" (HxW gray, HxWx3 RGB, HxWx4 RGBA)
+    or "rgb_planar" (3xHxW, the R, G and B planes)."""
+    if layout == "rgb_planar":
+        if not isinstance(m, np.ndarray) or m.dtype != np.uint8 or m.ndim != 3 or m.shape[0] != 3 or m.shape[1] <= 0 or m.shape[2] <= 0:
+            raise ValueError("mat %d: layout 'rgb_planar' expects a 3xHxW uint8 array" % i)
+        return _ffi.FDT_FMT_RGB_PLANAR
     if not isinstance(m, np.ndarray) or m.dtype != np.uint8 or m.ndim not in (2, 3) or m.shape[0] <= 0 or m.shape[1] <= 0:
         raise ValueError("mat %d: expected an HxW, HxWx3 or HxWx4 uint8 array" % i)
     mt = {1: _ffi.FDT_MAT_8UC1, 3: _ffi.FDT_MAT_8UC3, 4: _ffi.FDT_MAT_8UC4}.get(1 if m.ndim == 2 else m.shape[2])
     if mt is None:
         raise ValueError("mat %d: unsupported Mat type" % i)
+    if layout == "rgb":
+        mt = {_ffi.FDT_MAT_8UC3: _ffi.FDT_FMT_RGB, _ffi.FDT_MAT_8UC4: _ffi.FDT_FMT_RGBA}.get(mt, mt)
     return mt
 
 
@@ -68,15 +95,15 @@ def _frame_geometry(i: int, w, h, mt, stride):
     if not all(isinstance(v, (int, np.integer)) for v in (w, h, mt)) or w <= 0 or h <= 0:
         raise ValueError("frame %d: width, height and matType must be positive integers" % i)
     yuv = mt in _ffi.YUV_FORMATS
-    ch = 1 if yuv else _PACKED.get(mt)
-    if ch is None:
+    ch = _row_step(mt)
+    if ch == 0:
         raise ValueError("frame %d: unknown matType %r" % (i, mt))
     stride = w * ch if stride is None else stride
     if not isinstance(stride, (int, np.integer)) or stride < w * ch:
         raise ValueError("frame %d: rowStride smaller than width * channels" % i)
     if yuv and (w % 2 or h % 2):
         raise ValueError("frame %d: YUV 4:2:0 frames need an even width and height" % i)
-    return int(stride), (h * stride * 3 // 2 if yuv else h * stride)
+    return int(stride), _frame_bytes(mt, h, stride)
 
 
 def _orientation(o, what: str = "orientation") -> int:
@@ -187,7 +214,8 @@ class FaceDetector:
                                 mode: FaceDetectionMode = FaceDetectionMode.full, orientation: int = 1) -> List[Face]:
         """detectFacesFromMatBytes (face_detector.dart:588-609); the default mode is `full` like the reference's
         (detector + mesh + iris; the blendshape classifier is outside this path).  matType may also be one of the YUV 4:2:0
-        formats FDT_FMT_YUV_NV12 / _NV21 / _I420: `data` is then width * height * 3 / 2 bytes (cv2's (3H/2) x W Mat).
+        formats FDT_FMT_YUV_NV12 / _NV21 / _I420: `data` is then width * height * 3 / 2 bytes (cv2's (3H/2) x W Mat), or one of
+        the RGB formats FDT_FMT_RGB / _RGBA / _RGB_PLANAR (width * height * 3, * 4, or 3 * width * height bytes).
         orientation (EXIF 1..8, FDT_ORIENT_*): the frame is stored rotated / mirrored; width and height are the stored size,
         the faces are those of the upright image exif_transform(frame, orientation), normalised to its size."""
         if _orientation(orientation) != 1:
@@ -250,9 +278,16 @@ class FaceDetector:
         return out
 
     def detectFacesFromMat(self, mat: np.ndarray, *, mode: FaceDetectionMode = FaceDetectionMode.full,
-                           orientation: int = 1) -> List[Face]:
+                           orientation: int = 1, layout: str = "bgr") -> List[Face]:
         """detectFacesFromMat (face_detector.dart:559-572): `mat` is an HxW[xC] uint8 array (cv.Mat), stored in EXIF
-        `orientation` (see detectFacesFromMatBytes)."""
+        `orientation` (see detectFacesFromMatBytes).  layout: "bgr" (cv.Mat channel order), "rgb" (HxWx3 RGB, HxWx4 RGBA, HxW
+        gray: PIL, imageio, Flutter rawRgba) or "rgb_planar" (3xHxW, e.g. a decoded torchvision image moved to the host).  The
+        faces equal those of the BGR image."""
+        if _layout(layout) != "bgr":
+            mt = _mat_type(mat, 0, layout)
+            h, w = mat.shape[1:] if mt == _ffi.FDT_FMT_RGB_PLANAR else mat.shape[:2]
+            return self.detectFacesFromMatBytes(np.ascontiguousarray(mat), width=w, height=h, matType=mt, mode=mode,
+                                                orientation=orientation)
         ch = 1 if mat.ndim == 2 else mat.shape[2]
         mt = {1: _ffi.FDT_MAT_8UC1, 3: _ffi.FDT_MAT_8UC3, 4: _ffi.FDT_MAT_8UC4}.get(ch)
         if mt is None or mat.dtype != np.uint8:
@@ -281,23 +316,28 @@ class FaceDetector:
                        rowStride: Optional[int] = None, withIris: bool = False, orientation: int = 1):
         """fdt_detect_batch with array outputs: (FdtFace array, counts int32[count], mesh f32 or None) and, with
         withIris=True, a fourth element iris f32 [count, max_faces, 152, 3] (None unless mode is full).
-        `frames` may be a numpy array / bytes (host) or an integer device pointer with memKind=FDT_MEM_DEVICE.
-        YUV 4:2:0 formats: rowStride is the Y-plane stride (default: width) and a frame is height * rowStride * 3 / 2 bytes.
+        `frames` may be a numpy array / bytes (host) or an integer device pointer with memKind=FDT_MEM_DEVICE (a CUDA tensor:
+        t.data_ptr()).  YUV 4:2:0 formats: rowStride is the Y-plane stride (default: width) and a frame is
+        height * rowStride * 3 / 2 bytes.  FDT_FMT_RGB_PLANAR: rowStride is one plane's row stride (default: width) and a frame
+        is 3 * height * rowStride bytes.
         orientation (EXIF 1..8, FDT_ORIENT_*; fdt_detect_batch_oriented): every frame is stored rotated / mirrored.  width,
         height and rowStride describe the stored frames; faces are normalised to the upright image exif_transform(frame,
         orientation) and mesh / iris points are in its pixels."""
         orientation = _orientation(orientation)
         self._check()
         yuv = matType in _ffi.YUV_FORMATS
-        ch = 1 if yuv else {_ffi.FDT_MAT_8UC1: 1, _ffi.FDT_MAT_8UC3: 3, _ffi.FDT_MAT_8UC4: 4}.get(matType, 0)
+        ch = _row_step(matType)
         stride = rowStride if rowStride is not None else width * ch
-        frame_bytes = height * stride * 3 // 2 if yuv else height * stride
+        if ch and stride < width * ch:
+            raise ValueError("rowStride smaller than width * channels")
+        frame_bytes = _frame_bytes(matType, height, stride)
         if isinstance(frames, int):
             ptr = frames
         else:
             buf = np.ascontiguousarray(np.frombuffer(frames, np.uint8) if not isinstance(frames, np.ndarray) else frames.reshape(-1))
             if buf.size != count * frame_bytes:
-                raise ValueError("frames length does not equal count * height * rowStride%s" % (" * 3 / 2" if yuv else ""))   # helpers.dart:440-447
+                raise ValueError("frames length does not equal count * %sheight * rowStride%s" % (
+                    "3 * " if matType == _ffi.FDT_FMT_RGB_PLANAR else "", " * 3 / 2" if yuv else ""))   # helpers.dart:440-447
             ptr = buf.ctypes.data
         faces = (_ffi.FdtFace * max(1, count * self._max_faces))()
         counts = np.zeros(max(1, count), np.int32)
@@ -319,16 +359,26 @@ class FaceDetector:
 
     # -- mixed batches: frames of different sizes and formats, and encoded images, in one call ----------------------------
     def detectFacesFromMats(self, mats, *, mode: FaceDetectionMode = FaceDetectionMode.full,
-                            orientations=None) -> List[List[Face]]:
+                            orientations=None, layout: str = "bgr") -> List[List[Face]]:
         """detectFacesFromMat over a list of HxW / HxWx3 / HxWx4 uint8 arrays of any sizes, in one batched call
         (fdt_detect_frames).  A row-padded view (e.g. a crop of a larger array) goes in uncopied with strides[0] as its row
         stride.  Returns one list of faces per mat, each normalised to its own mat.  orientations: one EXIF orientation 1..8
-        per mat (fdt_detect_frames_oriented), or None for all upright; faces then refer to each mat's upright image."""
+        per mat (fdt_detect_frames_oriented), or None for all upright; faces then refer to each mat's upright image.
+        layout: as detectFacesFromMat, for every mat.  A 3xHxW view whose rows are padded but whose planes are height rows
+        apart (e.g. a crop of the columns of a larger CHW array) goes in uncopied; any other planar view is copied."""
         mats = list(mats)
+        layout = _layout(layout)
         orients = _orientations(orientations, len(mats))
         frames, keep = [], []
         for i, m in enumerate(mats):
-            mt = _mat_type(m, i)
+            mt = _mat_type(m, i, layout)
+            if mt == _ffi.FDT_FMT_RGB_PLANAR:
+                h, w = m.shape[1:]
+                if m.strides[2] != 1 or m.strides[1] < w or m.strides[0] != h * m.strides[1] or not _rows_in_buffer(m):
+                    m = np.ascontiguousarray(m)
+                keep.append(m)
+                frames.append((m.ctypes.data, w, h, m.strides[1], mt))
+                continue
             if m.strides[-1] != 1 or (m.ndim == 3 and m.strides[1] != m.shape[2]) or m.strides[0] < m.shape[1] * m.strides[1] \
                     or not _rows_in_buffer(m):
                 m = np.ascontiguousarray(m)
@@ -342,8 +392,9 @@ class FaceDetector:
     def detectFramesRaw(self, frames, *, mode: FaceDetectionMode = FaceDetectionMode.fast, memKind: int = _ffi.FDT_MEM_HOST,
                         orientations=None):
         """fdt_detect_frames with array outputs.  `frames` is a list of (data, width, height, matType[, rowStride]) tuples: data
-        is a numpy array / bytes of exactly height * rowStride bytes (YUV 4:2:0: height * rowStride * 3 / 2), or an integer
-        device pointer with memKind=FDT_MEM_DEVICE.  rowStride defaults to width * channels (YUV: width).  Returns
+        is a numpy array / bytes of exactly height * rowStride bytes (YUV 4:2:0: height * rowStride * 3 / 2; planar RGB:
+        3 * height * rowStride), or an integer device pointer with memKind=FDT_MEM_DEVICE.  rowStride defaults to
+        width * channels (YUV and planar RGB: width).  Returns
         (FdtFace array [n * max_faces], counts int32 [n], mesh f32 [n, max_faces, 468, 3] or None,
         iris f32 [n, max_faces, 152, 3] or None).  orientations: one EXIF orientation 1..8 per frame
         (fdt_detect_frames_oriented; results refer to each frame's upright image), or None for all upright."""
@@ -366,7 +417,8 @@ class FaceDetector:
                     raise ValueError("frame %d: host frames are numpy arrays or bytes" % i)
                 buf = np.ascontiguousarray(np.frombuffer(data, np.uint8) if not isinstance(data, np.ndarray) else data.reshape(-1))
                 if buf.dtype != np.uint8 or buf.size != nbytes:
-                    raise ValueError("frame %d: data length does not equal height * rowStride%s" % (i, " * 3 / 2" if mt in _ffi.YUV_FORMATS else ""))
+                    raise ValueError("frame %d: data length does not equal %sheight * rowStride%s" % (
+                        i, "3 * " if mt == _ffi.FDT_FMT_RGB_PLANAR else "", " * 3 / 2" if mt in _ffi.YUV_FORMATS else ""))
                 keep.append(buf)
                 ptr = buf.ctypes.data
             descs.append((ptr, w, h, stride, mt))

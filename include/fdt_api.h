@@ -84,6 +84,18 @@ enum { FDT_MAT_8UC1 = 0, FDT_MAT_8UC3 = 16, FDT_MAT_8UC4 = 24 };
  * MatType (at most 4095). */
 enum { FDT_FMT_YUV_NV12 = 0x1000, FDT_FMT_YUV_NV21 = 0x1001, FDT_FMT_YUV_I420 = 0x1002 };
 
+/* RGB-ordered frames (PIL, PyAV rgb24, imageio, Flutter rawRgba, browser ImageData, and torchvision / torchcodec GPU decoding,
+ * which hands over uint8 [3, H, W] tensors), accepted wherever mat_type is, except by fdt_extract_aligned_squares
+ * (FDT_ERR_BAD_ARG).  Every result equals the same call on the BGR image - cv::cvtColor(frame, COLOR_RGB2BGR) / COLOR_RGBA2BGR,
+ * or for planar frames the planes in reverse order interleaved (numpy: chw[::-1].transpose(1, 2, 0)) - bit for bit; the channel
+ * order and plane layout are read by the letterbox and crop kernels (no converted copy).
+ *   FDT_FMT_RGB        packed R, G, B; row_stride >= 3 * width; a frame is height * row_stride bytes.
+ *   FDT_FMT_RGBA       packed R, G, B, A (alpha ignored, as for 8UC4); row_stride >= 4 * width; height * row_stride bytes.
+ *   FDT_FMT_RGB_PLANAR an R plane, then a G plane, then a B plane, back to back, each height rows of row_stride >= width bytes;
+ *                      a frame is 3 * height * row_stride bytes (a contiguous [3, H, W] tensor has row_stride = W).  Any size.
+ * A row_stride below the minimum returns FDT_ERR_SIZE_MISMATCH. */
+enum { FDT_FMT_RGB = 0x1010, FDT_FMT_RGBA = 0x1011, FDT_FMT_RGB_PLANAR = 0x1012 };
+
 enum { FDT_MEM_HOST = 0, FDT_MEM_DEVICE = 1 };
 
 /* Frame orientation (fdt_detect_batch_oriented, fdt_detect_frames_oriented): the EXIF Orientation value of the STORED frame,
@@ -157,7 +169,7 @@ FDT_EXPORT int32_t fdt_destroy(fdt_handle* h);
 
 /* New batched entry point (Dart: detectFacesBatch).  `frames` is `batch` tightly laid out images
  * of height x row_stride bytes (row_stride >= width * channels(mat_type); YUV formats: height * row_stride * 3 / 2
- * bytes, see FDT_FMT_YUV_NV12), in host (pinned or
+ * bytes, see FDT_FMT_YUV_NV12; planar RGB: 3 * height * row_stride, see FDT_FMT_RGB), in host (pinned or
  * pageable) or device memory.  Replaces the per-frame sequence
  * _detectDetections -> applyDetectionGates -> computeFaceAlignment [-> extractAlignedSquare ->
  * FaceLandmark.callWithScore -> transformMeshToAbsolute]
@@ -177,7 +189,8 @@ typedef struct fdt_frame {
   const uint8_t* data;       /* host or device memory, per the call's mem_kind                                   */
   int32_t width, height;     /* image size                                                                        */
   int32_t row_stride;        /* as fdt_detect_batch: >= width * channels; YUV: the Y-plane stride                 */
-  int32_t mat_type;          /* FDT_MAT_8UC1 / _8UC3 / _8UC4 or FDT_FMT_YUV_NV12 / _NV21 / _I420                 */
+  int32_t mat_type;          /* FDT_MAT_8UC1 / _8UC3 / _8UC4, FDT_FMT_YUV_NV12 / _NV21 / _I420, FDT_FMT_RGB / _RGBA /
+                                _RGB_PLANAR                                                                       */
 } fdt_frame;                 /* 24 bytes */
 
 /* detectFacesFromMat over a list of frames of different sizes and formats (photos, mixed camera feeds), batched like
@@ -223,7 +236,8 @@ FDT_EXPORT int32_t fdt_detect_jpeg_batch(fdt_handle* h, const uint8_t* const* im
 
 /* detectFacesFromMatBytes (lib/src/face_detector.dart:588-609): one packed frame of
  * `nbytes` bytes; FDT_ERR_SIZE_MISMATCH when nbytes != width*height*channels
- * (matFromPackedBytes, lib/src/util/helpers.dart:432-450), or != width*height*3/2 for the YUV formats. */
+ * (matFromPackedBytes, lib/src/util/helpers.dart:432-450), or != width*height*3/2 for the YUV formats
+ * (FDT_FMT_RGB: width*height*3, FDT_FMT_RGBA: width*height*4, FDT_FMT_RGB_PLANAR: 3*width*height). */
 FDT_EXPORT int32_t fdt_detect_one(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int32_t width,
                                   int32_t height, int32_t mat_type, int32_t mode, fdt_face* out_faces,
                                   int32_t* out_count, float* out_mesh, float* out_iris);
@@ -315,8 +329,10 @@ FDT_EXPORT int64_t fdt_last_launch_count(fdt_handle* h);
  * and to the chroma plane(s) independently (720 -> 72: Y rows 10k+4, 10k+5 and chroma rows 5k+2).
  * Oriented frames (fdt_detect_batch_oriented): the rule is "the stored rows the upright image's taps read" - U's y taps for
  * orientations 1-4, U's x taps for 5-8 (a 1280x720 frame stored sideways still uploads 2 rows in 10), after the flips.  The two
- * axes clamp differently at the borders, so at some sizes that set differs from orientation 1's.  Mixed calls upload whole
- * frames. */
+ * axes clamp differently at the borders, so at some sizes that set differs from orientation 1's.  RGB and RGBA frames upload as
+ * BGR and BGRA do.  Planar RGB frames are read as 3 * height stacked rows: when height is a multiple of the period the same
+ * pattern runs through all three planes (1280x720: 552,960 bytes per frame, as BGR), otherwise whole frames go up.  Mixed calls
+ * upload whole frames. */
 FDT_EXPORT int64_t fdt_last_h2d_bytes(fdt_handle* h);
 /* Device time in ms of the named stage summed over the last call when stage timing was enabled
  * with fdt_set_stage_timing(h,1) (adds cudaEvent records; off by default).

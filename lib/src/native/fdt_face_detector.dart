@@ -190,7 +190,9 @@ class FdtFaceDetector {
   }
 
   /// New batched entry point: [frames] holds [count] packed frames (count * height * width * channels bytes), or [count]
-  /// YUV 4:2:0 frames of width * height * 3 / 2 bytes with matType kFdtFmtYuvNv12 / kFdtFmtYuvNv21 / kFdtFmtYuvI420.
+  /// YUV 4:2:0 frames of width * height * 3 / 2 bytes with matType kFdtFmtYuvNv12 / kFdtFmtYuvNv21 / kFdtFmtYuvI420, or RGB
+  /// frames with kFdtFmtRgb / kFdtFmtRgba / kFdtFmtRgbPlanar (a Flutter `ui.Image.toByteData(format: rawRgba)` buffer is one
+  /// kFdtFmtRgba frame as it is).
   /// One `fdt_detect_batch` call; results come back in frame order.  [orientation]: the EXIF orientation (kFdtOrient*) every
   /// frame is stored in (`fdt_detect_batch_oriented`); width / height are the stored size, faces refer to the upright image.  For sustained throughput keep the frames in a
   /// buffer from `fdt_alloc_pinned` (see [FdtPinnedFrames]) so the upload runs at PCIe speed.

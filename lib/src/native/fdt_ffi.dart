@@ -35,6 +35,13 @@ const int kFdtMemDevice = 1;
 const int kFdtFmtYuvNv12 = 0x1000;
 const int kFdtFmtYuvNv21 = 0x1001;
 const int kFdtFmtYuvI420 = 0x1002;
+/// RGB-ordered frame formats (fdt_api.h FDT_FMT_RGB*), accepted wherever a matType is, except by extractAlignedSquares;
+/// results equal those of the BGR image bit for bit.  kFdtFmtRgb: packed R, G, B; kFdtFmtRgba: packed R, G, B, A (alpha
+/// ignored) - `ui.Image.toByteData(format: ImageByteFormat.rawRgba)` goes in as it is, width * 4 bytes per row, no conversion;
+/// kFdtFmtRgbPlanar: an R, a G and a B plane of height rows of rowStride (>= width) bytes each, back to back.
+const int kFdtFmtRgb = 0x1010;
+const int kFdtFmtRgba = 0x1011;
+const int kFdtFmtRgbPlanar = 0x1012;
 
 /// Frame orientations (fdt_api.h FDT_ORIENT_*): the EXIF Orientation value of a stored frame, as OpenCV's ExifTransform
 /// applies it.  Results of the oriented calls refer to the upright image; for 5-8 its width is the stored height.  Camera
@@ -51,10 +58,14 @@ const int kFdtOrientRot90Ccw = 8;
 
 bool fdtIsYuv(int matType) => matType == kFdtFmtYuvNv12 || matType == kFdtFmtYuvNv21 || matType == kFdtFmtYuvI420;
 
-/// Row stride (Y-plane stride for the YUV formats) and size in bytes of one tightly packed frame of [matType].
-int fdtRowStride(int matType, int width) => fdtIsYuv(matType) ? width : width * (matType == 0 ? 1 : (matType == 24 ? 4 : 3));
-int fdtFrameBytes(int matType, int width, int height) =>
-    fdtIsYuv(matType) ? height * width * 3 ~/ 2 : height * fdtRowStride(matType, width);
+/// Row stride (Y-plane stride for the YUV formats, one plane's for planar RGB) and size in bytes of one tightly packed frame
+/// of [matType].
+int fdtRowStride(int matType, int width) => fdtIsYuv(matType) || matType == kFdtFmtRgbPlanar
+    ? width
+    : width * (matType == 0 ? 1 : (matType == 24 || matType == kFdtFmtRgba ? 4 : 3));
+int fdtFrameBytes(int matType, int width, int height) => fdtIsYuv(matType)
+    ? height * width * 3 ~/ 2
+    : (matType == kFdtFmtRgbPlanar ? 3 : 1) * height * fdtRowStride(matType, width);
 
 /// fdt_config: the named arguments of FaceDetector.create that touch the path (48 bytes).
 final class FdtConfig extends Struct {
