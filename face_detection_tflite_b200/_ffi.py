@@ -45,6 +45,13 @@ class FdtFrame(C.Structure):
                 ("mat_type", C.c_int32)]
 
 
+class FdtYuvPlanes(C.Structure):
+    """fdt_yuv_planes: one YUV 4:2:0 frame as a Y, a U and a V plane, each with its own base and row stride, U and V sharing a
+    pixel stride of 1 or 2 (fdt_detect_yuv_planes)."""
+    _fields_ = [("plane", C.c_void_p * 3), ("row_stride", C.c_int32 * 3), ("width", C.c_int32), ("height", C.c_int32),
+                ("pixel_stride", C.c_int32), ("reserved", C.c_int32)]
+
+
 # every symbol include/fdt_api.h declares: name -> (restype, argtypes)
 P = C.c_void_p
 u8p = C.POINTER(C.c_uint8)
@@ -64,6 +71,8 @@ SIGNATURES = {
                                               C.c_int32, C.POINTER(FdtFace), i32p, f32p, f32p]),
     "fdt_detect_frames_oriented": (C.c_int32, [P, C.POINTER(FdtFrame), i32p, C.c_int32, C.c_int32, C.c_int32, C.POINTER(FdtFace),
                                                i32p, f32p, f32p]),
+    "fdt_detect_yuv_planes": (C.c_int32, [P, C.POINTER(FdtYuvPlanes), i32p, C.c_int32, C.c_int32, C.c_int32, C.POINTER(FdtFace),
+                                          i32p, f32p, f32p]),
     "fdt_detect_jpeg_batch": (C.c_int32, [P, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_int32, C.c_int32, C.POINTER(FdtFace),
                                           i32p, f32p, f32p, i32p, i32p]),
     "fdt_detect_one": (C.c_int32, [P, P, C.c_size_t, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(FdtFace), i32p, f32p, f32p]),

@@ -6,6 +6,7 @@
 // mirroring _FaceDetectorCore.detectFacesDirect (lib/src/isolate/face_detector_core.dart:215-394).
 // In standard / full mode the host sits between the stages exactly where the reference's Dart code does (ROI
 // geometry with the host libm, presence gate); while it handles chunk c the other slot's stream runs chunk c + 1.
+#include <cuda.h>
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -534,6 +535,10 @@ struct Ragged {
   const fdt_frame* frames = nullptr;
   const int32_t* orientations = nullptr;   // [n] EXIF 1..8, or null: all upright
   std::vector<FrameLayout> lay;
+  // fdt_detect_yuv_planes: the descriptors, and `frames` points at pframes, one fdt_frame per descriptor that gives the size and
+  // the Y plane as the kernels read it (staged host frames: row stride = width); lay[i] is the staged layout (plane_layout)
+  const fdt_yuv_planes* planes = nullptr;
+  std::vector<fdt_frame> pframes;
   std::map<std::tuple<int, int, int>, SizeTaps> taps;   // (stored width, height, orientation)
   int orientation(int i) const { return orientations ? orientations[i] : 1; }
 };
@@ -562,11 +567,67 @@ void frame_size(const CallArgs& a, int i, double* w, double* hh) {
 }
 
 // d_desc: a mixed chunk's frame descriptors on the device (the crop warps read the frames through them); orientation: as
-// WarpP::orientation; d_pf: a mixed chunk's PixFmt table when it holds an RGB-family frame, else null
+// WarpP::orientation; d_pf: a mixed chunk's PixFmt table when it holds an RGB-family frame, else null; d_pl: a chunk's
+// YuvPlaneD table when its separate-plane device frames do not fit FrameD, else null
 struct ChunkJob {
   int off = 0, n = 0; const uint8_t* d_fr = nullptr; const FrameD* d_desc = nullptr; bool active = false; int orientation = 1;
   const PixFmt* d_pf = nullptr;
+  const YuvPlaneD* d_pl = nullptr;
 };
+
+// Bytes of the sampled columns of one chroma row of a separate-plane frame: (width / 2 - 1) * pixel_stride + 1.
+long long chroma_cols(const fdt_yuv_planes& f) { return (long long)(f.width / 2 - 1) * f.pixel_stride + 1; }
+
+// U and V interleaved in one chroma plane (NV12 / NV21, Android pixel stride 2 views of one buffer): pixel stride 2, one row
+// stride of at least width, V one byte behind or before U.  Each chroma row's width bytes from the lower of the two are then
+// exactly the two sampled extents' bytes in that row.
+bool interleaved_chroma(const fdt_yuv_planes& f) {
+  const uintptr_t u = reinterpret_cast<uintptr_t>(f.plane[1]), v = reinterpret_cast<uintptr_t>(f.plane[2]);
+  return f.pixel_stride == 2 && f.row_stride[1] == f.row_stride[2] && f.row_stride[1] >= f.width && (v == u + 1 || u == v + 1);
+}
+
+// A separate-plane frame as it is staged from host memory: the Y plane (width bytes per row), then the chroma, which FrameD
+// describes as it describes NV12 / NV21 and I420 frames.  Interleaved chroma: one area of height / 2 rows of width bytes (the
+// bytes fdt_detect_frames uploads for an NV12 frame).  Otherwise the U and then the V area, height / 2 rows of chroma_cols bytes
+// each, chroma step pixel_stride.
+FrameLayout plane_layout(const fdt_yuv_planes& f) {
+  FrameLayout L;
+  L.yuv = true;
+  L.c_off = (long long)f.width * f.height;
+  L.c_step = f.pixel_stride;
+  if (interleaved_chroma(f)) {
+    L.c_row_bytes = f.width; L.c_rows = f.height / 2;
+    L.u_off = f.plane[1] < f.plane[2] ? 0 : 1; L.v_off = 1 - L.u_off;
+    L.frame_bytes = L.c_off + (long long)(f.height / 2) * f.width;
+    return L;
+  }
+  const long long cc = chroma_cols(f);
+  L.planar = true;
+  L.c_row_bytes = (int)cc; L.c_rows = f.height; L.u_off = 0; L.v_off = (int)(f.height / 2 * cc);
+  L.frame_bytes = L.c_off + 2 * (f.height / 2) * cc;
+  return L;
+}
+
+// The sampled columns of every row, one 2-D copy per plane (interleaved chroma: one copy for U and V): nothing past a plane's
+// sampled extent is read.
+void upload_planes(uint8_t* dst, const fdt_yuv_planes& f, const FrameLayout& L, cudaStream_t s) {
+  cudaMemcpy2DAsync(dst, f.width, f.plane[0], f.row_stride[0], f.width, f.height, cudaMemcpyHostToDevice, s);
+  if (!L.planar) {
+    cudaMemcpy2DAsync(dst + L.c_off, L.c_row_bytes, std::min(f.plane[1], f.plane[2]), f.row_stride[1], L.c_row_bytes, f.height / 2,
+                      cudaMemcpyHostToDevice, s);
+    return;
+  }
+  for (int k = 1; k < 3; ++k)
+    cudaMemcpy2DAsync(dst + L.c_off + (k == 2 ? L.v_off : 0), L.c_row_bytes, f.plane[k], f.row_stride[k], L.c_row_bytes,
+                      f.height / 2, cudaMemcpyHostToDevice, s);
+}
+
+// Separate-plane device frames whose U and V share a row stride and lie less than 2^31 bytes apart (NVDEC NV12 surfaces,
+// contiguous I420 / NV21) are FrameD frames with the chroma base at the lower of the two; others need the YuvPlaneD table.
+bool fits_frame_desc(const fdt_yuv_planes& f) {
+  const long long d = (long long)(reinterpret_cast<uintptr_t>(f.plane[2]) - reinterpret_cast<uintptr_t>(f.plane[1]));
+  return f.row_stride[1] == f.row_stride[2] && d < INT32_MAX && d > -INT32_MAX;
+}
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
@@ -574,7 +635,7 @@ size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 // blob (frame descriptors, concatenated tap tables, decode geometry and, for a chunk with an RGB-family frame, every frame's
 // PixFmt) in one copy; then k_letterbox_multi.
 int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, const FrameD** d_desc, const double** d_geom,
-                 int* orientation, const PixFmt** d_pf) {
+                 int* orientation, const PixFmt** d_pf, const YuvPlaneD** d_pl) {
   cudaStream_t s = sl.stream;
   Ragged& rg = *a.rg;
   const fdt_frame* fr = rg.frames + off;
@@ -593,7 +654,8 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
     }
     for (int i = 0; i < n; ++i) {
       const size_t fb = (size_t)rg.lay[off + i].frame_bytes;
-      cudaMemcpyAsync(sl.d_frames + at[i], fr[i].data, fb, cudaMemcpyHostToDevice, s);
+      if (rg.planes) upload_planes(sl.d_frames + at[i], rg.planes[off + i], rg.lay[off + i], s);
+      else cudaMemcpyAsync(sl.d_frames + at[i], fr[i].data, fb, cudaMemcpyHostToDevice, s);
       h->h2d_bytes += (long long)fb;
       base[i] = sl.d_frames + at[i];
     }
@@ -617,10 +679,15 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
     if (tap_at.emplace(key, (int)ntaps).second) ntaps += it->second.t.size();
   }
   *orientation = upright ? 1 : 0;
+  const fdt_yuv_planes* pl = rg.planes ? rg.planes + off : nullptr;
+  bool table = false;
+  for (int i = 0; pl && a.mem_kind == FDT_MEM_DEVICE && i < n; ++i) table = table || !fits_frame_desc(pl[i]);
   const size_t taps_at = align_up((size_t)n * sizeof(FrameD), 16), geom_at = align_up(taps_at + ntaps * sizeof(int), 16);
-  // a chunk with an RGB-family frame also carries every frame's PixFmt (k_letterbox_multi<true, true>, k_warp_affine<., ., true>)
+  // a chunk with an RGB-family frame also carries every frame's PixFmt (k_letterbox_multi<true, true>, k_warp_affine<., ., true>);
+  // a chunk of separate-plane device frames that FrameD cannot describe, every frame's YuvPlaneD (the <., ., ., true> variants)
   const size_t pf_at = align_up(geom_at + (size_t)n * 6 * sizeof(double), 16);
-  const size_t bytes = rgb ? pf_at + (size_t)n * sizeof(PixFmt) : geom_at + (size_t)n * 6 * sizeof(double);
+  const size_t bytes = rgb ? pf_at + (size_t)n * sizeof(PixFmt)
+                           : table ? pf_at + (size_t)n * sizeof(YuvPlaneD) : geom_at + (size_t)n * 6 * sizeof(double);
   if (sl.blob_cap < bytes) {
     cudaStreamSynchronize(s);
     if (sl.h_blob) cudaFreeHost(sl.h_blob);
@@ -648,6 +715,17 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
     d.w = fr[i].width; d.h = fr[i].height; d.row_stride = fr[i].row_stride; d.channels = L.channels;
     d.c_row_stride = L.c_row_bytes; d.c_step = L.c_step; d.u_off = L.u_off; d.v_off = L.v_off;
     d.new_w = lp.new_w; d.new_h = lp.new_h; d.pad_top = lp.pad_top; d.pad_left = lp.pad_left; d.identity = st[i]->identity ? 1 : 0;
+    if (pl && a.mem_kind == FDT_MEM_DEVICE) {
+      const fdt_yuv_planes& f = pl[i];
+      if (table) {
+        d.c = nullptr;
+        reinterpret_cast<YuvPlaneD*>(sl.h_blob + pf_at)[i] = YuvPlaneD{f.plane[1], f.plane[2], f.row_stride[1], f.row_stride[2], f.pixel_stride, 0};
+      } else {
+        d.c = std::min(f.plane[1], f.plane[2]);
+        d.c_row_stride = f.row_stride[1]; d.c_step = f.pixel_stride;
+        d.u_off = (int)(f.plane[1] - d.c); d.v_off = (int)(f.plane[2] - d.c);
+      }
+    }
     d.orientation = rg.orientation(off + i);
     d.tx = tap_at[std::make_tuple(d.w, d.h, d.orientation)]; d.ty = d.tx + 4 * lp.new_w;
     // the values fill_decode derives from LbTables, computed the same way
@@ -664,10 +742,11 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
   *d_desc = reinterpret_cast<const FrameD*>(sl.d_blob);
   *d_geom = reinterpret_cast<const double*>(sl.d_blob + geom_at);
   *d_pf = rgb ? reinterpret_cast<const PixFmt*>(sl.d_blob + pf_at) : nullptr;
+  *d_pl = table ? reinterpret_cast<const YuvPlaneD*>(sl.d_blob + pf_at) : nullptr;
   StageTimer t(h, 0, s);
   LetterboxMultiP lb;
   lb.fr = *d_desc; lb.taps = reinterpret_cast<const int*>(sl.d_blob + taps_at); lb.out = sl.d_lb; lb.dst_w = S_w; lb.dst_h = S_h;
-  launch_letterbox_multi(lb, n, transposed, s, *d_pf);
+  launch_letterbox_multi(lb, n, transposed, s, *d_pf, *d_pl);
   t.launches = 1;
   return FDT_OK;
 }
@@ -779,7 +858,9 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
   const double* d_geom = nullptr;
   int orientation = a.orientation;
   const PixFmt* d_pf = nullptr;
-  const int rc = a.rg ? stage_ragged(h, sl, a, off, n, &d_desc, &d_geom, &orientation, &d_pf) : stage_uniform(h, sl, a, off, n, &d_fr);
+  const YuvPlaneD* d_pl = nullptr;
+  const int rc = a.rg ? stage_ragged(h, sl, a, off, n, &d_desc, &d_geom, &orientation, &d_pf, &d_pl)
+                      : stage_uniform(h, sl, a, off, n, &d_fr);
   if (rc != FDT_OK) return rc;
   {
     StageTimer t(h, 1, s);
@@ -809,7 +890,7 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
                       cudaMemcpyDeviceToHost, s);
   }
   job->off = off; job->n = n; job->d_fr = d_fr; job->d_desc = d_desc; job->active = true; job->orientation = orientation;
-  job->d_pf = d_pf;
+  job->d_pf = d_pf; job->d_pl = d_pl;
   return FDT_OK;
 }
 
@@ -887,7 +968,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
       wp.out_size = kMeshInput; wp.flip_odd = 0; wp.crops = sl.d_crops;
       set_warp_layout(wp, a.lay);
       wp.fr = job.d_desc; wp.orientation = job.orientation; wp.pf = d_pf;
-      launch_warp_affine(wp, s);
+      launch_warp_affine(wp, s, job.d_pl);
       t.launches = 1;
     }
     {
@@ -970,7 +1051,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
           wp.out_size = kIrisInput; wp.flip_odd = 1; wp.crops = sl.d_eye_crops;
           set_warp_layout(wp, a.lay);
           wp.fr = job.d_desc; wp.orientation = job.orientation; wp.pf = d_pf;
-          launch_warp_affine(wp, s);
+          launch_warp_affine(wp, s, job.d_pl);
           t.launches = 1;
         }
         {
@@ -1104,13 +1185,90 @@ int check_frames(fdt_handle* h, const fdt_frame* frames, const int32_t* orientat
   return FDT_OK;
 }
 
+// fdt_detect_yuv_planes' argument checks, every descriptor before any work; *lay receives the frames' staged layouts.
+int check_planes(fdt_handle* h, const fdt_yuv_planes* frames, const int32_t* orientations, int n, int mode, int mem_kind,
+                 const fdt_face* out_faces, const int32_t* out_counts, std::vector<FrameLayout>* lay) {
+  if (n < 0 || (n > 0 && !frames)) return fail(h, FDT_ERR_BAD_ARG, "bad frame list");
+  if (mem_kind != FDT_MEM_HOST && mem_kind != FDT_MEM_DEVICE) return fail(h, FDT_ERR_BAD_ARG, "unknown mem_kind");
+  if (int rc = check_mode(h, mode)) return rc;
+  if (n > 0 && (!out_faces || !out_counts)) return fail(h, FDT_ERR_BAD_ARG, "null output buffers");
+  static const char* const kPlane[3] = {"plane Y", "plane U", "plane V"};
+  lay->assign(n, FrameLayout());
+  for (int i = 0; i < n; ++i) {
+    const fdt_yuv_planes& f = frames[i];
+    auto at = [i] { return "frame " + std::to_string(i) + ": "; };   // built on failure only: the list can be thousands long
+    if (f.width <= 0 || f.height <= 0 || (f.width & 1) || (f.height & 1))
+      return fail(h, FDT_ERR_BAD_ARG, at() + "YUV 4:2:0 frames need an even, positive width and height");
+    for (int k = 0; k < 3; ++k)
+      if (!f.plane[k]) return fail(h, FDT_ERR_BAD_ARG, at() + kPlane[k] + " is NULL");
+    if (f.pixel_stride != 1 && f.pixel_stride != 2) return fail(h, FDT_ERR_BAD_ARG, at() + "pixel_stride must be 1 or 2");
+    for (int k = 0; k < 3; ++k)
+      if (f.row_stride[k] <= 0) return fail(h, FDT_ERR_BAD_ARG, at() + kPlane[k] + ": row_stride must be positive");
+    if (f.row_stride[0] < f.width) return fail(h, FDT_ERR_SIZE_MISMATCH, at() + "plane Y: row_stride smaller than width");
+    for (int k = 1; k < 3; ++k)
+      if (f.row_stride[k] < chroma_cols(f))
+        return fail(h, FDT_ERR_SIZE_MISMATCH, at() + kPlane[k] + ": row_stride smaller than (width / 2 - 1) * pixel_stride + 1");
+    if (orientations && (orientations[i] < 1 || orientations[i] > 8))
+      return fail(h, FDT_ERR_BAD_ARG, at() + "orientation must be an EXIF value 1..8");
+    (*lay)[i] = plane_layout(f);
+  }
+  return FDT_OK;
+}
+
+// FDT_MEM_DEVICE pointers of one call: p must be in the handle's device memory.  A pointer inside an allocation this call has
+// already checked needs no driver query: fdt_detect_yuv_planes checks three planes per frame, and decoder surfaces, tensors and
+// their planes usually share a few allocations.  `ranges` keeps the last few checked allocations (driver cuPointerGetAttributes,
+// resolved at run time like the tensor-map encoder; without it every pointer is queried).
+bool device_pointer_ok(fdt_handle* h, const void* p, std::vector<std::pair<uintptr_t, uintptr_t>>* ranges) {
+  const uintptr_t a = reinterpret_cast<uintptr_t>(p);
+  for (const auto& r : *ranges)
+    if (a >= r.first && a < r.second) return true;
+  cudaPointerAttributes pa;
+  const bool ok = cudaPointerGetAttributes(&pa, p) == cudaSuccess &&
+                  (pa.type == cudaMemoryTypeDevice || pa.type == cudaMemoryTypeManaged) && pa.device == h->cfg.device;
+  cudaGetLastError();
+  if (!ok) return false;
+  using AttrsFn = CUresult (*)(unsigned, CUpointer_attribute*, void**, CUdeviceptr);
+  static const AttrsFn attrs = [] {
+    void* f = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuPointerGetAttributes", &f, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) f = nullptr;
+    return reinterpret_cast<AttrsFn>(f);
+  }();
+  CUdeviceptr start = 0;
+  size_t size = 0;
+  CUpointer_attribute which[2] = {CU_POINTER_ATTRIBUTE_RANGE_START_ADDR, CU_POINTER_ATTRIBUTE_RANGE_SIZE};
+  void* out[2] = {&start, &size};
+  if (attrs && attrs(2, which, out, (CUdeviceptr)a) == CUDA_SUCCESS && size > 0 && a >= start && a < start + size) {
+    if (ranges->size() == 8) ranges->erase(ranges->begin());
+    ranges->emplace_back((uintptr_t)start, (uintptr_t)(start + size));
+  }
+  return true;
+}
+
+// What a ragged call was given: fdt_frame descriptors (fdt_detect_frames, the JPEG batch) or fdt_yuv_planes descriptors.
+enum class FrameList { kFrames, kYuvPlanes };
+
+// fdt_detect_frames (kFrames: `frames`) and fdt_detect_yuv_planes (kYuvPlanes: `planes`, frames unused) on one device.
 int detect_frames_single(fdt_handle* h, const fdt_frame* frames, const int32_t* orientations, int n, int mode, int mem_kind,
-                         fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris) {
+                         fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris,
+                         FrameList list = FrameList::kFrames, const fdt_yuv_planes* planes = nullptr) {
   if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
   Ragged rg;
-  if (int rc = check_frames(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, &rg.lay)) return rc;
+  if (list == FrameList::kYuvPlanes) {
+    if (int rc = check_planes(h, planes, orientations, n, mode, mem_kind, out_faces, out_counts, &rg.lay)) return rc;
+    rg.planes = planes;
+    rg.pframes.resize(n);
+    for (int i = 0; i < n; ++i) {
+      const fdt_yuv_planes& f = planes[i];
+      rg.pframes[i] = fdt_frame{f.plane[0], f.width, f.height, mem_kind == FDT_MEM_HOST ? f.width : f.row_stride[0], FDT_FMT_YUV_I420};
+    }
+    frames = rg.pframes.data();
+  } else if (int rc = check_frames(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, &rg.lay)) {
+    return rc;
+  }
   cudaSetDevice(h->cfg.device);
-  if (mem_kind == FDT_MEM_DEVICE)
+  if (mem_kind == FDT_MEM_DEVICE && list == FrameList::kFrames)
     for (int i = 0; i < n; ++i) {
       cudaPointerAttributes pa;
       const bool ok = cudaPointerGetAttributes(&pa, frames[i].data) == cudaSuccess &&
@@ -1118,6 +1276,14 @@ int detect_frames_single(fdt_handle* h, const fdt_frame* frames, const int32_t* 
       cudaGetLastError();
       if (!ok) return fail(h, FDT_ERR_BAD_ARG, "frame " + std::to_string(i) + ": FDT_MEM_DEVICE frames must be in the handle's device memory");
     }
+  if (mem_kind == FDT_MEM_DEVICE && list == FrameList::kYuvPlanes) {
+    static const char* const kPlane[3] = {"plane Y", "plane U", "plane V"};
+    std::vector<std::pair<uintptr_t, uintptr_t>> ranges;
+    for (int i = 0; i < n; ++i)
+      for (int k = 0; k < 3; ++k)
+        if (!device_pointer_ok(h, planes[i].plane[k], &ranges))
+          return fail(h, FDT_ERR_BAD_ARG, "frame " + std::to_string(i) + ": " + kPlane[k] + ": FDT_MEM_DEVICE planes must be in the handle's device memory");
+  }
   h->launches = 0;
   h->h2d_bytes = 0;
   for (int i = 0; i < kNumStages; ++i) { h->stage_ms[i] = 0; h->stage_launches[i] = 0; }
@@ -1177,6 +1343,20 @@ int detect_frames_multi(fdt_handle* h, const fdt_frame* frames, const int32_t* o
                                 out_faces + lo * mf, out_counts + lo,
                                 out_mesh ? out_mesh + lo * mf * FDT_MESH_FLOATS : nullptr,
                                 out_iris ? out_iris + lo * mf * FDT_IRIS_FLOATS : nullptr);
+  });
+}
+
+int detect_planes_multi(fdt_handle* h, const fdt_yuv_planes* planes, const int32_t* orientations, int n, int mode, int mem_kind,
+                        fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris) {
+  std::vector<FrameLayout> lay;
+  if (int rc = check_planes(h, planes, orientations, n, mode, mem_kind, out_faces, out_counts, &lay)) return rc;
+  if (mem_kind != FDT_MEM_HOST) return fail(h, FDT_ERR_UNSUPPORTED, "a multi-device handle takes host frames (device memory belongs to one device)");
+  return on_shards(h, n, [=](fdt_handle* sh, int lo, int hi) {
+    const size_t mf = (size_t)sh->max_faces;
+    return detect_frames_single(sh, nullptr, orientations ? orientations + lo : nullptr, hi - lo, mode, mem_kind,
+                                out_faces + lo * mf, out_counts + lo,
+                                out_mesh ? out_mesh + lo * mf * FDT_MESH_FLOATS : nullptr,
+                                out_iris ? out_iris + lo * mf * FDT_IRIS_FLOATS : nullptr, FrameList::kYuvPlanes, planes + lo);
   });
 }
 
@@ -1733,6 +1913,15 @@ int32_t fdt_detect_frames_oriented(fdt_handle* h, const fdt_frame* frames, const
   std::lock_guard<std::mutex> g(h->mu);
   if (!h->shards.empty()) return detect_frames_multi(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
   return detect_frames_single(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
+}
+
+int32_t fdt_detect_yuv_planes(fdt_handle* h, const fdt_yuv_planes* frames, const int32_t* orientations, int32_t n, int32_t mode,
+                              int32_t mem_kind, fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris) {
+  if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
+  std::lock_guard<std::mutex> g(h->mu);
+  if (!h->shards.empty()) return detect_planes_multi(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
+  return detect_frames_single(h, nullptr, orientations, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris,
+                              FrameList::kYuvPlanes, frames);
 }
 
 int32_t fdt_detect_jpeg_batch(fdt_handle* h, const uint8_t* const* images, const size_t* sizes, int32_t n, int32_t mode,

@@ -130,6 +130,20 @@ struct FrameD {
   int tx, ty;              // offsets (ints) of the frame's x taps [4][new_w] and y taps [6][new_h] in the chunk's tap table
   int orientation;         // EXIF 1..8: the upright image is exif_transform(stored frame, orientation); w, h are the stored size
 };
+// Separate-plane YUV 4:2:0 frames (fdt_detect_yuv_planes) in device memory whose U and V planes FrameD cannot describe (different
+// strides, or more than an int apart): the chroma samples of pixel (x, y) are u[(y / 2) * u_stride + (x / 2) * ps] and
+// v[(y / 2) * v_stride + (x / 2) * ps]; the frame's FrameD gives the Y plane.  One entry per frame of the chunk, in the chunk blob.
+struct YuvPlaneD {
+  const uint8_t* u;
+  const uint8_t* v;
+  int u_stride, v_stride, ps, reserved;
+};
+#ifdef __CUDACC__
+__device__ __forceinline__ void load_yuv_planes(const uint8_t* yrow, int crow, int x, const YuvPlaneD& q, int* v) {
+  const size_t cx = (size_t)(x >> 1) * q.ps;
+  yuv_to_bgr(yrow[x], q.u[(size_t)crow * q.u_stride + cx], q.v[(size_t)crow * q.v_stride + cx], v);
+}
+#endif
 // k_letterbox_multi: k_letterbox / k_letterbox_yuv per frame.  taps (host-built, resize_linear_taps): per distinct size and
 // orientation x0, x1, ax0, ax1 (new_w each), then y0, y1, by0, by1, cy0, cy1 (new_h each; cy = y / 2, read for YUV frames only),
 // all of the upright image with the flips folded in.  transposed = true launches the variant that also takes frames of
@@ -144,7 +158,10 @@ struct LetterboxMultiP {
 // frames; unused for YUV frames), FrameD::channels its pixel step.  Non-null launches the variant that reads every packed or planar
 // frame through pf, whatever its orientation.  (A kernel argument of its own, behind B: FrameD and LetterboxMultiP keep their
 // sizes, which the existing variants' code depends on.)
-void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s, const PixFmt* pf = nullptr);
+// pl (device, [B]): the chunk's frames are all separate-plane YUV frames read through their YuvPlaneD (any orientation; pf null).
+// (A kernel argument of its own, behind pfs, for the same reason.)
+void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s, const PixFmt* pf = nullptr,
+                            const YuvPlaneD* pl = nullptr);
 // k_letterbox_rgb: k_letterbox (transposed = 0) or k_letterbox_tr (transposed = 1, orientations 5-8) with every tap read through
 // pf; lb.channels unused.  (A struct of its own: the existing parameter blocks keep their layouts.)
 struct LetterboxRgbP {
@@ -370,7 +387,9 @@ struct WarpP {
   // makes for the existing instantiations.)
   const PixFmt* pf = nullptr;
 };
-void launch_warp_affine(const WarpP& p, cudaStream_t s);
+// pl: ragged chunks of separate-plane YUV frames (k_letterbox_multi's table, indexed like fr); non-null launches the instantiation
+// that reads every frame's chroma through it.  (A kernel argument of its own: WarpP has no room left, see pf.)
+void launch_warp_affine(const WarpP& p, cudaStream_t s, const YuvPlaneD* pl = nullptr);
 
 // ---- mesh / iris post-processing ----
 struct MeshPostP {

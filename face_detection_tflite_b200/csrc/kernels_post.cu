@@ -4,7 +4,7 @@
 //                      letterbox removal -> gates   (one block per image)
 //   k_warp_affine      cv::warpAffine(INTER_LINEAR, BORDER_CONSTANT 0) into square BGR crops (192 face / 64 eye);
 //                      YUV 4:2:0 frames are converted tap by tap (in-frame taps only); RGB, RGBA and planar RGB frames
-//                      are read through their PixFmt
+//                      are read through their PixFmt; separate-plane YUV frames through their YuvPlaneD
 //   k_mesh_post        _unpackLandmarks + transformMeshToAbsolute + face-flag sigmoid
 //   k_iris_post        _unpackLandmarks(clamp: false) + transformIrisNormToAbsolute + iris-centre eye keypoints
 #include "fdt_math.h"
@@ -227,8 +227,9 @@ __device__ __forceinline__ long long sat_round_ll(double v) { return (long long)
 // sample) it is.  Folding the orientation into the affine map instead would change the rint rounding above.
 // kFmt: the frame (uniform) or some frame of the chunk (ragged) is RGB / RGBA / planar RGB; every packed or planar frame's taps
 // are read through its PixFmt (p.pf[0], or p.pf[frame]), so a crop equals the crop of the BGR image.
-template <bool kRagged, bool kOriented, bool kFmt>
-__global__ void k_warp_affine(WarpP p) {
+// kPlanes (ragged only): every frame of the chunk is a separate-plane YUV frame, its chroma read through pl[frame].
+template <bool kRagged, bool kOriented, bool kFmt, bool kPlanes>
+__global__ void k_warp_affine(WarpP p, const YuvPlaneD* pl) {
   const int f = blockIdx.y;
   if (f >= p.ncrops) return;
   const int S = p.out_size;
@@ -241,6 +242,8 @@ __global__ void k_warp_affine(WarpP p) {
   const bool tr = orient >= 5;
   PixFmt pf;
   if (kFmt) pf = p.pf[kRagged ? p.crop_img[f] : 0];
+  YuvPlaneD q;
+  if (kPlanes) q = pl[p.crop_img[f]];
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < S * S; i += gridDim.x * blockDim.x) {
     int y = i / S, x = i - y * S;
     long long adelta = sat_round_ll(A[0] * x * 1024.0);
@@ -269,6 +272,12 @@ __global__ void k_warp_affine(WarpP p) {
         yy = tr ? fx : fy;
       }
       const int row_stride = kRagged ? d->row_stride : p.row_stride;
+      if (kPlanes) {
+        int v[3];
+        load_yuv_planes(src + (size_t)yy * row_stride, yy >> 1, xx, q, v);
+        acc[0] += v[0] * iw[t]; acc[1] += v[1] * iw[t]; acc[2] += v[2] * iw[t];
+        continue;
+      }
       if (kRagged ? d->channels == 0 : p.yuv) {
         const uint8_t* c = (kRagged ? d->c : src + p.c_off) + (size_t)(yy >> 1) * (kRagged ? d->c_row_stride : p.c_row_stride) +
                            (size_t)(xx >> 1) * (kRagged ? d->c_step : p.c_step);
@@ -393,19 +402,25 @@ void launch_decode_nms(const DecodeP& p, int B, cudaStream_t s) {
 
 template <bool kFmt> void launch_warp(const WarpP& p, dim3 grid, cudaStream_t s) {
   if (p.orientation != 1) {
-    if (p.fr) k_warp_affine<true, true, kFmt><<<grid, 256, 0, s>>>(p);
-    else k_warp_affine<false, true, kFmt><<<grid, 256, 0, s>>>(p);
+    if (p.fr) k_warp_affine<true, true, kFmt, false><<<grid, 256, 0, s>>>(p, nullptr);
+    else k_warp_affine<false, true, kFmt, false><<<grid, 256, 0, s>>>(p, nullptr);
   } else {
-    if (p.fr) k_warp_affine<true, false, kFmt><<<grid, 256, 0, s>>>(p);
-    else k_warp_affine<false, false, kFmt><<<grid, 256, 0, s>>>(p);
+    if (p.fr) k_warp_affine<true, false, kFmt, false><<<grid, 256, 0, s>>>(p, nullptr);
+    else k_warp_affine<false, false, kFmt, false><<<grid, 256, 0, s>>>(p, nullptr);
   }
 }
 
-void launch_warp_affine(const WarpP& p, cudaStream_t s) {
+void launch_warp_affine(const WarpP& p, cudaStream_t s, const YuvPlaneD* pl) {
   if (p.ncrops <= 0) return;
   dim3 grid((p.out_size * p.out_size + 255) / 256, p.ncrops);
-  if (p.pf) launch_warp<true>(p, grid, s);
-  else launch_warp<false>(p, grid, s);
+  if (pl) {
+    if (p.orientation != 1) k_warp_affine<true, true, false, true><<<grid, 256, 0, s>>>(p, pl);
+    else k_warp_affine<true, false, false, true><<<grid, 256, 0, s>>>(p, pl);
+  } else if (p.pf) {
+    launch_warp<true>(p, grid, s);
+  } else {
+    launch_warp<false>(p, grid, s);
+  }
 }
 
 void launch_mesh_post(const MeshPostP& p, cudaStream_t s) {

@@ -1,7 +1,7 @@
 // Preprocessing kernels: fused letterbox (cv::resize INTER_LINEAR 8U fixed point +
 // copyMakeBorder(0) + BGRA/GRAY->BGR, or cvtColor YUV2BGR for NV12 / NV21 / I420 frames; k_letterbox_multi for chunks of
 // frames of different sizes and formats; k_letterbox_tr for frames stored transposed; k_letterbox_rgb for RGB, RGBA and planar
-// RGB frames, read through their PixFmt) and the [-1,1] normalisation.
+// RGB frames, read through their PixFmt; k_letterbox_multi<., ., true> for separate-plane YUV frames) and the [-1,1] normalisation.
 // Reference: convertImageToTensor / bgrMatToSignedFloat32 (lib/src/util/helpers.dart:303-421).
 #include "kernels.h"
 
@@ -165,20 +165,24 @@ __global__ void __launch_bounds__(256) k_letterbox_tr(LetterboxTrP p, int B) {
 // folded into the taps.
 // kFmt: the chunk also holds RGB / RGBA / planar RGB frames; every packed or planar frame is read through its PixFmt pfs[b]
 // (launched with kTransposed = true, for a chunk of any orientations).
+// kPlanes: every frame of the chunk is a separate-plane YUV frame whose chroma is read through its YuvPlaneD pls[b] (launched with
+// kTransposed = true and kFmt = false); the chroma row of a tap is the same as above, only its address differs.
 template <bool kFmt>
 __device__ __forceinline__ void load_packed(const uint8_t* px, int channels, const PixFmt& pf, int* v) {
   if (kFmt) load_pix(px, pf, v);
   else load_bgr(px, channels, v);
 }
 
-template <bool kTransposed, bool kFmt>
-__global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int B, const PixFmt* pfs) {
+template <bool kTransposed, bool kFmt, bool kPlanes>
+__global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int B, const PixFmt* pfs, const YuvPlaneD* pls) {
   const int x = blockIdx.x * 64 + (threadIdx.x & 63), y = blockIdx.y * 4 + (threadIdx.x >> 6);
   if (x >= p.dst_w || y >= p.dst_h) return;
   for (int b = blockIdx.z; b < B; b += gridDim.z) {
     const FrameD f = p.fr[b];
     PixFmt pf;
     if (kFmt) pf = pfs[b];
+    YuvPlaneD pl;
+    if (kPlanes) pl = pls[b];
     const int dy = y - f.pad_top, dx = x - f.pad_left;
     uchar3 o = make_uchar3(0, 0, 0);
     if (dy >= 0 && dy < f.new_h && dx >= 0 && dx < f.new_w) {
@@ -191,7 +195,12 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
         int t00[3], t01[3], t10[3], t11[3];
         const uint8_t* r0 = f.y + (size_t)ra * f.row_stride;
         const uint8_t* r1 = f.y + (size_t)rb * f.row_stride;
-        if (f.channels) {
+        if (kPlanes) {
+          load_yuv_planes(r0, ra >> 1, ca, pl, t00);
+          load_yuv_planes(r1, rb >> 1, ca, pl, t01);
+          load_yuv_planes(r0, ra >> 1, cb, pl, t10);
+          load_yuv_planes(r1, rb >> 1, cb, pl, t11);
+        } else if (f.channels) {
           load_packed<kFmt>(r0 + (size_t)ca * f.channels, f.channels, pf, t00);
           load_packed<kFmt>(r1 + (size_t)ca * f.channels, f.channels, pf, t01);
           load_packed<kFmt>(r0 + (size_t)cb * f.channels, f.channels, pf, t10);
@@ -207,7 +216,8 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
 #pragma unroll
         for (int c = 0; c < 3; ++c) res[c] = resize_linear(t00[c], t01[c], t10[c], t11[c], wa, wb, va, vb);
       } else if (f.identity) {
-        if (f.channels) load_packed<kFmt>(f.y + (size_t)dy * f.row_stride + (size_t)dx * f.channels, f.channels, pf, res);
+        if (kPlanes) load_yuv_planes(f.y + (size_t)dy * f.row_stride, dy >> 1, dx, pl, res);
+        else if (f.channels) load_packed<kFmt>(f.y + (size_t)dy * f.row_stride + (size_t)dx * f.channels, f.channels, pf, res);
         else load_yuv(f.y + (size_t)dy * f.row_stride, f.c + (size_t)(dy >> 1) * f.c_row_stride, dx, f, res);
       } else {
         const int* tx = p.taps + f.tx;
@@ -217,7 +227,13 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
         int t00[3], t01[3], t10[3], t11[3];
         const uint8_t* r0 = f.y + (size_t)ya * f.row_stride;
         const uint8_t* r1 = f.y + (size_t)yb * f.row_stride;
-        if (f.channels) {
+        if (kPlanes) {
+          const int ca = ty[4 * f.new_h + dy], cb = ty[5 * f.new_h + dy];
+          load_yuv_planes(r0, ca, xa, pl, t00);
+          load_yuv_planes(r0, ca, xb, pl, t01);
+          load_yuv_planes(r1, cb, xa, pl, t10);
+          load_yuv_planes(r1, cb, xb, pl, t11);
+        } else if (f.channels) {
           load_packed<kFmt>(r0 + (size_t)xa * f.channels, f.channels, pf, t00);
           load_packed<kFmt>(r0 + (size_t)xb * f.channels, f.channels, pf, t01);
           load_packed<kFmt>(r1 + (size_t)xa * f.channels, f.channels, pf, t10);
@@ -320,12 +336,13 @@ void launch_letterbox_tr(const LetterboxTrP& p, int B, cudaStream_t s) {
   else k_letterbox_tr<false><<<grid, 256, 0, s>>>(p, B);
 }
 
-void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s, const PixFmt* pf) {
+void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s, const PixFmt* pf, const YuvPlaneD* pl) {
   if (B <= 0) return;
   dim3 grid((unsigned)((p.dst_w + 63) / 64), (unsigned)((p.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
-  if (pf) k_letterbox_multi<true, true><<<grid, 256, 0, s>>>(p, B, pf);
-  else if (transposed) k_letterbox_multi<true, false><<<grid, 256, 0, s>>>(p, B, pf);
-  else k_letterbox_multi<false, false><<<grid, 256, 0, s>>>(p, B, pf);
+  if (pl) k_letterbox_multi<true, false, true><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  else if (pf) k_letterbox_multi<true, true, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  else if (transposed) k_letterbox_multi<true, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  else k_letterbox_multi<false, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
 }
 
 void launch_letterbox_rgb(const LetterboxRgbP& p, int B, bool transposed, cudaStream_t s) {

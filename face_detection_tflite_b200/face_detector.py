@@ -122,6 +122,26 @@ def _orientations(orientations, n: int):
     return np.array([_orientation(o, "orientations[%d]" % i) for i, o in enumerate(orientations)], np.int32)
 
 
+def _plane_extents(i: int, strides, w, h, ps) -> tuple:
+    """The sampled extent in bytes of the Y, U and V plane of a separate-plane YUV 4:2:0 frame, (rows - 1) * stride +
+    (cols - 1) * step + 1; ValueError for the arguments fdt_detect_yuv_planes refuses."""
+    vals = (w, h, ps, *strides)
+    if len(strides) != 3 or not all(isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in vals):
+        raise ValueError("frame %d: width, height, pixel stride and the three row strides must be integers" % i)
+    if w <= 0 or h <= 0 or w % 2 or h % 2:
+        raise ValueError("frame %d: YUV 4:2:0 frames need an even, positive width and height" % i)
+    if ps not in (1, 2):
+        raise ValueError("frame %d: the chroma pixel stride must be 1 or 2, got %r" % (i, ps))
+    if min(strides) <= 0:
+        raise ValueError("frame %d: row strides must be positive (bottom-up frames are not supported)" % i)
+    cc = (w // 2 - 1) * ps + 1
+    if strides[0] < w:
+        raise ValueError("frame %d: Y row stride smaller than width" % i)
+    if strides[1] < cc or strides[2] < cc:
+        raise ValueError("frame %d: chroma row stride smaller than (width / 2 - 1) * pixelStride + 1" % i)
+    return (h - 1) * int(strides[0]) + w, (h // 2 - 1) * int(strides[1]) + cc, (h // 2 - 1) * int(strides[2]) + cc
+
+
 def _upright(w, h, orientation) -> tuple:
     """Size of the upright image of a w x h frame stored in `orientation`: 5-8 swap the axes."""
     return (h, w) if orientation >= 5 else (w, h)
@@ -424,6 +444,90 @@ class FaceDetector:
             descs.append((ptr, w, h, stride, mt))
         self._check()
         return self._detect_frames(descs, mode, memKind, orients)
+
+    # -- YUV 4:2:0 frames as three separate planes: decoder surfaces, AVFrames, Android YUV_420_888 images --------------------
+    def detectFacesFromYuvPlanes(self, frames, *, mode: FaceDetectionMode = FaceDetectionMode.full,
+                                 orientations=None) -> List[List[Face]]:
+        """Faces in YUV 4:2:0 frames given as (y, u, v) triples of 2-D uint8 arrays (fdt_detect_yuv_planes): Y is height x width,
+        U and V are height / 2 x width / 2.  strides[0] of each plane is its row stride; strides[1] is 1 for Y and the chroma
+        pixel stride, 1 or 2 and the same for U and V.  NumPy views describe every layout without a copy: an NV12 chroma plane
+        uv gives uv[:, 0::2], uv[:, 1::2]; an AVFrame gives its three planes; an Android YUV_420_888 image its three buffers
+        (pixelStride 2: U and V views into one interleaved buffer, or buffers that end at their last sample).  Returns one list
+        of faces per frame, normalised to its upright image.  orientations: one EXIF orientation 1..8 per frame, or None."""
+        frames = list(frames)
+        orients = _orientations(orientations, len(frames))
+        descs = []
+        for i, fr in enumerate(frames):
+            if not isinstance(fr, (tuple, list)) or len(fr) != 3 or \
+                    not all(isinstance(p, np.ndarray) and p.dtype == np.uint8 and p.ndim == 2 for p in fr):
+                raise ValueError("frame %d: expected (y, u, v), three 2-D uint8 arrays" % i)
+            y, u, v = fr
+            h, w = y.shape
+            if u.shape != (h // 2, w // 2) or v.shape != (h // 2, w // 2):
+                raise ValueError("frame %d: U and V must be height / 2 x width / 2 (Y is %d x %d)" % (i, h, w))
+            if y.strides[1] != 1:
+                raise ValueError("frame %d: the Y plane's pixels must be adjacent (strides[1] == 1)" % i)
+            if u.strides[1] != v.strides[1]:
+                raise ValueError("frame %d: U and V need the same pixel stride" % i)
+            strides = (y.strides[0], u.strides[0], v.strides[0])
+            _plane_extents(i, strides, w, h, u.strides[1])
+            descs.append(((y.ctypes.data, u.ctypes.data, v.ctypes.data), strides, w, h, u.strides[1]))
+        self._check()
+        faces, counts, mesh, iris = self._detect_planes(descs, mode, _ffi.FDT_MEM_HOST, orients)
+        sizes = [_upright(d[2], d[3], 1 if orients is None else orients[i]) for i, d in enumerate(descs)]
+        return self._faces_per_frame(faces, counts, mesh, iris, sizes)
+
+    def detectYuvPlanesRaw(self, frames, *, mode: FaceDetectionMode = FaceDetectionMode.fast, memKind: int = _ffi.FDT_MEM_HOST,
+                           orientations=None):
+        """fdt_detect_yuv_planes with array outputs, as detectFramesRaw.  `frames` is a list of
+        ((y, u, v), (yStride, uStride, vStride), width, height, pixelStride) tuples: the planes are integer device pointers with
+        memKind=FDT_MEM_DEVICE (e.g. torch CUDA tensors' data_ptr()), else numpy arrays or bytes, each holding at least its
+        plane's sampled extent from its first byte."""
+        if memKind not in (_ffi.FDT_MEM_HOST, _ffi.FDT_MEM_DEVICE):
+            raise ValueError("memKind must be FDT_MEM_HOST or FDT_MEM_DEVICE")
+        frames = list(frames)
+        orients = _orientations(orientations, len(frames))
+        descs, keep = [], []
+        for i, fr in enumerate(frames):
+            if not isinstance(fr, (tuple, list)) or len(fr) != 5 or not isinstance(fr[0], (tuple, list)) or len(fr[0]) != 3 \
+                    or not isinstance(fr[1], (tuple, list)):
+                raise ValueError("frame %d: expected ((y, u, v), (yStride, uStride, vStride), width, height, pixelStride)" % i)
+            planes, strides, w, h, ps = fr
+            extents = _plane_extents(i, tuple(strides), w, h, ps)
+            ptrs = []
+            for k, (p, ext) in enumerate(zip(planes, extents)):
+                if memKind == _ffi.FDT_MEM_DEVICE:
+                    if isinstance(p, bool) or not isinstance(p, int):
+                        raise ValueError("frame %d: FDT_MEM_DEVICE planes are integer device pointers" % i)
+                    ptrs.append(p)
+                    continue
+                if isinstance(p, int):
+                    raise ValueError("frame %d: host planes are numpy arrays or bytes" % i)
+                buf = np.frombuffer(p, np.uint8) if not isinstance(p, np.ndarray) else p
+                if buf.dtype != np.uint8 or not buf.flags.c_contiguous or buf.size < ext:
+                    raise ValueError("frame %d: plane %s is not a contiguous uint8 buffer of at least its sampled extent (%d bytes)"
+                                     % (i, "YUV"[k], ext))
+                keep.append(buf)
+                ptrs.append(buf.ctypes.data)
+            descs.append((tuple(ptrs), tuple(int(s) for s in strides), int(w), int(h), int(ps)))
+        self._check()
+        return self._detect_planes(descs, mode, memKind, orients)
+
+    def _detect_planes(self, descs, mode, memKind, orients):
+        n = len(descs)
+        arr = (_ffi.FdtYuvPlanes * max(1, n))()
+        for k, (ptrs, strides, w, h, ps) in enumerate(descs):
+            arr[k].plane = (C.c_void_p * 3)(*ptrs)
+            arr[k].row_stride = (C.c_int32 * 3)(*strides)
+            arr[k].width, arr[k].height, arr[k].pixel_stride = w, h, ps
+        faces, counts, mesh, iris = self._outputs(n, mode)
+        rc = self._lib.fdt_detect_yuv_planes(self._h, arr, orients.ctypes.data_as(_ffi.i32p) if orients is not None else None, n,
+                                             int(FaceDetectionMode(mode)), memKind, faces, counts.ctypes.data_as(_ffi.i32p),
+                                             mesh.ctypes.data_as(_ffi.f32p) if mesh is not None else None,
+                                             iris.ctypes.data_as(_ffi.f32p) if iris is not None else None)
+        if rc != _ffi.FDT_OK:
+            _raise(self._lib, self._h, rc)
+        return faces, counts[:n], mesh, iris
 
     def detectFacesFromBytesBatch(self, images, *, mode: FaceDetectionMode = FaceDetectionMode.full) -> List[Optional[List[Face]]]:
         """detectFacesFromBytes over a list of encoded images (JPEG) in one call (fdt_detect_jpeg_batch).  An image that

@@ -223,6 +223,47 @@ FDT_EXPORT int32_t fdt_detect_frames_oriented(fdt_handle* h, const fdt_frame* fr
                                               int32_t mode, int32_t mem_kind, fdt_face* out_faces, int32_t* out_counts,
                                               float* out_mesh, float* out_iris);
 
+/* One YUV 4:2:0 frame given as three planes, each with its own base pointer and row stride (fdt_detect_yuv_planes): hardware
+ * decoder surfaces (NVDEC / PyNvVideoCodec / FFmpeg cuda frames: pitched NV12 with the chroma at pitch * surface height), FFmpeg
+ * and PyAV AVFrames (data[] and linesize[] of yuv420p / nv12) and Android YUV_420_888 images (three plane buffers, rowStride,
+ * and a chroma pixelStride of 1 or 2).  The samples of pixel (x, y), x < width, y < height:
+ *   Y  plane[0][y * row_stride[0] + x]
+ *   U  plane[1][(y / 2) * row_stride[1] + (x / 2) * pixel_stride]
+ *   V  plane[2][(y / 2) * row_stride[2] + (x / 2) * pixel_stride]
+ * NV12 is U = chroma, V = chroma + 1, pixel_stride 2 (NV21 the other way round); I420 / YV12 are three planes with
+ * pixel_stride 1.  width and height must be even and positive, every plane non-NULL, pixel_stride 1 or 2 and every row_stride
+ * positive (else FDT_ERR_BAD_ARG; bottom-up frames with negative strides are not taken); row_stride[0] >= width and
+ * row_stride[1], row_stride[2] >= (width / 2 - 1) * pixel_stride + 1 (else FDT_ERR_SIZE_MISMATCH).
+ * The library reads only the sampled extent of each plane, (rows - 1) * row_stride + (cols - 1) * step + 1 bytes from its base
+ * (Y: rows = height, cols = width, step 1; U and V: rows = height / 2, cols = width / 2, step = pixel_stride), so a buffer that
+ * ends at its last sample (Android's truncated last chroma row) is complete. */
+typedef struct fdt_yuv_planes {
+  const uint8_t* plane[3];   /* Y, U, V; host or device memory, per the call's mem_kind                              */
+  int32_t row_stride[3];     /* bytes between rows of each plane                                                       */
+  int32_t width, height;     /* image size (even)                                                                      */
+  int32_t pixel_stride;      /* bytes between neighbouring chroma samples of U and V: 1 (planar) or 2 (interleaved)    */
+  int32_t reserved;          /* 0                                                                                      */
+} fdt_yuv_planes;            /* 56 bytes */
+
+/* fdt_detect_frames_oriented over separate-plane YUV 4:2:0 frames (fdt_yuv_planes): outputs, chunking, the two-slot pipeline,
+ * orientations (int32 [n], or NULL for all upright), modes and multi-device splitting (host frames only) as there.  Every result
+ * equals, bit for bit, fdt_detect_frames_oriented on the same samples packed into a contiguous FDT_FMT_YUV_I420 frame.  Every
+ * descriptor is checked before any work; the first bad one returns its code and fdt_last_error names its index and plane.
+ * n == 0 returns FDT_OK.
+ * Host frames: each plane's sampled columns of every row go up (width bytes of each Y row, (width / 2 - 1) * pixel_stride + 1
+ * bytes of each U and V row; no stride padding, nothing past a plane's extent).  Interleaved chroma - pixel_stride 2, U and V one
+ * byte apart with one row stride >= width (NV12, NV21, Android views of one buffer) - goes up as one area of width bytes per row,
+ * the two extents' bytes.  So fdt_last_h2d_bytes is the sum over the frames of width * height + (height / 2) * width for
+ * interleaved chroma (what fdt_detect_frames uploads for an NV12 frame), else width * height + 2 * (height / 2) *
+ * ((width / 2 - 1) * pixel_stride + 1).  No sparse row upload in fast mode.
+ * Device frames must be in the handle's device memory; each plane pointer is checked, each allocation queried once per call.
+ * A chunk whose frames all have U and V with one row stride and less than
+ * 2^31 bytes apart (NVDEC NV12 surfaces, contiguous I420) runs the fdt_detect_frames kernels; any other chunk runs their
+ * variants that read each frame's U and V planes through a per-frame plane table. */
+FDT_EXPORT int32_t fdt_detect_yuv_planes(fdt_handle* h, const fdt_yuv_planes* frames, const int32_t* orientations, int32_t n,
+                                         int32_t mode, int32_t mem_kind, fdt_face* out_faces, int32_t* out_counts,
+                                         float* out_mesh, float* out_iris);
+
 /* fdt_detect_jpeg over n encoded images in one call.  The host parses and Huffman-decodes them on a pool of
  * min(n, hardware threads) threads; the device decodes them into a handle-owned frame arena and detects them as one mixed
  * batch (chunks of up to max_batch images and max_batch * 8 MiB of decoded BGR).  out_status[i] is FDT_OK, FDT_ERR_FORMAT
@@ -332,7 +373,7 @@ FDT_EXPORT int64_t fdt_last_launch_count(fdt_handle* h);
  * axes clamp differently at the borders, so at some sizes that set differs from orientation 1's.  RGB and RGBA frames upload as
  * BGR and BGRA do.  Planar RGB frames are read as 3 * height stacked rows: when height is a multiple of the period the same
  * pattern runs through all three planes (1280x720: 552,960 bytes per frame, as BGR), otherwise whole frames go up.  Mixed calls
- * upload whole frames. */
+ * upload whole frames; fdt_detect_yuv_planes uploads each plane's sampled columns (see there). */
 FDT_EXPORT int64_t fdt_last_h2d_bytes(fdt_handle* h);
 /* Device time in ms of the named stage summed over the last call when stage timing was enabled
  * with fdt_set_stage_timing(h,1) (adds cudaEvent records; off by default).

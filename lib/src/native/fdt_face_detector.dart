@@ -333,6 +333,78 @@ class FdtFaceDetector {
     }
   }
 
+  /// Faces in YUV 4:2:0 frames given as three planes (`fdt_detect_yuv_planes`): an Android `YUV_420_888` CameraImage maps
+  /// planes[0..2].bytes to [y], [u], [v], their bytesPerRow to the row strides and planes[1].bytesPerPixel (1 or 2) to
+  /// [pixelStride]; the buffers may end at their last sample (pixelStride 2 leaves the last chroma row short).  The sample of
+  /// pixel (x, y) is y[y * yStride + x], u[(y ~/ 2) * uStride + (x ~/ 2) * pixelStride], likewise v.  [orientations]: one
+  /// EXIF orientation (kFdtOrient*) per frame, or null for all upright; each result list refers to its frame's upright image.
+  Future<List<List<Face>>> detectFacesFromYuvPlanes(
+    List<({Uint8List y, Uint8List u, Uint8List v, int yStride, int uStride, int vStride, int pixelStride, int width, int height})> frames, {
+    FaceDetectionMode mode = FaceDetectionMode.full,
+    List<int>? orientations,
+  }) async {
+    if (orientations != null) {
+      if (orientations.length != frames.length) {
+        throw ArgumentError('orientations: one EXIF orientation per frame (${frames.length})');
+      }
+      orientations.forEach(_checkOrientation);
+    }
+    _check();
+    for (int i = 0; i < frames.length; i++) {
+      final f = frames[i];
+      if (f.width <= 0 || f.height <= 0 || f.width.isOdd || f.height.isOdd) {
+        throw ArgumentError('frame $i: YUV 4:2:0 frames need an even, positive width and height');
+      }
+      if (f.pixelStride != 1 && f.pixelStride != 2) throw ArgumentError('frame $i: pixelStride must be 1 or 2');
+      final int cols = (f.width ~/ 2 - 1) * f.pixelStride + 1;
+      if (f.yStride < f.width || f.uStride < cols || f.vStride < cols) throw ArgumentError('frame $i: row stride too small');
+      if (f.y.length < (f.height - 1) * f.yStride + f.width ||
+          f.u.length < (f.height ~/ 2 - 1) * f.uStride + cols ||
+          f.v.length < (f.height ~/ 2 - 1) * f.vStride + cols) {
+        throw ArgumentError('frame $i: a plane is shorter than its sampled extent');
+      }
+    }
+    final int n = frames.length;
+    if (n == 0) return <List<Face>>[];
+    final arena = Arena();
+    try {
+      final Pointer<FdtYuvPlanes> desc = arena<FdtYuvPlanes>(n);
+      for (int i = 0; i < n; i++) {
+        final f = frames[i];
+        final planes = [f.y, f.u, f.v];
+        final strides = [f.yStride, f.uStride, f.vStride];
+        for (int k = 0; k < 3; k++) {
+          final Pointer<Uint8> src = arena<Uint8>(planes[k].length);
+          src.asTypedList(planes[k].length).setAll(0, planes[k]);
+          desc[i].plane[k] = src;
+          desc[i].rowStride[k] = strides[k];
+        }
+        desc[i].width = f.width;
+        desc[i].height = f.height;
+        desc[i].pixelStride = f.pixelStride;
+        desc[i].reserved = 0;
+      }
+      final out = _outputs(arena, n, mode);
+      Pointer<Int32> ors = nullptr;
+      if (orientations != null) {
+        ors = arena<Int32>(n);
+        ors.asTypedList(n).setAll(0, orientations);
+      }
+      final int rc = _lib.detectYuvPlanes(_h, desc, ors, n, mode.index, kFdtMemHost, out.faces, out.counts, out.mesh, out.iris);
+      if (rc != FdtStatus.ok) {
+        _lib.throwFor(rc, _h); // ArgumentError naming the first bad frame and plane
+      }
+      return <List<Face>>[
+        for (int b = 0; b < n; b++)
+          (orientations != null && orientations[b] >= 5)
+              ? _facesOf(out, b, frames[b].height, frames[b].width)
+              : _facesOf(out, b, frames[b].width, frames[b].height),
+      ];
+    } finally {
+      arena.releaseAll();
+    }
+  }
+
   /// detectFacesFromBytes over a list of encoded images (JPEG) in one `fdt_detect_jpeg_batch` call.  An image that cannot
   /// be decoded gives `null` in its place instead of throwing, so one bad photo does not discard the batch.
   Future<List<List<Face>?>> detectFacesFromBytesBatch(

@@ -128,6 +128,23 @@ final class FdtFrame extends Struct {
   external int matType;
 }
 
+/// fdt_yuv_planes: one YUV 4:2:0 frame as a Y, a U and a V plane with their own base and row stride, U and V sharing a pixel
+/// stride of 1 or 2 (fdt_detect_yuv_planes; an Android `YUV_420_888` CameraImage's three planes); 56 bytes.
+final class FdtYuvPlanes extends Struct {
+  @Array(3)
+  external Array<Pointer<Uint8>> plane;
+  @Array(3)
+  external Array<Int32> rowStride;
+  @Int32()
+  external int width;
+  @Int32()
+  external int height;
+  @Int32()
+  external int pixelStride;
+  @Int32()
+  external int reserved;
+}
+
 typedef _DefaultConfigC = Void Function(Pointer<FdtConfig>);
 typedef _DefaultConfigD = void Function(Pointer<FdtConfig>);
 typedef _CreateExC = Int32 Function(Pointer<FdtConfig>, Pointer<Uint8>, Size, Pointer<Uint8>, Size, Pointer<Uint8>, Size,
@@ -177,6 +194,10 @@ typedef _DetectJpegBatchC = Int32 Function(Pointer<Void>, Pointer<Pointer<Uint8>
     Pointer<Int32>, Pointer<Float>, Pointer<Float>, Pointer<Int32>, Pointer<Int32>);
 typedef _DetectJpegBatchD = int Function(Pointer<Void>, Pointer<Pointer<Uint8>>, Pointer<Size>, int, int, Pointer<FdtFace>,
     Pointer<Int32>, Pointer<Float>, Pointer<Float>, Pointer<Int32>, Pointer<Int32>);
+typedef _DetectYuvPlanesC = Int32 Function(Pointer<Void>, Pointer<FdtYuvPlanes>, Pointer<Int32>, Int32, Int32, Int32,
+    Pointer<FdtFace>, Pointer<Int32>, Pointer<Float>, Pointer<Float>);
+typedef _DetectYuvPlanesD = int Function(Pointer<Void>, Pointer<FdtYuvPlanes>, Pointer<Int32>, int, int, int, Pointer<FdtFace>,
+    Pointer<Int32>, Pointer<Float>, Pointer<Float>);
 typedef _NumDevicesC = Int32 Function(Pointer<Void>);
 typedef _NumDevicesD = int Function(Pointer<Void>);
 
@@ -199,6 +220,7 @@ class FdtLibrary {
         detectBatchOriented = _lib.lookupFunction<_DetectBatchOrientedC, _DetectBatchOrientedD>('fdt_detect_batch_oriented'),
         detectFramesOriented = _lib.lookupFunction<_DetectFramesOrientedC, _DetectFramesOrientedD>('fdt_detect_frames_oriented'),
         detectJpegBatch = _lib.lookupFunction<_DetectJpegBatchC, _DetectJpegBatchD>('fdt_detect_jpeg_batch'),
+        detectYuvPlanes = _lib.lookupFunction<_DetectYuvPlanesC, _DetectYuvPlanesD>('fdt_detect_yuv_planes'),
         numDevices = _lib.lookupFunction<_NumDevicesC, _NumDevicesD>('fdt_num_devices');
 
   final DynamicLibrary _lib;
@@ -218,6 +240,7 @@ class FdtLibrary {
   final _DetectBatchOrientedD detectBatchOriented;
   final _DetectFramesOrientedD detectFramesOriented;
   final _DetectJpegBatchD detectJpegBatch;
+  final _DetectYuvPlanesD detectYuvPlanes;
   final _NumDevicesD numDevices;
 
   static FdtLibrary? _instance;
