@@ -22,6 +22,9 @@ FDT_MEM_HOST, FDT_MEM_DEVICE = 0, 1
 # oracle.jpeg_ops.exif_transform(stored, orientation)
 (FDT_ORIENT_UPRIGHT, FDT_ORIENT_MIRROR_H, FDT_ORIENT_ROT180, FDT_ORIENT_MIRROR_V, FDT_ORIENT_TRANSPOSE, FDT_ORIENT_ROT90_CW,
  FDT_ORIENT_TRANSVERSE, FDT_ORIENT_ROT90_CCW) = range(1, 9)
+# face crops of the detect calls (fdt_set_face_crops): kinds and layout flags (0 = u8 HWC BGR)
+FDT_CROP_EMBEDDING, FDT_CROP_FACE = 0, 1
+FDT_CROP_RGB, FDT_CROP_CHW, FDT_CROP_F32 = 1, 2, 4
 FDT_MAX_FACES = 100
 FDT_MESH_FLOATS = 1404
 FDT_IRIS_FLOATS = 456
@@ -50,6 +53,12 @@ class FdtYuvPlanes(C.Structure):
     pixel stride of 1 or 2 (fdt_detect_yuv_planes)."""
     _fields_ = [("plane", C.c_void_p * 3), ("row_stride", C.c_int32 * 3), ("width", C.c_int32), ("height", C.c_int32),
                 ("pixel_stride", C.c_int32), ("reserved", C.c_int32)]
+
+
+class FdtCropSpec(C.Structure):
+    """fdt_crop_spec: the face crops every detect call returns (fdt_set_face_crops), 40 bytes."""
+    _fields_ = [("struct_size", C.c_int32), ("kind", C.c_int32), ("out_size", C.c_int32), ("layout", C.c_int32),
+                ("scale", C.c_float * 3), ("bias", C.c_float * 3)]
 
 
 # every symbol include/fdt_api.h declares: name -> (restype, argtypes)
@@ -123,6 +132,9 @@ SIGNATURES = {
     "fdt_host_decode_box": (C.c_int32, [P, C.c_double, C.c_double, C.c_double, P, P]),
     "fdt_host_face_roi": (C.c_int32, [P, C.c_double, C.c_double, C.c_int32, P]),
     "fdt_host_tile_walk": (C.c_int32, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, P]),
+    "fdt_set_face_crops": (C.c_int32, [P, C.POINTER(FdtCropSpec)]),
+    "fdt_get_face_crops": (C.c_int32, [P, C.POINTER(C.c_int64), C.POINTER(P)]),
+    "fdt_copy_face_crops": (C.c_int32, [P, P, C.c_size_t, C.c_int32, i32p]),
     "fdt_last_error": (C.c_char_p, [P]),
     "fdt_version": (C.c_char_p, []),
 }

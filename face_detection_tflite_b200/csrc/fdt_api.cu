@@ -33,6 +33,7 @@ using namespace fdt;
 static_assert(sizeof(fdt_face) == 160, "fdt_face wire layout (bindings rely on it)");
 static_assert(sizeof(fdt_config) == 48, "fdt_config layout");
 static_assert(sizeof(fdt_frame) == 24, "fdt_frame layout (bindings rely on it)");
+static_assert(sizeof(fdt_crop_spec) == 40, "fdt_crop_spec layout (bindings rely on it)");
 
 namespace {
 
@@ -41,7 +42,8 @@ constexpr int kMeshInput = 192;           // face_landmark input
 constexpr int kIrisInput = 64;            // iris_landmark input
 constexpr double kMinScore = 0.5;         // lib/src/shared/face_model_config.dart:53
 constexpr double kMinSuppression = 0.3;   // lib/src/shared/face_model_config.dart:77
-constexpr int kNumStages = 9;
+constexpr int kNumStages = 10;
+constexpr int kCropStage = 9;             // fdt_get_stage_ms stage of the face-crop warps
 constexpr int kEagerSlots = 4;            // result slots per frame copied to the host with the chunk (more on demand)
 // Mixed batches: a chunk of host frames (fdt_detect_frames) or of decoded JPEGs stages at most max_batch * this many bytes,
 // e.g. 256 frames of 1920x1080 BGRA; a larger frame runs as a chunk of its own.
@@ -142,6 +144,10 @@ struct Slot {
   cudaEvent_t ev_blob = nullptr;
   double *h_eye_wh = nullptr, *d_eye_wh = nullptr;    // frame size per iris face [F][2]
   PixFmt *h_pf = nullptr, *d_pf = nullptr;             // uniform RGB-family calls: the frames' pixel rule for the crop warps
+  // face crops (fdt_set_face_crops): one pass's frame indices and inverse maps; ev_fc follows their upload
+  int *h_fc_img = nullptr, *d_fc_img = nullptr;
+  double *h_fc_aff = nullptr, *d_fc_aff = nullptr;
+  cudaEvent_t ev_fc = nullptr;
 };
 
 }  // namespace
@@ -184,6 +190,13 @@ struct fdt_handle {
   uint16_t* d_jq = nullptr;
   int jw = 0, jh = 0;                        // size of the frame in d_jframe
   uint8_t* d_jarena = nullptr; size_t jarena_cap = 0;   // fdt_detect_jpeg_batch: one chunk's decoded frames
+  // face crops of the detect calls (fdt_set_face_crops): the spec, and the last call's crops packed in a device arena
+  bool crops_on = false;
+  fdt_crop_spec crop_spec = {};
+  int crop_cap = 0;                          // faces per crop pass (the slots' ROI buffers)
+  uint8_t* d_crop_arena = nullptr; size_t crop_arena_cap = 0;
+  long long crop_n = 0;
+  std::vector<int32_t> crop_ok;
   bool ready = false;
 };
 
@@ -553,6 +566,7 @@ struct CallArgs {
   Ragged* rg = nullptr;                   // mixed call: per-frame sizes and layouts (the uniform fields above are unused)
   int orientation = 1;                    // EXIF orientation of every frame; w, hh are the stored size, uw, uh the upright one
   int uw = 0, uh = 0;
+  bool crops = false;                     // face crops on (fdt_set_face_crops): fast mode runs a host stage per chunk too
 };
 
 // Upright size of frame i of the call: faces are normalised to it, the mesh and iris stages map their points into it.
@@ -758,7 +772,7 @@ int stage_uniform(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, co
   cudaStream_t s = sl.stream;
   const LbTables* tb = a.tb;
   const int S_w = h->det.in_w(), S_h = h->det.in_h();
-  const bool fast_host = a.mem_kind == FDT_MEM_HOST && a.mode == FDT_MODE_FAST;
+  const bool fast_host = a.mem_kind == FDT_MEM_HOST && a.mode == FDT_MODE_FAST && !a.crops;   // the crop warps read whole frames
   const bool sparse = fast_host && !a.lay.yuv && tb->sparse;
   // YUV frames: the Y plane and the chroma area go up independently, each compacted when its tap rows are periodic
   const bool y_sparse = fast_host && a.lay.yuv && tb->sparse, c_sparse = fast_host && a.lay.yuv && tb->c_sparse;
@@ -878,7 +892,7 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
   }
   const size_t pitch = (size_t)h->max_faces * sizeof(fdt_face);
   const size_t eager = (size_t)std::min(kEagerSlots, h->max_faces) * sizeof(fdt_face);
-  if (a.mode != FDT_MODE_FAST) {
+  if (a.mode != FDT_MODE_FAST || a.crops) {
     cudaMemcpyAsync(sl.h_counts, h->d_counts + off, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, s);
     cudaMemcpy2DAsync(sl.h_faces, pitch, h->d_faces + (size_t)off * h->max_faces, pitch, eager, n, cudaMemcpyDeviceToHost, s);
     cudaEventRecord(sl.ev_det, s);
@@ -919,6 +933,137 @@ void eye_rois_from_corners(const double* c8, double* out8 /* (cx, cy, size, thet
   }
 }
 
+// The crop warps' PixFmt: a mixed chunk's table, or for a uniform RGB-family call the frames' own (whole frames).
+const PixFmt* warp_pix_fmt(Slot& sl, const CallArgs& a, const ChunkJob& job) {
+  if (!a.lay.rgb) return job.d_pf;
+  *sl.h_pf = a.lay.px;
+  cudaMemcpyAsync(sl.d_pf, sl.h_pf, sizeof(PixFmt), cudaMemcpyHostToDevice, sl.stream);
+  return sl.d_pf;
+}
+
+// A crop warp over a chunk's frames: where they are on the device and how to read them.  The warps read whole frames: host frames
+// go up unsparsified whenever a crop warp follows the detector.
+WarpP chunk_warp(const CallArgs& a, const ChunkJob& job, const PixFmt* d_pf) {
+  WarpP wp;
+  wp.frames = job.d_fr; wp.frame_stride = a.frame_stride; wp.row_stride = a.row_stride; wp.channels = a.channels;
+  wp.src_w = a.uw; wp.src_h = a.uh;
+  set_warp_layout(wp, a.lay);
+  wp.fr = job.d_desc; wp.orientation = job.orientation; wp.pf = d_pf;
+  return wp;
+}
+
+size_t crop_bytes(const fdt_crop_spec& sp) { return (size_t)3 * sp.out_size * sp.out_size * ((sp.layout & FDT_CROP_F32) ? 4 : 1); }
+
+// computeEmbeddingAlignment (lib/src/models/face_embedding.dart:362-384): out4 = theta, cx, cy, size from the eye points in pixels.
+void embedding_alignment(const double* l, const double* r, double* out4) {
+  const double dx = r[0] - l[0], dy = r[1] - l[1];
+  const double theta = std::atan2(dy, dx);
+  const double eye_dist = std::sqrt(dx * dx + dy * dy);
+  const double size = eye_dist * 2.5;
+  const double ecx = (l[0] + r[0]) * 0.5, ecy = (l[1] + r[1]) * 0.5;
+  const double ct = std::cos(theta), st = std::sin(theta);
+  const double oy = size * 0.15;
+  out4[0] = theta; out4[1] = ecx - oy * st; out4[2] = ecy + oy * ct; out4[3] = size;
+}
+
+// Grows the crop arena to `need` bytes, keeping the crops earlier chunks of the call wrote.  Both slots' streams may still be
+// writing crops, so they drain first; growth is geometric, so this happens a few times per handle.
+bool grow_crop_arena(fdt_handle* h, size_t need) {
+  if (need <= h->crop_arena_cap) return true;
+  for (int i = 0; i < kSlots; ++i)
+    if (!cuda_ok(h, cudaStreamSynchronize(h->slots[i].stream), "face crops")) return false;
+  const size_t cap = std::max(need, 2 * h->crop_arena_cap);
+  uint8_t* p = nullptr;
+  if (!cuda_ok(h, cudaMalloc(&p, cap), "cudaMalloc(face crops)")) return false;
+  const size_t used = (size_t)h->crop_n * crop_bytes(h->crop_spec);
+  cudaStream_t s = h->slots[0].stream;
+  if (used && (!cuda_ok(h, cudaMemcpyAsync(p, h->d_crop_arena, used, cudaMemcpyDeviceToDevice, s), "face crop arena") ||
+               !cuda_ok(h, cudaStreamSynchronize(s), "face crop arena"))) {
+    cudaFree(p);
+    return false;
+  }
+  if (h->d_crop_arena) cudaFree(h->d_crop_arena);
+  h->d_crop_arena = p; h->crop_arena_cap = cap;
+  return true;
+}
+
+// One returned face of a chunk: its frame within the chunk and its record as the caller receives it.
+struct FaceAt { int b; const fdt_face* fc; };
+
+// Face crops of a chunk's returned faces, in output order (fdt_set_face_crops): ROIs on the host with the host libm from the
+// returned records' keypoints in upright pixels, then one crop warp per pass of up to crop_cap faces, writing crops
+// crop_n .. crop_n + nf - 1 of the arena.  Chunks finish in order, so the running count is the face's index in the flattened result.
+int launch_face_crops(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job, const PixFmt* d_pf,
+                      const std::vector<FaceAt>& faces) {
+  cudaStream_t s = sl.stream;
+  const fdt_crop_spec& sp = h->crop_spec;
+  const size_t cb = crop_bytes(sp);
+  for (size_t skip = 0; skip < faces.size(); skip += h->crop_cap) {
+    const int nf = (int)std::min<size_t>(h->crop_cap, faces.size() - skip);
+    if (!grow_crop_arena(h, (size_t)(h->crop_n + nf) * cb)) return FDT_ERR_CUDA;
+    if (!cuda_ok(h, cudaEventSynchronize(sl.ev_fc), "face crop ROIs")) return FDT_ERR_CUDA;   // the last upload from these buffers
+    std::vector<int> degenerate;
+    for (int f = 0; f < nf; ++f) {
+      const FaceAt& r = faces[skip + f];
+      const double* kp = r.fc->keypoints;
+      double fw, fh, theta, cx, cy, size;
+      frame_size(a, job.off + r.b, &fw, &fh);
+      if (sp.kind == FDT_CROP_FACE) {
+        face_alignment(kp, fw, fh, &theta, &cx, &cy, &size);
+      } else {
+        // Detection.landmarks: the normalised keypoints times the image size, in f64
+        const double le[2] = {kp[0] * fw, kp[1] * fh}, re[2] = {kp[2] * fw, kp[3] * fh};
+        double e[4];
+        embedding_alignment(le, re, e);
+        theta = e[0]; cx = e[1]; cy = e[2]; size = e[3];
+      }
+      sl.h_fc_img[f] = r.b;
+      const bool ok = aligned_square_inverse(cx, cy, size, -theta, sp.out_size, sl.h_fc_aff + 6 * f);
+      if (!ok) {
+        for (int k = 0; k < 6; ++k) sl.h_fc_aff[6 * f + k] = 0.0;
+        degenerate.push_back(f);
+      }
+      h->crop_ok.push_back(ok ? 1 : 0);
+    }
+    cudaMemcpyAsync(sl.d_fc_img, sl.h_fc_img, (size_t)nf * sizeof(int), cudaMemcpyHostToDevice, s);
+    cudaMemcpyAsync(sl.d_fc_aff, sl.h_fc_aff, (size_t)nf * 6 * sizeof(double), cudaMemcpyHostToDevice, s);
+    cudaEventRecord(sl.ev_fc, s);
+    {
+      StageTimer t(h, kCropStage, s);
+      WarpP wp = chunk_warp(a, job, d_pf);
+      wp.crop_img = sl.d_fc_img; wp.affine = sl.d_fc_aff; wp.ncrops = nf; wp.out_size = sp.out_size; wp.flip_odd = 0;
+      wp.crops = nullptr;
+      CropOutP o;
+      o.dst = h->d_crop_arena; o.first = h->crop_n; o.layout = sp.layout;
+      for (int c = 0; c < 3; ++c) { o.scale[c] = sp.scale[c]; o.bias[c] = sp.bias[c]; }
+      launch_warp_affine(wp, s, job.d_pl, &o);
+      t.launches = 1;
+    }
+    // the reference returns null for these: the crop is all zero bytes (its ok flag says so)
+    for (int f : degenerate) cudaMemsetAsync(h->d_crop_arena + (size_t)(h->crop_n + f) * cb, 0, cb, s);
+    h->crop_n += nf;
+  }
+  return FDT_OK;
+}
+
+// The host stage of a fast-mode chunk with face crops on: the records reach the caller here instead of through the detector
+// stage's copies (the same bytes: every frame's eager slots, then the faces past them), then the crop warp.
+int finish_crops(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job) {
+  const int n = job.n, off = job.off;
+  if (!cuda_ok(h, cudaEventSynchronize(sl.ev_det), "detector stage")) return FDT_ERR_CUDA;
+  if (fetch_overflow_faces(h, sl.h_counts, sl.h_faces, off, n) != FDT_OK) return FDT_ERR_CUDA;
+  const int eager = std::min(kEagerSlots, h->max_faces);
+  std::vector<FaceAt> faces;
+  for (int b = 0; b < n; ++b) {
+    const int c = sl.h_counts[b];
+    fdt_face* dst = a.out_faces + (size_t)(off + b) * h->max_faces;
+    std::memcpy(dst, sl.h_faces + (size_t)b * h->max_faces, (size_t)std::max(c, eager) * sizeof(fdt_face));
+    a.out_counts[off + b] = c;
+    for (int j = 0; j < c; ++j) faces.push_back({b, dst + j});
+  }
+  return launch_face_crops(h, sl, a, job, warp_pix_fmt(sl, a, job), faces);
+}
+
 // Stages 2-3 of a chunk (standard / full): host-built ROI lists between the device stages, presence gate, assembly.
 int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job) {
   cudaStream_t s = sl.stream;
@@ -933,15 +1078,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
   const long long total = (long long)list.size();
   const bool full = a.mode == FDT_MODE_FULL;
   const double gate = h->cfg.min_face_presence;
-  // the warp reads whole frames: host frames were uploaded unsparsified in these modes
-  const long long dev_frame_stride = a.frame_stride;
-  // the crop warps' PixFmt: a mixed chunk's table, or for a uniform RGB-family call the frames' own (whole frames)
-  const PixFmt* d_pf = job.d_pf;
-  if (a.lay.rgb) {
-    *sl.h_pf = a.lay.px;
-    cudaMemcpyAsync(sl.d_pf, sl.h_pf, sizeof(PixFmt), cudaMemcpyHostToDevice, s);
-    d_pf = sl.d_pf;
-  }
+  const PixFmt* d_pf = warp_pix_fmt(sl, a, job);
   for (long long skip = 0; skip < total; skip += h->mesh_cap) {
     const int nf = (int)std::min<long long>(h->mesh_cap, total - skip);
     // ---- face ROIs on the host: computeFaceAlignment + extractAlignedSquare's matrix (face_detector_core.dart:478-507)
@@ -962,12 +1099,9 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
     cudaMemcpyAsync(sl.d_roi, sl.h_roi, (size_t)nf * 6 * sizeof(double), cudaMemcpyHostToDevice, s);
     {
       StageTimer t(h, 3, s);
-      WarpP wp;
-      wp.frames = job.d_fr; wp.frame_stride = dev_frame_stride; wp.row_stride = a.row_stride; wp.channels = a.channels;
-      wp.src_w = a.uw; wp.src_h = a.uh; wp.crop_img = sl.d_crop_img; wp.affine = sl.d_affine; wp.ncrops = nf;
-      wp.out_size = kMeshInput; wp.flip_odd = 0; wp.crops = sl.d_crops;
-      set_warp_layout(wp, a.lay);
-      wp.fr = job.d_desc; wp.orientation = job.orientation; wp.pf = d_pf;
+      WarpP wp = chunk_warp(a, job, d_pf);
+      wp.crop_img = sl.d_crop_img; wp.affine = sl.d_affine; wp.ncrops = nf; wp.out_size = kMeshInput; wp.flip_odd = 0;
+      wp.crops = sl.d_crops;
       launch_warp_affine(wp, s, job.d_pl);
       t.launches = 1;
     }
@@ -1045,12 +1179,9 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
         if (a.rg) cudaMemcpyAsync(sl.d_eye_wh, sl.h_eye_wh, (size_t)nfi * 2 * sizeof(double), cudaMemcpyHostToDevice, s);
         {
           StageTimer t(h, 6, s);
-          WarpP wp;
-          wp.frames = job.d_fr; wp.frame_stride = dev_frame_stride; wp.row_stride = a.row_stride; wp.channels = a.channels;
-          wp.src_w = a.uw; wp.src_h = a.uh; wp.crop_img = sl.d_eye_img; wp.affine = sl.d_eye_affine; wp.ncrops = ne;
-          wp.out_size = kIrisInput; wp.flip_odd = 1; wp.crops = sl.d_eye_crops;
-          set_warp_layout(wp, a.lay);
-          wp.fr = job.d_desc; wp.orientation = job.orientation; wp.pf = d_pf;
+          WarpP wp = chunk_warp(a, job, d_pf);
+          wp.crop_img = sl.d_eye_img; wp.affine = sl.d_eye_affine; wp.ncrops = ne; wp.out_size = kIrisInput; wp.flip_odd = 1;
+          wp.crops = sl.d_eye_crops;
           launch_warp_affine(wp, s, job.d_pl);
           t.launches = 1;
         }
@@ -1091,6 +1222,13 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
         }
       }
     }
+    // ---- face crops of the pass's returned faces (after the presence gate; full mode: with the iris-refined eyes)
+    if (a.crops) {
+      std::vector<FaceAt> kf;
+      for (int f = 0; f < nf; ++f)
+        if (slot_of[f] >= 0) kf.push_back({list[(size_t)(skip + f)].b, a.out_faces + (size_t)off * h->max_faces + slot_of[f]});
+      if (int rc = launch_face_crops(h, sl, a, job, d_pf, kf)) return rc;
+    }
   }
   for (int b = 0; b < n; ++b) a.out_counts[off + b] = kept[b];
   return FDT_OK;
@@ -1103,6 +1241,11 @@ int run_chunks(fdt_handle* h, const CallArgs& a, const std::vector<int>& bounds)
   h->slot0_first_chunk = nchunks <= kSlots;             // chunk c runs on slot c % kSlots
   h->last_mesh_faces = 0; h->last_iris_faces = 0;
 
+  // the host stage of a chunk: mesh / iris (standard, full) or, in fast mode with face crops on, the records and the crop warp
+  const bool host_stage = mode != FDT_MODE_FAST || a.crops;
+  auto finish = [&](int i, const ChunkJob& job) {
+    return mode == FDT_MODE_FAST ? finish_crops(h, h->slots[i], a, job) : finish_mesh(h, h->slots[i], a, job);
+  };
   ChunkJob jobs[kSlots];
   int rc = FDT_OK;
   for (int c = 0; c < nchunks && rc == FDT_OK; ++c) {
@@ -1110,21 +1253,21 @@ int run_chunks(fdt_handle* h, const CallArgs& a, const std::vector<int>& bounds)
     Slot& sl = h->slots[c % kSlots];
     // software pipeline: chunk c is queued on its slot, then the host turns to chunk c - 1 on the other slot
     rc = enqueue_detect(h, sl, a, off, n, c == 0, &jobs[c % kSlots]);
-    if (rc == FDT_OK && mode != FDT_MODE_FAST && c > 0) {
+    if (rc == FDT_OK && host_stage && c > 0) {
       ChunkJob& prev = jobs[(c - 1) % kSlots];
-      rc = finish_mesh(h, h->slots[(c - 1) % kSlots], a, prev);
+      rc = finish((c - 1) % kSlots, prev);
       prev.active = false;
     }
   }
-  if (rc == FDT_OK && mode != FDT_MODE_FAST) {
+  if (rc == FDT_OK && host_stage) {
     for (int i = 0; i < kSlots && rc == FDT_OK; ++i)
-      if (jobs[i].active) { rc = finish_mesh(h, h->slots[i], a, jobs[i]); jobs[i].active = false; }
+      if (jobs[i].active) { rc = finish(i, jobs[i]); jobs[i].active = false; }
   }
   if (rc != FDT_OK) { for (int i = 0; i < kSlots; ++i) cudaStreamSynchronize(h->slots[i].stream); return rc; }
   if (!a.keep_on_device) {
     for (int i = 0; i < kSlots; ++i)
       if (!cuda_ok(h, cudaStreamSynchronize(h->slots[i].stream), "pipeline")) return FDT_ERR_CUDA;
-    if (mode == FDT_MODE_FAST && fetch_overflow_faces(h, a.out_counts, a.out_faces, 0, a.batch) != FDT_OK) return FDT_ERR_CUDA;
+    if (mode == FDT_MODE_FAST && !a.crops && fetch_overflow_faces(h, a.out_counts, a.out_faces, 0, a.batch) != FDT_OK) return FDT_ERR_CUDA;
   }
   if (!cuda_ok(h, cudaGetLastError(), "kernel launch")) return FDT_ERR_CUDA;
   if (h->det.failed() || h->mesh.failed() || h->iris.failed()) { h->err = "a kernel of the plan could not be launched (tensor map encoding / unsupported shape)"; return FDT_ERR_CUDA; }
@@ -1154,6 +1297,7 @@ int detect_single(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh
   a.mem_kind = mem_kind; a.out_faces = out_faces; a.out_counts = out_counts; a.out_mesh = out_mesh; a.out_iris = out_iris;
   a.keep_on_device = keep_on_device;
   a.orientation = orientation;
+  a.crops = h->crops_on;
   upright_size(w, hh, orientation, &a.uw, &a.uh);
   a.tb = get_tables(h, w, hh, orientation);
   if (!a.tb) return fail(h, FDT_ERR_CUDA, "letterbox table upload failed");
@@ -1294,7 +1438,7 @@ int detect_frames_single(fdt_handle* h, const fdt_frame* frames, const int32_t* 
   CallArgs a;
   a.frames = nullptr; a.batch = n; a.w = 0; a.hh = 0; a.row_stride = 0; a.channels = 0; a.mode = mode; a.mem_kind = mem_kind;
   a.out_faces = out_faces; a.out_counts = out_counts; a.out_mesh = out_mesh; a.out_iris = out_iris;
-  a.keep_on_device = false; a.tb = nullptr; a.frame_stride = 0; a.rg = &rg;
+  a.keep_on_device = false; a.tb = nullptr; a.frame_stride = 0; a.rg = &rg; a.crops = h->crops_on;
   // a chunk closes at max_batch frames, or (host frames) before its staged bytes would pass the budget
   const long long budget = (long long)h->chunk * kStageBytesPerFrame;
   std::vector<int> bounds(1, 0);
@@ -1407,6 +1551,16 @@ int detect_impl(fdt_handle* h, const uint8_t* frames, int batch, int w, int hh, 
 
 // the replica debug taps and profiling entries address (replica 0 of a multi-device handle)
 fdt_handle* primary(fdt_handle* h) { return (h && !h->shards.empty()) ? h->shards[0] : h; }
+
+// Every detect entry point replaces the face crops of the previous call (on every replica), whatever it returns.
+void reset_crops(fdt_handle* h) {
+  h->crop_n = 0;
+  h->crop_ok.clear();
+  for (fdt_handle* sh : h->shards) reset_crops(sh);
+}
+
+// The replicas whose crops a handle holds, in frame order.
+std::vector<fdt_handle*> replicas(fdt_handle* h) { return h->shards.empty() ? std::vector<fdt_handle*>{h} : h->shards; }
 
 int create_single(const fdt_config& cfg, const uint8_t* det_tflite, size_t det_len, const uint8_t* mesh_tflite, size_t mesh_len,
                   const uint8_t* iris_tflite, size_t iris_len, fdt_handle** out);
@@ -1730,7 +1884,8 @@ int create_single(const fdt_config& cfg, const uint8_t* det_tflite, size_t det_l
     if (!h->det.make_ctx(h->chunk, &sl.det_ctx, &err)) return bail(FDT_ERR_CUDA, err);
     bool ok = dalloc(h, &sl.d_lb, (size_t)h->chunk * h->det.in_h() * h->det.in_w() * 4) &&     // BGRX
               dalloc(h, &sl.d_cand_idx, (size_t)h->chunk * h->cand_cap) && dalloc(h, &sl.d_cand_n, (size_t)h->chunk) &&
-              palloc(h, &sl.h_counts, (size_t)h->chunk) && palloc(h, &sl.h_faces, (size_t)h->chunk * h->max_faces);
+              palloc(h, &sl.h_counts, (size_t)h->chunk) && palloc(h, &sl.h_faces, (size_t)h->chunk * h->max_faces) &&
+              dalloc(h, &sl.d_pf, 1) && palloc(h, &sl.h_pf, 1);
     if (!ok) return bail(FDT_ERR_CUDA, "detector stage allocation failed");
     cudaMemset(sl.d_cand_n, 0, (size_t)h->chunk * sizeof(int));
     if (with_mesh) {
@@ -1740,7 +1895,7 @@ int create_single(const fdt_config& cfg, const uint8_t* det_tflite, size_t det_l
            dalloc(h, &sl.d_roi, mc * 6) && palloc(h, &sl.h_roi, mc * 6) && dalloc(h, &sl.d_crops, mc * kMeshInput * kMeshInput * 4) &&
            dalloc(h, &sl.d_mesh_out, mc * FDT_MESH_FLOATS) && palloc(h, &sl.h_mesh_out, mc * FDT_MESH_FLOATS) &&
            dalloc(h, &sl.d_mesh_score, mc) && palloc(h, &sl.h_mesh_score, mc) && dalloc(h, &sl.d_eye_corners, mc * 8) &&
-           palloc(h, &sl.h_eye_corners, mc * 8) && dalloc(h, &sl.d_pf, 1) && palloc(h, &sl.h_pf, 1);
+           palloc(h, &sl.h_eye_corners, mc * 8);
       if (!ok) return bail(FDT_ERR_CUDA, "mesh stage allocation failed");
     }
     if (with_iris) {
@@ -1755,6 +1910,7 @@ int create_single(const fdt_config& cfg, const uint8_t* det_tflite, size_t det_l
     }
   }
   h->has_mesh = with_mesh; h->has_iris = with_iris;
+  h->crop_cap = std::max(64, h->chunk * 2);
   cudaEventCreate(&h->ev[0]);
   cudaEventCreate(&h->ev[1]);
   for (int i = 0; i < 3; ++i) cudaEventCreate(&h->tev[i]);
@@ -1789,6 +1945,7 @@ int32_t fdt_destroy(fdt_handle* h) {
       if (sl.stream) cudaStreamDestroy(sl.stream);
       if (sl.ev_det) cudaEventDestroy(sl.ev_det);
       if (sl.ev_blob) cudaEventDestroy(sl.ev_blob);
+      if (sl.ev_fc) cudaEventDestroy(sl.ev_fc);
       if (sl.h_blob) cudaFreeHost(sl.h_blob);
       if (sl.d_blob) cudaFree(sl.d_blob);
     }
@@ -1798,6 +1955,7 @@ int32_t fdt_destroy(fdt_handle* h) {
     if (h->d_jframe) cudaFree(h->d_jframe);
     if (h->d_jq) cudaFree(h->d_jq);
     if (h->d_jarena) cudaFree(h->d_jarena);
+    if (h->d_crop_arena) cudaFree(h->d_crop_arena);
     for (void* p : h->pin_allocs) cudaFreeHost(p);
     void* dev[] = {h->d_faces, h->d_counts, h->d_anchors};
     for (void* p : dev) if (p) cudaFree(p);
@@ -1825,6 +1983,7 @@ int32_t fdt_detect_batch_oriented(fdt_handle* h, const uint8_t* frames, int32_t 
                                   fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris) {
   if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
   std::lock_guard<std::mutex> g(h->mu);
+  reset_crops(h);
   if (orientation < 1 || orientation > 8) return fail(h, FDT_ERR_BAD_ARG, "orientation must be an EXIF value 1..8");
   return detect_impl(h, frames, batch, width, height, row_stride, mat_type, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris,
                      false, orientation);
@@ -1834,6 +1993,7 @@ int32_t fdt_detect_one(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int32
                        int32_t mode, fdt_face* out_faces, int32_t* out_count, float* out_mesh, float* out_iris) {
   if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
   std::lock_guard<std::mutex> g(h->mu);
+  reset_crops(h);
   if (width <= 0 || height <= 0) return fail(h, FDT_ERR_BAD_ARG, "bad frame arguments");
   const int row_stride = width * row_step(mat_type);
   FrameLayout lay;
@@ -1849,6 +2009,8 @@ int32_t fdt_detect_batch_device(fdt_handle* h, const uint8_t* d_frames, int32_t 
                                 const int32_t** d_counts) {
   if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
   std::lock_guard<std::mutex> g(h->mu);
+  reset_crops(h);
+  if (h->crops_on) return fail(h, FDT_ERR_UNSUPPORTED, "face crops need the results on the host: fdt_set_face_crops(h, NULL) first");
   int rc = detect_impl(h, d_frames, batch, width, height, row_stride, mat_type, mode, FDT_MEM_DEVICE, nullptr, nullptr, nullptr, nullptr, true);
   if (rc == FDT_OK) {
     if (d_faces) *d_faces = h->d_faces;
@@ -1888,6 +2050,7 @@ int32_t fdt_detect_jpeg(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int3
                         float* out_mesh, float* out_iris, int32_t* out_wh) {
   if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
   std::lock_guard<std::mutex> g(h->mu);
+  reset_crops(h);
   fdt_handle* p = primary(h);
   if (!p->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
   int w = 0, hh = 0;
@@ -1911,6 +2074,7 @@ int32_t fdt_detect_frames_oriented(fdt_handle* h, const fdt_frame* frames, const
                                    int32_t mem_kind, fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris) {
   if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
   std::lock_guard<std::mutex> g(h->mu);
+  reset_crops(h);
   if (!h->shards.empty()) return detect_frames_multi(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
   return detect_frames_single(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
 }
@@ -1919,6 +2083,7 @@ int32_t fdt_detect_yuv_planes(fdt_handle* h, const fdt_yuv_planes* frames, const
                               int32_t mem_kind, fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris) {
   if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
   std::lock_guard<std::mutex> g(h->mu);
+  reset_crops(h);
   if (!h->shards.empty()) return detect_planes_multi(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris);
   return detect_frames_single(h, nullptr, orientations, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris,
                               FrameList::kYuvPlanes, frames);
@@ -1929,6 +2094,7 @@ int32_t fdt_detect_jpeg_batch(fdt_handle* h, const uint8_t* const* images, const
                               int32_t* out_status) {
   if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
   std::lock_guard<std::mutex> g(h->mu);
+  reset_crops(h);
   if (!h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
   if (n < 0 || (n > 0 && (!images || !sizes || !out_faces || !out_counts || !out_status))) return fail(h, FDT_ERR_BAD_ARG, "bad image list");
   if (int rc = check_mode(h, mode)) return rc;
@@ -2340,6 +2506,84 @@ int32_t fdt_extract_aligned_squares(fdt_handle* h, const uint8_t* frame, int32_t
   return rc;
 }
 
+// ---- face crops of the detect calls -----------------------------------------------------------------
+namespace {
+int set_crops_single(fdt_handle* h, const fdt_crop_spec* spec) {
+  cudaSetDevice(h->cfg.device);
+  for (int i = 0; spec && i < kSlots; ++i) {
+    Slot& sl = h->slots[i];
+    if (sl.d_fc_img) continue;
+    const size_t cc = (size_t)h->crop_cap;
+    if (!dalloc(h, &sl.d_fc_img, cc) || !palloc(h, &sl.h_fc_img, cc) || !dalloc(h, &sl.d_fc_aff, cc * 6) ||
+        !palloc(h, &sl.h_fc_aff, cc * 6) || cudaEventCreateWithFlags(&sl.ev_fc, cudaEventDisableTiming) != cudaSuccess) {
+      sl.d_fc_img = nullptr;
+      return fail(h, FDT_ERR_CUDA, "face crop allocation failed");
+    }
+  }
+  h->crops_on = spec != nullptr;
+  if (spec) h->crop_spec = *spec;
+  reset_crops(h);
+  return FDT_OK;
+}
+}  // namespace
+
+int32_t fdt_set_face_crops(fdt_handle* h, const fdt_crop_spec* spec) {
+  if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
+  std::lock_guard<std::mutex> g(h->mu);
+  if (spec) {
+    if (spec->struct_size != (int32_t)sizeof(fdt_crop_spec)) return fail(h, FDT_ERR_BAD_ARG, "fdt_crop_spec.struct_size mismatch");
+    if (spec->kind != FDT_CROP_EMBEDDING && spec->kind != FDT_CROP_FACE) return fail(h, FDT_ERR_BAD_ARG, "unknown crop kind");
+    if (spec->layout & ~(FDT_CROP_RGB | FDT_CROP_CHW | FDT_CROP_F32)) return fail(h, FDT_ERR_BAD_ARG, "unknown crop layout bit");
+    if (spec->out_size <= 0 || spec->out_size > 4096) return fail(h, FDT_ERR_BAD_ARG, "crop out_size must be 1..4096");
+    for (int c = 0; c < 3; ++c)
+      if (!std::isfinite(spec->scale[c]) || !std::isfinite(spec->bias[c])) return fail(h, FDT_ERR_BAD_ARG, "crop scale and bias must be finite");
+  }
+  for (fdt_handle* r : replicas(h)) {
+    std::unique_lock<std::mutex> gl(r->mu, std::defer_lock);
+    if (r != h) gl.lock();
+    if (int rc = set_crops_single(r, spec)) { if (r != h) h->err = r->err; return rc; }
+  }
+  h->crops_on = spec != nullptr;
+  if (spec) h->crop_spec = *spec;
+  return FDT_OK;
+}
+
+int32_t fdt_get_face_crops(fdt_handle* h, int64_t* out_n, const void** out_dev) {
+  if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
+  std::lock_guard<std::mutex> g(h->mu);
+  if (out_dev && !h->shards.empty()) return fail(h, FDT_ERR_UNSUPPORTED, "the crops of a multi-device handle lie on several devices: fdt_copy_face_crops");
+  long long n = 0;
+  for (fdt_handle* r : replicas(h)) n += r->crop_n;
+  if (out_n) *out_n = n;
+  if (out_dev) *out_dev = h->d_crop_arena;
+  return FDT_OK;
+}
+
+int32_t fdt_copy_face_crops(fdt_handle* h, void* dst, size_t capacity, int32_t mem_kind, int32_t* out_ok) {
+  if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
+  std::lock_guard<std::mutex> g(h->mu);
+  if (mem_kind != FDT_MEM_HOST && mem_kind != FDT_MEM_DEVICE) return fail(h, FDT_ERR_BAD_ARG, "unknown mem_kind");
+  if (mem_kind == FDT_MEM_DEVICE && !h->shards.empty())
+    return fail(h, FDT_ERR_UNSUPPORTED, "a multi-device handle copies its crops to host memory only");
+  const std::vector<fdt_handle*> reps = replicas(h);
+  size_t total = 0;
+  for (fdt_handle* r : reps) total += (size_t)r->crop_n * crop_bytes(r->crop_spec);
+  if (total && !dst) return fail(h, FDT_ERR_BAD_ARG, "null destination");
+  if (capacity < total) return fail(h, FDT_ERR_SIZE_MISMATCH, "capacity smaller than n * crop bytes");
+  size_t at = 0, k = 0;
+  for (fdt_handle* r : reps) {
+    const size_t bytes = (size_t)r->crop_n * crop_bytes(r->crop_spec);
+    if (bytes) {
+      cudaSetDevice(r->cfg.device);
+      const cudaMemcpyKind kind = mem_kind == FDT_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+      if (!cuda_ok(h, cudaMemcpy(static_cast<uint8_t*>(dst) + at, r->d_crop_arena, bytes, kind), "face crop copy")) return FDT_ERR_CUDA;
+    }
+    if (out_ok) std::copy(r->crop_ok.begin(), r->crop_ok.end(), out_ok + k);
+    at += bytes; k += r->crop_ok.size();
+  }
+  return FDT_OK;
+}
+
 int64_t fdt_last_launch_count(fdt_handle* h) { return h ? h->launches : 0; }
 int64_t fdt_last_h2d_bytes(fdt_handle* h) { return h ? h->h2d_bytes : 0; }
 
@@ -2598,15 +2842,7 @@ int32_t fdt_host_eye_rois(const double* corners8, double* out8) {
 
 int32_t fdt_host_embedding_roi(const double* l, const double* r, double* out4) {
   if (!l || !r || !out4) return FDT_ERR_BAD_ARG;
-  // computeEmbeddingAlignment (lib/src/models/face_embedding.dart:362-384)
-  const double dx = r[0] - l[0], dy = r[1] - l[1];
-  const double theta = std::atan2(dy, dx);
-  const double eye_dist = std::sqrt(dx * dx + dy * dy);
-  const double size = eye_dist * 2.5;
-  const double ecx = (l[0] + r[0]) * 0.5, ecy = (l[1] + r[1]) * 0.5;
-  const double ct = std::cos(theta), st = std::sin(theta);
-  const double oy = size * 0.15;
-  out4[0] = theta; out4[1] = ecx - oy * st; out4[2] = ecy + oy * ct; out4[3] = size;
+  embedding_alignment(l, r, out4);
   return FDT_OK;
 }
 

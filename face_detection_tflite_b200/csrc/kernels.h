@@ -387,9 +387,19 @@ struct WarpP {
   // makes for the existing instantiations.)
   const PixFmt* pf = nullptr;
 };
+// Face crops of the detect calls (fdt_set_face_crops): the warp's epilogue writes crop f of the pass as crop first + f of a packed
+// arena, in the caller's layout (FDT_CROP_* flags: RGB channel order, CHW planes, f32 = (float)u8 * scale[c] + bias[c] rounded
+// per operation, c in output order), instead of BGRX into WarpP::crops.  (A kernel argument of its own: WarpP has no room left.)
+struct CropOutP {
+  void* dst = nullptr;
+  long long first = 0;
+  int layout = 0;
+  float scale[3] = {1.f, 1.f, 1.f}, bias[3] = {0.f, 0.f, 0.f};
+};
 // pl: ragged chunks of separate-plane YUV frames (k_letterbox_multi's table, indexed like fr); non-null launches the instantiation
 // that reads every frame's chroma through it.  (A kernel argument of its own: WarpP has no room left, see pf.)
-void launch_warp_affine(const WarpP& p, cudaStream_t s, const YuvPlaneD* pl = nullptr);
+// out: non-null launches the face-crop instantiation that writes the packed arena out->dst (WarpP::crops and flip_odd unused).
+void launch_warp_affine(const WarpP& p, cudaStream_t s, const YuvPlaneD* pl = nullptr, const CropOutP* out = nullptr);
 
 // ---- mesh / iris post-processing ----
 struct MeshPostP {

@@ -228,8 +228,10 @@ __device__ __forceinline__ long long sat_round_ll(double v) { return (long long)
 // kFmt: the frame (uniform) or some frame of the chunk (ragged) is RGB / RGBA / planar RGB; every packed or planar frame's taps
 // are read through its PixFmt (p.pf[0], or p.pf[frame]), so a crop equals the crop of the BGR image.
 // kPlanes (ragged only): every frame of the chunk is a separate-plane YUV frame, its chroma read through pl[frame].
-template <bool kRagged, bool kOriented, bool kFmt, bool kPlanes>
-__global__ void k_warp_affine(WarpP p, const YuvPlaneD* pl) {
+// kOut: a face crop of the detect calls.  Only the epilogue differs: crop f goes to crop out.first + f of the packed arena in
+// out.layout (FDT_CROP_RGB / _CHW / _F32); a warp's 32 pixels are consecutive in each CHW plane.
+template <bool kRagged, bool kOriented, bool kFmt, bool kPlanes, bool kOut>
+__global__ void k_warp_affine(WarpP p, const YuvPlaneD* pl, CropOutP out) {
   const int f = blockIdx.y;
   if (f >= p.ncrops) return;
   const int S = p.out_size;
@@ -303,6 +305,18 @@ __global__ void k_warp_affine(WarpP p, const YuvPlaneD* pl) {
     for (int c = 0; c < 3; ++c) {
       int v = (acc[c] + 16384) >> 15;
       o[c] = (uint8_t)(v < 0 ? 0 : (v > 255 ? 255 : v));
+    }
+    if (kOut) {
+      const size_t px = (size_t)S * S, k = (size_t)out.first + f;
+      const bool chw = out.layout & FDT_CROP_CHW;
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        const uint8_t v = o[(out.layout & FDT_CROP_RGB) ? 2 - c : c];
+        const size_t at = chw ? (3 * k + c) * px + i : (k * px + i) * 3 + c;
+        if (out.layout & FDT_CROP_F32) reinterpret_cast<float*>(out.dst)[at] = __fadd_rn(__fmul_rn((float)v, out.scale[c]), out.bias[c]);
+        else reinterpret_cast<uint8_t*>(out.dst)[at] = v;
+      }
+      continue;
     }
     const int xo = flip ? S - 1 - x : x;
     reinterpret_cast<uchar4*>(p.crops)[(size_t)f * S * S + (size_t)y * S + xo] = make_uchar4(o[0], o[1], o[2], 0);
@@ -400,27 +414,32 @@ void launch_decode_nms(const DecodeP& p, int B, cudaStream_t s) {
   k_decode_nms<<<B, kDecodeThreads, smem, s>>>(p);
 }
 
-template <bool kFmt> void launch_warp(const WarpP& p, dim3 grid, cudaStream_t s) {
+template <bool kFmt, bool kOut> void launch_warp(const WarpP& p, dim3 grid, cudaStream_t s, const CropOutP& o) {
   if (p.orientation != 1) {
-    if (p.fr) k_warp_affine<true, true, kFmt, false><<<grid, 256, 0, s>>>(p, nullptr);
-    else k_warp_affine<false, true, kFmt, false><<<grid, 256, 0, s>>>(p, nullptr);
+    if (p.fr) k_warp_affine<true, true, kFmt, false, kOut><<<grid, 256, 0, s>>>(p, nullptr, o);
+    else k_warp_affine<false, true, kFmt, false, kOut><<<grid, 256, 0, s>>>(p, nullptr, o);
   } else {
-    if (p.fr) k_warp_affine<true, false, kFmt, false><<<grid, 256, 0, s>>>(p, nullptr);
-    else k_warp_affine<false, false, kFmt, false><<<grid, 256, 0, s>>>(p, nullptr);
+    if (p.fr) k_warp_affine<true, false, kFmt, false, kOut><<<grid, 256, 0, s>>>(p, nullptr, o);
+    else k_warp_affine<false, false, kFmt, false, kOut><<<grid, 256, 0, s>>>(p, nullptr, o);
   }
 }
 
-void launch_warp_affine(const WarpP& p, cudaStream_t s, const YuvPlaneD* pl) {
+template <bool kOut> void launch_warp_any(const WarpP& p, dim3 grid, cudaStream_t s, const YuvPlaneD* pl, const CropOutP& o) {
+  if (pl) {
+    if (p.orientation != 1) k_warp_affine<true, true, false, true, kOut><<<grid, 256, 0, s>>>(p, pl, o);
+    else k_warp_affine<true, false, false, true, kOut><<<grid, 256, 0, s>>>(p, pl, o);
+  } else if (p.pf) {
+    launch_warp<true, kOut>(p, grid, s, o);
+  } else {
+    launch_warp<false, kOut>(p, grid, s, o);
+  }
+}
+
+void launch_warp_affine(const WarpP& p, cudaStream_t s, const YuvPlaneD* pl, const CropOutP* out) {
   if (p.ncrops <= 0) return;
   dim3 grid((p.out_size * p.out_size + 255) / 256, p.ncrops);
-  if (pl) {
-    if (p.orientation != 1) k_warp_affine<true, true, false, true><<<grid, 256, 0, s>>>(p, pl);
-    else k_warp_affine<true, false, false, true><<<grid, 256, 0, s>>>(p, pl);
-  } else if (p.pf) {
-    launch_warp<true>(p, grid, s);
-  } else {
-    launch_warp<false>(p, grid, s);
-  }
+  if (out) launch_warp_any<true>(p, grid, s, pl, *out);
+  else launch_warp_any<false>(p, grid, s, pl, CropOutP());
 }
 
 void launch_mesh_post(const MeshPostP& p, cudaStream_t s) {

@@ -147,6 +147,67 @@ def _upright(w, h, orientation) -> tuple:
     return (h, w) if orientation >= 5 else (w, h)
 
 
+class FaceCropSpec:
+    """The aligned face crop every detect call returns once FaceDetector.setFaceCrops(spec) is on (fdt_crop_spec).
+    kind: "embedding" (computeEmbeddingAlignment on the eye keypoints: the crop getFaceEmbedding feeds MobileFaceNet) or "face"
+    (computeFaceAlignment: the face-mesh ROI).  size: the side S, 1..4096.  order: "bgr" (extractAlignedSquare's) or "rgb".
+    chw: three S x S planes instead of S x S x 3.  dtype: np.uint8, or np.float32 with out = np.float32(u8) * scale[c] + bias[c]
+    (c in output order; a float32 multiply then a float32 add, as numpy computes it).  A bad argument raises ValueError."""
+    KINDS = {"embedding": _ffi.FDT_CROP_EMBEDDING, "face": _ffi.FDT_CROP_FACE}
+
+    def __init__(self, kind: str = "embedding", size: int = 112, order: str = "bgr", chw: bool = False, dtype=np.uint8,
+                 scale=(1.0, 1.0, 1.0), bias=(0.0, 0.0, 0.0)):
+        if not isinstance(kind, str) or kind not in self.KINDS:
+            raise ValueError("kind must be 'embedding' or 'face', got %r" % (kind,))
+        if isinstance(size, bool) or not isinstance(size, (int, np.integer)) or not 1 <= size <= 4096:
+            raise ValueError("size must be an integer 1..4096, got %r" % (size,))
+        if not isinstance(order, str) or order not in ("bgr", "rgb"):
+            raise ValueError("order must be 'bgr' or 'rgb', got %r" % (order,))
+        if not isinstance(chw, (bool, np.bool_)):
+            raise ValueError("chw must be a bool, got %r" % (chw,))
+        try:
+            dt = np.dtype(dtype)
+        except TypeError:
+            raise ValueError("dtype must be np.uint8 or np.float32, got %r" % (dtype,)) from None
+        if dt not in (np.dtype(np.uint8), np.dtype(np.float32)):
+            raise ValueError("dtype must be np.uint8 or np.float32, got %r" % (dtype,))
+        sc, bi = (self._triple(v, name) for v, name in ((scale, "scale"), (bias, "bias")))
+        self.kind, self.size, self.order, self.chw, self.dtype, self.scale, self.bias = kind, int(size), order, bool(chw), dt, sc, bi
+
+    @staticmethod
+    def _triple(v, name):
+        try:
+            a = np.asarray(v, np.float64)
+        except (TypeError, ValueError):
+            raise ValueError("%s must be three finite numbers, got %r" % (name, v)) from None
+        if a.shape == ():
+            a = np.repeat(a, 3)
+        with np.errstate(over="ignore"):
+            finite = a.shape == (3,) and np.all(np.isfinite(a.astype(np.float32)))
+        if not finite:
+            raise ValueError("%s must be three finite numbers, got %r" % (name, v))
+        return tuple(float(x) for x in a.astype(np.float32))
+
+    @property
+    def layout(self) -> int:
+        return ((_ffi.FDT_CROP_RGB if self.order == "rgb" else 0) | (_ffi.FDT_CROP_CHW if self.chw else 0) |
+                (_ffi.FDT_CROP_F32 if self.dtype == np.float32 else 0))
+
+    def shape(self, n: int) -> tuple:
+        return (n, 3, self.size, self.size) if self.chw else (n, self.size, self.size, 3)
+
+    @property
+    def cropBytes(self) -> int:
+        return 3 * self.size * self.size * self.dtype.itemsize
+
+    def _struct(self):
+        c = _ffi.FdtCropSpec()
+        c.struct_size, c.kind, c.out_size, c.layout = C.sizeof(_ffi.FdtCropSpec), self.KINDS[self.kind], self.size, self.layout
+        c.scale = (C.c_float * 3)(*self.scale)
+        c.bias = (C.c_float * 3)(*self.bias)
+        return c
+
+
 class FaceDetector:
     modelVersion = "1.1.1"   # lib/src/face_detector.dart:54-64
 
@@ -626,6 +687,46 @@ class FaceDetector:
         if not ok[0]:
             raise StateError("Failed to extract aligned face crop for embedding")
         return crops[0]
+
+    # -- face crops of the detect calls (fdt_set_face_crops) ----------------------------------------------------
+    def setFaceCrops(self, spec: Optional[FaceCropSpec]) -> None:
+        """Every later detect call also returns one aligned crop per returned face (spec), or none (None, the default).  The
+        crops are warped on the device from the frame the call already holds there; faceCrops() / copyFaceCropsRaw() fetch them.
+        Fast mode then runs a host stage per chunk and uploads host frames whole; detectBatchRaw on device frames is unaffected,
+        fdt_detect_batch_device refuses."""
+        if spec is not None and not isinstance(spec, FaceCropSpec):
+            raise ValueError("spec must be a FaceCropSpec or None")
+        self._check()
+        self._rc(self._lib.fdt_set_face_crops(self._h, C.byref(spec._struct()) if spec is not None else None))
+        self._crop_spec = spec
+
+    def faceCrops(self):
+        """The crops of the last detect call, one per returned face in output order (frame by frame, then slot by slot):
+        (array [F, S, S, 3] or [F, 3, S, S] of the spec's dtype, ok bool [F]).  ok is False where the ROI was degenerate
+        (the crop is then zeros)."""
+        self._check()
+        spec = getattr(self, "_crop_spec", None)
+        n = C.c_int64(0)
+        self._rc(self._lib.fdt_get_face_crops(self._h, C.byref(n), None))
+        if spec is None:
+            return np.zeros((0, 0, 0, 3), np.uint8), np.zeros(0, bool)
+        out = np.empty(spec.shape(n.value), spec.dtype)
+        ok = np.zeros(n.value, np.int32)
+        self._rc(self._lib.fdt_copy_face_crops(self._h, out.ctypes.data, out.nbytes, _ffi.FDT_MEM_HOST, ok.ctypes.data_as(_ffi.i32p)))
+        return out, ok.astype(bool)
+
+    def copyFaceCropsRaw(self, ptr: int, capacity: int, memKind: int = _ffi.FDT_MEM_DEVICE) -> int:
+        """fdt_copy_face_crops into caller memory: ptr is an integer address (e.g. a torch CUDA tensor's data_ptr() with
+        memKind=FDT_MEM_DEVICE), capacity its size in bytes.  Returns the number of crops copied."""
+        if isinstance(ptr, bool) or not isinstance(ptr, int) or isinstance(capacity, bool) or not isinstance(capacity, int) or capacity < 0:
+            raise ValueError("ptr and capacity must be integers (capacity >= 0)")
+        if memKind not in (_ffi.FDT_MEM_HOST, _ffi.FDT_MEM_DEVICE):
+            raise ValueError("memKind must be FDT_MEM_HOST or FDT_MEM_DEVICE")
+        self._check()
+        n = C.c_int64(0)
+        self._rc(self._lib.fdt_get_face_crops(self._h, C.byref(n), None))
+        self._rc(self._lib.fdt_copy_face_crops(self._h, ptr or None, capacity, memKind, None))
+        return n.value
 
     # -- parity taps (tests only) -----------------------------------------------------------------
     # The detector taps describe the first n frames of the last call's first chunk (min(count, maxBatch) frames).  After a

@@ -275,6 +275,55 @@ FDT_EXPORT int32_t fdt_detect_jpeg_batch(fdt_handle* h, const uint8_t* const* im
                                          int32_t mode, fdt_face* out_faces, int32_t* out_counts, float* out_mesh,
                                          float* out_iris, int32_t* out_wh, int32_t* out_status);
 
+/* ---- Aligned face crops of the detect calls (the input of a second model: recognition, attributes, liveness) ----
+ * With crops on (fdt_set_face_crops), every detect call - fdt_detect_batch[_oriented], fdt_detect_one, fdt_detect_frames[_oriented],
+ * fdt_detect_yuv_planes, fdt_detect_jpeg, fdt_detect_jpeg_batch - also warps one square crop per returned face on the device,
+ * straight from the frame it already holds there, in every format, orientation and memory kind.
+ *   Which faces: every face the call returns (the out_counts[b] records of each frame, after the gates; in standard and full mode
+ *     after the presence gate), packed in output order, frame by frame and then slot by slot: crop k is the k-th face of the
+ *     flattened result.  No max_faces padding.
+ *   ROI: built on the host from the RETURNED record's keypoints in pixels of the upright image (kp[2i] * width, kp[2i+1] * height,
+ *     f64; in full mode the eyes are iris-refined):
+ *       FDT_CROP_EMBEDDING  computeEmbeddingAlignment on the two eye keypoints (fdt_host_embedding_roi), then
+ *                           extractAlignedSquare(cx, cy, size, -theta, out_size): the crop getFaceEmbedding feeds MobileFaceNet
+ *                           (face_detector_core.dart:419-452; with layout 0 and out_size 112 it equals FaceDetector.embeddingCrop);
+ *       FDT_CROP_FACE       computeFaceAlignment on the keypoints (fdt_host_face_roi), then extractAlignedSquare(cx, cy, size,
+ *                           -theta, out_size): the face-mesh ROI (at out_size 192 the standard-mode mesh crop).
+ *   Pixels: each crop equals extractAlignedSquare on the upright BGR image bit for bit.  layout 0 is u8 HWC BGR; the flags only
+ *     reorder and convert: FDT_CROP_RGB reverses the channel order, FDT_CROP_CHW stores three S x S planes, FDT_CROP_F32 stores
+ *     float (float)u8 * scale[c] + bias[c], a rounded multiply then a rounded add (no fused multiply-add), c in OUTPUT order.
+ *     A crop of out_size S takes 3 * S * S bytes, times 4 with FDT_CROP_F32.
+ *   Degenerate ROI (round(size) <= 0, where the reference returns null): the crop is all zero bytes and its ok flag 0.  The
+ *     detector drops faces whose face ROI is degenerate, so detector output should not reach this.
+ *   Lifetime: the crops of the last detect call (any of the entry points above); each such call and fdt_set_face_crops replace
+ *     them.  With crops off the count is 0.
+ *   Fast mode with crops on runs the standard-mode pipeline shape (faces to the host after the detector, then a host stage per
+ *     chunk that writes the records and launches the crop warp), so host frames go up whole: fdt_last_h2d_bytes is the frames'
+ *     full size.  fdt_detect_batch_device returns FDT_ERR_UNSUPPORTED while crops are on (its results never reach the host).
+ *   Nothing else changes: with crops on, records, mesh, iris, counts and every debug tap are bitwise those of crops off.  The crop
+ *     warps count in fdt_last_launch_count and are stage 9 of fdt_get_stage_ms. */
+enum { FDT_CROP_EMBEDDING = 0, FDT_CROP_FACE = 1 };                 /* fdt_crop_spec.kind                                    */
+enum { FDT_CROP_RGB = 1, FDT_CROP_CHW = 2, FDT_CROP_F32 = 4 };      /* fdt_crop_spec.layout flags; 0 = u8 HWC BGR            */
+typedef struct fdt_crop_spec {
+  int32_t struct_size;       /* sizeof(fdt_crop_spec)                                                                    */
+  int32_t kind;              /* FDT_CROP_EMBEDDING / FDT_CROP_FACE                                                       */
+  int32_t out_size;          /* S, 1..4096 (as fdt_extract_aligned_squares)                                              */
+  int32_t layout;            /* FDT_CROP_* flags                                                                         */
+  float scale[3], bias[3];   /* FDT_CROP_F32: out = (float)u8 * scale[c] + bias[c], c in output order; finite            */
+} fdt_crop_spec;             /* 40 bytes */
+/* spec NULL: crops off (the default).  A bad struct_size, kind, layout bit or out_size, or a non-finite scale or bias, returns
+ * FDT_ERR_BAD_ARG and leaves the setting as it was.  A multi-device handle applies the spec to every replica. */
+FDT_EXPORT int32_t fdt_set_face_crops(fdt_handle* h, const fdt_crop_spec* spec);
+/* *out_n (optional): the crops of the last detect call.  *out_dev (optional): their packed array in a handle-owned device arena,
+ * valid until the next detect call or fdt_set_face_crops; single-device handles only (a non-NULL out_dev returns
+ * FDT_ERR_UNSUPPORTED on a multi-device handle). */
+FDT_EXPORT int32_t fdt_get_face_crops(fdt_handle* h, int64_t* out_n, const void** out_dev);
+/* Copies all crops to dst: host memory (mem_kind FDT_MEM_HOST) or the handle's device memory (FDT_MEM_DEVICE, single-device
+ * handles only, else FDT_ERR_UNSUPPORTED).  capacity (bytes) below n * crop bytes returns FDT_ERR_SIZE_MISMATCH.  A multi-device
+ * handle concatenates its replicas' crops in frame order.  out_ok (optional): int32 [n], 1 per crop, 0 where the ROI was
+ * degenerate. */
+FDT_EXPORT int32_t fdt_copy_face_crops(fdt_handle* h, void* dst, size_t capacity, int32_t mem_kind, int32_t* out_ok);
+
 /* detectFacesFromMatBytes (lib/src/face_detector.dart:588-609): one packed frame of
  * `nbytes` bytes; FDT_ERR_SIZE_MISMATCH when nbytes != width*height*channels
  * (matFromPackedBytes, lib/src/util/helpers.dart:432-450), or != width*height*3/2 for the YUV formats
@@ -285,7 +334,8 @@ FDT_EXPORT int32_t fdt_detect_one(fdt_handle* h, const uint8_t* bytes, size_t nb
 
 /* Throughput variant used by the benchmark: frames already resident in device memory, results
  * left in device memory (no host transfer, no sync); `*d_faces` / `*d_counts` receive internal
- * device pointers valid until the next call.  Same computation as fdt_detect_batch(fast). */
+ * device pointers valid until the next call.  Same computation as fdt_detect_batch(fast).
+ * FDT_ERR_UNSUPPORTED while face crops are on (fdt_set_face_crops). */
 FDT_EXPORT int32_t fdt_detect_batch_device(fdt_handle* h, const uint8_t* d_frames, int32_t batch,
                                            int32_t width, int32_t height, int32_t row_stride,
                                            int32_t mat_type, int32_t mode, const fdt_face** d_faces,
@@ -377,7 +427,8 @@ FDT_EXPORT int64_t fdt_last_launch_count(fdt_handle* h);
 FDT_EXPORT int64_t fdt_last_h2d_bytes(fdt_handle* h);
 /* Device time in ms of the named stage summed over the last call when stage timing was enabled
  * with fdt_set_stage_timing(h,1) (adds cudaEvent records; off by default).
- * stage: 0 letterbox, 1 conv stack, 2 decode+nms, 3 warp, 4 mesh net, 5 mesh post, 6 eye warp, 7 iris net, 8 iris post */
+ * stage: 0 letterbox, 1 conv stack, 2 decode+nms, 3 warp, 4 mesh net, 5 mesh post, 6 eye warp, 7 iris net, 8 iris post,
+ * 9 face crops (fdt_set_face_crops) */
 FDT_EXPORT int32_t fdt_set_stage_timing(fdt_handle* h, int32_t enable);
 FDT_EXPORT int32_t fdt_get_stage_ms(fdt_handle* h, int32_t stage, float* ms, int32_t* launches);
 

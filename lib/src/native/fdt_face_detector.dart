@@ -502,6 +502,64 @@ class FdtFaceDetector {
     }
   }
 
+  /// Every later detect call also warps one aligned crop per returned face on the device (fdt_set_face_crops), or none
+  /// (spec == null, the default).  kind: kFdtCropEmbedding (the MobileFaceNet input of getFaceEmbedding) or kFdtCropFace;
+  /// layout: kFdtCrop* flags; scale / bias (three each) apply with kFdtCropF32.
+  void setFaceCrops({int? kind, int outSize = 112, int layout = 0, List<double> scale = const [1, 1, 1],
+      List<double> bias = const [0, 0, 0]}) {
+    _check();
+    final arena = Arena();
+    try {
+      Pointer<FdtCropSpec> spec = nullptr;
+      if (kind != null) {
+        spec = arena<FdtCropSpec>();
+        spec.ref
+          ..structSize = sizeOf<FdtCropSpec>()
+          ..kind = kind
+          ..outSize = outSize
+          ..layout = layout;
+        for (int c = 0; c < 3; c++) {
+          spec.ref.scale[c] = scale[c];
+          spec.ref.bias[c] = bias[c];
+        }
+      }
+      final int rc = _lib.setFaceCrops(_h, spec);
+      if (rc != FdtStatus.ok) {
+        _lib.throwFor(rc, _h);
+      }
+      _cropBytes = kind == null ? 0 : 3 * outSize * outSize * ((layout & kFdtCropF32) != 0 ? 4 : 1);
+    } finally {
+      arena.releaseAll();
+    }
+  }
+
+  int _cropBytes = 0;
+
+  /// The crops of the last detect call, one per returned face in output order (frame by frame, then slot by slot), packed
+  /// in the layout setFaceCrops chose (bytes of float32 values with kFdtCropF32), and one ok flag per crop (false: the ROI
+  /// was degenerate and the crop is zeros).
+  ({Uint8List crops, List<bool> ok}) faceCrops() {
+    _check();
+    final arena = Arena();
+    try {
+      final Pointer<Int64> n = arena<Int64>();
+      int rc = _lib.getFaceCrops(_h, n, nullptr);
+      if (rc != FdtStatus.ok) {
+        _lib.throwFor(rc, _h);
+      }
+      final int bytes = n.value * _cropBytes;
+      final Pointer<Uint8> dst = arena<Uint8>(bytes > 0 ? bytes : 1);
+      final Pointer<Int32> ok = arena<Int32>(n.value > 0 ? n.value : 1);
+      rc = _lib.copyFaceCrops(_h, dst.cast(), bytes, kFdtMemHost, ok);
+      if (rc != FdtStatus.ok) {
+        _lib.throwFor(rc, _h);
+      }
+      return (crops: Uint8List.fromList(dst.asTypedList(bytes)), ok: [for (int k = 0; k < n.value; k++) ok[k] != 0]);
+    } finally {
+      arena.releaseAll();
+    }
+  }
+
   /// FaceDetector.dispose (face_detector.dart:1061-1081).
   Future<void> dispose() async {
     if (_h != nullptr) {

@@ -145,6 +145,27 @@ final class FdtYuvPlanes extends Struct {
   external int reserved;
 }
 
+/// fdt_crop_spec: the aligned face crop every detect call returns once fdt_set_face_crops is on; 40 bytes.
+/// kind: kFdtCropEmbedding / kFdtCropFace; layout: kFdtCrop* flags (0 = u8 HWC BGR); with kFdtCropF32,
+/// out = (float)u8 * scale[c] + bias[c], c in output order.
+final class FdtCropSpec extends Struct {
+  @Int32()
+  external int structSize;
+  @Int32()
+  external int kind;
+  @Int32()
+  external int outSize;
+  @Int32()
+  external int layout;
+  @Array(3)
+  external Array<Float> scale;
+  @Array(3)
+  external Array<Float> bias;
+}
+
+const int kFdtCropEmbedding = 0, kFdtCropFace = 1;
+const int kFdtCropRgb = 1, kFdtCropChw = 2, kFdtCropF32 = 4;
+
 typedef _DefaultConfigC = Void Function(Pointer<FdtConfig>);
 typedef _DefaultConfigD = void Function(Pointer<FdtConfig>);
 typedef _CreateExC = Int32 Function(Pointer<FdtConfig>, Pointer<Uint8>, Size, Pointer<Uint8>, Size, Pointer<Uint8>, Size,
@@ -198,6 +219,12 @@ typedef _DetectYuvPlanesC = Int32 Function(Pointer<Void>, Pointer<FdtYuvPlanes>,
     Pointer<FdtFace>, Pointer<Int32>, Pointer<Float>, Pointer<Float>);
 typedef _DetectYuvPlanesD = int Function(Pointer<Void>, Pointer<FdtYuvPlanes>, Pointer<Int32>, int, int, int, Pointer<FdtFace>,
     Pointer<Int32>, Pointer<Float>, Pointer<Float>);
+typedef _SetFaceCropsC = Int32 Function(Pointer<Void>, Pointer<FdtCropSpec>);
+typedef _SetFaceCropsD = int Function(Pointer<Void>, Pointer<FdtCropSpec>);
+typedef _GetFaceCropsC = Int32 Function(Pointer<Void>, Pointer<Int64>, Pointer<Pointer<Void>>);
+typedef _GetFaceCropsD = int Function(Pointer<Void>, Pointer<Int64>, Pointer<Pointer<Void>>);
+typedef _CopyFaceCropsC = Int32 Function(Pointer<Void>, Pointer<Void>, Size, Int32, Pointer<Int32>);
+typedef _CopyFaceCropsD = int Function(Pointer<Void>, Pointer<Void>, int, int, Pointer<Int32>);
 typedef _NumDevicesC = Int32 Function(Pointer<Void>);
 typedef _NumDevicesD = int Function(Pointer<Void>);
 
@@ -221,6 +248,9 @@ class FdtLibrary {
         detectFramesOriented = _lib.lookupFunction<_DetectFramesOrientedC, _DetectFramesOrientedD>('fdt_detect_frames_oriented'),
         detectJpegBatch = _lib.lookupFunction<_DetectJpegBatchC, _DetectJpegBatchD>('fdt_detect_jpeg_batch'),
         detectYuvPlanes = _lib.lookupFunction<_DetectYuvPlanesC, _DetectYuvPlanesD>('fdt_detect_yuv_planes'),
+        setFaceCrops = _lib.lookupFunction<_SetFaceCropsC, _SetFaceCropsD>('fdt_set_face_crops'),
+        getFaceCrops = _lib.lookupFunction<_GetFaceCropsC, _GetFaceCropsD>('fdt_get_face_crops'),
+        copyFaceCrops = _lib.lookupFunction<_CopyFaceCropsC, _CopyFaceCropsD>('fdt_copy_face_crops'),
         numDevices = _lib.lookupFunction<_NumDevicesC, _NumDevicesD>('fdt_num_devices');
 
   final DynamicLibrary _lib;
@@ -238,6 +268,9 @@ class FdtLibrary {
   final _DetectJpegD detectJpeg;
   final _DetectFramesD detectFrames;
   final _DetectBatchOrientedD detectBatchOriented;
+  final _SetFaceCropsD setFaceCrops;
+  final _GetFaceCropsD getFaceCrops;
+  final _CopyFaceCropsD copyFaceCrops;
   final _DetectFramesOrientedD detectFramesOriented;
   final _DetectJpegBatchD detectJpegBatch;
   final _DetectYuvPlanesD detectYuvPlanes;
