@@ -17,6 +17,10 @@ YUV_FORMATS = (FDT_FMT_YUV_NV12, FDT_FMT_YUV_NV21, FDT_FMT_YUV_I420)
 # rowStride bytes each, back to back (3 * height * rowStride bytes; a contiguous [3, H, W] tensor has rowStride = W)
 FDT_FMT_RGB, FDT_FMT_RGBA, FDT_FMT_RGB_PLANAR = 0x1010, 0x1011, 0x1012
 RGB_FORMATS = (FDT_FMT_RGB, FDT_FMT_RGBA, FDT_FMT_RGB_PLANAR)
+# packed YUV 4:2:2 (V4L2 webcams: YUYV; capture cards: UYVY; GStreamer YUY2 / UYVY / YVYU): 2 bytes per pixel, even width,
+# height * rowStride bytes with rowStride >= 2 * width (cv2's HxW CV_8UC2 Mat, an HxWx2 array)
+FDT_FMT_YUYV, FDT_FMT_UYVY, FDT_FMT_YVYU = 0x1020, 0x1021, 0x1022
+YUV422_FORMATS = (FDT_FMT_YUYV, FDT_FMT_UYVY, FDT_FMT_YVYU)
 FDT_MEM_HOST, FDT_MEM_DEVICE = 0, 1
 # EXIF orientation of a stored frame (fdt_detect_batch_oriented / fdt_detect_frames_oriented): the upright image is
 # oracle.jpeg_ops.exif_transform(stored, orientation)

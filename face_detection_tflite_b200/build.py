@@ -34,6 +34,7 @@ SOURCES = {
     "kernels_pre.cu": [],
     # f64 geometry must be evaluated operation by operation (no fused multiply-add contraction)
     "kernels_post.cu": ["-fmad=false"],
+    "kernels_warp422.cu": ["-fmad=false"],
 }
 
 

@@ -225,10 +225,13 @@ int channels_of(int mat_type) {
 
 bool is_yuv(int mat_type) { return mat_type == FDT_FMT_YUV_NV12 || mat_type == FDT_FMT_YUV_NV21 || mat_type == FDT_FMT_YUV_I420; }
 bool is_rgb(int mat_type) { return mat_type == FDT_FMT_RGB || mat_type == FDT_FMT_RGBA || mat_type == FDT_FMT_RGB_PLANAR; }
+bool is_yuv422(int mat_type) { return mat_type == FDT_FMT_YUYV || mat_type == FDT_FMT_UYVY || mat_type == FDT_FMT_YVYU; }
 
-// Bytes of one pixel within a row: the packed formats' channels, 1 for planar RGB and YUV (a row is one plane's); 0: unknown.
+// Bytes of one pixel within a row: the packed formats' channels, 1 for planar RGB and YUV 4:2:0 (a row is one plane's), 2 for
+// packed YUV 4:2:2; 0: unknown.
 int row_step(int mat_type) {
   if (is_yuv(mat_type) || mat_type == FDT_FMT_RGB_PLANAR) return 1;
+  if (is_yuv422(mat_type)) return 2;
   if (mat_type == FDT_FMT_RGB) return 3;
   if (mat_type == FDT_FMT_RGBA) return 4;
   return channels_of(mat_type);
@@ -238,9 +241,10 @@ int row_step(int mat_type) {
 // chroma area at c_off: c_rows rows of c_row_bytes (NV12 / NV21: h / 2 interleaved rows; I420: the h / 2 rows of U, then those
 // of V), the chroma of pixel (x, y) at row y / 2 (+ h / 2 for V of I420), byte (x / 2) * c_step + u_off / v_off.
 struct FrameLayout {
-  int channels = 0;          // packed formats (RGB family: the pixel step); 0 for YUV
+  int channels = 0;          // packed formats (RGB family and YUV 4:2:2: the pixel step); 0 for YUV 4:2:0
   bool yuv = false;
-  bool rgb = false;          // FDT_FMT_RGB / _RGBA / _RGB_PLANAR: read through px by k_letterbox_rgb and the format-aware warps
+  bool rgb = false;          // FDT_FMT_RGB / _RGBA / _RGB_PLANAR and packed YUV 4:2:2: read through px by k_letterbox_rgb and the
+                             // format-aware warps
   int planes = 1;            // planar RGB: 3 planes of height rows of row_stride, back to back
   PixFmt px;                 // every non-YUV format: pixel step and B, G, R offsets, P = one plane of the whole frame
   long long frame_bytes = 0;
@@ -249,11 +253,16 @@ struct FrameLayout {
   bool planar = false;       // I420: V is a plane of its own, h / 2 rows behind U
 };
 
-// The pixel rule of a non-YUV format (kernels.h, PixFmt); plane = bytes of one plane where the frame lies.
+// The pixel rule of a non-YUV 4:2:0 format (kernels.h, PixFmt); plane = bytes of one plane where the frame lies.
 PixFmt pix_fmt(int mat_type, long long plane) {
   PixFmt f;
   f.step = row_step(mat_type);
-  if (mat_type == FDT_FMT_RGB_PLANAR) { f.b = 2 * plane; f.g = plane; f.r = 0; }
+  f.yuv422 = is_yuv422(mat_type) ? 1 : 0;
+  // packed YUV 4:2:2: Y from byte 2x, U and V from the macropixel (kernels.h, load_422)
+  if (mat_type == FDT_FMT_YUYV) { f.b = 0; f.g = 1; f.r = 3; }
+  else if (mat_type == FDT_FMT_UYVY) { f.b = 1; f.g = 0; f.r = 2; }
+  else if (mat_type == FDT_FMT_YVYU) { f.b = 0; f.g = 3; f.r = 1; }
+  else if (mat_type == FDT_FMT_RGB_PLANAR) { f.b = 2 * plane; f.g = plane; f.r = 0; }
   else if (mat_type == FDT_FMT_RGB || mat_type == FDT_FMT_RGBA) { f.b = 2; f.g = 1; f.r = 0; }
   else if (f.step > 1) { f.b = 0; f.g = 1; f.r = 2; }
   return f;
@@ -265,11 +274,14 @@ int frame_layout(int mat_type, int w, int hh, int row_stride, FrameLayout* L, co
   if (!is_yuv(mat_type)) {
     L->channels = row_step(mat_type);
     if (L->channels == 0) { *msg = "bad frame arguments"; return FDT_ERR_BAD_ARG; }
+    if (is_yuv422(mat_type) && (w & 1)) { *msg = "YUV 4:2:2 frames need an even width"; return FDT_ERR_BAD_ARG; }
     if (row_stride < w * L->channels) {
-      *msg = L->channels == 1 && is_rgb(mat_type) ? "row_stride smaller than width" : "row_stride smaller than width * channels";
+      *msg = L->channels == 1 && is_rgb(mat_type) ? "row_stride smaller than width"
+             : is_yuv422(mat_type)                ? "row_stride smaller than 2 * width"
+                                                  : "row_stride smaller than width * channels";
       return FDT_ERR_SIZE_MISMATCH;
     }
-    L->rgb = is_rgb(mat_type);
+    L->rgb = is_rgb(mat_type) || is_yuv422(mat_type);
     L->planes = mat_type == FDT_FMT_RGB_PLANAR ? 3 : 1;
     L->frame_bytes = (long long)L->planes * hh * row_stride;
     L->px = pix_fmt(mat_type, (long long)hh * row_stride);
@@ -581,11 +593,13 @@ void frame_size(const CallArgs& a, int i, double* w, double* hh) {
 }
 
 // d_desc: a mixed chunk's frame descriptors on the device (the crop warps read the frames through them); orientation: as
-// WarpP::orientation; d_pf: a mixed chunk's PixFmt table when it holds an RGB-family frame, else null; d_pl: a chunk's
-// YuvPlaneD table when its separate-plane device frames do not fit FrameD, else null
+// WarpP::orientation; d_pf: a mixed chunk's PixFmt table when it holds an RGB-family or YUV 4:2:2 frame, else null; d_pl: a
+// chunk's YuvPlaneD table when its separate-plane device frames do not fit FrameD, else null; yuv422: the chunk holds a packed
+// YUV 4:2:2 frame (the crop warps' launch_warp_affine flag)
 struct ChunkJob {
   int off = 0, n = 0; const uint8_t* d_fr = nullptr; const FrameD* d_desc = nullptr; bool active = false; int orientation = 1;
   const PixFmt* d_pf = nullptr;
+  bool yuv422 = false;
   const YuvPlaneD* d_pl = nullptr;
 };
 
@@ -649,7 +663,7 @@ size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 // blob (frame descriptors, concatenated tap tables, decode geometry and, for a chunk with an RGB-family frame, every frame's
 // PixFmt) in one copy; then k_letterbox_multi.
 int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, const FrameD** d_desc, const double** d_geom,
-                 int* orientation, const PixFmt** d_pf, const YuvPlaneD** d_pl) {
+                 int* orientation, const PixFmt** d_pf, const YuvPlaneD** d_pl, bool* yuv422) {
   cudaStream_t s = sl.stream;
   Ragged& rg = *a.rg;
   const fdt_frame* fr = rg.frames + off;
@@ -681,8 +695,10 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
   std::vector<const SizeTaps*> st(n);
   size_t ntaps = 0;
   bool upright = true, transposed = false, rgb = false;
+  *yuv422 = false;
   for (int i = 0; i < n; ++i) {
     rgb = rgb || rg.lay[off + i].rgb;
+    *yuv422 = *yuv422 || rg.lay[off + i].px.yuv422;
     const int o = rg.orientation(off + i);
     upright = upright && o == 1;
     transposed = transposed || orient_transposed(o);
@@ -697,7 +713,8 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
   bool table = false;
   for (int i = 0; pl && a.mem_kind == FDT_MEM_DEVICE && i < n; ++i) table = table || !fits_frame_desc(pl[i]);
   const size_t taps_at = align_up((size_t)n * sizeof(FrameD), 16), geom_at = align_up(taps_at + ntaps * sizeof(int), 16);
-  // a chunk with an RGB-family frame also carries every frame's PixFmt (k_letterbox_multi<true, true>, k_warp_affine<., ., true>);
+  // a chunk with an RGB-family or YUV 4:2:2 frame also carries every frame's PixFmt (k_letterbox_multi<true, true>,
+  // k_warp_affine<., ., true>; with a YUV 4:2:2 frame, k_letterbox_multi<true, true, false, true> and yuv422::k_warp_affine);
   // a chunk of separate-plane device frames that FrameD cannot describe, every frame's YuvPlaneD (the <., ., ., true> variants)
   const size_t pf_at = align_up(geom_at + (size_t)n * 6 * sizeof(double), 16);
   const size_t bytes = rgb ? pf_at + (size_t)n * sizeof(PixFmt)
@@ -760,7 +777,7 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
   StageTimer t(h, 0, s);
   LetterboxMultiP lb;
   lb.fr = *d_desc; lb.taps = reinterpret_cast<const int*>(sl.d_blob + taps_at); lb.out = sl.d_lb; lb.dst_w = S_w; lb.dst_h = S_h;
-  launch_letterbox_multi(lb, n, transposed, s, *d_pf, *d_pl);
+  launch_letterbox_multi(lb, n, transposed, s, *d_pf, *d_pl, *yuv422);
   t.launches = 1;
   return FDT_OK;
 }
@@ -873,7 +890,8 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
   int orientation = a.orientation;
   const PixFmt* d_pf = nullptr;
   const YuvPlaneD* d_pl = nullptr;
-  const int rc = a.rg ? stage_ragged(h, sl, a, off, n, &d_desc, &d_geom, &orientation, &d_pf, &d_pl)
+  bool yuv422 = a.lay.px.yuv422 != 0;
+  const int rc = a.rg ? stage_ragged(h, sl, a, off, n, &d_desc, &d_geom, &orientation, &d_pf, &d_pl, &yuv422)
                       : stage_uniform(h, sl, a, off, n, &d_fr);
   if (rc != FDT_OK) return rc;
   {
@@ -904,7 +922,7 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
                       cudaMemcpyDeviceToHost, s);
   }
   job->off = off; job->n = n; job->d_fr = d_fr; job->d_desc = d_desc; job->active = true; job->orientation = orientation;
-  job->d_pf = d_pf; job->d_pl = d_pl;
+  job->d_pf = d_pf; job->d_pl = d_pl; job->yuv422 = yuv422;
   return FDT_OK;
 }
 
@@ -933,7 +951,7 @@ void eye_rois_from_corners(const double* c8, double* out8 /* (cx, cy, size, thet
   }
 }
 
-// The crop warps' PixFmt: a mixed chunk's table, or for a uniform RGB-family call the frames' own (whole frames).
+// The crop warps' PixFmt: a mixed chunk's table, or for a uniform RGB-family or YUV 4:2:2 call the frames' own (whole frames).
 const PixFmt* warp_pix_fmt(Slot& sl, const CallArgs& a, const ChunkJob& job) {
   if (!a.lay.rgb) return job.d_pf;
   *sl.h_pf = a.lay.px;
@@ -1036,7 +1054,7 @@ int launch_face_crops(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob
       CropOutP o;
       o.dst = h->d_crop_arena; o.first = h->crop_n; o.layout = sp.layout;
       for (int c = 0; c < 3; ++c) { o.scale[c] = sp.scale[c]; o.bias[c] = sp.bias[c]; }
-      launch_warp_affine(wp, s, job.d_pl, &o);
+      launch_warp_affine(wp, s, job.d_pl, &o, job.yuv422);
       t.launches = 1;
     }
     // the reference returns null for these: the crop is all zero bytes (its ok flag says so)
@@ -1102,7 +1120,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
       WarpP wp = chunk_warp(a, job, d_pf);
       wp.crop_img = sl.d_crop_img; wp.affine = sl.d_affine; wp.ncrops = nf; wp.out_size = kMeshInput; wp.flip_odd = 0;
       wp.crops = sl.d_crops;
-      launch_warp_affine(wp, s, job.d_pl);
+      launch_warp_affine(wp, s, job.d_pl, nullptr, job.yuv422);
       t.launches = 1;
     }
     {
@@ -1182,7 +1200,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
           WarpP wp = chunk_warp(a, job, d_pf);
           wp.crop_img = sl.d_eye_img; wp.affine = sl.d_eye_affine; wp.ncrops = ne; wp.out_size = kIrisInput; wp.flip_odd = 1;
           wp.crops = sl.d_eye_crops;
-          launch_warp_affine(wp, s, job.d_pl);
+          launch_warp_affine(wp, s, job.d_pl, nullptr, job.yuv422);
           t.launches = 1;
         }
         {

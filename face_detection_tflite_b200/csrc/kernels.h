@@ -111,12 +111,22 @@ void launch_letterbox_tr(const LetterboxTrP& p, int B, cudaStream_t s);
 // of its B, G and R samples from the pixel's first byte (row + x * step):
 //   BGR 3: 0, 1, 2   RGB 3: 2, 1, 0   BGRA 4: 0, 1, 2   RGBA 4: 2, 1, 0   GRAY 1: 0, 0, 0   planar RGB 1: 2P, P, 0
 // with P the bytes of one plane as it lies on the device (after a compacted upload, the compacted plane).
+// Packed YUV 4:2:2 frames (FDT_FMT_YUYV / _UYVY / _YVYU, yuv422 = 1): step 2, and b, g, r are the offsets of the pixel's Y from
+// byte 2x of its row and of U and V from its 4-byte macropixel, byte 4 * (x / 2):  YUYV 0, 1, 3   UYVY 1, 0, 2   YVYU 0, 3, 1.
+// They are read by load_422 (k_letterbox_rgb<., true>, k_letterbox_multi<., ., ., true>, yuv422::k_warp_affine), which needs the
+// pixel's column as well as its row.
 struct PixFmt {
   long long b = 0, g = 0, r = 0;
   int step = 0;            // 0: no PixFmt (the existing formats' own kernels)
+  int yuv422 = 0;          // 1: packed YUV 4:2:2 (in the struct's tail padding: PixFmt keeps its 32 bytes)
 };
 #ifdef __CUDACC__
 __device__ __forceinline__ void load_pix(const uint8_t* px, const PixFmt& f, int* v) { v[0] = px[f.b]; v[1] = px[f.g]; v[2] = px[f.r]; }
+// Pixel x of a packed YUV 4:2:2 row, converted as cv::cvtColor COLOR_YUV2BGR_YUYV / _UYVY / _YVYU converts it.
+__device__ __forceinline__ void load_422(const uint8_t* row, int x, const PixFmt& f, int* v) {
+  const uint8_t* m = row + (size_t)(x >> 1) * 4;
+  yuv_to_bgr(row[(size_t)x * 2 + f.b], m[f.g], m[f.r], v);
+}
 #endif
 // Ragged batches (fdt_detect_frames): one descriptor per frame of a chunk.  It says where the frame's bytes are and how the
 // letterbox maps it; the crop warps read the same table, indexed by WarpP::crop_img.
@@ -124,7 +134,7 @@ struct FrameD {
   const uint8_t* y;        // the packed frame, or the Y plane
   const uint8_t* c;        // YUV 4:2:0: the chroma area, addressed as in LetterboxYuvP (v_off relative to it)
   int w, h, row_stride;
-  int channels;            // 1 / 3 / 4 (RGB-family frames: their pixel step); 0: YUV 4:2:0
+  int channels;            // 1 / 3 / 4 (RGB-family frames: their pixel step); 2: packed YUV 4:2:2; 0: YUV 4:2:0
   int c_row_stride, c_step, u_off, v_off;
   int new_w, new_h, pad_top, pad_left, identity;
   int tx, ty;              // offsets (ints) of the frame's x taps [4][new_w] and y taps [6][new_h] in the chunk's tap table
@@ -160,10 +170,12 @@ struct LetterboxMultiP {
 // sizes, which the existing variants' code depends on.)
 // pl (device, [B]): the chunk's frames are all separate-plane YUV frames read through their YuvPlaneD (any orientation; pf null).
 // (A kernel argument of its own, behind pfs, for the same reason.)
+// yuv422: the chunk holds a packed YUV 4:2:2 frame (pf non-null); launches the variant that also knows that pixel rule.
 void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s, const PixFmt* pf = nullptr,
-                            const YuvPlaneD* pl = nullptr);
+                            const YuvPlaneD* pl = nullptr, bool yuv422 = false);
 // k_letterbox_rgb: k_letterbox (transposed = 0) or k_letterbox_tr (transposed = 1, orientations 5-8) with every tap read through
-// pf; lb.channels unused.  (A struct of its own: the existing parameter blocks keep their layouts.)
+// pf; lb.channels unused.  pf.yuv422 launches the instantiation that reads the taps with load_422.  (A struct of its own: the
+// existing parameter blocks keep their layouts.)
 struct LetterboxRgbP {
   LetterboxP lb;
   PixFmt pf;
@@ -399,7 +411,12 @@ struct CropOutP {
 // pl: ragged chunks of separate-plane YUV frames (k_letterbox_multi's table, indexed like fr); non-null launches the instantiation
 // that reads every frame's chroma through it.  (A kernel argument of its own: WarpP has no room left, see pf.)
 // out: non-null launches the face-crop instantiation that writes the packed arena out->dst (WarpP::crops and flip_odd unused).
-void launch_warp_affine(const WarpP& p, cudaStream_t s, const YuvPlaneD* pl = nullptr, const CropOutP* out = nullptr);
+// yuv422: the frame (uniform) or some frame of the chunk (ragged) is packed YUV 4:2:2 (p.pf non-null); launches the crop warps of
+// kernels_warp422.cu, which read such frames with load_422.  (WarpP has no room for the flag, see pf.)
+void launch_warp_affine(const WarpP& p, cudaStream_t s, const YuvPlaneD* pl = nullptr, const CropOutP* out = nullptr,
+                        bool yuv422 = false);
+// kernels_warp422.cu: yuv422::k_warp_affine on launch_warp_affine's grid (out: the face-crop epilogue, else BGRX crops).
+void launch_warp_affine_422(const WarpP& p, dim3 grid, cudaStream_t s, const CropOutP* out);
 
 // ---- mesh / iris post-processing ----
 struct MeshPostP {

@@ -1,7 +1,8 @@
 // Preprocessing kernels: fused letterbox (cv::resize INTER_LINEAR 8U fixed point +
 // copyMakeBorder(0) + BGRA/GRAY->BGR, or cvtColor YUV2BGR for NV12 / NV21 / I420 frames; k_letterbox_multi for chunks of
 // frames of different sizes and formats; k_letterbox_tr for frames stored transposed; k_letterbox_rgb for RGB, RGBA and planar
-// RGB frames, read through their PixFmt; k_letterbox_multi<., ., true> for separate-plane YUV frames) and the [-1,1] normalisation.
+// RGB frames, read through their PixFmt, and packed YUV 4:2:2 frames; k_letterbox_multi<., ., true> for separate-plane YUV frames)
+// and the [-1,1] normalisation.
 // Reference: convertImageToTensor / bgrMatToSignedFloat32 (lib/src/util/helpers.dart:303-421).
 #include "kernels.h"
 
@@ -167,13 +168,21 @@ __global__ void __launch_bounds__(256) k_letterbox_tr(LetterboxTrP p, int B) {
 // (launched with kTransposed = true, for a chunk of any orientations).
 // kPlanes: every frame of the chunk is a separate-plane YUV frame whose chroma is read through its YuvPlaneD pls[b] (launched with
 // kTransposed = true and kFmt = false); the chroma row of a tap is the same as above, only its address differs.
+// k422: the chunk also holds packed YUV 4:2:2 frames (launched with kTransposed = kFmt = true); their taps are read with load_422,
+// which needs the tap's column as well as its row.
 template <bool kFmt>
 __device__ __forceinline__ void load_packed(const uint8_t* px, int channels, const PixFmt& pf, int* v) {
   if (kFmt) load_pix(px, pf, v);
   else load_bgr(px, channels, v);
 }
+// pixel x of a packed or planar frame's row; k422: the chunk also holds packed YUV 4:2:2 frames (pf.yuv422, block-uniform)
+template <bool kFmt, bool k422>
+__device__ __forceinline__ void load_packed_at(const uint8_t* row, int x, int channels, const PixFmt& pf, int* v) {
+  if (k422 && pf.yuv422) load_422(row, x, pf, v);
+  else load_packed<kFmt>(row + (size_t)x * channels, channels, pf, v);
+}
 
-template <bool kTransposed, bool kFmt, bool kPlanes>
+template <bool kTransposed, bool kFmt, bool kPlanes, bool k422>
 __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int B, const PixFmt* pfs, const YuvPlaneD* pls) {
   const int x = blockIdx.x * 64 + (threadIdx.x & 63), y = blockIdx.y * 4 + (threadIdx.x >> 6);
   if (x >= p.dst_w || y >= p.dst_h) return;
@@ -201,10 +210,10 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
           load_yuv_planes(r0, ra >> 1, cb, pl, t10);
           load_yuv_planes(r1, rb >> 1, cb, pl, t11);
         } else if (f.channels) {
-          load_packed<kFmt>(r0 + (size_t)ca * f.channels, f.channels, pf, t00);
-          load_packed<kFmt>(r1 + (size_t)ca * f.channels, f.channels, pf, t01);
-          load_packed<kFmt>(r0 + (size_t)cb * f.channels, f.channels, pf, t10);
-          load_packed<kFmt>(r1 + (size_t)cb * f.channels, f.channels, pf, t11);
+          load_packed_at<kFmt, k422>(r0, ca, f.channels, pf, t00);
+          load_packed_at<kFmt, k422>(r1, ca, f.channels, pf, t01);
+          load_packed_at<kFmt, k422>(r0, cb, f.channels, pf, t10);
+          load_packed_at<kFmt, k422>(r1, cb, f.channels, pf, t11);
         } else {
           const uint8_t* c0 = f.c + (size_t)(ra >> 1) * f.c_row_stride;
           const uint8_t* c1 = f.c + (size_t)(rb >> 1) * f.c_row_stride;
@@ -217,7 +226,7 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
         for (int c = 0; c < 3; ++c) res[c] = resize_linear(t00[c], t01[c], t10[c], t11[c], wa, wb, va, vb);
       } else if (f.identity) {
         if (kPlanes) load_yuv_planes(f.y + (size_t)dy * f.row_stride, dy >> 1, dx, pl, res);
-        else if (f.channels) load_packed<kFmt>(f.y + (size_t)dy * f.row_stride + (size_t)dx * f.channels, f.channels, pf, res);
+        else if (f.channels) load_packed_at<kFmt, k422>(f.y + (size_t)dy * f.row_stride, dx, f.channels, pf, res);
         else load_yuv(f.y + (size_t)dy * f.row_stride, f.c + (size_t)(dy >> 1) * f.c_row_stride, dx, f, res);
       } else {
         const int* tx = p.taps + f.tx;
@@ -234,10 +243,10 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
           load_yuv_planes(r1, cb, xa, pl, t10);
           load_yuv_planes(r1, cb, xb, pl, t11);
         } else if (f.channels) {
-          load_packed<kFmt>(r0 + (size_t)xa * f.channels, f.channels, pf, t00);
-          load_packed<kFmt>(r0 + (size_t)xb * f.channels, f.channels, pf, t01);
-          load_packed<kFmt>(r1 + (size_t)xa * f.channels, f.channels, pf, t10);
-          load_packed<kFmt>(r1 + (size_t)xb * f.channels, f.channels, pf, t11);
+          load_packed_at<kFmt, k422>(r0, xa, f.channels, pf, t00);
+          load_packed_at<kFmt, k422>(r0, xb, f.channels, pf, t01);
+          load_packed_at<kFmt, k422>(r1, xa, f.channels, pf, t10);
+          load_packed_at<kFmt, k422>(r1, xb, f.channels, pf, t11);
         } else {
           const uint8_t* c0 = f.c + (size_t)ty[4 * f.new_h + dy] * f.c_row_stride;
           const uint8_t* c1 = f.c + (size_t)ty[5 * f.new_h + dy] * f.c_row_stride;
@@ -255,11 +264,19 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
   }
 }
 
+// pixel x of a row through its PixFmt: load_pix, or for packed YUV 4:2:2 frames (k422) load_422
+template <bool k422>
+__device__ __forceinline__ void load_fmt(const uint8_t* row, int x, int step, const PixFmt& pf, int* v) {
+  if (k422) load_422(row, x, pf, v);
+  else load_pix(row + (size_t)x * step, pf, v);
+}
+
 // RGB, RGBA and planar RGB frames (uniform chunks): the grid, taps and fixed-point resize of k_letterbox (kTransposed = false,
 // identity branch included) or of k_letterbox_tr (true, orientations 5-8: x taps name stored rows, y taps stored columns), with
 // every tap's B, G, R read through p.pf.  Swapping channels or reading three planes only changes which bytes a tap loads, so the
-// output equals letterboxing the BGR image.
-template <bool kTransposed>
+// output equals letterboxing the BGR image.  k422: packed YUV 4:2:2 frames, every tap converted as cvtColor converts it before
+// it is weighted (as k_letterbox_yuv does), so the output equals letterboxing the converted frame.
+template <bool kTransposed, bool k422>
 __global__ void __launch_bounds__(256) k_letterbox_rgb(LetterboxRgbP p, int B) {
   const LetterboxP& q = p.lb;
   const int x = blockIdx.x * 64 + (threadIdx.x & 63), y = blockIdx.y * 4 + (threadIdx.x >> 6);
@@ -272,7 +289,7 @@ __global__ void __launch_bounds__(256) k_letterbox_rgb(LetterboxRgbP p, int B) {
       const uint8_t* src = q.frames + (size_t)b * q.frame_stride;
       int res[3];
       if (!kTransposed && q.identity) {
-        load_pix(src + (size_t)dy * q.row_stride + (size_t)dx * step, p.pf, res);
+        load_fmt<k422>(src + (size_t)dy * q.row_stride, dx, step, p.pf, res);
       } else {
         const int xa = q.x0[dx], xb = q.x1[dx], wa = q.ax0[dx], wb = q.ax1[dx];
         const int ya = q.y0[dy], yb = q.y1[dy], va = q.by0[dy], vb = q.by1[dy];
@@ -280,17 +297,17 @@ __global__ void __launch_bounds__(256) k_letterbox_rgb(LetterboxRgbP p, int B) {
         if (kTransposed) {
           const uint8_t* r0 = src + (size_t)xa * q.row_stride;
           const uint8_t* r1 = src + (size_t)xb * q.row_stride;
-          load_pix(r0 + (size_t)ya * step, p.pf, t00);
-          load_pix(r1 + (size_t)ya * step, p.pf, t01);
-          load_pix(r0 + (size_t)yb * step, p.pf, t10);
-          load_pix(r1 + (size_t)yb * step, p.pf, t11);
+          load_fmt<k422>(r0, ya, step, p.pf, t00);
+          load_fmt<k422>(r1, ya, step, p.pf, t01);
+          load_fmt<k422>(r0, yb, step, p.pf, t10);
+          load_fmt<k422>(r1, yb, step, p.pf, t11);
         } else {
           const uint8_t* r0 = src + (size_t)ya * q.row_stride;
           const uint8_t* r1 = src + (size_t)yb * q.row_stride;
-          load_pix(r0 + (size_t)xa * step, p.pf, t00);
-          load_pix(r0 + (size_t)xb * step, p.pf, t01);
-          load_pix(r1 + (size_t)xa * step, p.pf, t10);
-          load_pix(r1 + (size_t)xb * step, p.pf, t11);
+          load_fmt<k422>(r0, xa, step, p.pf, t00);
+          load_fmt<k422>(r0, xb, step, p.pf, t01);
+          load_fmt<k422>(r1, xa, step, p.pf, t10);
+          load_fmt<k422>(r1, xb, step, p.pf, t11);
         }
 #pragma unroll
         for (int c = 0; c < 3; ++c) res[c] = resize_linear(t00[c], t01[c], t10[c], t11[c], wa, wb, va, vb);
@@ -336,20 +353,27 @@ void launch_letterbox_tr(const LetterboxTrP& p, int B, cudaStream_t s) {
   else k_letterbox_tr<false><<<grid, 256, 0, s>>>(p, B);
 }
 
-void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s, const PixFmt* pf, const YuvPlaneD* pl) {
+void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s, const PixFmt* pf, const YuvPlaneD* pl,
+                            bool yuv422) {
   if (B <= 0) return;
   dim3 grid((unsigned)((p.dst_w + 63) / 64), (unsigned)((p.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
-  if (pl) k_letterbox_multi<true, false, true><<<grid, 256, 0, s>>>(p, B, pf, pl);
-  else if (pf) k_letterbox_multi<true, true, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
-  else if (transposed) k_letterbox_multi<true, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
-  else k_letterbox_multi<false, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  if (pl) k_letterbox_multi<true, false, true, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  else if (pf && yuv422) k_letterbox_multi<true, true, false, true><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  else if (pf) k_letterbox_multi<true, true, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  else if (transposed) k_letterbox_multi<true, false, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  else k_letterbox_multi<false, false, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
 }
 
 void launch_letterbox_rgb(const LetterboxRgbP& p, int B, bool transposed, cudaStream_t s) {
   if (B <= 0) return;
   dim3 grid((unsigned)((p.lb.dst_w + 63) / 64), (unsigned)((p.lb.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
-  if (transposed) k_letterbox_rgb<true><<<grid, 256, 0, s>>>(p, B);
-  else k_letterbox_rgb<false><<<grid, 256, 0, s>>>(p, B);
+  if (p.pf.yuv422) {
+    if (transposed) k_letterbox_rgb<true, true><<<grid, 256, 0, s>>>(p, B);
+    else k_letterbox_rgb<false, true><<<grid, 256, 0, s>>>(p, B);
+  } else {
+    if (transposed) k_letterbox_rgb<true, false><<<grid, 256, 0, s>>>(p, B);
+    else k_letterbox_rgb<false, false><<<grid, 256, 0, s>>>(p, B);
+  }
 }
 
 void launch_normalize(const uint8_t* in, TV out, int B, cudaStream_t s) {

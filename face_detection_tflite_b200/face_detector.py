@@ -41,13 +41,15 @@ def _raise(lib, handle, code: int):
     raise RuntimeError(msg)
 
 
-_PACKED = {_ffi.FDT_MAT_8UC1: 1, _ffi.FDT_MAT_8UC3: 3, _ffi.FDT_MAT_8UC4: 4, _ffi.FDT_FMT_RGB: 3, _ffi.FDT_FMT_RGBA: 4}
-LAYOUTS = ("bgr", "rgb", "rgb_planar")
+_PACKED = {_ffi.FDT_MAT_8UC1: 1, _ffi.FDT_MAT_8UC3: 3, _ffi.FDT_MAT_8UC4: 4, _ffi.FDT_FMT_RGB: 3, _ffi.FDT_FMT_RGBA: 4,
+           _ffi.FDT_FMT_YUYV: 2, _ffi.FDT_FMT_UYVY: 2, _ffi.FDT_FMT_YVYU: 2}
+_YUV422_LAYOUTS = {"yuyv": _ffi.FDT_FMT_YUYV, "uyvy": _ffi.FDT_FMT_UYVY, "yvyu": _ffi.FDT_FMT_YVYU}
+LAYOUTS = ("bgr", "rgb", "rgb_planar") + tuple(_YUV422_LAYOUTS)
 
 
 def _row_step(mt) -> int:
-    """Bytes of one pixel within a row: the packed formats' channels, 1 for YUV and planar RGB (a row is one plane's); 0 when
-    matType is unknown."""
+    """Bytes of one pixel within a row: the packed formats' channels (2 for packed YUV 4:2:2), 1 for YUV 4:2:0 and planar RGB
+    (a row is one plane's); 0 when matType is unknown."""
     return 1 if mt in _ffi.YUV_FORMATS or mt == _ffi.FDT_FMT_RGB_PLANAR else _PACKED.get(mt, 0)
 
 
@@ -64,8 +66,15 @@ def _layout(layout) -> str:
 
 
 def _mat_type(m, i: int, layout: str = "bgr") -> int:
-    """The matType of a mat in `layout`: "bgr" (cv.Mat: HxW gray, HxWx3 BGR, HxWx4 BGRA), "rgb" (HxW gray, HxWx3 RGB, HxWx4 RGBA)
-    or "rgb_planar" (3xHxW, the R, G and B planes)."""
+    """The matType of a mat in `layout`: "bgr" (cv.Mat: HxW gray, HxWx3 BGR, HxWx4 BGRA), "rgb" (HxW gray, HxWx3 RGB, HxWx4 RGBA),
+    "rgb_planar" (3xHxW, the R, G and B planes) or "yuyv" / "uyvy" / "yvyu" (HxWx2, cv2's CV_8UC2 form of a packed YUV 4:2:2
+    frame, W even)."""
+    if layout in _YUV422_LAYOUTS:
+        if not isinstance(m, np.ndarray) or m.dtype != np.uint8 or m.ndim != 3 or m.shape[2] != 2 or m.shape[0] <= 0 or m.shape[1] <= 0:
+            raise ValueError("mat %d: layout %r expects an HxWx2 uint8 array" % (i, layout))
+        if m.shape[1] % 2:
+            raise ValueError("mat %d: YUV 4:2:2 frames need an even width" % i)
+        return _YUV422_LAYOUTS[layout]
     if layout == "rgb_planar":
         if not isinstance(m, np.ndarray) or m.dtype != np.uint8 or m.ndim != 3 or m.shape[0] != 3 or m.shape[1] <= 0 or m.shape[2] <= 0:
             raise ValueError("mat %d: layout 'rgb_planar' expects a 3xHxW uint8 array" % i)
@@ -103,6 +112,8 @@ def _frame_geometry(i: int, w, h, mt, stride):
         raise ValueError("frame %d: rowStride smaller than width * channels" % i)
     if yuv and (w % 2 or h % 2):
         raise ValueError("frame %d: YUV 4:2:0 frames need an even width and height" % i)
+    if mt in _ffi.YUV422_FORMATS and w % 2:
+        raise ValueError("frame %d: YUV 4:2:2 frames need an even width" % i)
     return int(stride), _frame_bytes(mt, h, stride)
 
 
@@ -296,9 +307,12 @@ class FaceDetector:
         """detectFacesFromMatBytes (face_detector.dart:588-609); the default mode is `full` like the reference's
         (detector + mesh + iris; the blendshape classifier is outside this path).  matType may also be one of the YUV 4:2:0
         formats FDT_FMT_YUV_NV12 / _NV21 / _I420: `data` is then width * height * 3 / 2 bytes (cv2's (3H/2) x W Mat), or one of
-        the RGB formats FDT_FMT_RGB / _RGBA / _RGB_PLANAR (width * height * 3, * 4, or 3 * width * height bytes).
+        the RGB formats FDT_FMT_RGB / _RGBA / _RGB_PLANAR (width * height * 3, * 4, or 3 * width * height bytes), or one of the
+        packed YUV 4:2:2 formats FDT_FMT_YUYV / _UYVY / _YVYU (width * height * 2 bytes, width even).
         orientation (EXIF 1..8, FDT_ORIENT_*): the frame is stored rotated / mirrored; width and height are the stored size,
         the faces are those of the upright image exif_transform(frame, orientation), normalised to its size."""
+        if matType in _ffi.YUV422_FORMATS and width % 2:
+            raise ValueError("YUV 4:2:2 frames need an even width")
         if _orientation(orientation) != 1:
             self._check()
             return self.detectFacesBatch(data, count=1, width=width, height=height, matType=matType, mode=mode,
@@ -307,6 +321,8 @@ class FaceDetector:
         buf = np.ascontiguousarray(np.frombuffer(data, np.uint8) if not isinstance(data, np.ndarray) else data.reshape(-1))
         if matType in _ffi.YUV_FORMATS and buf.size != width * height * 3 // 2:
             raise ValueError("bytes length does not equal width * height * 3 / 2")        # helpers.dart:440-447
+        if matType in _ffi.YUV422_FORMATS and buf.size != width * height * 2:
+            raise ValueError("bytes length does not equal width * height * 2")
         faces = (_ffi.FdtFace * self._max_faces)()
         count = C.c_int32(0)
         mode = FaceDetectionMode(mode)
@@ -362,8 +378,9 @@ class FaceDetector:
                            orientation: int = 1, layout: str = "bgr") -> List[Face]:
         """detectFacesFromMat (face_detector.dart:559-572): `mat` is an HxW[xC] uint8 array (cv.Mat), stored in EXIF
         `orientation` (see detectFacesFromMatBytes).  layout: "bgr" (cv.Mat channel order), "rgb" (HxWx3 RGB, HxWx4 RGBA, HxW
-        gray: PIL, imageio, Flutter rawRgba) or "rgb_planar" (3xHxW, e.g. a decoded torchvision image moved to the host).  The
-        faces equal those of the BGR image."""
+        gray: PIL, imageio, Flutter rawRgba), "rgb_planar" (3xHxW, e.g. a decoded torchvision image moved to the host) or
+        "yuyv" / "uyvy" / "yvyu" (HxWx2 packed YUV 4:2:2, W even: V4L2 webcams, capture cards, GStreamer; cv2's CV_8UC2 Mat).
+        The faces equal those of the BGR image (for YUV 4:2:2: of cv2.cvtColor(mat, COLOR_YUV2BGR_YUYV / _UYVY / _YVYU))."""
         if _layout(layout) != "bgr":
             mt = _mat_type(mat, 0, layout)
             h, w = mat.shape[1:] if mt == _ffi.FDT_FMT_RGB_PLANAR else mat.shape[:2]
@@ -379,7 +396,8 @@ class FaceDetector:
     def detectFacesBatch(self, frames, *, count: int, width: int, height: int, matType: int = 16,
                          mode: FaceDetectionMode = FaceDetectionMode.fast, orientation: int = 1) -> List[List[Face]]:
         """New batched entry point: `frames` holds `count` packed frames (bytes / uint8 array), or `count` YUV 4:2:0 frames of
-        width * height * 3 / 2 bytes with matType FDT_FMT_YUV_NV12 / _NV21 / _I420.  orientation: EXIF 1..8 of every frame
+        width * height * 3 / 2 bytes with matType FDT_FMT_YUV_NV12 / _NV21 / _I420 (packed YUV 4:2:2, FDT_FMT_YUYV / _UYVY /
+        _YVYU: width * height * 2 bytes).  orientation: EXIF 1..8 of every frame
         (see detectBatchRaw); the faces refer to the upright image."""
         uw, uh = _upright(width, height, _orientation(orientation))
         self._check()
@@ -400,7 +418,7 @@ class FaceDetector:
         `frames` may be a numpy array / bytes (host) or an integer device pointer with memKind=FDT_MEM_DEVICE (a CUDA tensor:
         t.data_ptr()).  YUV 4:2:0 formats: rowStride is the Y-plane stride (default: width) and a frame is
         height * rowStride * 3 / 2 bytes.  FDT_FMT_RGB_PLANAR: rowStride is one plane's row stride (default: width) and a frame
-        is 3 * height * rowStride bytes.
+        is 3 * height * rowStride bytes.  FDT_FMT_YUYV / _UYVY / _YVYU: width even, rowStride >= 2 * width (default 2 * width).
         orientation (EXIF 1..8, FDT_ORIENT_*; fdt_detect_batch_oriented): every frame is stored rotated / mirrored.  width,
         height and rowStride describe the stored frames; faces are normalised to the upright image exif_transform(frame,
         orientation) and mesh / iris points are in its pixels."""
@@ -411,6 +429,8 @@ class FaceDetector:
         stride = rowStride if rowStride is not None else width * ch
         if ch and stride < width * ch:
             raise ValueError("rowStride smaller than width * channels")
+        if matType in _ffi.YUV422_FORMATS and width % 2:
+            raise ValueError("YUV 4:2:2 frames need an even width")
         frame_bytes = _frame_bytes(matType, height, stride)
         if isinstance(frames, int):
             ptr = frames
@@ -441,7 +461,8 @@ class FaceDetector:
     # -- mixed batches: frames of different sizes and formats, and encoded images, in one call ----------------------------
     def detectFacesFromMats(self, mats, *, mode: FaceDetectionMode = FaceDetectionMode.full,
                             orientations=None, layout: str = "bgr") -> List[List[Face]]:
-        """detectFacesFromMat over a list of HxW / HxWx3 / HxWx4 uint8 arrays of any sizes, in one batched call
+        """detectFacesFromMat over a list of HxW / HxWx3 / HxWx4 (or, with a YUV 4:2:2 layout, HxWx2) uint8 arrays of any sizes,
+        in one batched call
         (fdt_detect_frames).  A row-padded view (e.g. a crop of a larger array) goes in uncopied with strides[0] as its row
         stride.  Returns one list of faces per mat, each normalised to its own mat.  orientations: one EXIF orientation 1..8
         per mat (fdt_detect_frames_oriented), or None for all upright; faces then refer to each mat's upright image.

@@ -96,6 +96,19 @@ enum { FDT_FMT_YUV_NV12 = 0x1000, FDT_FMT_YUV_NV21 = 0x1001, FDT_FMT_YUV_I420 = 
  * A row_stride below the minimum returns FDT_ERR_SIZE_MISMATCH. */
 enum { FDT_FMT_RGB = 0x1010, FDT_FMT_RGBA = 0x1011, FDT_FMT_RGB_PLANAR = 0x1012 };
 
+/* Packed YUV 4:2:2 frames (USB / UVC webcams through V4L2: YUYV; SDI / HDMI capture cards, DeckLink 2vuy: UYVY; GStreamer
+ * YUY2 / UYVY / YVYU caps), accepted wherever mat_type is, except by fdt_extract_aligned_squares (FDT_ERR_BAD_ARG).  Every
+ * result equals the same call on cv::cvtColor(frame, COLOR_YUV2BGR_YUYV / _UYVY / _YVYU) as a BGR frame, bit for bit (BT.601
+ * limited range, as the YUV 4:2:0 formats); the conversion is fused into the letterbox and crop kernels (no converted copy).
+ * Pixel (x, y) lies in row frame + y * row_stride, in the 4-byte macropixel at byte 4 * (x / 2), which two pixels share:
+ *   FDT_FMT_YUYV (= YUY2)  Y0 U Y1 V   Y of pixel x at byte 2x,     U at 4 * (x / 2) + 1, V at 4 * (x / 2) + 3
+ *   FDT_FMT_UYVY           U Y0 V Y1   Y of pixel x at byte 2x + 1, U at 4 * (x / 2),     V at 4 * (x / 2) + 2
+ *   FDT_FMT_YVYU           Y0 V Y1 U   Y of pixel x at byte 2x,     U at 4 * (x / 2) + 3, V at 4 * (x / 2) + 1
+ * width must be even (else FDT_ERR_BAD_ARG; for orientations 5-8 the stored width); height may be any positive value.
+ * row_stride >= 2 * width (else FDT_ERR_SIZE_MISMATCH), odd strides included; a frame is height * row_stride bytes (cv2's
+ * H x W CV_8UC2 Mat when row_stride = 2 * width). */
+enum { FDT_FMT_YUYV = 0x1020, FDT_FMT_UYVY = 0x1021, FDT_FMT_YVYU = 0x1022 };
+
 enum { FDT_MEM_HOST = 0, FDT_MEM_DEVICE = 1 };
 
 /* Frame orientation (fdt_detect_batch_oriented, fdt_detect_frames_oriented): the EXIF Orientation value of the STORED frame,
@@ -169,7 +182,8 @@ FDT_EXPORT int32_t fdt_destroy(fdt_handle* h);
 
 /* New batched entry point (Dart: detectFacesBatch).  `frames` is `batch` tightly laid out images
  * of height x row_stride bytes (row_stride >= width * channels(mat_type); YUV formats: height * row_stride * 3 / 2
- * bytes, see FDT_FMT_YUV_NV12; planar RGB: 3 * height * row_stride, see FDT_FMT_RGB), in host (pinned or
+ * bytes, see FDT_FMT_YUV_NV12; planar RGB: 3 * height * row_stride, see FDT_FMT_RGB; packed YUV 4:2:2: row_stride >= 2 * width,
+ * see FDT_FMT_YUYV), in host (pinned or
  * pageable) or device memory.  Replaces the per-frame sequence
  * _detectDetections -> applyDetectionGates -> computeFaceAlignment [-> extractAlignedSquare ->
  * FaceLandmark.callWithScore -> transformMeshToAbsolute]
@@ -190,7 +204,7 @@ typedef struct fdt_frame {
   int32_t width, height;     /* image size                                                                        */
   int32_t row_stride;        /* as fdt_detect_batch: >= width * channels; YUV: the Y-plane stride                 */
   int32_t mat_type;          /* FDT_MAT_8UC1 / _8UC3 / _8UC4, FDT_FMT_YUV_NV12 / _NV21 / _I420, FDT_FMT_RGB / _RGBA /
-                                _RGB_PLANAR                                                                       */
+                                _RGB_PLANAR, FDT_FMT_YUYV / _UYVY / _YVYU                                         */
 } fdt_frame;                 /* 24 bytes */
 
 /* detectFacesFromMat over a list of frames of different sizes and formats (photos, mixed camera feeds), batched like
@@ -327,7 +341,8 @@ FDT_EXPORT int32_t fdt_copy_face_crops(fdt_handle* h, void* dst, size_t capacity
 /* detectFacesFromMatBytes (lib/src/face_detector.dart:588-609): one packed frame of
  * `nbytes` bytes; FDT_ERR_SIZE_MISMATCH when nbytes != width*height*channels
  * (matFromPackedBytes, lib/src/util/helpers.dart:432-450), or != width*height*3/2 for the YUV formats
- * (FDT_FMT_RGB: width*height*3, FDT_FMT_RGBA: width*height*4, FDT_FMT_RGB_PLANAR: 3*width*height). */
+ * (FDT_FMT_RGB: width*height*3, FDT_FMT_RGBA: width*height*4, FDT_FMT_RGB_PLANAR: 3*width*height,
+ * FDT_FMT_YUYV / _UYVY / _YVYU: 2*width*height). */
 FDT_EXPORT int32_t fdt_detect_one(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int32_t width,
                                   int32_t height, int32_t mat_type, int32_t mode, fdt_face* out_faces,
                                   int32_t* out_count, float* out_mesh, float* out_iris);
@@ -422,7 +437,8 @@ FDT_EXPORT int64_t fdt_last_launch_count(fdt_handle* h);
  * orientations 1-4, U's x taps for 5-8 (a 1280x720 frame stored sideways still uploads 2 rows in 10), after the flips.  The two
  * axes clamp differently at the borders, so at some sizes that set differs from orientation 1's.  RGB and RGBA frames upload as
  * BGR and BGRA do.  Planar RGB frames are read as 3 * height stacked rows: when height is a multiple of the period the same
- * pattern runs through all three planes (1280x720: 552,960 bytes per frame, as BGR), otherwise whole frames go up.  Mixed calls
+ * pattern runs through all three planes (1280x720: 552,960 bytes per frame, as BGR), otherwise whole frames go up.  Packed YUV
+ * 4:2:2 frames upload as a packed format of 2 bytes per pixel (1280x720: rows 10k+4, 10k+5, 368,640 bytes per frame).  Mixed calls
  * upload whole frames; fdt_detect_yuv_planes uploads each plane's sampled columns (see there). */
 FDT_EXPORT int64_t fdt_last_h2d_bytes(fdt_handle* h);
 /* Device time in ms of the named stage summed over the last call when stage timing was enabled

@@ -43,6 +43,14 @@ const int kFdtFmtRgb = 0x1010;
 const int kFdtFmtRgba = 0x1011;
 const int kFdtFmtRgbPlanar = 0x1012;
 
+/// Packed YUV 4:2:2 frames (fdt_api.h FDT_FMT_YUYV / _UYVY / _YVYU): a USB webcam's V4L2 YUYV buffer, a capture card's UYVY
+/// frame or a GStreamer YUY2 / UYVY / YVYU buffer goes in as it is.  2 bytes per pixel (two pixels share one 4-byte
+/// macropixel), width even, rowStride >= 2 * width; results equal those of cvtColor(COLOR_YUV2BGR_YUYV / _UYVY / _YVYU).
+const int kFdtFmtYuyv = 0x1020;
+const int kFdtFmtUyvy = 0x1021;
+const int kFdtFmtYvyu = 0x1022;
+bool fdtIsYuv422(int matType) => matType == kFdtFmtYuyv || matType == kFdtFmtUyvy || matType == kFdtFmtYvyu;
+
 /// Frame orientations (fdt_api.h FDT_ORIENT_*): the EXIF Orientation value of a stored frame, as OpenCV's ExifTransform
 /// applies it.  Results of the oriented calls refer to the upright image; for 5-8 its width is the stored height.  Camera
 /// frames that must be rotated R degrees clockwise to display: 1, 6, 3, 8 for R = 0, 90, 180, 270; rotated R degrees clockwise
@@ -62,7 +70,7 @@ bool fdtIsYuv(int matType) => matType == kFdtFmtYuvNv12 || matType == kFdtFmtYuv
 /// of [matType].
 int fdtRowStride(int matType, int width) => fdtIsYuv(matType) || matType == kFdtFmtRgbPlanar
     ? width
-    : width * (matType == 0 ? 1 : (matType == 24 || matType == kFdtFmtRgba ? 4 : 3));
+    : width * (matType == 0 ? 1 : (fdtIsYuv422(matType) ? 2 : (matType == 24 || matType == kFdtFmtRgba ? 4 : 3)));
 int fdtFrameBytes(int matType, int width, int height) => fdtIsYuv(matType)
     ? height * width * 3 ~/ 2
     : (matType == kFdtFmtRgbPlanar ? 3 : 1) * height * fdtRowStride(matType, width);
