@@ -21,6 +21,11 @@ RGB_FORMATS = (FDT_FMT_RGB, FDT_FMT_RGBA, FDT_FMT_RGB_PLANAR)
 # height * rowStride bytes with rowStride >= 2 * width (cv2's HxW CV_8UC2 Mat, an HxWx2 array)
 FDT_FMT_YUYV, FDT_FMT_UYVY, FDT_FMT_YVYU = 0x1020, 0x1021, 0x1022
 YUV422_FORMATS = (FDT_FMT_YUYV, FDT_FMT_UYVY, FDT_FMT_YVYU)
+# 16-bit YUV 4:2:0 with the value in the high bits (P010 / P012 / P016: NVDEC, DXGI, hwdownload): NV12's layout of 16-bit words,
+# even width, height and rowStride >= 2 * width, height * rowStride * 3 / 2 bytes (cv2's (3H/2) x W CV_16UC1 Mat); each sample
+# is read as its high byte.  16-bit planes (yuv420p10le / p12le, P016 surfaces) go to fdt_detect_yuv_planes16 with sampleBits.
+FDT_FMT_P010 = 0x1003
+SAMPLE_BITS = (10, 12, 16)
 FDT_MEM_HOST, FDT_MEM_DEVICE = 0, 1
 # EXIF orientation of a stored frame (fdt_detect_batch_oriented / fdt_detect_frames_oriented): the upright image is
 # oracle.jpeg_ops.exif_transform(stored, orientation)
@@ -86,6 +91,8 @@ SIGNATURES = {
                                                i32p, f32p, f32p]),
     "fdt_detect_yuv_planes": (C.c_int32, [P, C.POINTER(FdtYuvPlanes), i32p, C.c_int32, C.c_int32, C.c_int32, C.POINTER(FdtFace),
                                           i32p, f32p, f32p]),
+    "fdt_detect_yuv_planes16": (C.c_int32, [P, C.POINTER(FdtYuvPlanes), i32p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                            C.POINTER(FdtFace), i32p, f32p, f32p]),
     "fdt_detect_jpeg_batch": (C.c_int32, [P, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_int32, C.c_int32, C.POINTER(FdtFace),
                                           i32p, f32p, f32p, i32p, i32p]),
     "fdt_detect_one": (C.c_int32, [P, P, C.c_size_t, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(FdtFace), i32p, f32p, f32p]),

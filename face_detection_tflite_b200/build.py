@@ -35,6 +35,7 @@ SOURCES = {
     # f64 geometry must be evaluated operation by operation (no fused multiply-add contraction)
     "kernels_post.cu": ["-fmad=false"],
     "kernels_warp422.cu": ["-fmad=false"],
+    "kernels_warp16.cu": ["-fmad=false"],
 }
 
 

@@ -228,10 +228,10 @@ bool is_rgb(int mat_type) { return mat_type == FDT_FMT_RGB || mat_type == FDT_FM
 bool is_yuv422(int mat_type) { return mat_type == FDT_FMT_YUYV || mat_type == FDT_FMT_UYVY || mat_type == FDT_FMT_YVYU; }
 
 // Bytes of one pixel within a row: the packed formats' channels, 1 for planar RGB and YUV 4:2:0 (a row is one plane's), 2 for
-// packed YUV 4:2:2; 0: unknown.
+// packed YUV 4:2:2 and P010 (a Y row of 16-bit words); 0: unknown.
 int row_step(int mat_type) {
   if (is_yuv(mat_type) || mat_type == FDT_FMT_RGB_PLANAR) return 1;
-  if (is_yuv422(mat_type)) return 2;
+  if (is_yuv422(mat_type) || mat_type == FDT_FMT_P010) return 2;
   if (mat_type == FDT_FMT_RGB) return 3;
   if (mat_type == FDT_FMT_RGBA) return 4;
   return channels_of(mat_type);
@@ -251,6 +251,8 @@ struct FrameLayout {
   long long c_off = 0;
   int c_row_bytes = 0, c_rows = 0, c_step = 0, u_off = 0, v_off = 0;
   bool planar = false;       // I420: V is a plane of its own, h / 2 rows behind U
+  bool p010 = false;         // FDT_FMT_P010: laid out as NV12 of 2-byte samples; c_step 4, u_off 1, v_off 3 name the chroma
+                             // words' high bytes, and the k16 kernels read the Y word's high byte
 };
 
 // The pixel rule of a non-YUV 4:2:0 format (kernels.h, PixFmt); plane = bytes of one plane where the frame lies.
@@ -271,6 +273,16 @@ PixFmt pix_fmt(int mat_type, long long plane) {
 // Validates the frame arguments (w, hh > 0 checked by the caller); *msg names the failure.
 int frame_layout(int mat_type, int w, int hh, int row_stride, FrameLayout* L, const char** msg) {
   *L = FrameLayout();
+  if (mat_type == FDT_FMT_P010) {
+    if ((w & 1) || (hh & 1)) { *msg = "P010 frames need an even width and height"; return FDT_ERR_BAD_ARG; }
+    if (row_stride & 1) { *msg = "P010 frames need an even row_stride"; return FDT_ERR_BAD_ARG; }
+    if (row_stride < 2 * w) { *msg = "row_stride smaller than 2 * width"; return FDT_ERR_SIZE_MISMATCH; }
+    L->yuv = true; L->p010 = true;
+    L->frame_bytes = (long long)hh * row_stride * 3 / 2;
+    L->c_off = (long long)hh * row_stride;
+    L->c_row_bytes = row_stride; L->c_rows = hh / 2; L->c_step = 4; L->u_off = 1; L->v_off = 3;
+    return FDT_OK;
+  }
   if (!is_yuv(mat_type)) {
     L->channels = row_step(mat_type);
     if (L->channels == 0) { *msg = "bad frame arguments"; return FDT_ERR_BAD_ARG; }
@@ -564,6 +576,7 @@ struct Ragged {
   // the Y plane as the kernels read it (staged host frames: row stride = width); lay[i] is the staged layout (plane_layout)
   const fdt_yuv_planes* planes = nullptr;
   std::vector<fdt_frame> pframes;
+  int bits = 0;                                         // fdt_detect_yuv_planes16: the call's sample_bits; 0: 8-bit planes
   std::map<std::tuple<int, int, int>, SizeTaps> taps;   // (stored width, height, orientation)
   int orientation(int i) const { return orientations ? orientations[i] : 1; }
 };
@@ -595,41 +608,45 @@ void frame_size(const CallArgs& a, int i, double* w, double* hh) {
 // d_desc: a mixed chunk's frame descriptors on the device (the crop warps read the frames through them); orientation: as
 // WarpP::orientation; d_pf: a mixed chunk's PixFmt table when it holds an RGB-family or YUV 4:2:2 frame, else null; d_pl: a
 // chunk's YuvPlaneD table when its separate-plane device frames do not fit FrameD, else null; yuv422: the chunk holds a packed
-// YUV 4:2:2 frame (the crop warps' launch_warp_affine flag)
+// YUV 4:2:2 frame (the crop warps' launch_warp_affine flag); yuv16: the chunk holds a P010 frame or fdt_detect_yuv_planes16
+// frames (the same for the yuv16 flags)
 struct ChunkJob {
   int off = 0, n = 0; const uint8_t* d_fr = nullptr; const FrameD* d_desc = nullptr; bool active = false; int orientation = 1;
   const PixFmt* d_pf = nullptr;
-  bool yuv422 = false;
+  bool yuv422 = false, yuv16 = false;
   const YuvPlaneD* d_pl = nullptr;
 };
 
-// Bytes of the sampled columns of one chroma row of a separate-plane frame: (width / 2 - 1) * pixel_stride + 1.
+// Samples of the sampled columns of one chroma row of a separate-plane frame: (width / 2 - 1) * pixel_stride + 1 (bytes for
+// 8-bit planes; fdt_detect_yuv_planes16's 16-bit planes take twice as many).
 long long chroma_cols(const fdt_yuv_planes& f) { return (long long)(f.width / 2 - 1) * f.pixel_stride + 1; }
 
-// U and V interleaved in one chroma plane (NV12 / NV21, Android pixel stride 2 views of one buffer): pixel stride 2, one row
-// stride of at least width, V one byte behind or before U.  Each chroma row's width bytes from the lower of the two are then
-// exactly the two sampled extents' bytes in that row.
-bool interleaved_chroma(const fdt_yuv_planes& f) {
+// U and V interleaved in one chroma plane (NV12 / NV21, Android pixel stride 2 views of one buffer; P016 surfaces with bps = 2):
+// pixel stride 2, one row stride of at least width samples, V one sample behind or before U.  Each chroma row's width samples
+// from the lower of the two are then exactly the two sampled extents' bytes in that row.  bps: bytes per sample, 1 or 2.
+bool interleaved_chroma(const fdt_yuv_planes& f, int bps) {
   const uintptr_t u = reinterpret_cast<uintptr_t>(f.plane[1]), v = reinterpret_cast<uintptr_t>(f.plane[2]);
-  return f.pixel_stride == 2 && f.row_stride[1] == f.row_stride[2] && f.row_stride[1] >= f.width && (v == u + 1 || u == v + 1);
+  return f.pixel_stride == 2 && f.row_stride[1] == f.row_stride[2] && f.row_stride[1] >= f.width * bps &&
+         (v == u + bps || u == v + bps);
 }
 
-// A separate-plane frame as it is staged from host memory: the Y plane (width bytes per row), then the chroma, which FrameD
-// describes as it describes NV12 / NV21 and I420 frames.  Interleaved chroma: one area of height / 2 rows of width bytes (the
-// bytes fdt_detect_frames uploads for an NV12 frame).  Otherwise the U and then the V area, height / 2 rows of chroma_cols bytes
-// each, chroma step pixel_stride.
-FrameLayout plane_layout(const fdt_yuv_planes& f) {
+// A separate-plane frame as it is staged from host memory: the Y plane (width samples per row), then the chroma, which FrameD
+// describes as it describes NV12 / NV21 and I420 frames.  Interleaved chroma: one area of height / 2 rows of width samples (the
+// bytes fdt_detect_frames uploads for an NV12 frame).  Otherwise the U and then the V area, height / 2 rows of chroma_cols
+// samples each, chroma step pixel_stride.  bps: bytes per sample (2: fdt_detect_yuv_planes16, whose staged chroma the kernels
+// read through YuvPlaneD with u_off, v_off and c_row_bytes in bytes).
+FrameLayout plane_layout(const fdt_yuv_planes& f, int bps) {
   FrameLayout L;
   L.yuv = true;
-  L.c_off = (long long)f.width * f.height;
-  L.c_step = f.pixel_stride;
-  if (interleaved_chroma(f)) {
-    L.c_row_bytes = f.width; L.c_rows = f.height / 2;
-    L.u_off = f.plane[1] < f.plane[2] ? 0 : 1; L.v_off = 1 - L.u_off;
-    L.frame_bytes = L.c_off + (long long)(f.height / 2) * f.width;
+  L.c_off = (long long)f.width * bps * f.height;
+  L.c_step = f.pixel_stride * bps;
+  if (interleaved_chroma(f, bps)) {
+    L.c_row_bytes = f.width * bps; L.c_rows = f.height / 2;
+    L.u_off = f.plane[1] < f.plane[2] ? 0 : bps; L.v_off = bps - L.u_off;
+    L.frame_bytes = L.c_off + (long long)(f.height / 2) * L.c_row_bytes;
     return L;
   }
-  const long long cc = chroma_cols(f);
+  const long long cc = chroma_cols(f) * bps;
   L.planar = true;
   L.c_row_bytes = (int)cc; L.c_rows = f.height; L.u_off = 0; L.v_off = (int)(f.height / 2 * cc);
   L.frame_bytes = L.c_off + 2 * (f.height / 2) * cc;
@@ -637,9 +654,10 @@ FrameLayout plane_layout(const fdt_yuv_planes& f) {
 }
 
 // The sampled columns of every row, one 2-D copy per plane (interleaved chroma: one copy for U and V): nothing past a plane's
-// sampled extent is read.
-void upload_planes(uint8_t* dst, const fdt_yuv_planes& f, const FrameLayout& L, cudaStream_t s) {
-  cudaMemcpy2DAsync(dst, f.width, f.plane[0], f.row_stride[0], f.width, f.height, cudaMemcpyHostToDevice, s);
+// sampled extent is read.  bps: bytes per sample.
+void upload_planes(uint8_t* dst, const fdt_yuv_planes& f, const FrameLayout& L, int bps, cudaStream_t s) {
+  const size_t y_row = (size_t)f.width * bps;
+  cudaMemcpy2DAsync(dst, y_row, f.plane[0], f.row_stride[0], y_row, f.height, cudaMemcpyHostToDevice, s);
   if (!L.planar) {
     cudaMemcpy2DAsync(dst + L.c_off, L.c_row_bytes, std::min(f.plane[1], f.plane[2]), f.row_stride[1], L.c_row_bytes, f.height / 2,
                       cudaMemcpyHostToDevice, s);
@@ -663,7 +681,7 @@ size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 // blob (frame descriptors, concatenated tap tables, decode geometry and, for a chunk with an RGB-family frame, every frame's
 // PixFmt) in one copy; then k_letterbox_multi.
 int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, const FrameD** d_desc, const double** d_geom,
-                 int* orientation, const PixFmt** d_pf, const YuvPlaneD** d_pl, bool* yuv422) {
+                 int* orientation, const PixFmt** d_pf, const YuvPlaneD** d_pl, bool* yuv422, bool* yuv16) {
   cudaStream_t s = sl.stream;
   Ragged& rg = *a.rg;
   const fdt_frame* fr = rg.frames + off;
@@ -682,7 +700,7 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
     }
     for (int i = 0; i < n; ++i) {
       const size_t fb = (size_t)rg.lay[off + i].frame_bytes;
-      if (rg.planes) upload_planes(sl.d_frames + at[i], rg.planes[off + i], rg.lay[off + i], s);
+      if (rg.planes) upload_planes(sl.d_frames + at[i], rg.planes[off + i], rg.lay[off + i], rg.bits ? 2 : 1, s);
       else cudaMemcpyAsync(sl.d_frames + at[i], fr[i].data, fb, cudaMemcpyHostToDevice, s);
       h->h2d_bytes += (long long)fb;
       base[i] = sl.d_frames + at[i];
@@ -696,9 +714,11 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
   size_t ntaps = 0;
   bool upright = true, transposed = false, rgb = false;
   *yuv422 = false;
+  *yuv16 = rg.bits != 0;
   for (int i = 0; i < n; ++i) {
     rgb = rgb || rg.lay[off + i].rgb;
     *yuv422 = *yuv422 || rg.lay[off + i].px.yuv422;
+    *yuv16 = *yuv16 || rg.lay[off + i].p010;
     const int o = rg.orientation(off + i);
     upright = upright && o == 1;
     transposed = transposed || orient_transposed(o);
@@ -710,7 +730,8 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
   }
   *orientation = upright ? 1 : 0;
   const fdt_yuv_planes* pl = rg.planes ? rg.planes + off : nullptr;
-  bool table = false;
+  // fdt_detect_yuv_planes16 frames, host or device, always go through the table (it carries their shift)
+  bool table = rg.bits != 0;
   for (int i = 0; pl && a.mem_kind == FDT_MEM_DEVICE && i < n; ++i) table = table || !fits_frame_desc(pl[i]);
   const size_t taps_at = align_up((size_t)n * sizeof(FrameD), 16), geom_at = align_up(taps_at + ntaps * sizeof(int), 16);
   // a chunk with an RGB-family or YUV 4:2:2 frame also carries every frame's PixFmt (k_letterbox_multi<true, true>,
@@ -746,16 +767,19 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
     d.w = fr[i].width; d.h = fr[i].height; d.row_stride = fr[i].row_stride; d.channels = L.channels;
     d.c_row_stride = L.c_row_bytes; d.c_step = L.c_step; d.u_off = L.u_off; d.v_off = L.v_off;
     d.new_w = lp.new_w; d.new_h = lp.new_h; d.pad_top = lp.pad_top; d.pad_left = lp.pad_left; d.identity = st[i]->identity ? 1 : 0;
-    if (pl && a.mem_kind == FDT_MEM_DEVICE) {
+    if (pl && table) {
       const fdt_yuv_planes& f = pl[i];
-      if (table) {
-        d.c = nullptr;
-        reinterpret_cast<YuvPlaneD*>(sl.h_blob + pf_at)[i] = YuvPlaneD{f.plane[1], f.plane[2], f.row_stride[1], f.row_stride[2], f.pixel_stride, 0};
-      } else {
-        d.c = std::min(f.plane[1], f.plane[2]);
-        d.c_row_stride = f.row_stride[1]; d.c_step = f.pixel_stride;
-        d.u_off = (int)(f.plane[1] - d.c); d.v_off = (int)(f.plane[2] - d.c);
+      d.c = nullptr;
+      YuvPlaneD q{f.plane[1], f.plane[2], f.row_stride[1], f.row_stride[2], f.pixel_stride, rg.bits ? rg.bits - 8 : 0};
+      if (a.mem_kind == FDT_MEM_HOST) {   // fdt_detect_yuv_planes16: the staged chroma (plane_layout)
+        q.u = base[i] + L.c_off + L.u_off; q.v = base[i] + L.c_off + L.v_off; q.u_stride = q.v_stride = L.c_row_bytes;
       }
+      reinterpret_cast<YuvPlaneD*>(sl.h_blob + pf_at)[i] = q;
+    } else if (pl && a.mem_kind == FDT_MEM_DEVICE) {
+      const fdt_yuv_planes& f = pl[i];
+      d.c = std::min(f.plane[1], f.plane[2]);
+      d.c_row_stride = f.row_stride[1]; d.c_step = f.pixel_stride;
+      d.u_off = (int)(f.plane[1] - d.c); d.v_off = (int)(f.plane[2] - d.c);
     }
     d.orientation = rg.orientation(off + i);
     d.tx = tap_at[std::make_tuple(d.w, d.h, d.orientation)]; d.ty = d.tx + 4 * lp.new_w;
@@ -777,7 +801,7 @@ int stage_ragged(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, con
   StageTimer t(h, 0, s);
   LetterboxMultiP lb;
   lb.fr = *d_desc; lb.taps = reinterpret_cast<const int*>(sl.d_blob + taps_at); lb.out = sl.d_lb; lb.dst_w = S_w; lb.dst_h = S_h;
-  launch_letterbox_multi(lb, n, transposed, s, *d_pf, *d_pl, *yuv422);
+  launch_letterbox_multi(lb, n, transposed, s, *d_pf, *d_pl, *yuv422, *yuv16);
   t.launches = 1;
   return FDT_OK;
 }
@@ -865,12 +889,12 @@ int stage_uniform(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, co
         lb.yp = LetterboxYuvP();
         fill_letterbox(lb.yp.lb, tb, d_fr, dev_frame_stride, a.row_stride, a.channels, a.w, a.hh, sl.d_lb, S_w, S_h, sparse);
       }
-      launch_letterbox_tr(lb, n, s);
+      launch_letterbox_tr(lb, n, s, a.lay.p010);
     } else if (a.lay.yuv) {
       if (!d_c) d_c = d_fr + a.lay.c_off;     // whole frames
       LetterboxYuvP lb;
       fill_letterbox_yuv(lb, tb, a.lay, d_fr, y_stride, y_sparse, d_c, c_stride, c_sparse, a.row_stride, a.w, a.hh, sl.d_lb, S_w, S_h);
-      launch_letterbox_yuv(lb, n, s);
+      launch_letterbox_yuv(lb, n, s, a.lay.p010);
     } else {
       LetterboxP lb;
       fill_letterbox(lb, tb, d_fr, dev_frame_stride, a.row_stride, a.channels, a.w, a.hh, sl.d_lb, S_w, S_h, sparse);
@@ -890,8 +914,8 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
   int orientation = a.orientation;
   const PixFmt* d_pf = nullptr;
   const YuvPlaneD* d_pl = nullptr;
-  bool yuv422 = a.lay.px.yuv422 != 0;
-  const int rc = a.rg ? stage_ragged(h, sl, a, off, n, &d_desc, &d_geom, &orientation, &d_pf, &d_pl, &yuv422)
+  bool yuv422 = a.lay.px.yuv422 != 0, yuv16 = a.lay.p010;
+  const int rc = a.rg ? stage_ragged(h, sl, a, off, n, &d_desc, &d_geom, &orientation, &d_pf, &d_pl, &yuv422, &yuv16)
                       : stage_uniform(h, sl, a, off, n, &d_fr);
   if (rc != FDT_OK) return rc;
   {
@@ -922,7 +946,7 @@ int enqueue_detect(fdt_handle* h, Slot& sl, const CallArgs& a, int off, int n, b
                       cudaMemcpyDeviceToHost, s);
   }
   job->off = off; job->n = n; job->d_fr = d_fr; job->d_desc = d_desc; job->active = true; job->orientation = orientation;
-  job->d_pf = d_pf; job->d_pl = d_pl; job->yuv422 = yuv422;
+  job->d_pf = d_pf; job->d_pl = d_pl; job->yuv422 = yuv422; job->yuv16 = yuv16;
   return FDT_OK;
 }
 
@@ -1054,7 +1078,7 @@ int launch_face_crops(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob
       CropOutP o;
       o.dst = h->d_crop_arena; o.first = h->crop_n; o.layout = sp.layout;
       for (int c = 0; c < 3; ++c) { o.scale[c] = sp.scale[c]; o.bias[c] = sp.bias[c]; }
-      launch_warp_affine(wp, s, job.d_pl, &o, job.yuv422);
+      launch_warp_affine(wp, s, job.d_pl, &o, job.yuv422, job.yuv16);
       t.launches = 1;
     }
     // the reference returns null for these: the crop is all zero bytes (its ok flag says so)
@@ -1120,7 +1144,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
       WarpP wp = chunk_warp(a, job, d_pf);
       wp.crop_img = sl.d_crop_img; wp.affine = sl.d_affine; wp.ncrops = nf; wp.out_size = kMeshInput; wp.flip_odd = 0;
       wp.crops = sl.d_crops;
-      launch_warp_affine(wp, s, job.d_pl, nullptr, job.yuv422);
+      launch_warp_affine(wp, s, job.d_pl, nullptr, job.yuv422, job.yuv16);
       t.launches = 1;
     }
     {
@@ -1200,7 +1224,7 @@ int finish_mesh(fdt_handle* h, Slot& sl, const CallArgs& a, const ChunkJob& job)
           WarpP wp = chunk_warp(a, job, d_pf);
           wp.crop_img = sl.d_eye_img; wp.affine = sl.d_eye_affine; wp.ncrops = ne; wp.out_size = kIrisInput; wp.flip_odd = 1;
           wp.crops = sl.d_eye_crops;
-          launch_warp_affine(wp, s, job.d_pl, nullptr, job.yuv422);
+          launch_warp_affine(wp, s, job.d_pl, nullptr, job.yuv422, job.yuv16);
           t.launches = 1;
         }
         {
@@ -1348,8 +1372,9 @@ int check_frames(fdt_handle* h, const fdt_frame* frames, const int32_t* orientat
 }
 
 // fdt_detect_yuv_planes' argument checks, every descriptor before any work; *lay receives the frames' staged layouts.
+// bits: fdt_detect_yuv_planes16's sample_bits (16-bit words: extents of 2 bytes per sample, even pointers and strides); 0: 8-bit.
 int check_planes(fdt_handle* h, const fdt_yuv_planes* frames, const int32_t* orientations, int n, int mode, int mem_kind,
-                 const fdt_face* out_faces, const int32_t* out_counts, std::vector<FrameLayout>* lay) {
+                 const fdt_face* out_faces, const int32_t* out_counts, std::vector<FrameLayout>* lay, int bits = 0) {
   if (n < 0 || (n > 0 && !frames)) return fail(h, FDT_ERR_BAD_ARG, "bad frame list");
   if (mem_kind != FDT_MEM_HOST && mem_kind != FDT_MEM_DEVICE) return fail(h, FDT_ERR_BAD_ARG, "unknown mem_kind");
   if (int rc = check_mode(h, mode)) return rc;
@@ -1366,13 +1391,20 @@ int check_planes(fdt_handle* h, const fdt_yuv_planes* frames, const int32_t* ori
     if (f.pixel_stride != 1 && f.pixel_stride != 2) return fail(h, FDT_ERR_BAD_ARG, at() + "pixel_stride must be 1 or 2");
     for (int k = 0; k < 3; ++k)
       if (f.row_stride[k] <= 0) return fail(h, FDT_ERR_BAD_ARG, at() + kPlane[k] + ": row_stride must be positive");
-    if (f.row_stride[0] < f.width) return fail(h, FDT_ERR_SIZE_MISMATCH, at() + "plane Y: row_stride smaller than width");
+    const int bps = bits ? 2 : 1;
+    if (bits)
+      for (int k = 0; k < 3; ++k)
+        if ((reinterpret_cast<uintptr_t>(f.plane[k]) | (uintptr_t)f.row_stride[k]) & 1)
+          return fail(h, FDT_ERR_BAD_ARG, at() + kPlane[k] + ": 16-bit planes need an even pointer and row_stride");
+    if (f.row_stride[0] < (long long)f.width * bps)
+      return fail(h, FDT_ERR_SIZE_MISMATCH, at() + (bits ? "plane Y: row_stride smaller than 2 * width" : "plane Y: row_stride smaller than width"));
     for (int k = 1; k < 3; ++k)
-      if (f.row_stride[k] < chroma_cols(f))
-        return fail(h, FDT_ERR_SIZE_MISMATCH, at() + kPlane[k] + ": row_stride smaller than (width / 2 - 1) * pixel_stride + 1");
+      if (f.row_stride[k] < chroma_cols(f) * bps)
+        return fail(h, FDT_ERR_SIZE_MISMATCH, at() + kPlane[k] + (bits ? ": row_stride smaller than 2 * ((width / 2 - 1) * pixel_stride + 1)"
+                                                                       : ": row_stride smaller than (width / 2 - 1) * pixel_stride + 1"));
     if (orientations && (orientations[i] < 1 || orientations[i] > 8))
       return fail(h, FDT_ERR_BAD_ARG, at() + "orientation must be an EXIF value 1..8");
-    (*lay)[i] = plane_layout(f);
+    (*lay)[i] = plane_layout(f, bps);
   }
   return FDT_OK;
 }
@@ -1411,19 +1443,22 @@ bool device_pointer_ok(fdt_handle* h, const void* p, std::vector<std::pair<uintp
 // What a ragged call was given: fdt_frame descriptors (fdt_detect_frames, the JPEG batch) or fdt_yuv_planes descriptors.
 enum class FrameList { kFrames, kYuvPlanes };
 
-// fdt_detect_frames (kFrames: `frames`) and fdt_detect_yuv_planes (kYuvPlanes: `planes`, frames unused) on one device.
+// fdt_detect_frames (kFrames: `frames`) and fdt_detect_yuv_planes (kYuvPlanes: `planes`, frames unused) on one device; bits:
+// fdt_detect_yuv_planes16's sample_bits, 0 for 8-bit planes.
 int detect_frames_single(fdt_handle* h, const fdt_frame* frames, const int32_t* orientations, int n, int mode, int mem_kind,
                          fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris,
-                         FrameList list = FrameList::kFrames, const fdt_yuv_planes* planes = nullptr) {
+                         FrameList list = FrameList::kFrames, const fdt_yuv_planes* planes = nullptr, int bits = 0) {
   if (!h || !h->ready) return fail(h, FDT_ERR_NOT_READY, "detector is not initialised");
   Ragged rg;
   if (list == FrameList::kYuvPlanes) {
-    if (int rc = check_planes(h, planes, orientations, n, mode, mem_kind, out_faces, out_counts, &rg.lay)) return rc;
+    if (int rc = check_planes(h, planes, orientations, n, mode, mem_kind, out_faces, out_counts, &rg.lay, bits)) return rc;
     rg.planes = planes;
+    rg.bits = bits;
     rg.pframes.resize(n);
+    const int bps = bits ? 2 : 1;
     for (int i = 0; i < n; ++i) {
       const fdt_yuv_planes& f = planes[i];
-      rg.pframes[i] = fdt_frame{f.plane[0], f.width, f.height, mem_kind == FDT_MEM_HOST ? f.width : f.row_stride[0], FDT_FMT_YUV_I420};
+      rg.pframes[i] = fdt_frame{f.plane[0], f.width, f.height, mem_kind == FDT_MEM_HOST ? f.width * bps : f.row_stride[0], FDT_FMT_YUV_I420};
     }
     frames = rg.pframes.data();
   } else if (int rc = check_frames(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, &rg.lay)) {
@@ -1509,16 +1544,16 @@ int detect_frames_multi(fdt_handle* h, const fdt_frame* frames, const int32_t* o
 }
 
 int detect_planes_multi(fdt_handle* h, const fdt_yuv_planes* planes, const int32_t* orientations, int n, int mode, int mem_kind,
-                        fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris) {
+                        fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris, int bits = 0) {
   std::vector<FrameLayout> lay;
-  if (int rc = check_planes(h, planes, orientations, n, mode, mem_kind, out_faces, out_counts, &lay)) return rc;
+  if (int rc = check_planes(h, planes, orientations, n, mode, mem_kind, out_faces, out_counts, &lay, bits)) return rc;
   if (mem_kind != FDT_MEM_HOST) return fail(h, FDT_ERR_UNSUPPORTED, "a multi-device handle takes host frames (device memory belongs to one device)");
   return on_shards(h, n, [=](fdt_handle* sh, int lo, int hi) {
     const size_t mf = (size_t)sh->max_faces;
     return detect_frames_single(sh, nullptr, orientations ? orientations + lo : nullptr, hi - lo, mode, mem_kind,
                                 out_faces + lo * mf, out_counts + lo,
                                 out_mesh ? out_mesh + lo * mf * FDT_MESH_FLOATS : nullptr,
-                                out_iris ? out_iris + lo * mf * FDT_IRIS_FLOATS : nullptr, FrameList::kYuvPlanes, planes + lo);
+                                out_iris ? out_iris + lo * mf * FDT_IRIS_FLOATS : nullptr, FrameList::kYuvPlanes, planes + lo, bits);
   });
 }
 
@@ -2107,6 +2142,19 @@ int32_t fdt_detect_yuv_planes(fdt_handle* h, const fdt_yuv_planes* frames, const
                               FrameList::kYuvPlanes, frames);
 }
 
+int32_t fdt_detect_yuv_planes16(fdt_handle* h, const fdt_yuv_planes* frames, const int32_t* orientations, int32_t n,
+                                int32_t sample_bits, int32_t mode, int32_t mem_kind, fdt_face* out_faces, int32_t* out_counts,
+                                float* out_mesh, float* out_iris) {
+  if (!h) return fail(nullptr, FDT_ERR_NOT_READY, "null handle");
+  std::lock_guard<std::mutex> g(h->mu);
+  reset_crops(h);
+  if (sample_bits != 10 && sample_bits != 12 && sample_bits != 16) return fail(h, FDT_ERR_BAD_ARG, "sample_bits must be 10, 12 or 16");
+  if (!h->shards.empty())
+    return detect_planes_multi(h, frames, orientations, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris, sample_bits);
+  return detect_frames_single(h, nullptr, orientations, n, mode, mem_kind, out_faces, out_counts, out_mesh, out_iris,
+                              FrameList::kYuvPlanes, frames, sample_bits);
+}
+
 int32_t fdt_detect_jpeg_batch(fdt_handle* h, const uint8_t* const* images, const size_t* sizes, int32_t n, int32_t mode,
                               fdt_face* out_faces, int32_t* out_counts, float* out_mesh, float* out_iris, int32_t* out_wh,
                               int32_t* out_status) {
@@ -2681,7 +2729,7 @@ int32_t fdt_profile_chunk(fdt_handle* h, const uint8_t* d_frames, int32_t n, int
       LetterboxYuvP lb;
       fill_letterbox_yuv(lb, tb, lay, d_frames, lay.frame_bytes, false, d_frames + lay.c_off, lay.frame_bytes, false, row_stride,
                          width, height, sl.d_lb, S_w, S_h);
-      launch_letterbox_yuv(lb, n, s);
+      launch_letterbox_yuv(lb, n, s, lay.p010);
     } else {
       LetterboxP lb;
       fill_letterbox(lb, tb, d_frames, lay.frame_bytes, row_stride, lay.channels, width, height, sl.d_lb, S_w, S_h, false);

@@ -96,7 +96,9 @@ struct LetterboxYuvP {
   int c_row_stride, c_step, u_off, v_off;
   const int* cy0; const int* cy1;
 };
-void launch_letterbox_yuv(const LetterboxYuvP& p, int B, cudaStream_t s);
+// p010: the frames are FDT_FMT_P010 (c_step 4, u_off 1, v_off 3: the chroma words' high bytes); launches k_letterbox_yuv<true>,
+// which reads the Y sample of pixel x as byte 2x + 1 of its row.
+void launch_letterbox_yuv(const LetterboxYuvP& p, int B, cudaStream_t s, bool p010 = false);
 // Frames stored transposed (EXIF orientations 5-8, see fdt_detect_batch_oriented), k_letterbox_tr: the letterbox of the upright
 // image U.  The tables are U's (x taps from U's width, y taps from U's height, flips folded in on the host), but the x taps,
 // indexed by the output column, name stored ROWS and the y taps, indexed by the output row, stored COLUMNS.  YUV frames (yuv = 1):
@@ -106,7 +108,8 @@ struct LetterboxTrP {
   LetterboxYuvP yp;
   int yuv;
 };
-void launch_letterbox_tr(const LetterboxTrP& p, int B, cudaStream_t s);
+// p010 (with yuv = 1): FDT_FMT_P010 frames, as for launch_letterbox_yuv.
+void launch_letterbox_tr(const LetterboxTrP& p, int B, cudaStream_t s, bool p010 = false);
 // RGB, RGBA and planar RGB frames (FDT_FMT_RGB / _RGBA / _RGB_PLANAR): every non-YUV format is a pixel step and the byte offsets
 // of its B, G and R samples from the pixel's first byte (row + x * step):
 //   BGR 3: 0, 1, 2   RGB 3: 2, 1, 0   BGRA 4: 0, 1, 2   RGBA 4: 2, 1, 0   GRAY 1: 0, 0, 0   planar RGB 1: 2P, P, 0
@@ -135,6 +138,8 @@ struct FrameD {
   const uint8_t* c;        // YUV 4:2:0: the chroma area, addressed as in LetterboxYuvP (v_off relative to it)
   int w, h, row_stride;
   int channels;            // 1 / 3 / 4 (RGB-family frames: their pixel step); 2: packed YUV 4:2:2; 0: YUV 4:2:0
+  // YUV 4:2:0: c_step 4 (u_off 1, v_off 3) is a P010 frame, 16-bit words read by their high bytes (the Y sample of pixel x at
+  // byte 2x + 1 of its row); only the k16 variants (k_letterbox_multi<., ., ., ., true>, yuv16::k_warp_affine) take such frames
   int c_row_stride, c_step, u_off, v_off;
   int new_w, new_h, pad_top, pad_left, identity;
   int tx, ty;              // offsets (ints) of the frame's x taps [4][new_w] and y taps [6][new_h] in the chunk's tap table
@@ -143,15 +148,26 @@ struct FrameD {
 // Separate-plane YUV 4:2:0 frames (fdt_detect_yuv_planes) in device memory whose U and V planes FrameD cannot describe (different
 // strides, or more than an int apart): the chroma samples of pixel (x, y) are u[(y / 2) * u_stride + (x / 2) * ps] and
 // v[(y / 2) * v_stride + (x / 2) * ps]; the frame's FrameD gives the Y plane.  One entry per frame of the chunk, in the chunk blob.
+// fdt_detect_yuv_planes16 (every frame, host or device, through this table): the planes hold 16-bit words, strides count bytes,
+// ps and x count samples, and shift = sample_bits - 8 (load_yuv_planes16).  8-bit frames leave shift 0 and unread.
 struct YuvPlaneD {
   const uint8_t* u;
   const uint8_t* v;
-  int u_stride, v_stride, ps, reserved;
+  int u_stride, v_stride, ps, shift;
 };
 #ifdef __CUDACC__
 __device__ __forceinline__ void load_yuv_planes(const uint8_t* yrow, int crow, int x, const YuvPlaneD& q, int* v) {
   const size_t cx = (size_t)(x >> 1) * q.ps;
   yuv_to_bgr(yrow[x], q.u[(size_t)crow * q.u_stride + cx], q.v[(size_t)crow * q.v_stride + cx], v);
+}
+// The 8-bit sample of a 16-bit word with shift + 8 significant bits from bit 0: (s >> shift) & 0xFF (truncation; bits above the
+// significant ones are ignored).
+__device__ __forceinline__ int sample16(const uint8_t* p, int shift) { return (*reinterpret_cast<const uint16_t*>(p) >> shift) & 0xFF; }
+// load_yuv_planes over planes of 16-bit words: every sample reduced to 8 bits first, then the 8-bit conversion.
+__device__ __forceinline__ void load_yuv_planes16(const uint8_t* yrow, int crow, int x, const YuvPlaneD& q, int* v) {
+  const size_t cx = (size_t)(x >> 1) * q.ps * 2;
+  yuv_to_bgr(sample16(yrow + (size_t)x * 2, q.shift), sample16(q.u + (size_t)crow * q.u_stride + cx, q.shift),
+             sample16(q.v + (size_t)crow * q.v_stride + cx, q.shift), v);
 }
 #endif
 // k_letterbox_multi: k_letterbox / k_letterbox_yuv per frame.  taps (host-built, resize_linear_taps): per distinct size and
@@ -171,8 +187,10 @@ struct LetterboxMultiP {
 // pl (device, [B]): the chunk's frames are all separate-plane YUV frames read through their YuvPlaneD (any orientation; pf null).
 // (A kernel argument of its own, behind pfs, for the same reason.)
 // yuv422: the chunk holds a packed YUV 4:2:2 frame (pf non-null); launches the variant that also knows that pixel rule.
+// yuv16: the chunk holds a P010 frame (FrameD::c_step 4), or its frames are fdt_detect_yuv_planes16 frames (pl non-null, every
+// frame's shift set); launches the k16 variant, which reduces every 16-bit sample to 8 bits before the conversion.
 void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s, const PixFmt* pf = nullptr,
-                            const YuvPlaneD* pl = nullptr, bool yuv422 = false);
+                            const YuvPlaneD* pl = nullptr, bool yuv422 = false, bool yuv16 = false);
 // k_letterbox_rgb: k_letterbox (transposed = 0) or k_letterbox_tr (transposed = 1, orientations 5-8) with every tap read through
 // pf; lb.channels unused.  pf.yuv422 launches the instantiation that reads the taps with load_422.  (A struct of its own: the
 // existing parameter blocks keep their layouts.)
@@ -413,10 +431,14 @@ struct CropOutP {
 // out: non-null launches the face-crop instantiation that writes the packed arena out->dst (WarpP::crops and flip_odd unused).
 // yuv422: the frame (uniform) or some frame of the chunk (ragged) is packed YUV 4:2:2 (p.pf non-null); launches the crop warps of
 // kernels_warp422.cu, which read such frames with load_422.  (WarpP has no room for the flag, see pf.)
+// yuv16: the frame (uniform) or some frame of the chunk (ragged) is P010 (c_step 4), or pl holds fdt_detect_yuv_planes16 frames;
+// launches the crop warps of kernels_warp16.cu, which reduce every 16-bit sample to 8 bits before the conversion.
 void launch_warp_affine(const WarpP& p, cudaStream_t s, const YuvPlaneD* pl = nullptr, const CropOutP* out = nullptr,
-                        bool yuv422 = false);
+                        bool yuv422 = false, bool yuv16 = false);
 // kernels_warp422.cu: yuv422::k_warp_affine on launch_warp_affine's grid (out: the face-crop epilogue, else BGRX crops).
 void launch_warp_affine_422(const WarpP& p, dim3 grid, cudaStream_t s, const CropOutP* out);
+// kernels_warp16.cu: yuv16::k_warp_affine on launch_warp_affine's grid (pl: the plane table of fdt_detect_yuv_planes16 frames).
+void launch_warp_affine_16(const WarpP& p, dim3 grid, cudaStream_t s, const YuvPlaneD* pl, const CropOutP* out);
 
 // ---- mesh / iris post-processing ----
 struct MeshPostP {

@@ -219,6 +219,7 @@ __global__ void __launch_bounds__(kDecodeThreads) k_decode_nms(DecodeP p) {
 
 // ------------------------------------------------------------------------------------------
 constexpr bool kWarpYuv422 = false;   // warp_affine.cuh: chunks with a packed YUV 4:2:2 frame take kernels_warp422.cu
+constexpr bool kWarp16 = false;       // and chunks with a 16-bit YUV 4:2:0 frame kernels_warp16.cu
 #include "warp_affine.cuh"
 
 // ------------------------------------------------------------------------------------------
@@ -323,8 +324,10 @@ template <bool kFmt, bool kOut> void launch_warp(const WarpP& p, dim3 grid, cuda
 }
 
 template <bool kOut> void launch_warp_any(const WarpP& p, dim3 grid, cudaStream_t s, const YuvPlaneD* pl, const CropOutP& o,
-                                          bool yuv422) {
-  if (pl) {
+                                          bool yuv422, bool yuv16) {
+  if (yuv16) {
+    launch_warp_affine_16(p, grid, s, pl, kOut ? &o : nullptr);
+  } else if (pl) {
     if (p.orientation != 1) k_warp_affine<true, true, false, true, kOut><<<grid, 256, 0, s>>>(p, pl, o);
     else k_warp_affine<true, false, false, true, kOut><<<grid, 256, 0, s>>>(p, pl, o);
   } else if (p.pf && yuv422) {
@@ -336,11 +339,11 @@ template <bool kOut> void launch_warp_any(const WarpP& p, dim3 grid, cudaStream_
   }
 }
 
-void launch_warp_affine(const WarpP& p, cudaStream_t s, const YuvPlaneD* pl, const CropOutP* out, bool yuv422) {
+void launch_warp_affine(const WarpP& p, cudaStream_t s, const YuvPlaneD* pl, const CropOutP* out, bool yuv422, bool yuv16) {
   if (p.ncrops <= 0) return;
   dim3 grid((p.out_size * p.out_size + 255) / 256, p.ncrops);
-  if (out) launch_warp_any<true>(p, grid, s, pl, *out, yuv422);
-  else launch_warp_any<false>(p, grid, s, pl, CropOutP(), yuv422);
+  if (out) launch_warp_any<true>(p, grid, s, pl, *out, yuv422, yuv16);
+  else launch_warp_any<false>(p, grid, s, pl, CropOutP(), yuv422, yuv16);
 }
 
 void launch_mesh_post(const MeshPostP& p, cudaStream_t s) {

@@ -1,8 +1,8 @@
 // Preprocessing kernels: fused letterbox (cv::resize INTER_LINEAR 8U fixed point +
 // copyMakeBorder(0) + BGRA/GRAY->BGR, or cvtColor YUV2BGR for NV12 / NV21 / I420 frames; k_letterbox_multi for chunks of
 // frames of different sizes and formats; k_letterbox_tr for frames stored transposed; k_letterbox_rgb for RGB, RGBA and planar
-// RGB frames, read through their PixFmt, and packed YUV 4:2:2 frames; k_letterbox_multi<., ., true> for separate-plane YUV frames)
-// and the [-1,1] normalisation.
+// RGB frames, read through their PixFmt, and packed YUV 4:2:2 frames; k_letterbox_multi<., ., true> for separate-plane YUV frames;
+// the k16 variants for 16-bit YUV 4:2:0, P010 and fdt_detect_yuv_planes16 frames) and the [-1,1] normalisation.
 // Reference: convertImageToTensor / bgrMatToSignedFloat32 (lib/src/util/helpers.dart:303-421).
 #include "kernels.h"
 
@@ -65,19 +65,29 @@ __global__ void __launch_bounds__(256) k_letterbox(LetterboxP p, int B) {
   }
 }
 
+// The Y sample of pixel x: its byte, or for P010 (k16) the high byte of its 16-bit word, (s >> 8) & 0xFF.  A P010 frame's chroma
+// step and offsets (4, 1, 3) already name the high bytes of its U and V words.
+template <bool k16>
+__device__ __forceinline__ int y_sample(const uint8_t* yrow, int x) { return k16 ? yrow[(size_t)x * 2 + 1] : yrow[x]; }
+
 // One YUV 4:2:0 tap: the Y byte and the chroma pair of its 2x2 block, converted to BGR (cvtColor first, then resize).
+template <bool k16 = false>
 __device__ __forceinline__ void load_yuv(const uint8_t* yrow, const uint8_t* crow, int x, const LetterboxYuvP& p, int* v) {
   const uint8_t* c = crow + (size_t)(x >> 1) * p.c_step;
-  yuv_to_bgr(yrow[x], c[p.u_off], c[p.v_off], v);
+  yuv_to_bgr(y_sample<k16>(yrow, x), c[p.u_off], c[p.v_off], v);
 }
 // the same for a frame of a ragged chunk
+template <bool k16 = false>
 __device__ __forceinline__ void load_yuv(const uint8_t* yrow, const uint8_t* crow, int x, const FrameD& f, int* v) {
   const uint8_t* c = crow + (size_t)(x >> 1) * f.c_step;
-  yuv_to_bgr(yrow[x], c[f.u_off], c[f.v_off], v);
+  yuv_to_bgr(y_sample<k16>(yrow, x), c[f.u_off], c[f.v_off], v);
 }
 
 // k_letterbox for NV12 / NV21 / I420 frames: same grid and fixed-point resize; every tap is converted before it is weighted
 // (the conversion is per pixel, so this equals resizing the converted frame).  Padding stays BGR 0.
+// k16: P010 frames; each tap's samples are reduced to 8 bits on load (y_sample), so the output equals that of the NV12 frame
+// made of the words' high bytes.
+template <bool k16>
 __global__ void __launch_bounds__(256) k_letterbox_yuv(LetterboxYuvP p, int B) {
   const LetterboxP& q = p.lb;
   const int x = blockIdx.x * 64 + (threadIdx.x & 63), y = blockIdx.y * 4 + (threadIdx.x >> 6);
@@ -90,7 +100,7 @@ __global__ void __launch_bounds__(256) k_letterbox_yuv(LetterboxYuvP p, int B) {
       const uint8_t* cs = p.chroma + (size_t)b * p.c_frame_stride;
       if (q.identity) {
         int v[3];
-        load_yuv(ys + (size_t)dy * q.row_stride, cs + (size_t)(dy >> 1) * p.c_row_stride, dx, p, v);
+        load_yuv<k16>(ys + (size_t)dy * q.row_stride, cs + (size_t)(dy >> 1) * p.c_row_stride, dx, p, v);
         o = make_uchar3((unsigned char)v[0], (unsigned char)v[1], (unsigned char)v[2]);
       } else {
         const int xa = q.x0[dx], xb = q.x1[dx], wa = q.ax0[dx], wb = q.ax1[dx];
@@ -101,10 +111,10 @@ __global__ void __launch_bounds__(256) k_letterbox_yuv(LetterboxYuvP p, int B) {
         const uint8_t* r1 = ys + (size_t)yb * q.row_stride;
         const uint8_t* c0 = cs + (size_t)ca * p.c_row_stride;
         const uint8_t* c1 = cs + (size_t)cb * p.c_row_stride;
-        load_yuv(r0, c0, xa, p, t00);
-        load_yuv(r0, c0, xb, p, t01);
-        load_yuv(r1, c1, xa, p, t10);
-        load_yuv(r1, c1, xb, p, t11);
+        load_yuv<k16>(r0, c0, xa, p, t00);
+        load_yuv<k16>(r0, c0, xb, p, t01);
+        load_yuv<k16>(r1, c1, xa, p, t10);
+        load_yuv<k16>(r1, c1, xb, p, t11);
         int res[3];
 #pragma unroll
         for (int c = 0; c < 3; ++c) res[c] = resize_linear(t00[c], t01[c], t10[c], t11[c], wa, wb, va, vb);
@@ -120,7 +130,8 @@ __global__ void __launch_bounds__(256) k_letterbox_yuv(LetterboxYuvP p, int B) {
 // So U's four taps t00 = U(xa, ya), t01 = U(xb, ya), t10 = U(xa, yb), t11 = U(xb, yb) are read from stored rows xa / xb and stored
 // columns ya / yb, and resize_linear weights them exactly as it weights an upright frame's taps: the output bytes are those of
 // letterboxing U itself.  No identity branch: at equal sizes the taps are (i, weight 2048 / 0), which resize_linear returns exactly.
-template <bool kYuv>
+// k16 (with kYuv): P010 frames, read as k_letterbox_yuv<true> reads them.
+template <bool kYuv, bool k16>
 __global__ void __launch_bounds__(256) k_letterbox_tr(LetterboxTrP p, int B) {
   const LetterboxP& q = p.yp.lb;
   const int x = blockIdx.x * 64 + (threadIdx.x & 63), y = blockIdx.y * 4 + (threadIdx.x >> 6);
@@ -139,10 +150,10 @@ __global__ void __launch_bounds__(256) k_letterbox_tr(LetterboxTrP p, int B) {
         const uint8_t* cs = p.yp.chroma + (size_t)b * p.yp.c_frame_stride;
         const uint8_t* c0 = cs + (size_t)p.yp.cy0[dx] * p.yp.c_row_stride;
         const uint8_t* c1 = cs + (size_t)p.yp.cy1[dx] * p.yp.c_row_stride;
-        load_yuv(r0, c0, ca, p.yp, t00);
-        load_yuv(r1, c1, ca, p.yp, t01);
-        load_yuv(r0, c0, cb, p.yp, t10);
-        load_yuv(r1, c1, cb, p.yp, t11);
+        load_yuv<k16>(r0, c0, ca, p.yp, t00);
+        load_yuv<k16>(r1, c1, ca, p.yp, t01);
+        load_yuv<k16>(r0, c0, cb, p.yp, t10);
+        load_yuv<k16>(r1, c1, cb, p.yp, t11);
       } else {
         load_bgr(r0 + (size_t)ca * q.channels, q.channels, t00);
         load_bgr(r1 + (size_t)ca * q.channels, q.channels, t01);
@@ -170,6 +181,9 @@ __global__ void __launch_bounds__(256) k_letterbox_tr(LetterboxTrP p, int B) {
 // kTransposed = true and kFmt = false); the chroma row of a tap is the same as above, only its address differs.
 // k422: the chunk also holds packed YUV 4:2:2 frames (launched with kTransposed = kFmt = true); their taps are read with load_422,
 // which needs the tap's column as well as its row.
+// k16 (launched with kTransposed = true): the chunk holds P010 frames (c_step 4), whose Y samples are read by y_sample<true>, or
+// (with kPlanes) every frame is an fdt_detect_yuv_planes16 frame, read with load_yuv_planes16 and its YuvPlaneD::shift.  Only the
+// loads differ; every tap's samples are 8-bit before yuv_to_bgr, so the output is that of the 8-bit frame.
 template <bool kFmt>
 __device__ __forceinline__ void load_packed(const uint8_t* px, int channels, const PixFmt& pf, int* v) {
   if (kFmt) load_pix(px, pf, v);
@@ -181,8 +195,20 @@ __device__ __forceinline__ void load_packed_at(const uint8_t* row, int x, int ch
   if (k422 && pf.yuv422) load_422(row, x, pf, v);
   else load_packed<kFmt>(row + (size_t)x * channels, channels, pf, v);
 }
+// a YUV 4:2:0 tap of a ragged chunk's frame; k16: the chunk may hold P010 frames (c_step 4, block-uniform)
+template <bool k16>
+__device__ __forceinline__ void load_yuv_frame(const uint8_t* yrow, const uint8_t* crow, int x, const FrameD& f, int* v) {
+  if (k16 && f.c_step == 4) load_yuv<true>(yrow, crow, x, f, v);
+  else load_yuv(yrow, crow, x, f, v);
+}
+// a tap of a separate-plane frame; k16: planes of 16-bit words
+template <bool k16>
+__device__ __forceinline__ void load_planes(const uint8_t* yrow, int crow, int x, const YuvPlaneD& q, int* v) {
+  if (k16) load_yuv_planes16(yrow, crow, x, q, v);
+  else load_yuv_planes(yrow, crow, x, q, v);
+}
 
-template <bool kTransposed, bool kFmt, bool kPlanes, bool k422>
+template <bool kTransposed, bool kFmt, bool kPlanes, bool k422, bool k16>
 __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int B, const PixFmt* pfs, const YuvPlaneD* pls) {
   const int x = blockIdx.x * 64 + (threadIdx.x & 63), y = blockIdx.y * 4 + (threadIdx.x >> 6);
   if (x >= p.dst_w || y >= p.dst_h) return;
@@ -205,10 +231,10 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
         const uint8_t* r0 = f.y + (size_t)ra * f.row_stride;
         const uint8_t* r1 = f.y + (size_t)rb * f.row_stride;
         if (kPlanes) {
-          load_yuv_planes(r0, ra >> 1, ca, pl, t00);
-          load_yuv_planes(r1, rb >> 1, ca, pl, t01);
-          load_yuv_planes(r0, ra >> 1, cb, pl, t10);
-          load_yuv_planes(r1, rb >> 1, cb, pl, t11);
+          load_planes<k16>(r0, ra >> 1, ca, pl, t00);
+          load_planes<k16>(r1, rb >> 1, ca, pl, t01);
+          load_planes<k16>(r0, ra >> 1, cb, pl, t10);
+          load_planes<k16>(r1, rb >> 1, cb, pl, t11);
         } else if (f.channels) {
           load_packed_at<kFmt, k422>(r0, ca, f.channels, pf, t00);
           load_packed_at<kFmt, k422>(r1, ca, f.channels, pf, t01);
@@ -217,17 +243,17 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
         } else {
           const uint8_t* c0 = f.c + (size_t)(ra >> 1) * f.c_row_stride;
           const uint8_t* c1 = f.c + (size_t)(rb >> 1) * f.c_row_stride;
-          load_yuv(r0, c0, ca, f, t00);
-          load_yuv(r1, c1, ca, f, t01);
-          load_yuv(r0, c0, cb, f, t10);
-          load_yuv(r1, c1, cb, f, t11);
+          load_yuv_frame<k16>(r0, c0, ca, f, t00);
+          load_yuv_frame<k16>(r1, c1, ca, f, t01);
+          load_yuv_frame<k16>(r0, c0, cb, f, t10);
+          load_yuv_frame<k16>(r1, c1, cb, f, t11);
         }
 #pragma unroll
         for (int c = 0; c < 3; ++c) res[c] = resize_linear(t00[c], t01[c], t10[c], t11[c], wa, wb, va, vb);
       } else if (f.identity) {
-        if (kPlanes) load_yuv_planes(f.y + (size_t)dy * f.row_stride, dy >> 1, dx, pl, res);
+        if (kPlanes) load_planes<k16>(f.y + (size_t)dy * f.row_stride, dy >> 1, dx, pl, res);
         else if (f.channels) load_packed_at<kFmt, k422>(f.y + (size_t)dy * f.row_stride, dx, f.channels, pf, res);
-        else load_yuv(f.y + (size_t)dy * f.row_stride, f.c + (size_t)(dy >> 1) * f.c_row_stride, dx, f, res);
+        else load_yuv_frame<k16>(f.y + (size_t)dy * f.row_stride, f.c + (size_t)(dy >> 1) * f.c_row_stride, dx, f, res);
       } else {
         const int* tx = p.taps + f.tx;
         const int* ty = p.taps + f.ty;
@@ -238,10 +264,10 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
         const uint8_t* r1 = f.y + (size_t)yb * f.row_stride;
         if (kPlanes) {
           const int ca = ty[4 * f.new_h + dy], cb = ty[5 * f.new_h + dy];
-          load_yuv_planes(r0, ca, xa, pl, t00);
-          load_yuv_planes(r0, ca, xb, pl, t01);
-          load_yuv_planes(r1, cb, xa, pl, t10);
-          load_yuv_planes(r1, cb, xb, pl, t11);
+          load_planes<k16>(r0, ca, xa, pl, t00);
+          load_planes<k16>(r0, ca, xb, pl, t01);
+          load_planes<k16>(r1, cb, xa, pl, t10);
+          load_planes<k16>(r1, cb, xb, pl, t11);
         } else if (f.channels) {
           load_packed_at<kFmt, k422>(r0, xa, f.channels, pf, t00);
           load_packed_at<kFmt, k422>(r0, xb, f.channels, pf, t01);
@@ -250,10 +276,10 @@ __global__ void __launch_bounds__(256) k_letterbox_multi(LetterboxMultiP p, int 
         } else {
           const uint8_t* c0 = f.c + (size_t)ty[4 * f.new_h + dy] * f.c_row_stride;
           const uint8_t* c1 = f.c + (size_t)ty[5 * f.new_h + dy] * f.c_row_stride;
-          load_yuv(r0, c0, xa, f, t00);
-          load_yuv(r0, c0, xb, f, t01);
-          load_yuv(r1, c1, xa, f, t10);
-          load_yuv(r1, c1, xb, f, t11);
+          load_yuv_frame<k16>(r0, c0, xa, f, t00);
+          load_yuv_frame<k16>(r0, c0, xb, f, t01);
+          load_yuv_frame<k16>(r1, c1, xa, f, t10);
+          load_yuv_frame<k16>(r1, c1, xb, f, t11);
         }
 #pragma unroll
         for (int c = 0; c < 3; ++c) res[c] = resize_linear(t00[c], t01[c], t10[c], t11[c], wa, wb, va, vb);
@@ -340,28 +366,35 @@ void launch_letterbox(const LetterboxP& p, int B, cudaStream_t s) {
   k_letterbox<<<grid, 256, 0, s>>>(p, B);
 }
 
-void launch_letterbox_yuv(const LetterboxYuvP& p, int B, cudaStream_t s) {
+void launch_letterbox_yuv(const LetterboxYuvP& p, int B, cudaStream_t s, bool p010) {
   if (B <= 0) return;
   dim3 grid((unsigned)((p.lb.dst_w + 63) / 64), (unsigned)((p.lb.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
-  k_letterbox_yuv<<<grid, 256, 0, s>>>(p, B);
+  if (p010) k_letterbox_yuv<true><<<grid, 256, 0, s>>>(p, B);
+  else k_letterbox_yuv<false><<<grid, 256, 0, s>>>(p, B);
 }
 
-void launch_letterbox_tr(const LetterboxTrP& p, int B, cudaStream_t s) {
+void launch_letterbox_tr(const LetterboxTrP& p, int B, cudaStream_t s, bool p010) {
   if (B <= 0) return;
   dim3 grid((unsigned)((p.yp.lb.dst_w + 63) / 64), (unsigned)((p.yp.lb.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
-  if (p.yuv) k_letterbox_tr<true><<<grid, 256, 0, s>>>(p, B);
-  else k_letterbox_tr<false><<<grid, 256, 0, s>>>(p, B);
+  if (p.yuv && p010) k_letterbox_tr<true, true><<<grid, 256, 0, s>>>(p, B);
+  else if (p.yuv) k_letterbox_tr<true, false><<<grid, 256, 0, s>>>(p, B);
+  else k_letterbox_tr<false, false><<<grid, 256, 0, s>>>(p, B);
 }
 
 void launch_letterbox_multi(const LetterboxMultiP& p, int B, bool transposed, cudaStream_t s, const PixFmt* pf, const YuvPlaneD* pl,
-                            bool yuv422) {
+                            bool yuv422, bool yuv16) {
   if (B <= 0) return;
   dim3 grid((unsigned)((p.dst_w + 63) / 64), (unsigned)((p.dst_h + 3) / 4), (unsigned)(B < 65535 ? B : 65535));
-  if (pl) k_letterbox_multi<true, false, true, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
-  else if (pf && yuv422) k_letterbox_multi<true, true, false, true><<<grid, 256, 0, s>>>(p, B, pf, pl);
-  else if (pf) k_letterbox_multi<true, true, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
-  else if (transposed) k_letterbox_multi<true, false, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
-  else k_letterbox_multi<false, false, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  if (yuv16) {
+    if (pl) k_letterbox_multi<true, false, true, false, true><<<grid, 256, 0, s>>>(p, B, pf, pl);
+    else if (pf && yuv422) k_letterbox_multi<true, true, false, true, true><<<grid, 256, 0, s>>>(p, B, pf, pl);
+    else if (pf) k_letterbox_multi<true, true, false, false, true><<<grid, 256, 0, s>>>(p, B, pf, pl);
+    else k_letterbox_multi<true, false, false, false, true><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  } else if (pl) k_letterbox_multi<true, false, true, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  else if (pf && yuv422) k_letterbox_multi<true, true, false, true, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  else if (pf) k_letterbox_multi<true, true, false, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  else if (transposed) k_letterbox_multi<true, false, false, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
+  else k_letterbox_multi<false, false, false, false, false><<<grid, 256, 0, s>>>(p, B, pf, pl);
 }
 
 void launch_letterbox_rgb(const LetterboxRgbP& p, int B, bool transposed, cudaStream_t s) {

@@ -10,6 +10,7 @@ namespace {
 namespace yuv422 {
 
 constexpr bool kWarpYuv422 = true;
+constexpr bool kWarp16 = false;
 #include "warp_affine.cuh"
 
 template <bool kOut> void launch(const WarpP& p, dim3 grid, cudaStream_t s, const CropOutP& o) {

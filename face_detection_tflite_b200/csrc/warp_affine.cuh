@@ -1,7 +1,8 @@
 // k_warp_affine: cv::warpAffine(INTER_LINEAR, BORDER_CONSTANT 0) of a list of ROIs into square crops.  Included by
-// kernels_post.cu with kWarpYuv422 = false (the crop warps of every format but packed YUV 4:2:2) and by kernels_warp422.cu, inside
-// namespace yuv422, with kWarpYuv422 = true (a chunk or frame that holds packed YUV 4:2:2), so both translation units compile the
-// same source and the first keeps its code.  Both compile with -fmad=false: the f64 map is evaluated operation by operation.
+// kernels_post.cu with kWarpYuv422 = kWarp16 = false (the crop warps of every 8-bit format but packed YUV 4:2:2), by
+// kernels_warp422.cu, inside namespace yuv422, with kWarpYuv422 = true (a chunk or frame that holds packed YUV 4:2:2), and by
+// kernels_warp16.cu, inside namespace yuv16, with both true (a chunk or frame that holds 16-bit YUV 4:2:0), so every translation
+// unit compiles the same source and the first keeps its code.  Both compile with -fmad=false: the f64 map is evaluated operation by operation.
 // Included inside an anonymous namespace of fdt, after kernels.h and fdt_math.h.
 
 __device__ __forceinline__ long long sat_round_ll(double v) { return (long long)rint(v); }
@@ -19,6 +20,9 @@ __device__ __forceinline__ long long sat_round_ll(double v) { return (long long)
 // out.layout (FDT_CROP_RGB / _CHW / _F32); a warp's 32 pixels are consecutive in each CHW plane.
 // kWarpYuv422 (a constexpr bool of the including scope): with kFmt, a frame whose PixFmt says yuv422 has its taps read with
 // load_422 (the stored column, after the orientation mapping, picks the macropixel).
+// kWarp16 (a constexpr bool of the including scope): a YUV 4:2:0 frame with c_step 4 is P010 (its Y sample the high byte of the
+// word, byte 2x + 1; the chroma offsets already name high bytes), and kPlanes frames are fdt_detect_yuv_planes16 frames
+// (load_yuv_planes16).  Every sample is 8-bit before yuv_to_bgr, so a crop equals the crop of the 8-bit frame.
 template <bool kRagged, bool kOriented, bool kFmt, bool kPlanes, bool kOut>
 __global__ void k_warp_affine(WarpP p, const YuvPlaneD* pl, CropOutP out) {
   const int f = blockIdx.y;
@@ -65,7 +69,8 @@ __global__ void k_warp_affine(WarpP p, const YuvPlaneD* pl, CropOutP out) {
       const int row_stride = kRagged ? d->row_stride : p.row_stride;
       if (kPlanes) {
         int v[3];
-        load_yuv_planes(src + (size_t)yy * row_stride, yy >> 1, xx, q, v);
+        if (kWarp16) load_yuv_planes16(src + (size_t)yy * row_stride, yy >> 1, xx, q, v);
+        else load_yuv_planes(src + (size_t)yy * row_stride, yy >> 1, xx, q, v);
         acc[0] += v[0] * iw[t]; acc[1] += v[1] * iw[t]; acc[2] += v[2] * iw[t];
         continue;
       }
@@ -73,7 +78,9 @@ __global__ void k_warp_affine(WarpP p, const YuvPlaneD* pl, CropOutP out) {
         const uint8_t* c = (kRagged ? d->c : src + p.c_off) + (size_t)(yy >> 1) * (kRagged ? d->c_row_stride : p.c_row_stride) +
                            (size_t)(xx >> 1) * (kRagged ? d->c_step : p.c_step);
         int v[3];
-        yuv_to_bgr(src[(size_t)yy * row_stride + xx], c[kRagged ? d->u_off : p.u_off], c[kRagged ? d->v_off : p.v_off], v);
+        const int ys = kWarp16 && (kRagged ? d->c_step : p.c_step) == 4 ? src[(size_t)yy * row_stride + (size_t)xx * 2 + 1]
+                                                                          : src[(size_t)yy * row_stride + xx];
+        yuv_to_bgr(ys, c[kRagged ? d->u_off : p.u_off], c[kRagged ? d->v_off : p.v_off], v);
         acc[0] += v[0] * iw[t]; acc[1] += v[1] * iw[t]; acc[2] += v[2] * iw[t];
         continue;
       }

@@ -44,19 +44,36 @@ def _raise(lib, handle, code: int):
 _PACKED = {_ffi.FDT_MAT_8UC1: 1, _ffi.FDT_MAT_8UC3: 3, _ffi.FDT_MAT_8UC4: 4, _ffi.FDT_FMT_RGB: 3, _ffi.FDT_FMT_RGBA: 4,
            _ffi.FDT_FMT_YUYV: 2, _ffi.FDT_FMT_UYVY: 2, _ffi.FDT_FMT_YVYU: 2}
 _YUV422_LAYOUTS = {"yuyv": _ffi.FDT_FMT_YUYV, "uyvy": _ffi.FDT_FMT_UYVY, "yvyu": _ffi.FDT_FMT_YVYU}
-LAYOUTS = ("bgr", "rgb", "rgb_planar") + tuple(_YUV422_LAYOUTS)
+LAYOUTS = ("bgr", "rgb", "rgb_planar") + tuple(_YUV422_LAYOUTS) + ("p010",)
 
 
 def _row_step(mt) -> int:
     """Bytes of one pixel within a row: the packed formats' channels (2 for packed YUV 4:2:2), 1 for YUV 4:2:0 and planar RGB
-    (a row is one plane's); 0 when matType is unknown."""
+    (a row is one plane's), 2 for P010 (a Y row of 16-bit words); 0 when matType is unknown."""
+    if mt == _ffi.FDT_FMT_P010:
+        return 2
     return 1 if mt in _ffi.YUV_FORMATS or mt == _ffi.FDT_FMT_RGB_PLANAR else _PACKED.get(mt, 0)
 
 
 def _frame_bytes(mt, h, stride) -> int:
-    if mt in _ffi.YUV_FORMATS:
+    if mt in _ffi.YUV_FORMATS or mt == _ffi.FDT_FMT_P010:
         return h * stride * 3 // 2
     return 3 * h * stride if mt == _ffi.FDT_FMT_RGB_PLANAR else h * stride
+
+
+def _p010_checks(w, h, stride, what: str = "") -> None:
+    """ValueError for the P010 geometry the library refuses: odd width, height or row stride."""
+    if w % 2 or h % 2:
+        raise ValueError(what + "P010 frames need an even width and height")
+    if stride % 2:
+        raise ValueError(what + "P010 frames need an even rowStride")
+
+
+def _frame_buffer(data, mt) -> np.ndarray:
+    """A host frame as a flat uint8 array (a P010 frame may also be a uint16 array: its bytes)."""
+    if mt == _ffi.FDT_FMT_P010 and isinstance(data, np.ndarray) and data.dtype == np.uint16:
+        return np.ascontiguousarray(data).reshape(-1).view(np.uint8)
+    return np.ascontiguousarray(np.frombuffer(data, np.uint8) if not isinstance(data, np.ndarray) else data.reshape(-1))
 
 
 def _layout(layout) -> str:
@@ -68,7 +85,13 @@ def _layout(layout) -> str:
 def _mat_type(m, i: int, layout: str = "bgr") -> int:
     """The matType of a mat in `layout`: "bgr" (cv.Mat: HxW gray, HxWx3 BGR, HxWx4 BGRA), "rgb" (HxW gray, HxWx3 RGB, HxWx4 RGBA),
     "rgb_planar" (3xHxW, the R, G and B planes) or "yuyv" / "uyvy" / "yvyu" (HxWx2, cv2's CV_8UC2 form of a packed YUV 4:2:2
-    frame, W even)."""
+    frame, W even) or "p010" ((3H/2)xW uint16, cv2's CV_16UC1 form of a P010 frame, H and W even)."""
+    if layout == "p010":
+        if not isinstance(m, np.ndarray) or m.dtype != np.uint16 or m.ndim != 2 or m.shape[0] <= 0 or m.shape[1] <= 0:
+            raise ValueError("mat %d: layout 'p010' expects a (3H/2)xW uint16 array" % i)
+        if m.shape[0] % 3 or m.shape[1] % 2:      # 3H/2 rows: a multiple of 3 exactly when H is even
+            raise ValueError("mat %d: P010 frames need an even width and height ((3H/2)xW: rows a multiple of 3, W even)" % i)
+        return _ffi.FDT_FMT_P010
     if layout in _YUV422_LAYOUTS:
         if not isinstance(m, np.ndarray) or m.dtype != np.uint8 or m.ndim != 3 or m.shape[2] != 2 or m.shape[0] <= 0 or m.shape[1] <= 0:
             raise ValueError("mat %d: layout %r expects an HxWx2 uint8 array" % (i, layout))
@@ -114,6 +137,8 @@ def _frame_geometry(i: int, w, h, mt, stride):
         raise ValueError("frame %d: YUV 4:2:0 frames need an even width and height" % i)
     if mt in _ffi.YUV422_FORMATS and w % 2:
         raise ValueError("frame %d: YUV 4:2:2 frames need an even width" % i)
+    if mt == _ffi.FDT_FMT_P010:
+        _p010_checks(w, h, stride, "frame %d: " % i)
     return int(stride), _frame_bytes(mt, h, stride)
 
 
@@ -133,9 +158,10 @@ def _orientations(orientations, n: int):
     return np.array([_orientation(o, "orientations[%d]" % i) for i, o in enumerate(orientations)], np.int32)
 
 
-def _plane_extents(i: int, strides, w, h, ps) -> tuple:
+def _plane_extents(i: int, strides, w, h, ps, bps: int = 1) -> tuple:
     """The sampled extent in bytes of the Y, U and V plane of a separate-plane YUV 4:2:0 frame, (rows - 1) * stride +
-    (cols - 1) * step + 1; ValueError for the arguments fdt_detect_yuv_planes refuses."""
+    (cols - 1) * step + 1 samples of bps bytes (2: fdt_detect_yuv_planes16, strides in bytes, ps in samples); ValueError for the
+    arguments fdt_detect_yuv_planes / _planes16 refuse."""
     vals = (w, h, ps, *strides)
     if len(strides) != 3 or not all(isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in vals):
         raise ValueError("frame %d: width, height, pixel stride and the three row strides must be integers" % i)
@@ -145,12 +171,22 @@ def _plane_extents(i: int, strides, w, h, ps) -> tuple:
         raise ValueError("frame %d: the chroma pixel stride must be 1 or 2, got %r" % (i, ps))
     if min(strides) <= 0:
         raise ValueError("frame %d: row strides must be positive (bottom-up frames are not supported)" % i)
-    cc = (w // 2 - 1) * ps + 1
-    if strides[0] < w:
-        raise ValueError("frame %d: Y row stride smaller than width" % i)
+    cc = ((w // 2 - 1) * ps + 1) * bps
+    if strides[0] < w * bps:
+        raise ValueError("frame %d: Y row stride smaller than %swidth" % (i, "2 * " if bps == 2 else ""))
     if strides[1] < cc or strides[2] < cc:
-        raise ValueError("frame %d: chroma row stride smaller than (width / 2 - 1) * pixelStride + 1" % i)
-    return (h - 1) * int(strides[0]) + w, (h // 2 - 1) * int(strides[1]) + cc, (h // 2 - 1) * int(strides[2]) + cc
+        raise ValueError("frame %d: chroma row stride smaller than %s(width / 2 - 1) * pixelStride + 1%s"
+                         % (i, "2 * (" if bps == 2 else "", ")" if bps == 2 else ""))
+    if bps == 2 and any(s % 2 for s in strides):
+        raise ValueError("frame %d: 16-bit planes need even row strides" % i)
+    return (h - 1) * int(strides[0]) + w * bps, (h // 2 - 1) * int(strides[1]) + cc, (h // 2 - 1) * int(strides[2]) + cc
+
+
+def _sample_bits(bits) -> int:
+    """fdt_detect_yuv_planes16's sample_bits: 10, 12 or 16; ValueError otherwise."""
+    if isinstance(bits, bool) or not isinstance(bits, (int, np.integer)) or bits not in _ffi.SAMPLE_BITS:
+        raise ValueError("sampleBits must be 10, 12 or 16 for 16-bit planes, got %r" % (bits,))
+    return int(bits)
 
 
 def _upright(w, h, orientation) -> tuple:
@@ -308,17 +344,22 @@ class FaceDetector:
         (detector + mesh + iris; the blendshape classifier is outside this path).  matType may also be one of the YUV 4:2:0
         formats FDT_FMT_YUV_NV12 / _NV21 / _I420: `data` is then width * height * 3 / 2 bytes (cv2's (3H/2) x W Mat), or one of
         the RGB formats FDT_FMT_RGB / _RGBA / _RGB_PLANAR (width * height * 3, * 4, or 3 * width * height bytes), or one of the
-        packed YUV 4:2:2 formats FDT_FMT_YUYV / _UYVY / _YVYU (width * height * 2 bytes, width even).
+        packed YUV 4:2:2 formats FDT_FMT_YUYV / _UYVY / _YVYU (width * height * 2 bytes, width even), or FDT_FMT_P010
+        (3 * width * height bytes, or a (3H/2) x W uint16 array; width and height even).
         orientation (EXIF 1..8, FDT_ORIENT_*): the frame is stored rotated / mirrored; width and height are the stored size,
         the faces are those of the upright image exif_transform(frame, orientation), normalised to its size."""
         if matType in _ffi.YUV422_FORMATS and width % 2:
             raise ValueError("YUV 4:2:2 frames need an even width")
+        if matType == _ffi.FDT_FMT_P010:
+            _p010_checks(width, height, 0)
         if _orientation(orientation) != 1:
             self._check()
             return self.detectFacesBatch(data, count=1, width=width, height=height, matType=matType, mode=mode,
                                          orientation=orientation)[0]
         self._check()
-        buf = np.ascontiguousarray(np.frombuffer(data, np.uint8) if not isinstance(data, np.ndarray) else data.reshape(-1))
+        buf = _frame_buffer(data, matType)
+        if matType == _ffi.FDT_FMT_P010 and buf.size != width * height * 3:
+            raise ValueError("bytes length does not equal width * height * 3")
         if matType in _ffi.YUV_FORMATS and buf.size != width * height * 3 // 2:
             raise ValueError("bytes length does not equal width * height * 3 / 2")        # helpers.dart:440-447
         if matType in _ffi.YUV422_FORMATS and buf.size != width * height * 2:
@@ -379,11 +420,15 @@ class FaceDetector:
         """detectFacesFromMat (face_detector.dart:559-572): `mat` is an HxW[xC] uint8 array (cv.Mat), stored in EXIF
         `orientation` (see detectFacesFromMatBytes).  layout: "bgr" (cv.Mat channel order), "rgb" (HxWx3 RGB, HxWx4 RGBA, HxW
         gray: PIL, imageio, Flutter rawRgba), "rgb_planar" (3xHxW, e.g. a decoded torchvision image moved to the host) or
-        "yuyv" / "uyvy" / "yvyu" (HxWx2 packed YUV 4:2:2, W even: V4L2 webcams, capture cards, GStreamer; cv2's CV_8UC2 Mat).
-        The faces equal those of the BGR image (for YUV 4:2:2: of cv2.cvtColor(mat, COLOR_YUV2BGR_YUYV / _UYVY / _YVYU))."""
+        "yuyv" / "uyvy" / "yvyu" (HxWx2 packed YUV 4:2:2, W even: V4L2 webcams, capture cards, GStreamer; cv2's CV_8UC2 Mat)
+        or "p010" ((3H/2)xW uint16, a P010 / P012 / P016 frame, H and W even: a downloaded NVDEC or DXGI surface).
+        The faces equal those of the BGR image (for YUV 4:2:2: of cv2.cvtColor(mat, COLOR_YUV2BGR_YUYV / _UYVY / _YVYU); for
+        P010: of the NV12 frame of the words' high bytes, (mat >> 8).astype(np.uint8))."""
         if _layout(layout) != "bgr":
             mt = _mat_type(mat, 0, layout)
             h, w = mat.shape[1:] if mt == _ffi.FDT_FMT_RGB_PLANAR else mat.shape[:2]
+            if mt == _ffi.FDT_FMT_P010:
+                h = h // 3 * 2
             return self.detectFacesFromMatBytes(np.ascontiguousarray(mat), width=w, height=h, matType=mt, mode=mode,
                                                 orientation=orientation)
         ch = 1 if mat.ndim == 2 else mat.shape[2]
@@ -397,7 +442,7 @@ class FaceDetector:
                          mode: FaceDetectionMode = FaceDetectionMode.fast, orientation: int = 1) -> List[List[Face]]:
         """New batched entry point: `frames` holds `count` packed frames (bytes / uint8 array), or `count` YUV 4:2:0 frames of
         width * height * 3 / 2 bytes with matType FDT_FMT_YUV_NV12 / _NV21 / _I420 (packed YUV 4:2:2, FDT_FMT_YUYV / _UYVY /
-        _YVYU: width * height * 2 bytes).  orientation: EXIF 1..8 of every frame
+        _YVYU: width * height * 2 bytes; FDT_FMT_P010: width * height * 3 bytes or uint16 words).  orientation: EXIF 1..8 of every frame
         (see detectBatchRaw); the faces refer to the upright image."""
         uw, uh = _upright(width, height, _orientation(orientation))
         self._check()
@@ -419,6 +464,8 @@ class FaceDetector:
         t.data_ptr()).  YUV 4:2:0 formats: rowStride is the Y-plane stride (default: width) and a frame is
         height * rowStride * 3 / 2 bytes.  FDT_FMT_RGB_PLANAR: rowStride is one plane's row stride (default: width) and a frame
         is 3 * height * rowStride bytes.  FDT_FMT_YUYV / _UYVY / _YVYU: width even, rowStride >= 2 * width (default 2 * width).
+        FDT_FMT_P010: width and height even, rowStride even and >= 2 * width (default 2 * width), height * rowStride * 3 / 2 bytes
+        (a uint16 array is taken as its bytes).
         orientation (EXIF 1..8, FDT_ORIENT_*; fdt_detect_batch_oriented): every frame is stored rotated / mirrored.  width,
         height and rowStride describe the stored frames; faces are normalised to the upright image exif_transform(frame,
         orientation) and mesh / iris points are in its pixels."""
@@ -431,14 +478,17 @@ class FaceDetector:
             raise ValueError("rowStride smaller than width * channels")
         if matType in _ffi.YUV422_FORMATS and width % 2:
             raise ValueError("YUV 4:2:2 frames need an even width")
+        if matType == _ffi.FDT_FMT_P010:
+            _p010_checks(width, height, stride)
         frame_bytes = _frame_bytes(matType, height, stride)
         if isinstance(frames, int):
             ptr = frames
         else:
-            buf = np.ascontiguousarray(np.frombuffer(frames, np.uint8) if not isinstance(frames, np.ndarray) else frames.reshape(-1))
+            buf = _frame_buffer(frames, matType)
             if buf.size != count * frame_bytes:
                 raise ValueError("frames length does not equal count * %sheight * rowStride%s" % (
-                    "3 * " if matType == _ffi.FDT_FMT_RGB_PLANAR else "", " * 3 / 2" if yuv else ""))   # helpers.dart:440-447
+                    "3 * " if matType == _ffi.FDT_FMT_RGB_PLANAR else "",
+                    " * 3 / 2" if yuv or matType == _ffi.FDT_FMT_P010 else ""))   # helpers.dart:440-447
             ptr = buf.ctypes.data
         faces = (_ffi.FdtFace * max(1, count * self._max_faces))()
         counts = np.zeros(max(1, count), np.int32)
@@ -461,8 +511,8 @@ class FaceDetector:
     # -- mixed batches: frames of different sizes and formats, and encoded images, in one call ----------------------------
     def detectFacesFromMats(self, mats, *, mode: FaceDetectionMode = FaceDetectionMode.full,
                             orientations=None, layout: str = "bgr") -> List[List[Face]]:
-        """detectFacesFromMat over a list of HxW / HxWx3 / HxWx4 (or, with a YUV 4:2:2 layout, HxWx2) uint8 arrays of any sizes,
-        in one batched call
+        """detectFacesFromMat over a list of HxW / HxWx3 / HxWx4 (or, with a YUV 4:2:2 layout, HxWx2; with "p010", (3H/2)xW
+        uint16) arrays of any sizes, in one batched call
         (fdt_detect_frames).  A row-padded view (e.g. a crop of a larger array) goes in uncopied with strides[0] as its row
         stride.  Returns one list of faces per mat, each normalised to its own mat.  orientations: one EXIF orientation 1..8
         per mat (fdt_detect_frames_oriented), or None for all upright; faces then refer to each mat's upright image.
@@ -481,6 +531,12 @@ class FaceDetector:
                 keep.append(m)
                 frames.append((m.ctypes.data, w, h, m.strides[1], mt))
                 continue
+            if mt == _ffi.FDT_FMT_P010:
+                if m.strides[1] != 2 or m.strides[0] % 2 or m.strides[0] < 2 * m.shape[1] or not _rows_in_buffer(m):
+                    m = np.ascontiguousarray(m)
+                keep.append(m)
+                frames.append((m.ctypes.data, m.shape[1], m.shape[0] // 3 * 2, m.strides[0], mt))
+                continue
             if m.strides[-1] != 1 or (m.ndim == 3 and m.strides[1] != m.shape[2]) or m.strides[0] < m.shape[1] * m.strides[1] \
                     or not _rows_in_buffer(m):
                 m = np.ascontiguousarray(m)
@@ -494,8 +550,9 @@ class FaceDetector:
     def detectFramesRaw(self, frames, *, mode: FaceDetectionMode = FaceDetectionMode.fast, memKind: int = _ffi.FDT_MEM_HOST,
                         orientations=None):
         """fdt_detect_frames with array outputs.  `frames` is a list of (data, width, height, matType[, rowStride]) tuples: data
-        is a numpy array / bytes of exactly height * rowStride bytes (YUV 4:2:0: height * rowStride * 3 / 2; planar RGB:
-        3 * height * rowStride), or an integer device pointer with memKind=FDT_MEM_DEVICE.  rowStride defaults to
+        is a numpy array / bytes of exactly height * rowStride bytes (YUV 4:2:0 and P010: height * rowStride * 3 / 2, a P010
+        frame also as a uint16 array; planar RGB: 3 * height * rowStride), or an integer device pointer with
+        memKind=FDT_MEM_DEVICE.  rowStride defaults to
         width * channels (YUV and planar RGB: width).  Returns
         (FdtFace array [n * max_faces], counts int32 [n], mesh f32 [n, max_faces, 468, 3] or None,
         iris f32 [n, max_faces, 152, 3] or None).  orientations: one EXIF orientation 1..8 per frame
@@ -517,10 +574,11 @@ class FaceDetector:
             else:
                 if isinstance(data, int):
                     raise ValueError("frame %d: host frames are numpy arrays or bytes" % i)
-                buf = np.ascontiguousarray(np.frombuffer(data, np.uint8) if not isinstance(data, np.ndarray) else data.reshape(-1))
+                buf = _frame_buffer(data, mt)
                 if buf.dtype != np.uint8 or buf.size != nbytes:
                     raise ValueError("frame %d: data length does not equal %sheight * rowStride%s" % (
-                        i, "3 * " if mt == _ffi.FDT_FMT_RGB_PLANAR else "", " * 3 / 2" if mt in _ffi.YUV_FORMATS else ""))
+                        i, "3 * " if mt == _ffi.FDT_FMT_RGB_PLANAR else "",
+                        " * 3 / 2" if mt in _ffi.YUV_FORMATS or mt == _ffi.FDT_FMT_P010 else ""))
                 keep.append(buf)
                 ptr = buf.ctypes.data
             descs.append((ptr, w, h, stride, mt))
@@ -529,73 +587,93 @@ class FaceDetector:
 
     # -- YUV 4:2:0 frames as three separate planes: decoder surfaces, AVFrames, Android YUV_420_888 images --------------------
     def detectFacesFromYuvPlanes(self, frames, *, mode: FaceDetectionMode = FaceDetectionMode.full,
-                                 orientations=None) -> List[List[Face]]:
+                                 orientations=None, sampleBits: Optional[int] = None) -> List[List[Face]]:
         """Faces in YUV 4:2:0 frames given as (y, u, v) triples of 2-D uint8 arrays (fdt_detect_yuv_planes): Y is height x width,
         U and V are height / 2 x width / 2.  strides[0] of each plane is its row stride; strides[1] is 1 for Y and the chroma
         pixel stride, 1 or 2 and the same for U and V.  NumPy views describe every layout without a copy: an NV12 chroma plane
         uv gives uv[:, 0::2], uv[:, 1::2]; an AVFrame gives its three planes; an Android YUV_420_888 image its three buffers
         (pixelStride 2: U and V views into one interleaved buffer, or buffers that end at their last sample).  Returns one list
-        of faces per frame, normalised to its upright image.  orientations: one EXIF orientation 1..8 per frame, or None."""
+        of faces per frame, normalised to its upright image.  orientations: one EXIF orientation 1..8 per frame, or None.
+        sampleBits (10, 12 or 16; required for, and only for, 16-bit planes): the planes are 2-D uint16 arrays
+        (fdt_detect_yuv_planes16), e.g. a PyAV yuv420p10le frame's planes (10) or a downloaded P016 surface's Y plane and
+        uv[:, 0::2], uv[:, 1::2] (16); each sample is read as (s >> (sampleBits - 8)) & 0xFF."""
         frames = list(frames)
         orients = _orientations(orientations, len(frames))
+        bits = None if sampleBits is None else _sample_bits(sampleBits)
+        dt, bps = (np.uint8, 1) if bits is None else (np.uint16, 2)
         descs = []
         for i, fr in enumerate(frames):
             if not isinstance(fr, (tuple, list)) or len(fr) != 3 or \
-                    not all(isinstance(p, np.ndarray) and p.dtype == np.uint8 and p.ndim == 2 for p in fr):
-                raise ValueError("frame %d: expected (y, u, v), three 2-D uint8 arrays" % i)
+                    not all(isinstance(p, np.ndarray) and p.dtype == dt and p.ndim == 2 for p in fr):
+                if bits is None and isinstance(fr, (tuple, list)) and len(fr) == 3 and \
+                        all(isinstance(p, np.ndarray) and p.dtype == np.uint16 for p in fr):
+                    raise ValueError("frame %d: uint16 planes need sampleBits (10, 12 or 16)" % i)
+                raise ValueError("frame %d: expected (y, u, v), three 2-D %s arrays" % (i, np.dtype(dt).name))
             y, u, v = fr
             h, w = y.shape
             if u.shape != (h // 2, w // 2) or v.shape != (h // 2, w // 2):
                 raise ValueError("frame %d: U and V must be height / 2 x width / 2 (Y is %d x %d)" % (i, h, w))
-            if y.strides[1] != 1:
-                raise ValueError("frame %d: the Y plane's pixels must be adjacent (strides[1] == 1)" % i)
+            if y.strides[1] != bps:
+                raise ValueError("frame %d: the Y plane's pixels must be adjacent (strides[1] == %d)" % (i, bps))
             if u.strides[1] != v.strides[1]:
                 raise ValueError("frame %d: U and V need the same pixel stride" % i)
+            if u.strides[1] % bps:
+                raise ValueError("frame %d: the chroma pixel stride must be a whole number of samples" % i)
             strides = (y.strides[0], u.strides[0], v.strides[0])
-            _plane_extents(i, strides, w, h, u.strides[1])
-            descs.append(((y.ctypes.data, u.ctypes.data, v.ctypes.data), strides, w, h, u.strides[1]))
+            _plane_extents(i, strides, w, h, u.strides[1] // bps, bps)
+            descs.append(((y.ctypes.data, u.ctypes.data, v.ctypes.data), strides, w, h, u.strides[1] // bps))
         self._check()
-        faces, counts, mesh, iris = self._detect_planes(descs, mode, _ffi.FDT_MEM_HOST, orients)
+        faces, counts, mesh, iris = self._detect_planes(descs, mode, _ffi.FDT_MEM_HOST, orients, bits)
         sizes = [_upright(d[2], d[3], 1 if orients is None else orients[i]) for i, d in enumerate(descs)]
         return self._faces_per_frame(faces, counts, mesh, iris, sizes)
 
     def detectYuvPlanesRaw(self, frames, *, mode: FaceDetectionMode = FaceDetectionMode.fast, memKind: int = _ffi.FDT_MEM_HOST,
-                           orientations=None):
+                           orientations=None, sampleBits: Optional[int] = None):
         """fdt_detect_yuv_planes with array outputs, as detectFramesRaw.  `frames` is a list of
         ((y, u, v), (yStride, uStride, vStride), width, height, pixelStride) tuples: the planes are integer device pointers with
         memKind=FDT_MEM_DEVICE (e.g. torch CUDA tensors' data_ptr()), else numpy arrays or bytes, each holding at least its
-        plane's sampled extent from its first byte."""
+        plane's sampled extent from its first byte.  sampleBits (10, 12 or 16): the planes hold 16-bit words
+        (fdt_detect_yuv_planes16): strides count bytes and must be even, pixelStride counts samples (2 for a P016 surface's
+        chroma, U = chroma, V = chroma + 2), host buffers may be uint8 or uint16 arrays and device pointers must be even."""
         if memKind not in (_ffi.FDT_MEM_HOST, _ffi.FDT_MEM_DEVICE):
             raise ValueError("memKind must be FDT_MEM_HOST or FDT_MEM_DEVICE")
         frames = list(frames)
         orients = _orientations(orientations, len(frames))
+        bits = None if sampleBits is None else _sample_bits(sampleBits)
+        bps = 1 if bits is None else 2
         descs, keep = [], []
         for i, fr in enumerate(frames):
             if not isinstance(fr, (tuple, list)) or len(fr) != 5 or not isinstance(fr[0], (tuple, list)) or len(fr[0]) != 3 \
                     or not isinstance(fr[1], (tuple, list)):
                 raise ValueError("frame %d: expected ((y, u, v), (yStride, uStride, vStride), width, height, pixelStride)" % i)
             planes, strides, w, h, ps = fr
-            extents = _plane_extents(i, tuple(strides), w, h, ps)
+            extents = _plane_extents(i, tuple(strides), w, h, ps, bps)
             ptrs = []
             for k, (p, ext) in enumerate(zip(planes, extents)):
                 if memKind == _ffi.FDT_MEM_DEVICE:
                     if isinstance(p, bool) or not isinstance(p, int):
                         raise ValueError("frame %d: FDT_MEM_DEVICE planes are integer device pointers" % i)
+                    if p % bps:
+                        raise ValueError("frame %d: plane %s: 16-bit planes need an even pointer" % (i, "YUV"[k]))
                     ptrs.append(p)
                     continue
                 if isinstance(p, int):
                     raise ValueError("frame %d: host planes are numpy arrays or bytes" % i)
                 buf = np.frombuffer(p, np.uint8) if not isinstance(p, np.ndarray) else p
+                if bits is not None and buf.dtype == np.uint16 and buf.flags.c_contiguous:
+                    buf = buf.reshape(-1).view(np.uint8)
                 if buf.dtype != np.uint8 or not buf.flags.c_contiguous or buf.size < ext:
-                    raise ValueError("frame %d: plane %s is not a contiguous uint8 buffer of at least its sampled extent (%d bytes)"
-                                     % (i, "YUV"[k], ext))
+                    raise ValueError("frame %d: plane %s is not a contiguous %s buffer of at least its sampled extent (%d bytes)"
+                                     % (i, "YUV"[k], "uint8" if bits is None else "uint8 / uint16", ext))
+                if buf.ctypes.data % bps:
+                    raise ValueError("frame %d: plane %s: 16-bit planes need an even address" % (i, "YUV"[k]))
                 keep.append(buf)
                 ptrs.append(buf.ctypes.data)
             descs.append((tuple(ptrs), tuple(int(s) for s in strides), int(w), int(h), int(ps)))
         self._check()
-        return self._detect_planes(descs, mode, memKind, orients)
+        return self._detect_planes(descs, mode, memKind, orients, bits)
 
-    def _detect_planes(self, descs, mode, memKind, orients):
+    def _detect_planes(self, descs, mode, memKind, orients, bits=None):
         n = len(descs)
         arr = (_ffi.FdtYuvPlanes * max(1, n))()
         for k, (ptrs, strides, w, h, ps) in enumerate(descs):
@@ -603,10 +681,13 @@ class FaceDetector:
             arr[k].row_stride = (C.c_int32 * 3)(*strides)
             arr[k].width, arr[k].height, arr[k].pixel_stride = w, h, ps
         faces, counts, mesh, iris = self._outputs(n, mode)
-        rc = self._lib.fdt_detect_yuv_planes(self._h, arr, orients.ctypes.data_as(_ffi.i32p) if orients is not None else None, n,
-                                             int(FaceDetectionMode(mode)), memKind, faces, counts.ctypes.data_as(_ffi.i32p),
-                                             mesh.ctypes.data_as(_ffi.f32p) if mesh is not None else None,
-                                             iris.ctypes.data_as(_ffi.f32p) if iris is not None else None)
+        orients_p = orients.ctypes.data_as(_ffi.i32p) if orients is not None else None
+        outs = (faces, counts.ctypes.data_as(_ffi.i32p), mesh.ctypes.data_as(_ffi.f32p) if mesh is not None else None,
+                iris.ctypes.data_as(_ffi.f32p) if iris is not None else None)
+        if bits is None:
+            rc = self._lib.fdt_detect_yuv_planes(self._h, arr, orients_p, n, int(FaceDetectionMode(mode)), memKind, *outs)
+        else:
+            rc = self._lib.fdt_detect_yuv_planes16(self._h, arr, orients_p, n, bits, int(FaceDetectionMode(mode)), memKind, *outs)
         if rc != _ffi.FDT_OK:
             _raise(self._lib, self._h, rc)
         return faces, counts[:n], mesh, iris

@@ -109,6 +109,24 @@ enum { FDT_FMT_RGB = 0x1010, FDT_FMT_RGBA = 0x1011, FDT_FMT_RGB_PLANAR = 0x1012 
  * H x W CV_8UC2 Mat when row_stride = 2 * width). */
 enum { FDT_FMT_YUYV = 0x1020, FDT_FMT_UYVY = 0x1021, FDT_FMT_YVYU = 0x1022 };
 
+/* High-bit-depth YUV 4:2:0 (HEVC Main10, AV1 / VP9 profile 2 and 10-bit capture: NVDEC P016 surfaces, Windows DXGI / Media
+ * Foundation P010, FFmpeg hwdownload).  Semi-planar 4:2:0 of little-endian 16-bit words with the value in the high bits; the one
+ * constant serves P010, P012 and P016.  Accepted wherever mat_type is, except by fdt_extract_aligned_squares (FDT_ERR_BAD_ARG).
+ *   Y plane: height rows of row_stride bytes, the Y word of pixel (x, y) at byte y * row_stride + 2x.
+ *   UV plane at height * row_stride: height / 2 rows of row_stride bytes; U of pixel (x, y) is the word at byte
+ *   (y / 2) * row_stride + 4 * (x / 2) of that plane, V the word 2 bytes behind it.
+ *   A frame is height * row_stride * 3 / 2 bytes (with row_stride = 2 * width, cv2's (3H/2) x W CV_16UC1 Mat).
+ * width, height and row_stride must be even (else FDT_ERR_BAD_ARG; for orientations 5-8, the stored size); row_stride >=
+ * 2 * width (else FDT_ERR_SIZE_MISMATCH).
+ * The sample rule, here and in fdt_detect_yuv_planes16: a 16-bit sample s with `bits` significant bits stored from bit 0 becomes
+ * the 8-bit sample (s >> (bits - 8)) & 0xFF; high-bit-aligned data (P010 / P012 / P016) is bits = 16, its high byte.  It
+ * truncates (what a caller's `>> 8` to uint8 computes, and P010 and P016 of one picture give one answer); the bits below the 8
+ * it keeps never affect a result, and bits above `bits` are ignored.  Every result (records, mesh, iris, the letterbox tap, the
+ * mesh / iris stage crops, face crops) equals, bit for bit, the same call on the 8-bit FDT_FMT_YUV_NV12 frame made by that rule,
+ * in every orientation, memory kind and mode.  Colour is then the NV12 path's BT.601 limited-range conversion: a detector input,
+ * not an HDR-correct one; BT.2020 primaries and PQ / HLG transfer functions are not applied. */
+enum { FDT_FMT_P010 = 0x1003 };
+
 enum { FDT_MEM_HOST = 0, FDT_MEM_DEVICE = 1 };
 
 /* Frame orientation (fdt_detect_batch_oriented, fdt_detect_frames_oriented): the EXIF Orientation value of the STORED frame,
@@ -204,7 +222,7 @@ typedef struct fdt_frame {
   int32_t width, height;     /* image size                                                                        */
   int32_t row_stride;        /* as fdt_detect_batch: >= width * channels; YUV: the Y-plane stride                 */
   int32_t mat_type;          /* FDT_MAT_8UC1 / _8UC3 / _8UC4, FDT_FMT_YUV_NV12 / _NV21 / _I420, FDT_FMT_RGB / _RGBA /
-                                _RGB_PLANAR, FDT_FMT_YUYV / _UYVY / _YVYU                                         */
+                                _RGB_PLANAR, FDT_FMT_YUYV / _UYVY / _YVYU, FDT_FMT_P010                           */
 } fdt_frame;                 /* 24 bytes */
 
 /* detectFacesFromMat over a list of frames of different sizes and formats (photos, mixed camera feeds), batched like
@@ -278,6 +296,28 @@ FDT_EXPORT int32_t fdt_detect_yuv_planes(fdt_handle* h, const fdt_yuv_planes* fr
                                          int32_t mode, int32_t mem_kind, fdt_face* out_faces, int32_t* out_counts,
                                          float* out_mesh, float* out_iris);
 
+/* fdt_detect_yuv_planes over planes of little-endian 16-bit words: NVDEC / PyNvVideoCodec P016 surfaces (pitched, the chroma
+ * at pitch * surface height: U = chroma, V = chroma + 2 bytes, pixel_stride 2) and FFmpeg / PyAV yuv420p10le / yuv420p12le
+ * frames (three planes, data[] and linesize[], pixel_stride 1).  The same fdt_yuv_planes descriptors: row_stride[] counts bytes,
+ * pixel_stride counts SAMPLES, so the words of pixel (x, y) are at
+ *   Y  plane[0] + y * row_stride[0] + 2x
+ *   U  plane[1] + (y / 2) * row_stride[1] + 2 * (x / 2) * pixel_stride,   V likewise from plane[2].
+ * sample_bits (10, 12 or 16 for the whole call, else FDT_ERR_BAD_ARG before any work) is the number of significant bits stored
+ * from bit 0: 10 / 12 for yuv420p10le / p12le, 16 for P010 / P016 surfaces; each sample becomes (s >> (sample_bits - 8)) & 0xFF,
+ * the rule of FDT_FMT_P010.  Every result equals, bit for bit, fdt_detect_yuv_planes on the 8-bit planes made by that rule.
+ * Checks as fdt_detect_yuv_planes, with the extents in samples x 2 bytes: row_stride[0] >= 2 * width and row_stride[1],
+ * row_stride[2] >= 2 * ((width / 2 - 1) * pixel_stride + 1) (else FDT_ERR_SIZE_MISMATCH); every plane pointer and row stride must
+ * be even (else FDT_ERR_BAD_ARG naming the frame and the plane).  Orientations, chunking, modes, face crops and multi-device
+ * splitting of host frames are as there.
+ * Host frames: each plane's sampled columns go up, twice the bytes of fdt_detect_yuv_planes' rule; interleaved chroma
+ * (pixel_stride 2, U and V 2 bytes apart with one row stride >= 2 * width) as one area of 2 * width bytes per row.  So
+ * fdt_last_h2d_bytes is the sum over the frames of 2 * width * height + (height / 2) * 2 * width for interleaved chroma, else
+ * 2 * width * height + 4 * (height / 2) * ((width / 2 - 1) * pixel_stride + 1).  Every chunk runs the plane-table variants of
+ * the letterbox and crop kernels. */
+FDT_EXPORT int32_t fdt_detect_yuv_planes16(fdt_handle* h, const fdt_yuv_planes* frames, const int32_t* orientations, int32_t n,
+                                           int32_t sample_bits, int32_t mode, int32_t mem_kind, fdt_face* out_faces,
+                                           int32_t* out_counts, float* out_mesh, float* out_iris);
+
 /* fdt_detect_jpeg over n encoded images in one call.  The host parses and Huffman-decodes them on a pool of
  * min(n, hardware threads) threads; the device decodes them into a handle-owned frame arena and detects them as one mixed
  * batch (chunks of up to max_batch images and max_batch * 8 MiB of decoded BGR).  out_status[i] is FDT_OK, FDT_ERR_FORMAT
@@ -342,7 +382,7 @@ FDT_EXPORT int32_t fdt_copy_face_crops(fdt_handle* h, void* dst, size_t capacity
  * `nbytes` bytes; FDT_ERR_SIZE_MISMATCH when nbytes != width*height*channels
  * (matFromPackedBytes, lib/src/util/helpers.dart:432-450), or != width*height*3/2 for the YUV formats
  * (FDT_FMT_RGB: width*height*3, FDT_FMT_RGBA: width*height*4, FDT_FMT_RGB_PLANAR: 3*width*height,
- * FDT_FMT_YUYV / _UYVY / _YVYU: 2*width*height). */
+ * FDT_FMT_YUYV / _UYVY / _YVYU: 2*width*height, FDT_FMT_P010: 3*width*height, row_stride 2 * width). */
 FDT_EXPORT int32_t fdt_detect_one(fdt_handle* h, const uint8_t* bytes, size_t nbytes, int32_t width,
                                   int32_t height, int32_t mat_type, int32_t mode, fdt_face* out_faces,
                                   int32_t* out_count, float* out_mesh, float* out_iris);
@@ -438,8 +478,10 @@ FDT_EXPORT int64_t fdt_last_launch_count(fdt_handle* h);
  * axes clamp differently at the borders, so at some sizes that set differs from orientation 1's.  RGB and RGBA frames upload as
  * BGR and BGRA do.  Planar RGB frames are read as 3 * height stacked rows: when height is a multiple of the period the same
  * pattern runs through all three planes (1280x720: 552,960 bytes per frame, as BGR), otherwise whole frames go up.  Packed YUV
- * 4:2:2 frames upload as a packed format of 2 bytes per pixel (1280x720: rows 10k+4, 10k+5, 368,640 bytes per frame).  Mixed calls
- * upload whole frames; fdt_detect_yuv_planes uploads each plane's sampled columns (see there). */
+ * 4:2:2 frames upload as a packed format of 2 bytes per pixel (1280x720: rows 10k+4, 10k+5, 368,640 bytes per frame).  FDT_FMT_P010
+ * frames keep the YUV rule on both planes, each row 2 * width bytes (1280x720: Y rows 10k+4, 10k+5 and chroma row 5k+2, 552,960
+ * bytes per frame, twice NV12's).  Mixed calls upload whole frames; fdt_detect_yuv_planes and fdt_detect_yuv_planes16 upload each
+ * plane's sampled columns (see there). */
 FDT_EXPORT int64_t fdt_last_h2d_bytes(fdt_handle* h);
 /* Device time in ms of the named stage summed over the last call when stage timing was enabled
  * with fdt_set_stage_timing(h,1) (adds cudaEvent records; off by default).

@@ -51,6 +51,13 @@ const int kFdtFmtUyvy = 0x1021;
 const int kFdtFmtYvyu = 0x1022;
 bool fdtIsYuv422(int matType) => matType == kFdtFmtYuyv || matType == kFdtFmtUyvy || matType == kFdtFmtYvyu;
 
+/// 16-bit YUV 4:2:0 with the value in the high bits (fdt_api.h FDT_FMT_P010; P010 / P012 / P016, e.g. a 10-bit HEVC frame
+/// from a hardware decoder): NV12's layout of little-endian 16-bit words, width, height and rowStride even, rowStride >=
+/// 2 * width, height * rowStride * 3 / 2 bytes.  Each sample is read as its high byte, so results equal those of the NV12 frame
+/// of the high bytes.  Separate 16-bit planes (yuv420p10le / p12le) go to `fdt_detect_yuv_planes16` (FdtLibrary.detectYuvPlanes16)
+/// with their sample bits.
+const int kFdtFmtP010 = 0x1003;
+
 /// Frame orientations (fdt_api.h FDT_ORIENT_*): the EXIF Orientation value of a stored frame, as OpenCV's ExifTransform
 /// applies it.  Results of the oriented calls refer to the upright image; for 5-8 its width is the stored height.  Camera
 /// frames that must be rotated R degrees clockwise to display: 1, 6, 3, 8 for R = 0, 90, 180, 270; rotated R degrees clockwise
@@ -70,9 +77,12 @@ bool fdtIsYuv(int matType) => matType == kFdtFmtYuvNv12 || matType == kFdtFmtYuv
 /// of [matType].
 int fdtRowStride(int matType, int width) => fdtIsYuv(matType) || matType == kFdtFmtRgbPlanar
     ? width
-    : width * (matType == 0 ? 1 : (fdtIsYuv422(matType) ? 2 : (matType == 24 || matType == kFdtFmtRgba ? 4 : 3)));
-int fdtFrameBytes(int matType, int width, int height) => fdtIsYuv(matType)
-    ? height * width * 3 ~/ 2
+    : width *
+        (matType == 0
+            ? 1
+            : (fdtIsYuv422(matType) || matType == kFdtFmtP010 ? 2 : (matType == 24 || matType == kFdtFmtRgba ? 4 : 3)));
+int fdtFrameBytes(int matType, int width, int height) => fdtIsYuv(matType) || matType == kFdtFmtP010
+    ? height * fdtRowStride(matType, width) * 3 ~/ 2
     : (matType == kFdtFmtRgbPlanar ? 3 : 1) * height * fdtRowStride(matType, width);
 
 /// fdt_config: the named arguments of FaceDetector.create that touch the path (48 bytes).
@@ -227,6 +237,10 @@ typedef _DetectYuvPlanesC = Int32 Function(Pointer<Void>, Pointer<FdtYuvPlanes>,
     Pointer<FdtFace>, Pointer<Int32>, Pointer<Float>, Pointer<Float>);
 typedef _DetectYuvPlanesD = int Function(Pointer<Void>, Pointer<FdtYuvPlanes>, Pointer<Int32>, int, int, int, Pointer<FdtFace>,
     Pointer<Int32>, Pointer<Float>, Pointer<Float>);
+typedef _DetectYuvPlanes16C = Int32 Function(Pointer<Void>, Pointer<FdtYuvPlanes>, Pointer<Int32>, Int32, Int32, Int32, Int32,
+    Pointer<FdtFace>, Pointer<Int32>, Pointer<Float>, Pointer<Float>);
+typedef _DetectYuvPlanes16D = int Function(Pointer<Void>, Pointer<FdtYuvPlanes>, Pointer<Int32>, int, int, int, int,
+    Pointer<FdtFace>, Pointer<Int32>, Pointer<Float>, Pointer<Float>);
 typedef _SetFaceCropsC = Int32 Function(Pointer<Void>, Pointer<FdtCropSpec>);
 typedef _SetFaceCropsD = int Function(Pointer<Void>, Pointer<FdtCropSpec>);
 typedef _GetFaceCropsC = Int32 Function(Pointer<Void>, Pointer<Int64>, Pointer<Pointer<Void>>);
@@ -256,6 +270,7 @@ class FdtLibrary {
         detectFramesOriented = _lib.lookupFunction<_DetectFramesOrientedC, _DetectFramesOrientedD>('fdt_detect_frames_oriented'),
         detectJpegBatch = _lib.lookupFunction<_DetectJpegBatchC, _DetectJpegBatchD>('fdt_detect_jpeg_batch'),
         detectYuvPlanes = _lib.lookupFunction<_DetectYuvPlanesC, _DetectYuvPlanesD>('fdt_detect_yuv_planes'),
+        detectYuvPlanes16 = _lib.lookupFunction<_DetectYuvPlanes16C, _DetectYuvPlanes16D>('fdt_detect_yuv_planes16'),
         setFaceCrops = _lib.lookupFunction<_SetFaceCropsC, _SetFaceCropsD>('fdt_set_face_crops'),
         getFaceCrops = _lib.lookupFunction<_GetFaceCropsC, _GetFaceCropsD>('fdt_get_face_crops'),
         copyFaceCrops = _lib.lookupFunction<_CopyFaceCropsC, _CopyFaceCropsD>('fdt_copy_face_crops'),
@@ -282,6 +297,9 @@ class FdtLibrary {
   final _DetectFramesOrientedD detectFramesOriented;
   final _DetectJpegBatchD detectJpegBatch;
   final _DetectYuvPlanesD detectYuvPlanes;
+  /// fdt_detect_yuv_planes16(h, frames, orientations, n, sampleBits, mode, memKind, faces, counts, mesh, iris): FdtYuvPlanes of
+  /// 16-bit words (row strides in bytes, pixelStride in samples), sampleBits 10, 12 or 16.
+  final _DetectYuvPlanes16D detectYuvPlanes16;
   final _NumDevicesD numDevices;
 
   static FdtLibrary? _instance;
